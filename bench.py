@@ -3,7 +3,7 @@
 bench.py -- the PhaMers hot path (k-mer count -> normalise -> score) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--contigs C] [--k 4]
-                    [--workload shipped|enlarged|count] [--refs R] [--canonical]
+                    [--workload shipped|enlarged|count] [--refs R] [--canonical] [--dump-outputs DIR]
 
 A "step" is one pass of the whole hot path over one batch of synthetic contigs: BASELINE.json configs[1]
 ("synthetic metagenome 1M contigs, 1-100 kb lognormal lengths, k=4 tetranucleotide, 1xB200"), scored against the shipped
@@ -54,7 +54,18 @@ def parse_args():
     ap.add_argument("--no-configs", action="store_true", help="skip the short runs of BASELINE configs[2] and configs[4] after the main region")
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--cpu-sample-contigs", type=int, default=2400, help="oracle-port sample on rank 0 (about 12 s of one core)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB in all): "
+                         "counts, knn, kmeans, combo (counts, freq for --workload count).  An array cut to a seeded sample of its "
+                         "rows has their row numbers in DIR/<name>.row_index.npy.  With several GPUs, combo holds the gathered "
+                         "scores of every rank; the other arrays are rank 0's shard only.  git ignores bench_outputs/ at the top "
+                         "of the tree")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of --impl b200")
+    return args
 
 
 def ncu_traffic():
@@ -75,6 +86,28 @@ def measured_peaks():
         return {"hbm_gbs": p["hbm_gbs"], "bf16_tflops": p["bf16_tflops"],
                 "bf16_tflops_sustained": p.get("bf16_tflops_sustained", p["bf16_tflops"]), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, outputs):
+    """--dump-outputs: each (name, CUDA tensor) of `outputs` goes to directory/<name>.npy, float64 as float64 and everything else as
+    float32 (counts stay below 2^24, so they convert exactly).  Every array gets an equal share of DUMP_BYTES; one larger than its
+    share keeps a sample of its rows, drawn with SEED and sorted, whose row numbers go to <name>.row_index.npy.  The sample
+    depends on the row count only, so two builds run with the same arguments dump the same rows."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_BYTES // len(outputs) - 4096                            # room for the .npy headers
+    for name, t in outputs:
+        dtype = torch.float64 if t.dtype == torch.float64 else torch.float32
+        row_bytes = int(np.prod(t.shape[1:], dtype=np.int64)) * dtype.itemsize
+        if t.shape[0] * row_bytes > share:
+            rows = np.sort(np.random.default_rng(SEED).choice(t.shape[0], size=share // (row_bytes + 8), replace=False))
+            np.save(os.path.join(directory, name + ".row_index.npy"), rows.astype(np.float64))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        np.save(os.path.join(directory, name + ".npy"), t.to(dtype).cpu().numpy())
 
 
 class ClockSampler(object):
@@ -358,7 +391,10 @@ def run_b200(args, rank, local_rank, world):
             gathered = combo
         if timed:
             step.events.append((e0, e1))
-        return counts, gathered
+        # what a caller of this path receives (the all-gathered combo scores when several GPUs score)
+        outputs = ([("counts", counts), ("knn", knn), ("kmeans", km), ("combo", gathered)] if scoring
+                   else [("counts", counts), ("freq", freq)])
+        return counts, gathered, outputs
     step.events = []
 
     sampler = ClockSampler(local_rank)
@@ -378,7 +414,7 @@ def run_b200(args, rank, local_rank, world):
     wall_begin = time.time()
     t_start.record(stream)
     for _ in range(args.steps):
-        counts, gathered = step(True)
+        counts, gathered, outputs = step(True)
     t_end.record(stream)
     torch.cuda.synchronize()
     if world > 1:
@@ -405,6 +441,8 @@ def run_b200(args, rank, local_rank, world):
     assert args.no_check or bool((counts.sum(dim=1, dtype=torch.int64) == lengths - (args.k - 1)).all()), "count row sums are wrong"
     if scoring and not args.no_check:
         assert bool(torch.isfinite(gathered).all()) and gathered.numel() == (sum(shard_sizes) if shard_sizes else n * world)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- end to end through the public API with HOST buffers (copies inside the timed region) ----
     e2e = None

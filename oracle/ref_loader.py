@@ -14,10 +14,10 @@ the import (SURVEY.md section 8(c)):
   5. empty ``basic`` module                         (phamer.py:28 ; basic.py is py2-only syntax)
   6. ``fileIO`` stub with get_fasta_ids/read_fasta  (kmer.py:18,125 ; fileIO.py is py2-only syntax)
 
-The reference tree only exists in the build container (/root/reference); nothing that
-runs on the GPU box may call this module.  It is used by tests/golden/make_golden.py to
-generate the committed golden vectors and by the ``not gpu`` tests (when the tree is
-present) to pin oracle/phamers_oracle.py against the real code.
+The original scripts are found through $PHAMERS_REF (their scripts/ directory); the
+repository does not carry them.  This module is used by tests/golden/make_golden.py to
+generate the committed golden vectors and, when $PHAMERS_REF is set, by
+tests/test_oracle.py to pin oracle/phamers_oracle.py against the real code as well.
 """
 import builtins
 import importlib
@@ -25,9 +25,9 @@ import os
 import sys
 import types
 
+# the scripts/ directory of an original PhaMers checkout; the repository does not carry one
 REF_CANDIDATES = [
     os.environ.get("PHAMERS_REF", ""),
-    "/root/reference/scripts",
 ]
 
 
@@ -135,7 +135,7 @@ def load_reference():
         return _cache["mods"]
     d = reference_scripts_dir()
     if d is None:
-        raise RuntimeError("reference tree not present (only available in the build container)")
+        raise RuntimeError("original PhaMers scripts not found: set PHAMERS_REF to their scripts/ directory")
     _install_shims(_contig_get_id)
     saved = {name: sys.modules.pop(name, None) for name in ("kmer", "learning", "phamer")}
     sys.path.insert(0, d)

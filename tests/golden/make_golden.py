@@ -1,11 +1,9 @@
 #!/usr/bin/env python
 """
 Generates the committed golden vectors from the UNMODIFIED PhaMers reference
-(/root/reference/scripts/{kmer,learning,phamer}.py imported through oracle/ref_loader.py).
+(scripts/{kmer,learning,phamer}.py imported through oracle/ref_loader.py):
 
-Run in the build container only (the reference tree does not exist on the GPU box):
-
-    python tests/golden/make_golden.py
+    PHAMERS_REF=<PhaMers checkout>/scripts python tests/golden/make_golden.py
 
 Outputs (all under tests/golden/):
   counting_golden.npz  adversarial + random sequences (laid end to end as seq_bytes + seq_offsets),

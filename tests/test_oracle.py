@@ -2,7 +2,7 @@
 Pins the oracle (oracle/phamers_oracle.py, oracle/kmer_oracle.c) against
   (a) the committed golden vectors, which tests/golden/make_golden.py produced by running the
       UNMODIFIED reference modules, and
-  (b) the live reference itself when /root/reference is present (build container only).
+  (b) the original scripts themselves when PHAMERS_REF names their directory.
 CPU only.
 """
 import os
@@ -134,8 +134,26 @@ def test_host_kmeans_reproduces_golden_centroids(scoring):
     assert np.max(np.abs(cn - g["centroids_neg"])) < 1e-9
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree only exists in the build container")
-def test_restatement_matches_live_reference():
+def test_restatement_matches_live_reference(counting, scoring):
+    # always: the original's stored answers (tests/golden/make_golden.py), with every restatement and every method as below
+    # -- here score_points clusters the references itself, as the original did when the golden scores were made
+    seqs = _seqs(counting)
+    for k in (3, 4, 5, 6):
+        want = counting["counts_k%d" % k]
+        assert np.array_equal(c_oracle.count(counting["seq_bytes"], counting["seq_offsets"], k), want)
+        for i, s in enumerate(seqs):
+            assert np.array_equal(po.count_string_np(s, k), want[i])
+            if len(s) <= 3001:
+                assert np.array_equal(po.count_string(s, k), want[i])
+    assert np.array_equal(po.normalize_counts(counting["counts_k4"]), counting["normalized_k4"], equal_nan=True)
+    g, pos, neg = scoring
+    pts = po.normalize_counts(g["query_counts"])
+    for method in ("knn", "kmeans", "combo"):
+        got = po.score_points(pts, pos, neg, method=method)
+        assert np.max(np.abs(got - g["scores_" + method])) <= 1e-9, method
+    if not ref_loader.reference_available():
+        return
+    # and, where the original scripts are installed (PHAMERS_REF), against them on fresh random inputs
     kmer, learning, phamer = ref_loader.load_reference()
     rng = np.random.default_rng(7)
     alphabet = np.frombuffer(b"ATGCATGCATGCATGCNatgcRY-", dtype=np.uint8)
