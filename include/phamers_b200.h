@@ -147,6 +147,42 @@ int phm_score_counts(const uint32_t *d_counts, int64_t n_points, int dim,
                      int k_neighbors, double *d_knn, double *d_kmeans, double *d_combo,
                      void *d_workspace, size_t workspace_bytes, void *stream);
 
+/* Neighbour report: the rows that decided each score, written by the same call that writes the scores.
+ *     For query row i, with k = k_neighbors and references in d_refs order (positives first):
+ *     d_ref_index[i*k .. i*k+k-1]       rows of d_refs of the k nearest references, ascending float64 Euclidean distance, ties to
+ *                                       the lower row first (the references whose labels cast the vote)
+ *     d_ref_distance[i*k .. i*k+k-1]    their distances: sqrt of the float64 direct-difference sum of squares (the arithmetic of
+ *                                       phm_distances, not the |a|^2 + |b|^2 - 2ab expansion)
+ *     d_centroid_index[2i], [2i+1]      row of d_cent_pos of the nearest positive centroid, row of d_cent_neg of the nearest negative
+ *                                       one (first on ties, like np.argmin; -1 when that centroid set is empty).  With centroids from
+ *                                       k-means, the row is the cluster label.
+ *     d_centroid_distance[2i], [2i+1]   their distances: the e_pos, e_neg of tanh((e_neg - e_pos)/(e_pos + e_neg))
+ *     A NaN query row reports index -1 and distance NaN in every slot.  Every member may be NULL. */
+typedef struct phm_neighbors {
+    int64_t *d_ref_index;          /* int64  [n_points * k_neighbors]  (may be NULL) */
+    double  *d_ref_distance;       /* float64[n_points * k_neighbors]  (may be NULL) */
+    int64_t *d_centroid_index;     /* int64  [n_points * 2]  nearest positive, nearest negative (may be NULL) */
+    double  *d_centroid_distance;  /* float64[n_points * 2]  (may be NULL) */
+} phm_neighbors;
+
+/* phm_score / phm_score_counts that also fill `nb` (same arguments, same workspace size from phm_score_workspace_bytes).  The
+ * scores are bit-identical to those of phm_score / phm_score_counts on the same inputs, and consistent with the report: the labels
+ * of the reported references give the vote, tanh((cd[1] - cd[0]) / (cd[0] + cd[1])) is the kmeans score.  On the tensor-core path
+ * every live row has its candidate band re-measured exactly (the vote alone may be settled by the error intervals; the order of the
+ * k nearest is not), which costs time; on the exhaustive path (other widths, k outside {1, 3, 5}) the k references are selected by
+ * the norm expansion and then re-measured, so at a near tie (gap below the expansion's rounding) that path may report the other
+ * member of the tie.  nb = NULL, or all members NULL: exactly phm_score / phm_score_counts. */
+int phm_score_neighbors(const double *d_points, int64_t n_points, int dim,
+                        const double *d_refs, int64_t n_refs, int64_t n_positive,
+                        const double *d_cent_pos, int64_t n_cent_pos, const double *d_cent_neg, int64_t n_cent_neg,
+                        int k_neighbors, double *d_knn, double *d_kmeans, double *d_combo, const phm_neighbors *nb,
+                        void *d_workspace, size_t workspace_bytes, void *stream);
+int phm_score_counts_neighbors(const uint32_t *d_counts, int64_t n_points, int dim,
+                               const double *d_refs, int64_t n_refs, int64_t n_positive,
+                               const double *d_cent_pos, int64_t n_cent_pos, const double *d_cent_neg, int64_t n_cent_neg,
+                               int k_neighbors, double *d_knn, double *d_kmeans, double *d_combo, const phm_neighbors *nb,
+                               void *d_workspace, size_t workspace_bytes, void *stream);
+
 /* learning.distances (scripts/learning.py:47-56): Euclidean distance, float64 by direct difference, of d_point[dim] to each of
  * d_rows[n_rows * dim] -> d_out[n_rows].  learning.closest_to (:59-66) is the row with the first smallest of them. */
 int phm_distances(const double *d_point, const double *d_rows, int64_t n_rows, int dim, double *d_out, void *stream);
@@ -224,7 +260,7 @@ int phm_set_option(const char *name, int64_t value);
 /* Kernels this library has launched in the calling process so far (bench.py reports the difference over its timed region). */
 uint64_t phm_kernel_launches(void);
 
-/* Mean device time (ms) of the launches (at most 64) of a hot kernel ("kmer_hist_kernel", "score_tc_kernel") since the previous
+/* Mean device time (ms) of the launches (at most 64) of a hot kernel ("kmer_hist_kernel", "score_tc_kernel", "score_decide_kernel") since the previous
  * call for that kernel; needs option "time_kernels" = 1 before the launches.  Synchronises on the last of them. */
 int phm_last_kernel_ms(const char *kernel, float *ms);
 

@@ -35,6 +35,10 @@ SIGNATURES = {
                           c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "phm_score_counts": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int64,
                                  c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_score_neighbors": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int64,
+                                    c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_score_counts_neighbors": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p,
+                                           c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "phm_count_score_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int64, c_int64]),
     "phm_count_score": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int64,
                                 c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
@@ -53,6 +57,12 @@ SIGNATURES = {
 
 class PhamersLibraryError(RuntimeError):
     pass
+
+
+class Neighbors(ctypes.Structure):
+    """phm_neighbors: device pointers of the neighbour report (NULL = not wanted)."""
+    _fields_ = [("d_ref_index", c_void_p), ("d_ref_distance", c_void_p), ("d_centroid_index", c_void_p),
+                ("d_centroid_distance", c_void_p)]
 
 
 class Caps(ctypes.Structure):

@@ -112,6 +112,7 @@ extern "C" uint64_t phm_kernel_launches(void) { return (uint64_t)kernel_launches
 extern "C" int phm_last_kernel_ms(const char *kernel, float *ms) {
     PHM_REQUIRE(kernel != nullptr && ms != nullptr, "null pointer");
     if (!strcmp(kernel, "score_tc_kernel")) return tc::score_tc_last_ms(ms);
+    if (!strcmp(kernel, "score_decide_kernel")) return tc::score_decide_last_ms(ms);
     if (!strcmp(kernel, "kmer_hist_kernel")) return kmer_hist_last_ms(ms);
     set_error("no timing hook for kernel '%s'", kernel);
     return PHM_E_ARG;

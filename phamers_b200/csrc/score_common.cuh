@@ -7,6 +7,14 @@
 
 namespace phm {
 
+// Where a scoring call reports the rows that decided each query (phm_neighbors of the header): the k nearest references as rows
+// of d_refs with their direct-difference distances, and the nearest centroid of each class.  Every member may be null.
+struct NeighborOut {
+    int64_t *ref_index = nullptr; double *ref_distance = nullptr;       // [n, k]
+    int64_t *cent_index = nullptr; double *cent_distance = nullptr;     // [n, 2]: nearest positive, nearest negative
+    __host__ __device__ bool any() const { return ref_index || ref_distance || cent_index || cent_distance; }
+};
+
 struct ScoreArgs {
     const double *points; int64_t n_points; int dim;
     const uint32_t *point_counts;             // optional: raw count rows instead of `points` (features = row / row sum, formed on the fly)
@@ -19,6 +27,7 @@ struct ScoreArgs {
     int64_t n_rows;                           // rows to score (upper bound when n_rows_dev is set)
     int k_neighbors;
     double *knn, *kmeans, *combo;
+    NeighborOut nb;                           // neighbour report (all null: scores only)
 };
 
 int launch_score_exact(const ScoreArgs &a, cudaStream_t st);
@@ -103,6 +112,7 @@ bool score_tc_supported(int dim, int k_neighbors, int64_t n_refs, int64_t n_cent
 size_t score_tc_workspace_bytes(int64_t n_points, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg);
 int score_tc(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, int *kernels_launched);
 int score_tc_last_ms(float *ms);
+int score_decide_last_ms(float *ms);
 int score_tc_stats(const void *ws, unsigned long long *fallback_rows, float *max_rank_error, cudaStream_t st);
 }  // namespace tc
 

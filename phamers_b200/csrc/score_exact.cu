@@ -65,6 +65,43 @@ __device__ __forceinline__ double direct_distance(const double *p, const double 
     return sqrt(s);
 }
 
+// Neighbour report of one row.  The selection ranks by the norm expansion; the k references it kept are re-measured by direct
+// difference and ordered by (distance, index), and the nearer of the two re-measured centroids of each class is reported (lower
+// index on ties).  At a near tie (a gap below the expansion's rounding) the selection may keep the other member of the tie than
+// the tensor-core path does.  A NaN row reports index -1 and distance NaN everywhere.
+__device__ void exact_neighbors(const ScoreArgs &a, int64_t q, bool nan_row, const int (&ki)[KNN_MAX + 1], const int (&ci)[4]) {
+    const int kn = a.k_neighbors;
+    const double *p = a.points + q * a.dim;
+    double d[KNN_MAX];
+    int64_t id[KNN_MAX];
+    for (int j = 0; j < kn; ++j) {
+        const bool ok = !nan_row && ki[j] >= 0;
+        id[j] = ok ? ki[j] : -1;
+        d[j] = ok ? direct_distance(p, a.refs + (int64_t)ki[j] * a.dim, a.dim) : NAN;
+        for (int s = j; s > 0 && (d[s] < d[s - 1] || (d[s] == d[s - 1] && id[s] < id[s - 1])); --s) {
+            const double td = d[s]; d[s] = d[s - 1]; d[s - 1] = td;
+            const int64_t ti = id[s]; id[s] = id[s - 1]; id[s - 1] = ti;
+        }
+    }
+    for (int j = 0; j < kn; ++j) {
+        if (a.nb.ref_index) a.nb.ref_index[q * kn + j] = id[j];
+        if (a.nb.ref_distance) a.nb.ref_distance[q * kn + j] = d[j];
+    }
+    for (int c = 0; c < 2; ++c) {
+        const double *cent = c ? a.cent_neg : a.cent_pos;
+        int64_t best = -1;
+        double bd = NAN;
+        for (int j = 0; j < 2 && !nan_row; ++j) {
+            const int i = ci[2 * c + j];
+            if (i < 0) continue;
+            const double e = direct_distance(p, cent + (int64_t)i * a.dim, a.dim);
+            if (best < 0 || e < bd || (e == bd && i < best)) { best = i; bd = e; }
+        }
+        if (a.nb.cent_index) a.nb.cent_index[q * 2 + c] = best;
+        if (a.nb.cent_distance) a.nb.cent_distance[q * 2 + c] = bd;
+    }
+}
+
 __global__ void __launch_bounds__(256) score_exact_kernel(ScoreArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     ExactSmem &sm = *reinterpret_cast<ExactSmem *>(smem_raw);
@@ -185,6 +222,7 @@ __global__ void __launch_bounds__(256) score_exact_kernel(ScoreArgs a) {
         if (a.knn) a.knn[q] = knn;
         if (a.kmeans) a.kmeans[q] = km;
         if (a.combo) a.combo[q] = knn + km;                           // phamer.py:313
+        if (a.nb.any()) exact_neighbors(a, q, isnan(qn), knn_i[tid], cen_i[tid]);
     }
 }
 
@@ -260,7 +298,7 @@ extern "C" size_t phm_score_workspace_bytes(int64_t n_points, int64_t n_refs, in
 static int score_any(const double *d_points, const uint32_t *d_point_counts, int64_t n_points, int dim,
                      const double *d_refs, int64_t n_refs, int64_t n_positive,
                      const double *d_cent_pos, int64_t n_cent_pos, const double *d_cent_neg, int64_t n_cent_neg,
-                     int k_neighbors, double *d_knn, double *d_kmeans, double *d_combo,
+                     int k_neighbors, double *d_knn, double *d_kmeans, double *d_combo, const phm_neighbors *nb,
                      void *d_workspace, size_t workspace_bytes, void *stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     PHM_REQUIRE(n_points >= 0 && dim > 0, "bad query shape");
@@ -283,6 +321,10 @@ static int score_any(const double *d_points, const uint32_t *d_point_counts, int
     a.row_list = nullptr; a.n_rows_dev = nullptr; a.n_rows = n_points;
     a.k_neighbors = k_neighbors;
     a.knn = d_knn; a.kmeans = d_kmeans; a.combo = d_combo;
+    if (nb) {
+        a.nb.ref_index = nb->d_ref_index; a.nb.ref_distance = nb->d_ref_distance;
+        a.nb.cent_index = nb->d_centroid_index; a.nb.cent_distance = nb->d_centroid_distance;
+    }
 
     const bool tc_ok = tc::score_tc_supported(dim, k_neighbors, n_refs, n_cent_pos, n_cent_neg);
     if (score_path == 2 && !tc_ok) { set_error("tensor-core scoring needs dim = 256, k_neighbors in {1, 3, 5} and both centroid sets"); return PHM_E_UNSUPPORTED; }
@@ -311,7 +353,7 @@ extern "C" int phm_score(const double *d_points, int64_t n_points, int dim,
                          void *d_workspace, size_t workspace_bytes, void *stream) {
     PHM_REQUIRE(d_points != nullptr || n_points == 0, "d_points is null");
     return score_any(d_points, nullptr, n_points, dim, d_refs, n_refs, n_positive, d_cent_pos, n_cent_pos, d_cent_neg, n_cent_neg,
-                     k_neighbors, d_knn, d_kmeans, d_combo, d_workspace, workspace_bytes, stream);
+                     k_neighbors, d_knn, d_kmeans, d_combo, nullptr, d_workspace, workspace_bytes, stream);
 }
 
 // Stages 2 + 3 fused: the query features are never materialised, every kernel forms count / row total on the fly.
@@ -322,7 +364,27 @@ extern "C" int phm_score_counts(const uint32_t *d_counts, int64_t n_points, int 
                                 void *d_workspace, size_t workspace_bytes, void *stream) {
     PHM_REQUIRE(d_counts != nullptr || n_points == 0, "d_counts is null");
     return score_any(nullptr, d_counts, n_points, dim, d_refs, n_refs, n_positive, d_cent_pos, n_cent_pos, d_cent_neg, n_cent_neg,
-                     k_neighbors, d_knn, d_kmeans, d_combo, d_workspace, workspace_bytes, stream);
+                     k_neighbors, d_knn, d_kmeans, d_combo, nullptr, d_workspace, workspace_bytes, stream);
+}
+
+extern "C" int phm_score_neighbors(const double *d_points, int64_t n_points, int dim,
+                                   const double *d_refs, int64_t n_refs, int64_t n_positive,
+                                   const double *d_cent_pos, int64_t n_cent_pos, const double *d_cent_neg, int64_t n_cent_neg,
+                                   int k_neighbors, double *d_knn, double *d_kmeans, double *d_combo, const phm_neighbors *nb,
+                                   void *d_workspace, size_t workspace_bytes, void *stream) {
+    PHM_REQUIRE(d_points != nullptr || n_points == 0, "d_points is null");
+    return score_any(d_points, nullptr, n_points, dim, d_refs, n_refs, n_positive, d_cent_pos, n_cent_pos, d_cent_neg, n_cent_neg,
+                     k_neighbors, d_knn, d_kmeans, d_combo, nb, d_workspace, workspace_bytes, stream);
+}
+
+extern "C" int phm_score_counts_neighbors(const uint32_t *d_counts, int64_t n_points, int dim,
+                                          const double *d_refs, int64_t n_refs, int64_t n_positive,
+                                          const double *d_cent_pos, int64_t n_cent_pos, const double *d_cent_neg, int64_t n_cent_neg,
+                                          int k_neighbors, double *d_knn, double *d_kmeans, double *d_combo, const phm_neighbors *nb,
+                                          void *d_workspace, size_t workspace_bytes, void *stream) {
+    PHM_REQUIRE(d_counts != nullptr || n_points == 0, "d_counts is null");
+    return score_any(nullptr, d_counts, n_points, dim, d_refs, n_refs, n_positive, d_cent_pos, n_cent_pos, d_cent_neg, n_cent_neg,
+                     k_neighbors, d_knn, d_kmeans, d_combo, nb, d_workspace, workspace_bytes, stream);
 }
 
 // Diagnostics of the last tensor-core phm_score call that used this workspace (synchronises the stream).

@@ -805,6 +805,7 @@ struct DecideParams {
     // rows with an overflowed buffer but a final threshold: handed to the list pass instead of the exhaustive kernels
     int64_t *list_rows; unsigned long long *list_count; int list_max_rows;
     float *list_thr; double *list_km;
+    NeighborOut nb;                    // neighbour report (score_decide_kernel<., true> only)
 };
 
 __device__ __forceinline__ double warp_exact_d2(const double (&x)[KDIM / 32], const double *__restrict__ b, int lane) {
@@ -843,7 +844,10 @@ __device__ __forceinline__ int64_t cand_ref_index(const DecideParams &p, uint32_
 #ifndef PHM_DECIDE_MIN_CTAS
 #define PHM_DECIDE_MIN_CTAS 3
 #endif
-template <bool FROM_COUNTS>
+// NEIGHBORS: the call also reports the k nearest references and the nearest centroid of each class (p.nb).  A row then counts as
+// settled only when its k nearest are identified, not merely its vote: every live row re-measures its band (ROW_OPEN), and a row
+// with a dropped candidate within reach goes to the overflow road even when its vote is unanimous.  The scores do not change.
+template <bool FROM_COUNTS, bool NEIGHBORS = false>
 __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(DecideParams p) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -911,10 +915,11 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 if (lost_neg || lost_pos) {
                     // a dropped candidate could still be among the k nearest: only a unanimous vote over kept AND dropped ones
                     // can be read off
-                    if (pos_mask == band && !lost_neg) my_knn = 1.0;
+                    if (NEIGHBORS) state = ROW_FALLBACK;
+                    else if (pos_mask == band && !lost_neg) my_knn = 1.0;
                     else if (pos_mask == 0u && !lost_pos) my_knn = -1.0;
                     else state = ROW_FALLBACK;
-                } else if (n_band == kn || pos_mask == 0u || pos_mask == band) {
+                } else if (!NEIGHBORS && (n_band == kn || pos_mask == 0u || pos_mask == band)) {
                     // the k nearest are exactly the band, or every possible member votes the same way
                     const int pos = (pos_mask == band) ? kn : ((pos_mask == 0u) ? 0 : __popc(pos_mask));
                     my_knn = (2 * pos > kn) ? 1.0 : -1.0;               // 2 * (predict - 0.5), scripts/learning.py:128
@@ -954,6 +959,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
 
         // ---------------- B: warp = row, for every live row of the batch ----------------
         double my_e0 = INFINITY, my_e1 = INFINITY;
+        int64_t my_c0 = -1, my_c1 = -1;                                 // NEIGHBORS: index of the nearest centroid of each class
         unsigned todo = __ballot_sync(FULL, my_live && (has_cent || state == ROW_OPEN || p.stats != nullptr));
         // the count row (or feature row) of the NEXT row to do is fetched while the current one is worked on: the loop is a chain of
         // dependent memory accesses per row otherwise
@@ -1016,6 +1022,10 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 const unsigned posm = __ballot_sync(FULL, in_band && my_idx < p.n_positive);
                 const double knn = (2 * __popc(top & posm) > kn) ? 1.0 : -1.0;
                 if (lane == rr) my_knn = knn;
+                if (NEIGHBORS && in_band && erank < kn) {
+                    if (p.nb.ref_index) p.nb.ref_index[row * kn + erank] = my_idx;
+                    if (p.nb.ref_distance) p.nb.ref_distance[row * kn + erank] = sqrt(my_d2);
+                }
                 if (p.rows_remeasured && lane == 0) atomicAdd(p.rows_remeasured, 1ull);
             }
             if (p.stats) {                    // diagnostics: how much of the proven interval the true value uses
@@ -1039,19 +1049,30 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
             }
             if (has_cent) {
                 double e2[2] = {INFINITY, INFINITY};
+                int64_t i2[2] = {INT64_MAX, INT64_MAX};                  // NEIGHBORS: argmin, first on ties
                 unsigned rest_p = (info >> 12) & 7u, rest_n = (info >> 15) & 7u;
                 if ((info >> 18) & 1u) {
-                    // every centroid, exactly (rare)
+                    // every centroid, exactly (rare); ascending index, so a strict '<' keeps the first of a tie
                     rest_p = 0u; rest_n = 0u;
                     for (int64_t c = 0; c < p.n_cent_pos; c += 2) {
                         const int64_t c1 = c + 1 < p.n_cent_pos ? c + 1 : c;
                         const double a0 = warp_exact_d2(x, p.cent_pos + c * KDIM, lane), a1 = warp_exact_d2(x, p.cent_pos + c1 * KDIM, lane);
-                        e2[0] = fmin(e2[0], fmin(a0, a1));
+                        if (NEIGHBORS) {
+                            if (a0 < e2[0]) { e2[0] = a0; i2[0] = c; }
+                            if (a1 < e2[0]) { e2[0] = a1; i2[0] = c1; }
+                        } else {
+                            e2[0] = fmin(e2[0], fmin(a0, a1));
+                        }
                     }
                     for (int64_t c = 0; c < p.n_cent_neg; c += 2) {
                         const int64_t c1 = c + 1 < p.n_cent_neg ? c + 1 : c;
                         const double a0 = warp_exact_d2(x, p.cent_neg + c * KDIM, lane), a1 = warp_exact_d2(x, p.cent_neg + c1 * KDIM, lane);
-                        e2[1] = fmin(e2[1], fmin(a0, a1));
+                        if (NEIGHBORS) {
+                            if (a0 < e2[1]) { e2[1] = a0; i2[1] = c; }
+                            if (a1 < e2[1]) { e2[1] = a1; i2[1] = c1; }
+                        } else {
+                            e2[1] = fmin(e2[1], fmin(a0, a1));
+                        }
                     }
                 }
                 bool first_round = true;                                 // the lowest kept slot of each class came along from part A
@@ -1070,12 +1091,19 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                     }
 #pragma unroll
                     for (int o = 16; o > 0; o >>= 1) { ap += __shfl_xor_sync(FULL, ap, o); an += __shfl_xor_sync(FULL, an, o); }
-                    if (rest_p) e2[0] = fmin(e2[0], ap);
-                    if (rest_n) e2[1] = fmin(e2[1], an);
+                    if (NEIGHBORS) {
+                        // kept slots are not in index order: the tie rule compares indices
+                        if (rest_p && (ap < e2[0] || (ap == e2[0] && (int64_t)ip < i2[0]))) { e2[0] = ap; i2[0] = ip; }
+                        if (rest_n && (an < e2[1] || (an == e2[1] && (int64_t)in_ < i2[1]))) { e2[1] = an; i2[1] = in_; }
+                    } else {
+                        if (rest_p) e2[0] = fmin(e2[0], ap);
+                        if (rest_n) e2[1] = fmin(e2[1], an);
+                    }
                     rest_p &= rest_p - 1;
                     rest_n &= rest_n - 1;
                 }
                 if (lane == rr) { my_e0 = e2[0]; my_e1 = e2[1]; }
+                if (NEIGHBORS && lane == rr) { my_c0 = i2[0]; my_c1 = i2[1]; }
             }
         }
 
@@ -1103,6 +1131,22 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 if (p.knn) p.knn[my_row] = my_knn;
                 if (p.kmeans) p.kmeans[my_row] = km;
                 if (p.combo) p.combo[my_row] = my_knn + km;                 // scripts/phamer.py:313
+            }
+            if (NEIGHBORS) {
+                // the centroid term of every live row is settled here, whichever road its references take; a NaN row reports
+                // nothing anywhere
+                const bool cen = my_live && has_cent;
+                if (p.nb.cent_index) { p.nb.cent_index[2 * my_row] = cen ? my_c0 : -1; p.nb.cent_index[2 * my_row + 1] = cen ? my_c1 : -1; }
+                if (p.nb.cent_distance) {
+                    p.nb.cent_distance[2 * my_row] = cen ? sqrt(my_e0) : NAN;
+                    p.nb.cent_distance[2 * my_row + 1] = cen ? sqrt(my_e1) : NAN;
+                }
+                if (!my_live) {
+                    for (int t = 0; t < kn; ++t) {
+                        if (p.nb.ref_index) p.nb.ref_index[my_row * kn + t] = -1;
+                        if (p.nb.ref_distance) p.nb.ref_distance[my_row * kn + t] = NAN;
+                    }
+                }
             }
         }
     }
@@ -1202,6 +1246,7 @@ struct ListDecideParams {
     double *knn, *kmeans, *combo;
     int64_t *fallback_rows; unsigned long long *fallback_count;
     unsigned long long *rows_listed;       // statistics: rows settled here
+    NeighborOut nb;                        // neighbour report: the k nearest references (the centroids were reported by score_decide_kernel)
 };
 
 constexpr int LD_K = 5;                    // k_neighbors <= 5 on the tensor-core path
@@ -1274,6 +1319,12 @@ __global__ void __launch_bounds__(256) score_list_decide_kernel(ListDecideParams
             if (p.knn) p.knn[row] = knn;
             if (p.kmeans) p.kmeans[row] = km;
             if (p.combo) p.combo[row] = knn + km;                       // scripts/phamer.py:313
+#pragma unroll
+            for (int t = 0; t < LD_K; ++t) {
+                if (t >= kn) break;
+                if (p.nb.ref_index) p.nb.ref_index[row * kn + t] = bi[t];
+                if (p.nb.ref_distance) p.nb.ref_distance[row * kn + t] = sqrt(bd[t]);
+            }
             atomicAdd(p.rows_listed, 1ull);
         }
     }
@@ -1301,6 +1352,7 @@ struct FallbackParams {
     unsigned int *tickets;                 // [FB_GRID], zero on entry, left zero on exit
     int k_neighbors;
     double *knn, *kmeans, *combo;
+    NeighborOut nb;                        // neighbour report: the k nearest references (the centroids were reported by score_decide_kernel)
 };
 
 // merge `n_lists` lists sorted by (distance, index) into the vote / score of one row (one thread)
@@ -1317,6 +1369,8 @@ __device__ __forceinline__ void fallback_finish(const FallbackParams &f, int64_t
         }
         if (best < 0) break;
         pos += lists[best].i[head[best]] < f.n_positive;
+        if (f.nb.ref_index) f.nb.ref_index[row * kn + t] = lists[best].i[head[best]];
+        if (f.nb.ref_distance) f.nb.ref_distance[row * kn + t] = sqrt(lists[best].d[head[best]]);
         ++head[best];
     }
     const double knn = (2 * pos > kn) ? 1.0 : -1.0;             // scripts/learning.py:128
@@ -1516,8 +1570,13 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
         for (int64_t c = 0; c < f.n_cent_neg; ++c) cn = fmin(cn, warp_exact_d2(x[q], f.cent_neg + c * KDIM, lane));
         if (lane == 0) {
             const int *li = s_i + (warp * QW + q) * FB_K;
+            const double *ld = s_d + (warp * QW + q) * FB_K;
             int pos = 0;
-            for (int t = 0; t < kn; ++t) pos += (li[t] >= 0 && li[t] < f.n_positive);
+            for (int t = 0; t < kn; ++t) {
+                pos += (li[t] >= 0 && li[t] < f.n_positive);
+                if (f.nb.ref_index) f.nb.ref_index[my_row[q] * kn + t] = li[t];
+                if (f.nb.ref_distance) f.nb.ref_distance[my_row[q] * kn + t] = sqrt(ld[t]);
+            }
             const double knn = (2 * pos > kn) ? 1.0 : -1.0;               // scripts/learning.py:128
             double km = NAN;
             if (f.n_cent_pos > 0 && f.n_cent_neg > 0) {
@@ -1677,6 +1736,7 @@ static int launch_prep(const double *src, const uint32_t *src_counts, int64_t n_
 }
 
 static EventRing g_tc_ring;      // brackets of the score_tc_kernel launches (option "time_kernels")
+static EventRing g_decide_ring;  // ... and of the score_decide_kernel launches
 
 template <int KN>
 static int launch_tc_list(const CUtensorMap &map_list, const TcParams &p, cudaStream_t st) {
@@ -1701,6 +1761,7 @@ static int launch_tc(const CUtensorMap &map_a, const TcParams &p, cudaStream_t s
 }
 
 int score_tc_last_ms(float *ms) { return g_tc_ring.mean_ms(ms); }
+int score_decide_last_ms(float *ms) { return g_decide_ring.mean_ms(ms); }
 
 static void ref_permutation(int64_t n_refs, int64_t *perm_a, int64_t *perm_c) {
     // golden-ratio stride coprime to n_refs (see tc_prep_rows_kernel)
@@ -1801,11 +1862,20 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     const bool use_list = score_list_pass != 0;
     r.list_rows = use_list ? w.list_rows : nullptr; r.list_count = w.list_count; r.list_max_rows = w.list_max_rows;
     r.list_thr = w.list_thr; r.list_km = w.list_km;
+    r.nb = a.nb;
     int64_t blocks = (n + 255) / 256;                                  // a warp takes 32 consecutive rows at a time
     if (blocks > 148 * 16) blocks = 148 * 16;
-    if (a.point_counts) score_decide_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(r);
-    else score_decide_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(r);
+    const bool timed = g_decide_ring.begin(st);
+    const bool nb = a.nb.any();
+    if (a.point_counts) {
+        if (nb) score_decide_kernel<true, true><<<(unsigned)blocks, 256, 0, st>>>(r);
+        else score_decide_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(r);
+    } else {
+        if (nb) score_decide_kernel<false, true><<<(unsigned)blocks, 256, 0, st>>>(r);
+        else score_decide_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(r);
+    }
     PHM_LAUNCH_CHECK();
+    if (timed) g_decide_ring.end(st);
 
     // rows whose candidate buffer overflowed but whose threshold is final: second tensor-core pass that lists every reference
     // under the threshold, then the exact decision over the lists (row count read on the device: no host synchronisation)
@@ -1842,6 +1912,7 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
         ld.knn = a.knn; ld.kmeans = a.kmeans; ld.combo = a.combo;
         ld.fallback_rows = w.fallback_rows; ld.fallback_count = w.fallback_count;
         ld.rows_listed = w.rows_listed;
+        ld.nb = a.nb;
         score_list_decide_kernel<<<sm_count() * 2, 256, 0, st>>>(ld);
         PHM_LAUNCH_CHECK();
     }
@@ -1855,6 +1926,7 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     f.k_neighbors = a.k_neighbors;
     f.knn = a.knn; f.kmeans = a.kmeans; f.combo = a.combo;
     f.parts = w.fb_parts; f.tickets = w.fb_tickets;
+    f.nb = a.nb;
     PHM_CUDA_CHECK(cudaMemsetAsync(w.fb_tickets, 0, sizeof(unsigned int) * FB_GRID, st));
     score_fallback_kernel<<<FB_GRID, 256, 0, st>>>(f);                 // few rows: column slices across CTAs
     PHM_LAUNCH_CHECK();

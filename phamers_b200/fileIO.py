@@ -5,6 +5,7 @@ scripts/id_parser.py the path touches:
     FASTA in        read_fasta :28, get_fasta_ids :62 (Bio.SeqIO tokenisation) + id_parser.get_id :89
     feature CSV     read_feature_file :134, save_counts :169  ('#' header lines, then id,c0,c1,...)
     score CSV       save_phamer_scores :241, read_phamer_output :256  ('# ' header, then 'id, score')
+    neighbour CSV   save_phamer_neighbors, read_phamer_neighbors  ('# ' header, then per contig its nearest references and clusters)
 
 Host-side only (bytes and text); no arithmetic happens here.
 """
@@ -283,3 +284,60 @@ def read_phamer_output(filename):
                 continue
             out[line.split(",")[0]] = float(line.split()[1])
     return out
+
+
+# ----------------------------------------------------------------------------------------------------------
+# neighbour CSV (phamer -neighbors): the references and clusters behind each score
+# ----------------------------------------------------------------------------------------------------------
+NEIGHBOR_CLASSES = {1: "phage", 0: "bacteria", -1: ""}
+
+
+def save_phamer_neighbors(ids, reference_ids, reference_labels, reference_distances, clusters, cluster_distances, file_name,
+                          args=None):
+    """'# '-prefixed header lines (header 'PhaMers neighbour file', then the column names), then per contig, in the order of the
+    score file: 'id, reference_1, class_1, distance_1, ..., reference_k, class_k, distance_k, phage_cluster,
+    phage_cluster_distance, bacteria_cluster, bacteria_cluster_distance'.  reference_* are [contigs, k] arrays nearest first,
+    labels 1 = phage / 0 = bacteria (-1: none), clusters / cluster_distances [contigs, 2] (phage, bacteria; cluster -1: none).
+    Distances are printed by numpy's float64 -> str conversion, which round-trips."""
+    header = "PhaMers neighbour file"
+    if args is not None:
+        header = generate_summary(args, header=header)
+    ref_ids = np.asarray(reference_ids).astype(str)
+    k = ref_ids.shape[1]
+    classes = np.vectorize(NEIGHBOR_CLASSES.get, otypes=[str])(np.asarray(reference_labels, dtype=np.int64))
+    ref_dist = np.asarray(reference_distances, dtype=np.float64).astype(str)
+    clusters = np.asarray(clusters, dtype=np.int64)
+    cl_dist = np.asarray(cluster_distances, dtype=np.float64).astype(str)
+    columns = ["id"] + ["%s_%d" % (c, j + 1) for j in range(k) for c in ("reference", "class", "distance")]
+    columns += ["phage_cluster", "phage_cluster_distance", "bacteria_cluster", "bacteria_cluster_distance"]
+    with open(file_name, "w") as fh:
+        for line in header.split("\n"):
+            fh.write("# " + line + "\n")
+        fh.write("# " + ", ".join(columns) + "\n")
+        for i, ident in enumerate(np.asarray(ids).astype(str)):
+            fields = [ident]
+            for j in range(k):
+                fields += [ref_ids[i, j], classes[i, j], ref_dist[i, j]]
+            fields += [str(clusters[i, 0]), cl_dist[i, 0], str(clusters[i, 1]), cl_dist[i, 1]]
+            fh.write(", ".join(fields) + "\n")
+
+
+def read_phamer_neighbors(filename):
+    """The file of save_phamer_neighbors -> (ids [contigs] str, reference_ids [contigs, k] str, reference_labels [contigs, k] int64,
+    reference_distances [contigs, k] float64, clusters [contigs, 2] int64, cluster_distances [contigs, 2] float64)."""
+    labels = {v: c for c, v in NEIGHBOR_CLASSES.items()}
+    rows = []
+    with open(filename, "r") as fh:
+        for line in fh:
+            if line.startswith("#") or not line.strip():
+                continue
+            rows.append(line.rstrip("\n").split(", "))
+    n = len(rows)
+    k = (len(rows[0]) - 5) // 3 if rows else 0
+    ids = np.array([r[0] for r in rows], dtype=str)
+    refs = np.array([[r[1 + 3 * j] for j in range(k)] for r in rows], dtype=str).reshape(n, k)
+    ref_labels = np.array([[labels[r[2 + 3 * j]] for j in range(k)] for r in rows], dtype=np.int64).reshape(n, k)
+    ref_dist = np.array([[float(r[3 + 3 * j]) for j in range(k)] for r in rows], dtype=np.float64).reshape(n, k)
+    clusters = np.array([[int(r[-4]), int(r[-2])] for r in rows], dtype=np.int64).reshape(n, 2)
+    cl_dist = np.array([[float(r[-3]), float(r[-1])] for r in rows], dtype=np.float64).reshape(n, 2)
+    return ids, refs, ref_labels, ref_dist, clusters, cl_dist

@@ -2,6 +2,7 @@
 Drop-in for the hot-path part of the reference's scripts/learning.py.
 
     knn            :118   brute-force k nearest neighbours + vote       -> CUDA (phm_score)
+    kneighbors            the neighbours themselves (scikit-learn's NearestNeighbors.kneighbors) -> CUDA (phm_score_neighbors)
     distances      :47, closest_to :59   distances of one point to a set of points / the nearest of them -> CUDA
                           (phm_distances; inside the scorer the same search is fused into phm_score)
     get_centroids  :69, kmeans :131   reference-set preprocessing         -> host scikit-learn, see references.py
@@ -34,6 +35,21 @@ def knn(queries, ref_data, ref_labels, k=3):
     empty = torch.empty((0, queries.shape[1]), dtype=torch.float64, device="cuda")
     votes, _, _ = ops.score_cuda(torch.from_numpy(queries).cuda(), torch.from_numpy(refs).cuda(), n_pos, empty, empty, k)
     return votes.cpu().numpy()
+
+
+def kneighbors(queries, ref_data, k=3):
+    """The k nearest rows of `ref_data` to each query, as scikit-learn's NearestNeighbors(algorithm="brute").kneighbors returns
+    them: (distances float64[n, k] ascending, indices int64[n, k] into ref_data), computed on the GPU (phm_score_neighbors).
+    Distances are float64 direct differences (as `distances`); equal distances list the lower row first.  k is 1..15."""
+    import torch
+    from . import ops, _lib
+    _lib.require_cuda()
+    queries = np.ascontiguousarray(np.atleast_2d(queries), dtype=np.float64)
+    refs = np.ascontiguousarray(ref_data, dtype=np.float64)
+    empty = torch.empty((0, queries.shape[1]), dtype=torch.float64, device="cuda")
+    # no labels, so no positives-first regrouping as in knn: the reported rows are already the caller's row numbers
+    out = ops.score_neighbors_cuda(torch.from_numpy(queries).cuda(), torch.from_numpy(refs).cuda(), 0, empty, empty, k)
+    return out[4].cpu().numpy(), out[3].cpu().numpy()
 
 
 def distances(vector, data):

@@ -150,6 +150,18 @@ def score_cuda(points, refs, n_positive, cent_pos, cent_neg, k_neighbors=3, out=
     inside the kernels and never materialised (tensor-core shapes only).
     Returns (knn, kmeans, combo) float64[n]; out = optional preallocated (knn, kmeans, combo)."""
     lib = _lib.require_cuda()
+    points, refs, cent_pos, cent_neg = _score_inputs(points, refs, cent_pos, cent_neg)
+    n, dim = points.shape
+    knn, kmeans, combo = (_result(t, (n,), torch.float64) for t in (out if out is not None else (None, None, None)))
+    ws = _score_workspace(lib, points, refs, cent_pos, cent_neg)
+    entry = lib.phm_score_counts if points.dtype == torch.int32 else lib.phm_score
+    check(entry(ptr(points), n, dim, ptr(refs), refs.shape[0], int(n_positive),
+                ptr(cent_pos), cent_pos.shape[0], ptr(cent_neg), cent_neg.shape[0], int(k_neighbors),
+                ptr(knn), ptr(kmeans), ptr(combo), ptr(ws), ws.numel(), stream_ptr()))
+    return knn, kmeans, combo
+
+
+def _score_inputs(points, refs, cent_pos, cent_neg):
     from_counts = points.dtype == torch.int32
     tensors = [points, refs, cent_pos, cent_neg]
     for t in tensors[1:] if from_counts else tensors:
@@ -158,18 +170,41 @@ def score_cuda(points, refs, n_positive, cent_pos, cent_neg, k_neighbors=3, out=
     if not points.is_cuda:
         raise TypeError("score_cuda takes CUDA tensors")
     points, refs, cent_pos, cent_neg = (t.contiguous() for t in tensors)
-    n, dim = points.shape
+    dim = points.shape[1]
     if refs.shape[1] != dim or (cent_pos.numel() and cent_pos.shape[1] != dim) or (cent_neg.numel() and cent_neg.shape[1] != dim):
         raise ValueError("feature widths differ")
-    knn, kmeans, combo = (_result(t, (n,), torch.float64) for t in (out if out is not None else (None, None, None)))
-    ws_bytes = lib.phm_score_workspace_bytes(n, refs.shape[0], cent_pos.shape[0], cent_neg.shape[0], dim)
+    return points, refs, cent_pos, cent_neg
+
+
+def _score_workspace(lib, points, refs, cent_pos, cent_neg):
+    ws_bytes = lib.phm_score_workspace_bytes(points.shape[0], refs.shape[0], cent_pos.shape[0], cent_neg.shape[0], points.shape[1])
     ws = _workspace("score", ws_bytes)
     _last_score_ws[0] = ws
-    entry = lib.phm_score_counts if from_counts else lib.phm_score
+    return ws
+
+
+def score_neighbors_cuda(points, refs, n_positive, cent_pos, cent_neg, k_neighbors=3):
+    """score_cuda that also reports the rows behind each score, from the same device call (phm_score_neighbors).  Returns
+    (knn, kmeans, combo float64[n] -- bit-identical to score_cuda --, ref_index int64[n, k] rows of `refs` of the k nearest references
+    by ascending distance (ties: lower row first), ref_distance float64[n, k] their Euclidean distances, centroid_index int64[n, 2]
+    rows of cent_pos / cent_neg of the nearest positive / negative centroid (-1 for an empty set), centroid_distance float64[n, 2]).
+    A NaN query row reports index -1 and distance NaN."""
+    lib = _lib.require_cuda()
+    points, refs, cent_pos, cent_neg = _score_inputs(points, refs, cent_pos, cent_neg)
+    n, dim = points.shape
+    k = int(k_neighbors)
+    knn, kmeans, combo = (torch.empty((n,), dtype=torch.float64, device="cuda") for _ in range(3))
+    ref_index = torch.empty((n, max(k, 0)), dtype=torch.int64, device="cuda")
+    ref_distance = torch.empty((n, max(k, 0)), dtype=torch.float64, device="cuda")
+    centroid_index = torch.empty((n, 2), dtype=torch.int64, device="cuda")
+    centroid_distance = torch.empty((n, 2), dtype=torch.float64, device="cuda")
+    nb = _lib.Neighbors(ref_index.data_ptr(), ref_distance.data_ptr(), centroid_index.data_ptr(), centroid_distance.data_ptr())
+    ws = _score_workspace(lib, points, refs, cent_pos, cent_neg)
+    entry = lib.phm_score_counts_neighbors if points.dtype == torch.int32 else lib.phm_score_neighbors
     check(entry(ptr(points), n, dim, ptr(refs), refs.shape[0], int(n_positive),
-                ptr(cent_pos), cent_pos.shape[0], ptr(cent_neg), cent_neg.shape[0], int(k_neighbors),
-                ptr(knn), ptr(kmeans), ptr(combo), ptr(ws), ws.numel(), stream_ptr()))
-    return knn, kmeans, combo
+                ptr(cent_pos), cent_pos.shape[0], ptr(cent_neg), cent_neg.shape[0], k,
+                ptr(knn), ptr(kmeans), ptr(combo), ctypes.byref(nb), ptr(ws), ws.numel(), stream_ptr()))
+    return knn, kmeans, combo, ref_index, ref_distance, centroid_index, centroid_distance
 
 
 def count_score_cuda(seq, offsets, refs, n_positive, cent_pos, cent_neg, k_neighbors=3, out_counts=None, out=None):
@@ -251,7 +286,8 @@ def synth_contigs(seed, first_contig, n_contigs):
 
 
 def last_kernel_ms(kernel="score_tc_kernel"):
-    """Mean device time of the launches of a hot kernel ('kmer_hist_kernel', 'score_tc_kernel') since the last call (after
+    """Mean device time of the launches of a hot kernel ('kmer_hist_kernel', 'score_tc_kernel', 'score_decide_kernel') since the
+    last call (after
     _lib.set_option('time_kernels', 1))."""
     ms = ctypes.c_float(0.0)
     check(_lib.require_cuda().phm_last_kernel_ms(kernel.encode(), ctypes.byref(ms)))

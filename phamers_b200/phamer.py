@@ -48,6 +48,13 @@ class phamer_scorer(object):
         self.k_clusters = 86                                 # :78
         self.k_neighbors = 3                                 # :79
         self.scores = None
+        # filled by score_neighbors(): per contig the k_neighbors nearest references (ids, 1 = phage / 0 = bacteria, distances)
+        # and the nearest phage / bacteria cluster (k-means label, -1 without centroids) with its distance
+        self.neighbor_ids = None
+        self.neighbor_labels = None
+        self.neighbor_distances = None
+        self.nearest_clusters = None
+        self.nearest_cluster_distances = None
 
     # ---- data -------------------------------------------------------------------------------------------
     def load_reference_data(self, positive_features_file=None, negative_features_file=None):
@@ -100,9 +107,9 @@ class phamer_scorer(object):
         self.num_positive = self.num_negative = num_ref
 
     # ---- scoring ----------------------------------------------------------------------------------------
-    def _device_scores(self):
+    def _device_inputs(self):
         import torch
-        from . import ops, _lib
+        from . import _lib
         _lib.require_cuda()
         pts = np.ascontiguousarray(self.data_points, dtype=np.float64)
         pos = np.ascontiguousarray(self.positive_data, dtype=np.float64)
@@ -112,9 +119,12 @@ class phamer_scorer(object):
         else:
             cpos = cneg = np.zeros((0, pts.shape[1]))
         refs = torch.from_numpy(np.vstack((pos, neg))).cuda()                         # :186
-        out = ops.score_cuda(torch.from_numpy(pts).cuda(), refs, pos.shape[0],
-                             torch.from_numpy(np.ascontiguousarray(cpos)).cuda(),
-                             torch.from_numpy(np.ascontiguousarray(cneg)).cuda(), self.k_neighbors)
+        return (torch.from_numpy(pts).cuda(), refs, pos.shape[0], torch.from_numpy(np.ascontiguousarray(cpos)).cuda(),
+                torch.from_numpy(np.ascontiguousarray(cneg)).cuda(), self.k_neighbors)
+
+    def _device_scores(self):
+        from . import ops
+        out = ops.score_cuda(*self._device_inputs())
         return [t.cpu().numpy() for t in out]
 
     def score_points(self):
@@ -131,6 +141,32 @@ class phamer_scorer(object):
                                       % self.scoring_method)
         knn, km, combo = self._device_scores()
         self.scores = {"knn": knn, "kmeans": km, "combo": combo}[self.scoring_method]
+        return self.scores
+
+    def score_neighbors(self):
+        """score_points that also fills neighbor_ids / neighbor_labels / neighbor_distances ([contigs, k_neighbors]: the references
+        that cast the kNN vote, nearest first) and nearest_clusters / nearest_cluster_distances ([contigs, 2]: the phage and the
+        bacteria cluster whose centroid distances enter the kmeans score), from the same device call.  The scores are those of
+        score_points.  A contig with no countable k-mer gets id "", label -1, cluster -1 and distance NaN."""
+        from . import ops
+        self.num_points = self.data_points.shape[0]
+        self.num_positive = self.positive_data.shape[0]
+        self.num_negative = self.negative_data.shape[0]
+        if self.scoring_method not in self.all_scoring_methods:
+            raise KeyError(self.scoring_method)
+        if self.scoring_method not in ("knn", "kmeans", "combo"):
+            raise NotImplementedError("scoring method %r is outside the B200 hot path (knn / kmeans / combo only)"
+                                      % self.scoring_method)
+        knn, km, combo, ref_i, ref_d, cen_i, cen_d = [t.cpu().numpy() for t in ops.score_neighbors_cuda(*self._device_inputs())]
+        self.scores = {"knn": knn, "kmeans": km, "combo": combo}[self.scoring_method]
+        pos_ids = self.positive_ids if self.positive_ids is not None else np.arange(self.num_positive)
+        neg_ids = self.negative_ids if self.negative_ids is not None else np.arange(self.num_negative)
+        all_ids = np.concatenate((np.asarray(pos_ids).astype(str), np.asarray(neg_ids).astype(str), [""]))
+        self.neighbor_ids = all_ids[ref_i]                        # index -1 (NaN row) picks the trailing ""
+        self.neighbor_labels = np.where(ref_i < 0, -1, (ref_i < self.num_positive).astype(np.int64))
+        self.neighbor_distances = ref_d
+        self.nearest_clusters = cen_i
+        self.nearest_cluster_distances = cen_d
         return self.scores
 
     def knn_score_points(self):
@@ -181,6 +217,12 @@ class phamer_scorer(object):
         self.phamer_output_filename = self.get_phamer_output_filename()
         fileIO.save_phamer_scores(self.data_ids, self.scores, self.phamer_output_filename, args=args)
 
+    def make_neighbors_file(self, args=None):
+        """<out>/phamer_neighbors.csv: the rows of phamer_scores.csv with the references and clusters behind each score."""
+        self.phamer_neighbors_filename = os.path.join(self.output_directory, "phamer_neighbors.csv")
+        fileIO.save_phamer_neighbors(self.data_ids, self.neighbor_ids, self.neighbor_labels, self.neighbor_distances,
+                                     self.nearest_clusters, self.nearest_cluster_distances, self.phamer_neighbors_filename, args=args)
+
 
 def score_points(scoring_data, positive_training_data, negative_training_data, method=None):
     """scripts/phamer.py:451-468."""
@@ -217,7 +259,8 @@ def decide_files(scorer, args):
 
 def main(argv=None):
     """The reference's command line (scripts/phamer.py:510-599) for the hot path: count the contigs of a FASTA (or read their
-    feature CSV), score them against the reference features, write <out>/phamer_scores.csv.  t-SNE and plots are out of scope."""
+    feature CSV), score them against the reference features, write <out>/phamer_scores.csv (and with -neighbors
+    <out>/phamer_neighbors.csv).  t-SNE and plots are out of scope."""
     import argparse
     parser = argparse.ArgumentParser(description="Scores contigs based on feature similarity (B200 path)",
                                      formatter_class=argparse.ArgumentDefaultsHelpFormatter)
@@ -232,6 +275,8 @@ def main(argv=None):
     parser.add_argument("-l", "--length_requirement", type=int, default=5000, help="Sequence length requirement")
     parser.add_argument("-equal", "--equalize_reference", action="store_true", help="Use same number of reference data from each")
     parser.add_argument("-m", "--method", default="combo", help="Learning algorithm name")
+    parser.add_argument("-neighbors", "--write_neighbors", action="store_true",
+                        help="Also write phamer_neighbors.csv: the nearest references and clusters behind each score")
     parser.add_argument("-do_tsne", "--do_tsne", action="store_true", help="(out of scope)")
     parser.add_argument("-plot", "--plot_tsne", action="store_true", help="(out of scope)")
     args = parser.parse_args(argv)
@@ -246,8 +291,14 @@ def main(argv=None):
         scorer.equalize_reference_data()
     if not os.path.isdir(scorer.output_directory):
         os.makedirs(scorer.output_directory)
-    scorer.scores = scorer.score_points()
-    scorer.make_summary_file(args=args)
+    if args.write_neighbors:
+        scorer.scores = scorer.score_neighbors()
+        scorer.make_neighbors_file(args=args)
+    else:
+        scorer.scores = scorer.score_points()
+    # the score file's header does not depend on whether neighbours were asked for
+    score_args = argparse.Namespace(**{k: v for k, v in vars(args).items() if k != "write_neighbors"})
+    scorer.make_summary_file(args=score_args)
     return scorer
 
 
