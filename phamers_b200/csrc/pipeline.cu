@@ -55,9 +55,8 @@ extern "C" int phm_count_score(const uint8_t *d_seq, const int64_t *d_offsets, i
     a.cent_pos = d_cent_pos; a.n_cent_pos = n_cent_pos;
     a.cent_neg = d_cent_neg; a.n_cent_neg = n_cent_neg;
     a.norm_points = a.norm_refs = a.norm_cpos = a.norm_cneg = nullptr;
-    a.row_list = nullptr; a.n_rows_dev = nullptr; a.n_rows = n_contigs;
-    a.k_neighbors = k_neighbors;
-    a.knn = d_knn; a.kmeans = d_kmeans; a.combo = d_combo;
+    a.out.k = k_neighbors;
+    a.out.knn = d_knn; a.out.kmeans = d_kmeans; a.out.combo = d_combo;
 
     tc::QueryEmit emit;
     int rc = tc::score_tc_begin(a, score_ws, score_ws_bytes, st, &emit);                          // references: rho, pmax, B operand

@@ -15,6 +15,53 @@ struct NeighborOut {
     __host__ __device__ bool any() const { return ref_index || ref_distance || cent_index || cent_distance; }
 };
 
+// What a scoring call writes for each row: the three scores (each may be null) and the neighbour report.
+struct ScoreOut {
+    int k;                                    // k_neighbors: report slots per row
+    double *knn, *kmeans, *combo;
+    NeighborOut nb;                           // all null: scores only
+};
+
+// ---- the rules of a row's outputs, the same on every road that finishes rows ----
+__device__ __forceinline__ double knn_vote(int n_pos, int k) {
+    return (2 * n_pos > k) ? 1.0 : -1.0;                               // 2 * (predict - 0.5), scripts/learning.py:128
+}
+// e_pos, e_neg: distances (not squares) to the nearest centroid of each class
+__device__ __forceinline__ double kmeans_score(double e_pos, double e_neg) {
+    return tanh((e_neg - e_pos) / (e_pos + e_neg));                    // scripts/phamer.py:206-209
+}
+__device__ __forceinline__ void put_scores(const ScoreOut &o, int64_t row, double knn, double km) {
+    if (o.knn) o.knn[row] = knn;
+    if (o.kmeans) o.kmeans[row] = km;
+    if (o.combo) o.combo[row] = knn + km;                              // scripts/phamer.py:313
+}
+// one reported (index, distance) pair: slot `at` of the reference report (row * k + j) or of the centroid report (row * 2 + class)
+__device__ __forceinline__ void put_neighbor(int64_t *index, double *distance, int64_t at, int64_t i, double d) {
+    if (index) index[at] = i;
+    if (distance) distance[at] = d;
+}
+// a NaN row reports index -1 and distance NaN everywhere
+__device__ __forceinline__ void put_nan_row(const ScoreOut &o, int64_t row) {
+    for (int j = 0; j < o.k; ++j) put_neighbor(o.nb.ref_index, o.nb.ref_distance, row * o.k + j, -1, NAN);
+    for (int c = 0; c < 2; ++c) put_neighbor(o.nb.cent_index, o.nb.cent_distance, row * 2 + c, -1, NAN);
+}
+
+// ---- the order of neighbours: distance, then the lower index ----
+// Roads that see candidates in ascending index (the exhaustive kernels, score_exact_kernel) keep with this comparator exactly
+// what a strict '<' on the distance keeps: a later candidate never wins a tie.
+template <typename I>
+__device__ __forceinline__ bool nearer(double d, I i, double e, I j) { return d < e || (d == e && i < j); }
+
+// insertion of (v, i) into a list of k entries sorted by nearer() (empty entries: INFINITY); drops the last entry
+template <typename I>
+__device__ __forceinline__ void list_insert(double *d, I *idx, int k, double v, I i) {
+    if (!nearer(v, i, d[k - 1], idx[k - 1])) return;
+    int s = k - 1;
+    for (; s > 0 && nearer(v, i, d[s - 1], idx[s - 1]); --s) { d[s] = d[s - 1]; idx[s] = idx[s - 1]; }
+    d[s] = v;
+    idx[s] = i;
+}
+
 struct ScoreArgs {
     const double *points; int64_t n_points; int dim;
     const uint32_t *point_counts;             // optional: raw count rows instead of `points` (features = row / row sum, formed on the fly)
@@ -22,12 +69,7 @@ struct ScoreArgs {
     const double *cent_pos; int64_t n_cent_pos;
     const double *cent_neg; int64_t n_cent_neg;
     const double *norm_points, *norm_refs, *norm_cpos, *norm_cneg;    // squared row norms (float64)
-    const int64_t *row_list;                  // optional: score only these rows
-    const unsigned long long *n_rows_dev;     // optional: number of rows in row_list, read on the device
-    int64_t n_rows;                           // rows to score (upper bound when n_rows_dev is set)
-    int k_neighbors;
-    double *knn, *kmeans, *combo;
-    NeighborOut nb;                           // neighbour report (all null: scores only)
+    ScoreOut out;
 };
 
 int launch_score_exact(const ScoreArgs &a, cudaStream_t st);
@@ -110,7 +152,7 @@ int score_tc_begin(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t s
 int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, bool queries_prepared);
 bool score_tc_supported(int dim, int k_neighbors, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg);
 size_t score_tc_workspace_bytes(int64_t n_points, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg);
-int score_tc(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, int *kernels_launched);
+int score_tc(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st);
 int score_tc_last_ms(float *ms);
 int score_decide_last_ms(float *ms);
 int score_tc_stats(const void *ws, unsigned long long *fallback_rows, float *max_rank_error, cudaStream_t st);

@@ -70,35 +70,33 @@ __device__ __forceinline__ double direct_distance(const double *p, const double 
 // index on ties).  At a near tie (a gap below the expansion's rounding) the selection may keep the other member of the tie than
 // the tensor-core path does.  A NaN row reports index -1 and distance NaN everywhere.
 __device__ void exact_neighbors(const ScoreArgs &a, int64_t q, bool nan_row, const int (&ki)[KNN_MAX + 1], const int (&ci)[4]) {
-    const int kn = a.k_neighbors;
+    const ScoreOut &o = a.out;
+    if (nan_row) { put_nan_row(o, q); return; }
+    const int kn = o.k;
     const double *p = a.points + q * a.dim;
     double d[KNN_MAX];
     int64_t id[KNN_MAX];
     for (int j = 0; j < kn; ++j) {
-        const bool ok = !nan_row && ki[j] >= 0;
+        const bool ok = ki[j] >= 0;
         id[j] = ok ? ki[j] : -1;
         d[j] = ok ? direct_distance(p, a.refs + (int64_t)ki[j] * a.dim, a.dim) : NAN;
-        for (int s = j; s > 0 && (d[s] < d[s - 1] || (d[s] == d[s - 1] && id[s] < id[s - 1])); --s) {
+        for (int s = j; s > 0 && nearer(d[s], id[s], d[s - 1], id[s - 1]); --s) {
             const double td = d[s]; d[s] = d[s - 1]; d[s - 1] = td;
             const int64_t ti = id[s]; id[s] = id[s - 1]; id[s - 1] = ti;
         }
     }
-    for (int j = 0; j < kn; ++j) {
-        if (a.nb.ref_index) a.nb.ref_index[q * kn + j] = id[j];
-        if (a.nb.ref_distance) a.nb.ref_distance[q * kn + j] = d[j];
-    }
+    for (int j = 0; j < kn; ++j) put_neighbor(o.nb.ref_index, o.nb.ref_distance, q * kn + j, id[j], d[j]);
     for (int c = 0; c < 2; ++c) {
         const double *cent = c ? a.cent_neg : a.cent_pos;
         int64_t best = -1;
         double bd = NAN;
-        for (int j = 0; j < 2 && !nan_row; ++j) {
+        for (int j = 0; j < 2; ++j) {
             const int i = ci[2 * c + j];
             if (i < 0) continue;
             const double e = direct_distance(p, cent + (int64_t)i * a.dim, a.dim);
-            if (best < 0 || e < bd || (e == bd && i < best)) { best = i; bd = e; }
+            if (best < 0 || nearer(e, (int64_t)i, bd, best)) { best = i; bd = e; }
         }
-        if (a.nb.cent_index) a.nb.cent_index[q * 2 + c] = best;
-        if (a.nb.cent_distance) a.nb.cent_distance[q * 2 + c] = bd;
+        put_neighbor(o.nb.cent_index, o.nb.cent_distance, q * 2 + c, best, bd);
     }
 }
 
@@ -112,14 +110,12 @@ __global__ void __launch_bounds__(256) score_exact_kernel(ScoreArgs a) {
     const int tid = threadIdx.x;
     const int tx = tid & 15, ty = tid >> 4;
     const int64_t q0 = (int64_t)blockIdx.x * TQ;
-    const int64_t n_rows = a.n_rows_dev ? (int64_t)*a.n_rows_dev : a.n_rows;
-    if (q0 >= n_rows) return;
     const int64_t n_cols = a.n_refs + a.n_cent_pos + a.n_cent_neg;
-    const int kn = a.k_neighbors;
+    const int kn = a.out.k;
 
     if (tid < TQ) {
         const int64_t r = q0 + tid;
-        qrow[tid] = (r < n_rows) ? (a.row_list ? a.row_list[r] : r) : -1;
+        qrow[tid] = (r < a.n_points) ? r : -1;
         for (int j = 0; j <= KNN_MAX; ++j) { knn_d[tid][j] = INFINITY; knn_i[tid][j] = -1; }
         for (int j = 0; j < 4; ++j) { cen_d[tid][j] = INFINITY; cen_i[tid][j] = -1; }
     }
@@ -175,16 +171,7 @@ __global__ void __launch_bounds__(256) score_exact_kernel(ScoreArgs a) {
                 if (col >= n_cols) break;
                 const double d = Ds[tid][j];
                 if (col < a.n_refs) {
-                    if (d < knn_d[tid][kn - 1]) {            // strict: earlier index wins ties
-                        int s = kn - 1;
-                        while (s > 0 && knn_d[tid][s - 1] > d) {
-                            knn_d[tid][s] = knn_d[tid][s - 1];
-                            knn_i[tid][s] = knn_i[tid][s - 1];
-                            --s;
-                        }
-                        knn_d[tid][s] = d;
-                        knn_i[tid][s] = (int)col;
-                    }
+                    list_insert(knn_d[tid], knn_i[tid], kn, d, (int)col);
                 } else {
                     const bool neg = col >= a.n_refs + a.n_cent_pos;
                     const int b = neg ? 2 : 0;
@@ -208,7 +195,7 @@ __global__ void __launch_bounds__(256) score_exact_kernel(ScoreArgs a) {
         if (!isnan(qn)) {
             int pos = 0;
             for (int j = 0; j < kn; ++j) pos += (knn_i[tid][j] >= 0 && knn_i[tid][j] < a.n_positive);
-            knn = (2 * pos > kn) ? 1.0 : -1.0;                      // 2 * (predict - 0.5), learning.py:128
+            knn = knn_vote(pos, kn);
             if (a.n_cent_pos > 0 && a.n_cent_neg > 0) {
                 const double *p = a.points + q * a.dim;
                 double e_pos = INFINITY, e_neg = INFINITY;
@@ -216,19 +203,17 @@ __global__ void __launch_bounds__(256) score_exact_kernel(ScoreArgs a) {
                     if (cen_i[tid][j] >= 0) e_pos = fmin(e_pos, direct_distance(p, a.cent_pos + (int64_t)cen_i[tid][j] * a.dim, a.dim));
                     if (cen_i[tid][2 + j] >= 0) e_neg = fmin(e_neg, direct_distance(p, a.cent_neg + (int64_t)cen_i[tid][2 + j] * a.dim, a.dim));
                 }
-                km = tanh((e_neg - e_pos) / (e_pos + e_neg));      // phamer.py:206-209
+                km = kmeans_score(e_pos, e_neg);
             }
         }
-        if (a.knn) a.knn[q] = knn;
-        if (a.kmeans) a.kmeans[q] = km;
-        if (a.combo) a.combo[q] = knn + km;                           // phamer.py:313
-        if (a.nb.any()) exact_neighbors(a, q, isnan(qn), knn_i[tid], cen_i[tid]);
+        put_scores(a.out, q, knn, km);
+        if (a.out.nb.any()) exact_neighbors(a, q, isnan(qn), knn_i[tid], cen_i[tid]);
     }
 }
 
 int launch_score_exact(const ScoreArgs &a, cudaStream_t st) {
-    if (a.n_rows == 0) return PHM_OK;
-    const int64_t blocks = (a.n_rows + TQ - 1) / TQ;
+    if (a.n_points == 0) return PHM_OK;
+    const int64_t blocks = (a.n_points + TQ - 1) / TQ;
     PHM_CUDA_CHECK(cudaFuncSetAttribute(score_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ExactSmem)));
     score_exact_kernel<<<(unsigned)blocks, 256, sizeof(ExactSmem), st>>>(a);
     PHM_LAUNCH_CHECK();
@@ -318,17 +303,16 @@ static int score_any(const double *d_points, const uint32_t *d_point_counts, int
     a.refs = d_refs; a.n_refs = n_refs; a.n_positive = n_positive;
     a.cent_pos = d_cent_pos; a.n_cent_pos = n_cent_pos;
     a.cent_neg = d_cent_neg; a.n_cent_neg = n_cent_neg;
-    a.row_list = nullptr; a.n_rows_dev = nullptr; a.n_rows = n_points;
-    a.k_neighbors = k_neighbors;
-    a.knn = d_knn; a.kmeans = d_kmeans; a.combo = d_combo;
+    a.out.k = k_neighbors;
+    a.out.knn = d_knn; a.out.kmeans = d_kmeans; a.out.combo = d_combo;
     if (nb) {
-        a.nb.ref_index = nb->d_ref_index; a.nb.ref_distance = nb->d_ref_distance;
-        a.nb.cent_index = nb->d_centroid_index; a.nb.cent_distance = nb->d_centroid_distance;
+        a.out.nb.ref_index = nb->d_ref_index; a.out.nb.ref_distance = nb->d_ref_distance;
+        a.out.nb.cent_index = nb->d_centroid_index; a.out.nb.cent_distance = nb->d_centroid_distance;
     }
 
     const bool tc_ok = tc::score_tc_supported(dim, k_neighbors, n_refs, n_cent_pos, n_cent_neg);
     if (score_path == 2 && !tc_ok) { set_error("tensor-core scoring needs dim = 256, k_neighbors in {1, 3, 5} and both centroid sets"); return PHM_E_UNSUPPORTED; }
-    if (score_path != 1 && tc_ok) return tc::score_tc(a, d_workspace, workspace_bytes, st, nullptr);
+    if (score_path != 1 && tc_ok) return tc::score_tc(a, d_workspace, workspace_bytes, st);
     if (d_point_counts) {
         set_error("scoring from raw counts needs the tensor-core path (dim = 256, k_neighbors in {1, 3, 5}, both centroid sets); "
                   "normalise first (phm_normalize_counts) and call phm_score");

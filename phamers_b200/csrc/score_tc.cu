@@ -150,11 +150,6 @@ __device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32
         : "r"(taddr) : "memory");
 }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ float tmem_ld1(uint32_t taddr) {
-    uint32_t r;
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];\n\ttcgen05.wait::ld.sync.aligned;" : "=r"(r) : "r"(taddr) : "memory");
-    return __uint_as_float(r);
-}
 __device__ __forceinline__ uint2 lds_v2(uint32_t addr) {
     uint2 v;
     asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(addr) : "memory");
@@ -222,10 +217,6 @@ __device__ __forceinline__ float pick32(const float (&v)[32], int j) {       // 
     }
 }
 
-// 32 accumulator columns of this thread's row (already in registers): lower bounds and their minimum against the row's
-// threshold; only if some lane of the warp has a hit are the hits looked at, one warp-uniform column at a time.
-// INSERT = false: the threshold is already final for these columns (second pass of a two-pass tile), hits are only collected.
-struct NoIssue { __device__ __forceinline__ void operator()() const {} };
 __device__ __forceinline__ float max32(const uint32_t (&r)[32]) {
     float g[8];
 #pragma unroll
@@ -237,18 +228,16 @@ __device__ __forceinline__ float max32(const uint32_t (&r)[32]) {
 // the chunk's smallest lower bound is minus the largest accumulator, and only if it beats the row's threshold in some lane of the
 // warp are the hits looked at, one warp-uniform column at a time.
 // INSERT = false: the threshold is already final for these columns (second pass of a two-pass tile), hits are only collected.
-// issue_next() is called as soon as the accumulators in `r` are no longer needed by the common path.
-template <int K, int CAP, bool INSERT, bool LABELLED, typename Issue = NoIssue>
+template <int K, int CAP, bool INSERT, bool LABELLED>
 __device__ __forceinline__ void scan_chunk(const uint32_t (&r)[32], uint32_t p_c, int col_c,
                                            int n_class, float C, uint32_t cand_addr, int first, float (&u)[K], int &cnt,
-                                           uint32_t &flags, float (&drop_lo)[2], Issue issue_next = Issue()) {
+                                           uint32_t &flags, float (&drop_lo)[2]) {
     const float limit0 = u[K - 1];
     const float m = -max32(r);
-    if (!__any_sync(FULL, m <= limit0)) { issue_next(); return; }
+    if (!__any_sync(FULL, m <= limit0)) return;
     float lo[32];
 #pragma unroll
     for (int j = 0; j < 32; ++j) lo[j] = -__uint_as_float(r[j]);
-    issue_next();
 
     // sign of (limit - lo) shifted in column by column: column 0 ends in the top bit, a clear bit is a hit (lo <= limit)
     uint32_t mq[4] = {0u, 0u, 0u, 0u};                   // four independent chains of 8 columns
@@ -601,7 +590,6 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, TcParams p) {
                 }
                 for (int nt = nt_lo; nt < nt_hi; ++nt, ++tile) {
                     const uint32_t set = tile & 1u;
-                    const uint32_t stg = sm_stg + set * (2 * BN * 4);
                     mbar_wait(bar_t_full + 8 * set, (tile >> 1) & 1u);
                     mbar_wait(bar_n_full + 8 * set, (tile >> 1) & 1u);      // P of the tile (hits only): issued with the MMAs, long there by now
                     tc_fence_after();
@@ -797,27 +785,40 @@ struct DecideParams {
     const double *cnorm_points;        // centred squared norms of the query rows (NaN = NaN feature row)
     const uint32_t *row_total;         // row totals of the count rows (written by whoever prepared the query operands)
     const uint2 *cand; const float *cand_up; const uint32_t *meta; const float2 *drop_lo; const float *thr;
-    int k_neighbors;
-    double *knn, *kmeans, *combo;
+    ScoreOut out;                      // the neighbour report is written by score_decide_kernel<., true> only
     int64_t *fallback_rows; unsigned long long *fallback_count;
     float *stats;                      // when non-null: [0] max |x - exact| / (C P) (must stay <= 1), [1] max |x - exact| in d2 units
     unsigned long long *rows_remeasured;
     // rows with an overflowed buffer but a final threshold: handed to the list pass instead of the exhaustive kernels
     int64_t *list_rows; unsigned long long *list_count; int list_max_rows;
     float *list_thr; double *list_km;
-    NeighborOut nb;                    // neighbour report (score_decide_kernel<., true> only)
 };
 
-__device__ __forceinline__ double warp_exact_d2(const double (&x)[KDIM / 32], const double *__restrict__ b, int lane) {
-    double acc = 0.0;
+// Squared float64 direct-difference distances of a query row (x: this lane's 8 features, lane-strided) to U rows at once.  Every
+// exact road measures its (row, reference) and (row, centroid) pairs with this: each lane's fma chain over its features in
+// ascending order, then the butterfly xor 16 ... 1, so that the roads agree bit for bit.  U > 1 keeps independent rows in flight
+// where a loop over rows is latency-bound.
+template <int U>
+__device__ __forceinline__ void warp_d2(const double (&x)[KDIM / 32], const double *const (&b)[U], int lane, double (&acc)[U]) {
 #pragma unroll
-    for (int i = 0; i < KDIM / 32; ++i) {
-        const double t = x[i] - b[lane + 32 * i];
-        acc = fma(t, t, acc);
-    }
+    for (int t = 0; t < U; ++t) acc[t] = 0.0;
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(FULL, acc, o);
-    return acc;
+    for (int i = 0; i < KDIM / 32; ++i)
+#pragma unroll
+        for (int t = 0; t < U; ++t) {
+            const double d = x[i] - b[t][lane + 32 * i];
+            acc[t] = fma(d, d, acc[t]);
+        }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+        for (int t = 0; t < U; ++t) acc[t] += __shfl_xor_sync(FULL, acc[t], o);
+}
+__device__ __forceinline__ double warp_d2(const double (&x)[KDIM / 32], const double *b, int lane) {
+    const double *const rows[1] = {b};
+    double acc[1];
+    warp_d2<1>(x, rows, lane, acc);
+    return acc[0];
 }
 
 __device__ __forceinline__ double warp_min_d(double v) {
@@ -852,7 +853,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    const int kn = p.k_neighbors;
+    const int kn = p.out.k;
     const bool has_cent = p.n_cent_pos > 0 && p.n_cent_neg > 0;
     for (int64_t base = warp * 32; base < p.n_points; base += n_warps * 32) {
         // ---------------- A: lane = row ----------------
@@ -922,7 +923,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 } else if (!NEIGHBORS && (n_band == kn || pos_mask == 0u || pos_mask == band)) {
                     // the k nearest are exactly the band, or every possible member votes the same way
                     const int pos = (pos_mask == band) ? kn : ((pos_mask == 0u) ? 0 : __popc(pos_mask));
-                    my_knn = (2 * pos > kn) ? 1.0 : -1.0;               // 2 * (predict - 0.5), scripts/learning.py:128
+                    my_knn = knn_vote(pos, kn);
                 } else {
                     state = ROW_OPEN;                                    // exact distances of the band decide (part B)
                 }
@@ -1005,7 +1006,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                     const int s = __ffs(rest) - 1;
                     rest &= rest - 1;
                     const int64_t idx = cand_ref_index(p, ent[s].y);
-                    const double d = warp_exact_d2(x, p.refs + idx * KDIM, lane);
+                    const double d = warp_d2(x, p.refs + idx * KDIM, lane);
                     if (lane == s) { my_d2 = d; my_idx = idx; }
                 }
                 int erank = 0;
@@ -1020,12 +1021,9 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 const bool in_band = lane < CAP_R && ((bnd >> lane) & 1u);
                 const unsigned top = __ballot_sync(FULL, in_band && erank < kn);
                 const unsigned posm = __ballot_sync(FULL, in_band && my_idx < p.n_positive);
-                const double knn = (2 * __popc(top & posm) > kn) ? 1.0 : -1.0;
+                const double knn = knn_vote(__popc(top & posm), kn);
                 if (lane == rr) my_knn = knn;
-                if (NEIGHBORS && in_band && erank < kn) {
-                    if (p.nb.ref_index) p.nb.ref_index[row * kn + erank] = my_idx;
-                    if (p.nb.ref_distance) p.nb.ref_distance[row * kn + erank] = sqrt(my_d2);
-                }
+                if (NEIGHBORS && in_band && erank < kn) put_neighbor(p.out.nb.ref_index, p.out.nb.ref_distance, row * kn + erank, my_idx, sqrt(my_d2));
                 if (p.rows_remeasured && lane == 0) atomicAdd(p.rows_remeasured, 1ull);
             }
             if (p.stats) {                    // diagnostics: how much of the proven interval the true value uses
@@ -1036,7 +1034,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 for (int s = 0; s < CAP_R && s < cnt_r; ++s) {
                     const uint2 e = ent[s];
                     const double lo_s = (double)__uint_as_float(e.x), w_s = (double)p.cand_up[row * NENT + s] - lo_s;
-                    const double d = warp_exact_d2(x, p.refs + cand_ref_index(p, e.y) * KDIM, lane);
+                    const double d = warp_d2(x, p.refs + cand_ref_index(p, e.y) * KDIM, lane);
                     const double exact = (d - na) * NORM_SCALE;                 // what the ranking value estimates
                     const double err = fabs(lo_s + 0.5 * w_s - exact);
                     worst_abs = fmaxf(worst_abs, (float)(err / NORM_SCALE));
@@ -1054,24 +1052,19 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 if ((info >> 18) & 1u) {
                     // every centroid, exactly (rare); ascending index, so a strict '<' keeps the first of a tie
                     rest_p = 0u; rest_n = 0u;
-                    for (int64_t c = 0; c < p.n_cent_pos; c += 2) {
-                        const int64_t c1 = c + 1 < p.n_cent_pos ? c + 1 : c;
-                        const double a0 = warp_exact_d2(x, p.cent_pos + c * KDIM, lane), a1 = warp_exact_d2(x, p.cent_pos + c1 * KDIM, lane);
-                        if (NEIGHBORS) {
-                            if (a0 < e2[0]) { e2[0] = a0; i2[0] = c; }
-                            if (a1 < e2[0]) { e2[0] = a1; i2[0] = c1; }
-                        } else {
-                            e2[0] = fmin(e2[0], fmin(a0, a1));
-                        }
-                    }
-                    for (int64_t c = 0; c < p.n_cent_neg; c += 2) {
-                        const int64_t c1 = c + 1 < p.n_cent_neg ? c + 1 : c;
-                        const double a0 = warp_exact_d2(x, p.cent_neg + c * KDIM, lane), a1 = warp_exact_d2(x, p.cent_neg + c1 * KDIM, lane);
-                        if (NEIGHBORS) {
-                            if (a0 < e2[1]) { e2[1] = a0; i2[1] = c; }
-                            if (a1 < e2[1]) { e2[1] = a1; i2[1] = c1; }
-                        } else {
-                            e2[1] = fmin(e2[1], fmin(a0, a1));
+#pragma unroll
+                    for (int cls = 0; cls < 2; ++cls) {
+                        const double *cent = cls ? p.cent_neg : p.cent_pos;
+                        const int64_t n_c = cls ? p.n_cent_neg : p.n_cent_pos;
+                        for (int64_t c = 0; c < n_c; c += 2) {
+                            const int64_t c1 = c + 1 < n_c ? c + 1 : c;
+                            const double a0 = warp_d2(x, cent + c * KDIM, lane), a1 = warp_d2(x, cent + c1 * KDIM, lane);
+                            if (NEIGHBORS) {
+                                if (a0 < e2[cls]) { e2[cls] = a0; i2[cls] = c; }
+                                if (a1 < e2[cls]) { e2[cls] = a1; i2[cls] = c1; }
+                            } else {
+                                e2[cls] = fmin(e2[cls], fmin(a0, a1));
+                            }
                         }
                     }
                 }
@@ -1080,17 +1073,10 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                     const int sp = rest_p ? __ffs(rest_p) - 1 : 0, sn = rest_n ? __ffs(rest_n) - 1 : 0;
                     const uint32_t ip = first_round ? cp0 : ent[CAP_R + sp].y, in_ = first_round ? cn0 : ent[CAP_R + CAP_C + sn].y;
                     first_round = false;
-                    const double *bp = p.cent_pos + (int64_t)(rest_p ? ip : 0u) * KDIM;
-                    const double *bn = p.cent_neg + (int64_t)(rest_n ? in_ : 0u) * KDIM;
-                    double ap = 0.0, an = 0.0;
-#pragma unroll
-                    for (int i = 0; i < KDIM / 32; ++i) {
-                        const double tp = x[i] - bp[lane + 32 * i], tn = x[i] - bn[lane + 32 * i];
-                        ap = fma(tp, tp, ap);
-                        an = fma(tn, tn, an);
-                    }
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1) { ap += __shfl_xor_sync(FULL, ap, o); an += __shfl_xor_sync(FULL, an, o); }
+                    const double *const b[2] = {p.cent_pos + (int64_t)(rest_p ? ip : 0u) * KDIM, p.cent_neg + (int64_t)(rest_n ? in_ : 0u) * KDIM};
+                    double a[2];
+                    warp_d2<2>(x, b, lane, a);
+                    const double ap = a[0], an = a[1];
                     if (NEIGHBORS) {
                         // kept slots are not in index order: the tie rule compares indices
                         if (rest_p && (ap < e2[0] || (ap == e2[0] && (int64_t)ip < i2[0]))) { e2[0] = ap; i2[0] = ip; }
@@ -1110,10 +1096,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
         // ---------------- C: lane = row ----------------
         if (my_row < p.n_points) {
             double km = NAN;
-            if (my_live && has_cent) {
-                const double e_pos = sqrt(my_e0), e_neg = sqrt(my_e1);
-                km = tanh((e_neg - e_pos) / (e_pos + e_neg));              // scripts/phamer.py:206-209
-            }
+            if (my_live && has_cent) km = kmeans_score(sqrt(my_e0), sqrt(my_e1));
             if (my_live && state == ROW_FALLBACK) {
                 bool listed = false;
                 if (p.list_rows) {
@@ -1128,24 +1111,15 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                     p.fallback_rows[slot_out] = my_row;
                 }
             } else {
-                if (p.knn) p.knn[my_row] = my_knn;
-                if (p.kmeans) p.kmeans[my_row] = km;
-                if (p.combo) p.combo[my_row] = my_knn + km;                 // scripts/phamer.py:313
+                put_scores(p.out, my_row, my_knn, km);
             }
             if (NEIGHBORS) {
-                // the centroid term of every live row is settled here, whichever road its references take; a NaN row reports
-                // nothing anywhere
-                const bool cen = my_live && has_cent;
-                if (p.nb.cent_index) { p.nb.cent_index[2 * my_row] = cen ? my_c0 : -1; p.nb.cent_index[2 * my_row + 1] = cen ? my_c1 : -1; }
-                if (p.nb.cent_distance) {
-                    p.nb.cent_distance[2 * my_row] = cen ? sqrt(my_e0) : NAN;
-                    p.nb.cent_distance[2 * my_row + 1] = cen ? sqrt(my_e1) : NAN;
-                }
+                // the centroid term of every live row is settled here, whichever road its references take
                 if (!my_live) {
-                    for (int t = 0; t < kn; ++t) {
-                        if (p.nb.ref_index) p.nb.ref_index[my_row * kn + t] = -1;
-                        if (p.nb.ref_distance) p.nb.ref_distance[my_row * kn + t] = NAN;
-                    }
+                    put_nan_row(p.out, my_row);
+                } else {
+                    put_neighbor(p.out.nb.cent_index, p.out.nb.cent_distance, 2 * my_row, has_cent ? my_c0 : -1, has_cent ? sqrt(my_e0) : NAN);
+                    put_neighbor(p.out.nb.cent_index, p.out.nb.cent_distance, 2 * my_row + 1, has_cent ? my_c1 : -1, has_cent ? sqrt(my_e1) : NAN);
                 }
             }
         }
@@ -1242,25 +1216,57 @@ struct ListDecideParams {
     int64_t perm_a, perm_c;
     const int64_t *list_rows; const unsigned long long *list_count; int list_max_rows;
     const uint32_t *list_n; const uint32_t *list_off; const uint32_t *list_cols; const double *list_km;
-    int k_neighbors;
-    double *knn, *kmeans, *combo;
+    ScoreOut out;                          // the reference report only (the centroids were reported by score_decide_kernel)
     int64_t *fallback_rows; unsigned long long *fallback_count;
     unsigned long long *rows_listed;       // statistics: rows settled here
-    NeighborOut nb;                        // neighbour report: the k nearest references (the centroids were reported by score_decide_kernel)
 };
 
-constexpr int LD_K = 5;                    // k_neighbors <= 5 on the tensor-core path
+constexpr int TC_KMAX = 5;                 // k_neighbors <= 5 on the tensor-core path
 constexpr int LD_U = 4;                    // listed references in flight per warp
 
-// One warp per listed row: float64 direct-difference distance (the arithmetic of every other exact path) to each listed
-// reference, k smallest by (distance, reference index), vote.  The centroid part of the score was settled by score_decide_kernel.
+// The K nearest (distance, index) pairs seen so far, ascending by nearer(); empty entries are (INFINITY, -1).  A branch-free
+// insertion network, so the list stays in registers.
+template <int K>
+struct TopK {
+    double d[K];
+    int i[K];
+    __device__ __forceinline__ void clear() {
+#pragma unroll
+        for (int s = 0; s < K; ++s) { d[s] = INFINITY; i[s] = -1; }
+    }
+    __device__ __forceinline__ void insert(double v, int id) {
+#pragma unroll
+        for (int s = K - 1; s > 0; --s) {
+            const bool shift = nearer(v, id, d[s - 1], i[s - 1]), here = nearer(v, id, d[s], i[s]);
+            i[s] = shift ? i[s - 1] : (here ? id : i[s]);
+            d[s] = shift ? d[s - 1] : (here ? v : d[s]);
+        }
+        if (nearer(v, id, d[0], i[0])) { d[0] = v; i[0] = id; }
+    }
+};
+
+// A row finished from its k nearest references (squared distances d2, ascending by nearer()) and its kmeans score: vote, scores
+// and the reference report.
+__device__ __forceinline__ void finish_row(const ScoreOut &o, int64_t row, const double *d2, const int *idx, int64_t n_positive, double km) {
+    int pos = 0;
+#pragma unroll
+    for (int t = 0; t < TC_KMAX; ++t) {
+        if (t >= o.k) break;
+        pos += idx[t] >= 0 && idx[t] < n_positive;
+        put_neighbor(o.nb.ref_index, o.nb.ref_distance, row * o.k + t, idx[t], sqrt(d2[t]));
+    }
+    put_scores(o, row, knn_vote(pos, o.k), km);
+}
+
+// One warp per listed row: float64 direct-difference distance (warp_d2) to each listed reference, k smallest by (distance,
+// reference index), vote.  The centroid part of the score was settled by score_decide_kernel.
 __global__ void __launch_bounds__(256) score_list_decide_kernel(ListDecideParams p) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     unsigned long long cnt = *p.list_count;
     if (cnt > (unsigned long long)p.list_max_rows) cnt = (unsigned long long)p.list_max_rows;
-    const int kn = p.k_neighbors;
+    const int kn = p.out.k;
     for (int64_t slot = warp; slot < (int64_t)cnt; slot += n_warps) {
         const int64_t row = p.list_rows[slot];
         const uint32_t n = p.list_n[slot], off = p.list_off[slot];
@@ -1270,61 +1276,28 @@ __global__ void __launch_bounds__(256) score_list_decide_kernel(ListDecideParams
         }
         double x[KDIM / 32];
         load_query_row(p.points, p.point_counts, row, lane, x);
-        double bd[LD_K];
-        int bi[LD_K];
-#pragma unroll
-        for (int i = 0; i < LD_K; ++i) { bd[i] = INFINITY; bi[i] = 0x7FFFFFFF; }
+        TopK<TC_KMAX> top;
+        top.clear();
         const uint32_t *cols = p.list_cols + off;
         for (uint32_t c0 = 0; c0 < n; c0 += LD_U) {
-            double acc[LD_U];
+            const double *b[LD_U];
             int idx[LD_U];
 #pragma unroll
             for (int t = 0; t < LD_U; ++t) {
                 const uint32_t c = c0 + t < n ? c0 + t : n - 1;
                 idx[t] = (int)((p.perm_a * (int64_t)cols[c] + p.perm_c) % p.n_refs);
-                const double *b = p.refs + (int64_t)idx[t] * KDIM;
-                double a = 0.0;
-#pragma unroll
-                for (int i = 0; i < KDIM / 32; ++i) {
-                    const double d = x[i] - b[lane + 32 * i];
-                    a = fma(d, d, a);
-                }
-                acc[t] = a;
+                b[t] = p.refs + (int64_t)idx[t] * KDIM;
             }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1)
-#pragma unroll
-                for (int t = 0; t < LD_U; ++t) acc[t] += __shfl_xor_sync(FULL, acc[t], o);
+            double acc[LD_U];
+            warp_d2<LD_U>(x, b, lane, acc);
 #pragma unroll
             for (int t = 0; t < LD_U; ++t) {
                 if (c0 + t >= n) break;
-                const double d = acc[t];
-                const int id = idx[t];
-#pragma unroll
-                for (int i = LD_K - 1; i > 0; --i) {
-                    const bool shift = d < bd[i - 1] || (d == bd[i - 1] && id < bi[i - 1]);
-                    const bool here = d < bd[i] || (d == bd[i] && id < bi[i]);
-                    bi[i] = shift ? bi[i - 1] : (here ? id : bi[i]);
-                    bd[i] = shift ? bd[i - 1] : (here ? d : bd[i]);
-                }
-                if (d < bd[0] || (d == bd[0] && id < bi[0])) { bd[0] = d; bi[0] = id; }
+                top.insert(acc[t], idx[t]);
             }
         }
         if (lane == 0) {
-            int pos = 0;
-#pragma unroll
-            for (int t = 0; t < LD_K; ++t) pos += (t < kn && (int64_t)bi[t] < p.n_positive);
-            const double knn = (2 * pos > kn) ? 1.0 : -1.0;               // scripts/learning.py:128
-            const double km = p.list_km[slot];
-            if (p.knn) p.knn[row] = knn;
-            if (p.kmeans) p.kmeans[row] = km;
-            if (p.combo) p.combo[row] = knn + km;                       // scripts/phamer.py:313
-#pragma unroll
-            for (int t = 0; t < LD_K; ++t) {
-                if (t >= kn) break;
-                if (p.nb.ref_index) p.nb.ref_index[row * kn + t] = bi[t];
-                if (p.nb.ref_distance) p.nb.ref_distance[row * kn + t] = sqrt(bd[t]);
-            }
+            finish_row(p.out, row, top.d, top.i, p.n_positive, p.list_km[slot]);
             atomicAdd(p.rows_listed, 1ull);
         }
     }
@@ -1336,12 +1309,11 @@ __global__ void __launch_bounds__(256) score_list_decide_kernel(ListDecideParams
 // inside a dense cloud of near-identical references), so the grid is small and persistent and reads the row count on the
 // device.  When there are fewer rows than CTAs each row is cut into up to FB_SLICES column slices handled by different CTAs;
 // the last CTA to finish a row (ticket counter) merges the slices.
-constexpr int FB_K = 5;
 constexpr int FB_U = 8;                    // reference rows in flight per warp
 constexpr int FB_SLICES = 16;
 constexpr int FB_GRID = 148 * 4;
 constexpr int FB_BLOCKED_MIN = FB_GRID;    // more fallback rows than this: blocked kernel (references streamed once per 32 rows)
-struct FallbackPart { double d[FB_K]; int i[FB_K]; int pad; double cp, cn; };
+struct FallbackPart { TopK<TC_KMAX> top; double cp, cn; };
 struct FallbackParams {
     const double *points; const uint32_t *point_counts;
     const double *refs; int64_t n_refs; int64_t n_positive;
@@ -1350,45 +1322,44 @@ struct FallbackParams {
     const int64_t *rows; const unsigned long long *count;
     FallbackPart *parts;                   // [FB_GRID][FB_SLICES], used only while rows < CTAs
     unsigned int *tickets;                 // [FB_GRID], zero on entry, left zero on exit
-    int k_neighbors;
-    double *knn, *kmeans, *combo;
-    NeighborOut nb;                        // neighbour report: the k nearest references (the centroids were reported by score_decide_kernel)
+    ScoreOut out;                          // the reference report only (the centroids were reported by score_decide_kernel)
 };
 
-// merge `n_lists` lists sorted by (distance, index) into the vote / score of one row (one thread)
-__device__ __forceinline__ void fallback_finish(const FallbackParams &f, int64_t row, const FallbackPart *lists, int n_lists) {
-    const int kn = f.k_neighbors;
-    int pos = 0, head[FB_SLICES];
+// kmeans score from the squared distances to the nearest centroid of each class (NaN without both classes)
+__device__ __forceinline__ double fallback_km(const FallbackParams &f, double cp, double cn) {
+    return (f.n_cent_pos > 0 && f.n_cent_neg > 0) ? kmeans_score(sqrt(cp), sqrt(cn)) : NAN;
+}
+
+// k-way merge of `n_lists` (<= FB_SLICES) lists sorted by nearer() -- a list ends at its first empty entry -- into one, with the
+// smallest centroid distances of all
+__device__ __forceinline__ FallbackPart merge_parts(const FallbackPart *lists, int n_lists) {
+    FallbackPart m;
+    int head[FB_SLICES];
     for (int w = 0; w < n_lists; ++w) head[w] = 0;
-    for (int t = 0; t < kn; ++t) {
+    for (int t = 0; t < TC_KMAX; ++t) {
         int best = -1;
         for (int w = 0; w < n_lists; ++w) {
-            if (head[w] >= FB_K || lists[w].i[head[w]] < 0) continue;
-            if (best < 0 || lists[w].d[head[w]] < lists[best].d[head[best]] ||
-                (lists[w].d[head[w]] == lists[best].d[head[best]] && lists[w].i[head[w]] < lists[best].i[head[best]])) best = w;
+            if (head[w] >= TC_KMAX || lists[w].top.i[head[w]] < 0) continue;
+            if (best < 0 || nearer(lists[w].top.d[head[w]], lists[w].top.i[head[w]], lists[best].top.d[head[best]], lists[best].top.i[head[best]]))
+                best = w;
         }
-        if (best < 0) break;
-        pos += lists[best].i[head[best]] < f.n_positive;
-        if (f.nb.ref_index) f.nb.ref_index[row * kn + t] = lists[best].i[head[best]];
-        if (f.nb.ref_distance) f.nb.ref_distance[row * kn + t] = sqrt(lists[best].d[head[best]]);
-        ++head[best];
+        m.top.d[t] = best < 0 ? INFINITY : lists[best].top.d[head[best]];
+        m.top.i[t] = best < 0 ? -1 : lists[best].top.i[head[best]];
+        if (best >= 0) ++head[best];
     }
-    const double knn = (2 * pos > kn) ? 1.0 : -1.0;             // scripts/learning.py:128
-    double km = NAN;
-    if (f.n_cent_pos > 0 && f.n_cent_neg > 0) {
-        double e_pos = INFINITY, e_neg = INFINITY;
-        for (int w = 0; w < n_lists; ++w) { e_pos = fmin(e_pos, lists[w].cp); e_neg = fmin(e_neg, lists[w].cn); }
-        e_pos = sqrt(e_pos); e_neg = sqrt(e_neg);
-        km = tanh((e_neg - e_pos) / (e_pos + e_neg));          // scripts/phamer.py:206-209
-    }
-    if (f.knn) f.knn[row] = knn;
-    if (f.kmeans) f.kmeans[row] = km;
-    if (f.combo) f.combo[row] = knn + km;
+    m.cp = INFINITY; m.cn = INFINITY;
+    for (int w = 0; w < n_lists; ++w) { m.cp = fmin(m.cp, lists[w].cp); m.cn = fmin(m.cn, lists[w].cn); }
+    return m;
+}
+
+// the vote / score of one row from `n_lists` partial lists (one thread)
+__device__ __forceinline__ void fallback_finish(const FallbackParams &f, int64_t row, const FallbackPart *lists, int n_lists) {
+    const FallbackPart m = merge_parts(lists, n_lists);
+    finish_row(f.out, row, m.top.d, m.top.i, f.n_positive, fallback_km(f, m.cp, m.cn));
 }
 
 __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
     __shared__ FallbackPart s_part[8];
-    __shared__ FallbackPart s_merged;
     __shared__ FallbackPart s_all[FB_SLICES];
     __shared__ unsigned int s_ticket;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1404,74 +1375,38 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
         const int64_t c_lo = f.n_refs * slice / slices, c_hi = f.n_refs * (slice + 1) / slices;
         double x[KDIM / 32];
         load_query_row(f.points, f.point_counts, row, lane, x);
-        double bd[FB_K];
-        int bi[FB_K];
+        TopK<TC_KMAX> top;
+        top.clear();
+        for (int64_t c0 = c_lo + warp; c0 < c_hi; c0 += 8 * FB_U) {   // ascending index per warp (see nearer)
+            const double *b[FB_U];
 #pragma unroll
-        for (int i = 0; i < FB_K; ++i) { bd[i] = INFINITY; bi[i] = -1; }
-        for (int64_t c0 = c_lo + warp; c0 < c_hi; c0 += 8 * FB_U) {   // ascending index per warp: strict '<' keeps the earlier of a tie
-            double acc[FB_U];
-#pragma unroll
-            for (int t = 0; t < FB_U; ++t) {                     // FB_U independent rows in flight: this loop is latency-bound
+            for (int t = 0; t < FB_U; ++t) {
                 const int64_t c = c0 + 8 * t;
-                const double *b = f.refs + (c < c_hi ? c : c0) * KDIM;
-                double a = 0.0;
-#pragma unroll
-                for (int i = 0; i < KDIM / 32; ++i) {
-                    const double d = x[i] - b[lane + 32 * i];
-                    a = fma(d, d, a);
-                }
-                acc[t] = a;
+                b[t] = f.refs + (c < c_hi ? c : c0) * KDIM;
             }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1)
-#pragma unroll
-                for (int t = 0; t < FB_U; ++t) acc[t] += __shfl_xor_sync(FULL, acc[t], o);
+            double acc[FB_U];
+            warp_d2<FB_U>(x, b, lane, acc);                     // FB_U independent rows in flight: this loop is latency-bound
 #pragma unroll
             for (int t = 0; t < FB_U; ++t) {
                 const int64_t c = c0 + 8 * t;
                 if (c >= c_hi) break;
-                const double d = acc[t];
-#pragma unroll
-                for (int i = FB_K - 1; i > 0; --i) {
-                    const bool shift = d < bd[i - 1], here = d < bd[i];
-                    bi[i] = shift ? bi[i - 1] : (here ? (int)c : bi[i]);
-                    bd[i] = shift ? bd[i - 1] : (here ? d : bd[i]);
-                }
-                if (d < bd[0]) { bd[0] = d; bi[0] = (int)c; }
+                top.insert(acc[t], (int)c);
             }
         }
         double cp = INFINITY, cn = INFINITY;
         if (slice == 0) {
-            for (int64_t c = warp; c < f.n_cent_pos; c += 8) cp = fmin(cp, warp_exact_d2(x, f.cent_pos + c * KDIM, lane));
-            for (int64_t c = warp; c < f.n_cent_neg; c += 8) cn = fmin(cn, warp_exact_d2(x, f.cent_neg + c * KDIM, lane));
+            for (int64_t c = warp; c < f.n_cent_pos; c += 8) cp = fmin(cp, warp_d2(x, f.cent_pos + c * KDIM, lane));
+            for (int64_t c = warp; c < f.n_cent_neg; c += 8) cn = fmin(cn, warp_d2(x, f.cent_neg + c * KDIM, lane));
         }
         __syncthreads();                                        // previous item's merge has finished reading shared memory
-        if (lane == 0) {
-#pragma unroll
-            for (int i = 0; i < FB_K; ++i) { s_part[warp].d[i] = bd[i]; s_part[warp].i[i] = bi[i]; }
-            s_part[warp].cp = cp; s_part[warp].cn = cn;
-        }
+        if (lane == 0) { s_part[warp].top = top; s_part[warp].cp = cp; s_part[warp].cn = cn; }
         __syncthreads();
         if (threadIdx.x == 0) {
             if (slices == 1) {
                 fallback_finish(f, row, s_part, 8);
             } else {
                 // this CTA's slice as one sorted list, published for whichever CTA finishes the row last
-                int head[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-                for (int t = 0; t < FB_K; ++t) {
-                    int best = -1;
-                    for (int w = 0; w < 8; ++w) {
-                        if (head[w] >= FB_K || s_part[w].i[head[w]] < 0) continue;
-                        if (best < 0 || s_part[w].d[head[w]] < s_part[best].d[head[best]] ||
-                            (s_part[w].d[head[w]] == s_part[best].d[head[best]] && s_part[w].i[head[w]] < s_part[best].i[head[best]])) best = w;
-                    }
-                    s_merged.d[t] = best < 0 ? INFINITY : s_part[best].d[head[best]];
-                    s_merged.i[t] = best < 0 ? -1 : s_part[best].i[head[best]];
-                    if (best >= 0) ++head[best];
-                }
-                s_merged.cp = INFINITY; s_merged.cn = INFINITY;
-                for (int w = 0; w < 8; ++w) { s_merged.cp = fmin(s_merged.cp, s_part[w].cp); s_merged.cn = fmin(s_merged.cn, s_part[w].cn); }
-                f.parts[ridx * FB_SLICES + slice] = s_merged;
+                f.parts[ridx * FB_SLICES + slice] = merge_parts(s_part, 8);
                 __threadfence();
                 s_ticket = atomicAdd(&f.tickets[ridx], 1u);
                 if (s_ticket == (unsigned)slices - 1) {
@@ -1479,7 +1414,7 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
                     // the other CTAs' slices, read past L1 (they were written by other SMs)
                     for (int w = 0; w < slices; ++w) {
                         const FallbackPart *src = f.parts + ridx * FB_SLICES + w;
-                        for (int i = 0; i < FB_K; ++i) { s_all[w].d[i] = __ldcg(&src->d[i]); s_all[w].i[i] = __ldcg(&src->i[i]); }
+                        for (int i = 0; i < TC_KMAX; ++i) { s_all[w].top.d[i] = __ldcg(&src->top.d[i]); s_all[w].top.i[i] = __ldcg(&src->top.i[i]); }
                         s_all[w].cp = __ldcg(&src->cp); s_all[w].cn = __ldcg(&src->cn);
                     }
                     fallback_finish(f, row, s_all, slices);
@@ -1493,15 +1428,15 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
 // Many fallback rows (an enlarged reference set that is a cloud of near-duplicates): 32 rows per CTA share every reference tile,
 // which is staged once in shared memory (transposed, padded: conflict-free for lane = reference), so the references are streamed
 // from HBM once per 32 rows instead of once per row.  Reference distances only ORDER the neighbours here; the centroid distances,
-// whose values reach the score, use the same warp_exact_d2 as every other path.
+// whose values reach the score, use the same warp_d2 as every other path.
 constexpr int FBB_ROWS = 32, FBB_TR = 32, FBB_PITCH = FBB_TR + 1;
-constexpr int FBB_SMEM = (FBB_ROWS * KDIM + KDIM * FBB_PITCH) * 8 + FBB_ROWS * FB_K * 12 + 64;
+constexpr int FBB_SMEM = (FBB_ROWS * KDIM + KDIM * FBB_PITCH) * 8 + FBB_ROWS * TC_KMAX * 12 + 64;
 
 template <int QW>                                                          // rows per warp
 __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned long long blk, unsigned long long count,
                                                double *s_rows, double *s_tile, double *s_d, int *s_i) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int kn = f.k_neighbors;
+    const int kn = f.out.k;
     __syncthreads();
     // this warp's rows into shared memory; their lists start empty
     int64_t my_row[QW];
@@ -1513,7 +1448,7 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
         if (my_row[q] >= 0) load_query_row(f.points, f.point_counts, my_row[q], lane, x[q]);
 #pragma unroll
         for (int i = 0; i < KDIM / 32; ++i) s_rows[(warp * QW + q) * KDIM + lane + 32 * i] = my_row[q] >= 0 ? x[q][i] : 0.0;
-        if (lane < FB_K) { s_d[(warp * QW + q) * FB_K + lane] = INFINITY; s_i[(warp * QW + q) * FB_K + lane] = -1; }
+        if (lane < TC_KMAX) { s_d[(warp * QW + q) * TC_KMAX + lane] = INFINITY; s_i[(warp * QW + q) * TC_KMAX + lane] = -1; }
     }
     double thr[QW];
 #pragma unroll
@@ -1548,14 +1483,9 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
                 const int src = __ffs(hit) - 1;
                 hit &= hit - 1;
                 const double d = __shfl_sync(FULL, acc[q], src);
-                double *ld = s_d + (warp * QW + q) * FB_K;
-                int *li = s_i + (warp * QW + q) * FB_K;
-                if (lane == 0 && d < ld[kn - 1]) {
-                    int p = kn - 1;
-                    while (p > 0 && ld[p - 1] > d) { ld[p] = ld[p - 1]; li[p] = li[p - 1]; --p; }   // strict: earlier index wins ties
-                    ld[p] = d;
-                    li[p] = (int)(c0 + src);
-                }
+                double *ld = s_d + (warp * QW + q) * TC_KMAX;
+                int *li = s_i + (warp * QW + q) * TC_KMAX;
+                if (lane == 0) list_insert(ld, li, kn, d, (int)(c0 + src));
                 __syncwarp();
                 thr[q] = ld[kn - 1];
             }
@@ -1566,26 +1496,11 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
     for (int q = 0; q < QW; ++q) {
         if (my_row[q] < 0) continue;
         double cp = INFINITY, cn = INFINITY;
-        for (int64_t c = 0; c < f.n_cent_pos; ++c) cp = fmin(cp, warp_exact_d2(x[q], f.cent_pos + c * KDIM, lane));
-        for (int64_t c = 0; c < f.n_cent_neg; ++c) cn = fmin(cn, warp_exact_d2(x[q], f.cent_neg + c * KDIM, lane));
+        for (int64_t c = 0; c < f.n_cent_pos; ++c) cp = fmin(cp, warp_d2(x[q], f.cent_pos + c * KDIM, lane));
+        for (int64_t c = 0; c < f.n_cent_neg; ++c) cn = fmin(cn, warp_d2(x[q], f.cent_neg + c * KDIM, lane));
         if (lane == 0) {
-            const int *li = s_i + (warp * QW + q) * FB_K;
-            const double *ld = s_d + (warp * QW + q) * FB_K;
-            int pos = 0;
-            for (int t = 0; t < kn; ++t) {
-                pos += (li[t] >= 0 && li[t] < f.n_positive);
-                if (f.nb.ref_index) f.nb.ref_index[my_row[q] * kn + t] = li[t];
-                if (f.nb.ref_distance) f.nb.ref_distance[my_row[q] * kn + t] = sqrt(ld[t]);
-            }
-            const double knn = (2 * pos > kn) ? 1.0 : -1.0;               // scripts/learning.py:128
-            double km = NAN;
-            if (f.n_cent_pos > 0 && f.n_cent_neg > 0) {
-                const double e_pos = sqrt(cp), e_neg = sqrt(cn);
-                km = tanh((e_neg - e_pos) / (e_pos + e_neg));              // scripts/phamer.py:206-209
-            }
-            if (f.knn) f.knn[my_row[q]] = knn;
-            if (f.kmeans) f.kmeans[my_row[q]] = km;
-            if (f.combo) f.combo[my_row[q]] = knn + km;
+            const int at = (warp * QW + q) * TC_KMAX;
+            finish_row(f.out, my_row[q], s_d + at, s_i + at, f.n_positive, fallback_km(f, cp, cn));
         }
     }
 }
@@ -1594,8 +1509,8 @@ __global__ void __launch_bounds__(256) score_fallback_blocked_kernel(FallbackPar
     extern __shared__ __align__(16) unsigned char fbb_raw[];
     double *s_rows = reinterpret_cast<double *>(fbb_raw);                     // [32][256]
     double *s_tile = s_rows + FBB_ROWS * KDIM;                                // [256][33]
-    double *s_d = s_tile + KDIM * FBB_PITCH;                                  // [32][FB_K]
-    int *s_i = reinterpret_cast<int *>(s_d + FBB_ROWS * FB_K);                // [32][FB_K]
+    double *s_d = s_tile + KDIM * FBB_PITCH;                                  // [32][TC_KMAX]
+    int *s_i = reinterpret_cast<int *>(s_d + FBB_ROWS * TC_KMAX);             // [32][TC_KMAX]
     const unsigned long long count = *f.count;
     if (count <= FB_BLOCKED_MIN) return;
     // rows per warp chosen so that one wave of CTAs covers all rows when it can (the work per CTA is proportional to its rows)
@@ -1738,23 +1653,21 @@ static int launch_prep(const double *src, const uint32_t *src_counts, int64_t n_
 static EventRing g_tc_ring;      // brackets of the score_tc_kernel launches (option "time_kernels")
 static EventRing g_decide_ring;  // ... and of the score_decide_kernel launches
 
-template <int KN>
-static int launch_tc_list(const CUtensorMap &map_list, const TcParams &p, cudaStream_t st) {
-    auto kern = score_tc_kernel<KN, true>;
-    PHM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    kern<<<sm_count(), NTHREADS, SMEM_BYTES, st>>>(map_list, p);       // persistent; the number of rows is read on the device
-    PHM_LAUNCH_CHECK();
-    return PHM_OK;
-}
-
-template <int KN>
-static int launch_tc(const CUtensorMap &map_a, const TcParams &p, cudaStream_t st) {
-    auto kern = score_tc_kernel<KN, false>;
+// score_tc_kernel for k_neighbors k: the first pass (one CTA per contig tile at most; timed for "time_kernels"), or the list pass
+// (persistent; the number of rows is read on the device)
+static int launch_tc(bool list, int k, const CUtensorMap &map, const TcParams &p, cudaStream_t st) {
+    void (*kern)(CUtensorMap, TcParams);
+    switch (k) {
+        case 1: kern = list ? score_tc_kernel<1, true> : score_tc_kernel<1, false>; break;
+        case 3: kern = list ? score_tc_kernel<3, true> : score_tc_kernel<3, false>; break;
+        case 5: kern = list ? score_tc_kernel<5, true> : score_tc_kernel<5, false>; break;
+        default: set_error("tensor-core scoring supports k_neighbors 1, 3, 5"); return PHM_E_UNSUPPORTED;
+    }
     PHM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     int grid = sm_count();
-    if (grid > p.n_mtiles) grid = p.n_mtiles;
-    const bool timed = g_tc_ring.begin(st);
-    kern<<<grid, NTHREADS, SMEM_BYTES, st>>>(map_a, p);
+    if (!list && grid > p.n_mtiles) grid = p.n_mtiles;
+    const bool timed = !list && g_tc_ring.begin(st);
+    kern<<<grid, NTHREADS, SMEM_BYTES, st>>>(map, p);
     PHM_LAUNCH_CHECK();
     if (timed) g_tc_ring.end(st);
     return PHM_OK;
@@ -1798,10 +1711,9 @@ int score_tc_begin(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t s
     return PHM_OK;
 }
 
-int score_tc(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, int *kernels_launched) {
+int score_tc(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st) {
     int rc = score_tc_begin(a, ws, ws_bytes, st, nullptr);
     if (rc != PHM_OK) return rc;
-    if (kernels_launched) *kernels_launched = 12;
     return score_tc_finish(a, ws, ws_bytes, st, false);
 }
 
@@ -1840,13 +1752,7 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     p.skip_scan = score_force_fallback;
     p.list_count = w.list_count; p.list_max_rows = w.list_max_rows; p.list_thr = w.list_thr; p.list_cnt = w.list_cnt;
     p.list_off = w.list_off; p.list_cols = nullptr;
-    switch (a.k_neighbors) {
-        case 1: rc = launch_tc<1>(map_a, p, st); break;
-        case 3: rc = launch_tc<3>(map_a, p, st); break;
-        case 5: rc = launch_tc<5>(map_a, p, st); break;
-        default: set_error("tensor-core scoring supports k_neighbors 1, 3, 5"); return PHM_E_UNSUPPORTED;
-    }
-    if (rc != PHM_OK) return rc;
+    if ((rc = launch_tc(false, a.out.k, map_a, p, st)) != PHM_OK) return rc;
 
     DecideParams r;
     r.points = a.points; r.point_counts = a.point_counts; r.n_points = n;
@@ -1854,19 +1760,17 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     r.perm_a = perm_a; r.perm_c = perm_c;
     r.cent_pos = a.cent_pos; r.n_cent_pos = a.n_cent_pos; r.cent_neg = a.cent_neg; r.n_cent_neg = a.n_cent_neg;
     r.cnorm_points = w.cnorm_points; r.row_total = w.row_total; r.cand = w.cand; r.cand_up = w.cand_up; r.meta = w.meta; r.drop_lo = w.drop_lo; r.thr = w.thr_out;
-    r.k_neighbors = a.k_neighbors;
-    r.knn = a.knn; r.kmeans = a.kmeans; r.combo = a.combo;
+    r.out = a.out;
     r.fallback_rows = w.fallback_rows; r.fallback_count = w.fallback_count;
     r.stats = score_collect_stats ? w.stats : nullptr;
     r.rows_remeasured = w.rows_remeasured;
     const bool use_list = score_list_pass != 0;
     r.list_rows = use_list ? w.list_rows : nullptr; r.list_count = w.list_count; r.list_max_rows = w.list_max_rows;
     r.list_thr = w.list_thr; r.list_km = w.list_km;
-    r.nb = a.nb;
     int64_t blocks = (n + 255) / 256;                                  // a warp takes 32 consecutive rows at a time
     if (blocks > 148 * 16) blocks = 148 * 16;
     const bool timed = g_decide_ring.begin(st);
-    const bool nb = a.nb.any();
+    const bool nb = a.out.nb.any();
     if (a.point_counts) {
         if (nb) score_decide_kernel<true, true><<<(unsigned)blocks, 256, 0, st>>>(r);
         else score_decide_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(r);
@@ -1890,12 +1794,7 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
         pl.ax_img = w.ax_list;
         for (int pass = 0; pass < 2; ++pass) {                           // count, prefix sum, fill
             pl.list_cols = pass ? w.list_cols : nullptr;
-            switch (a.k_neighbors) {
-                case 1: rc = launch_tc_list<1>(map_list, pl, st); break;
-                case 3: rc = launch_tc_list<3>(map_list, pl, st); break;
-                default: rc = launch_tc_list<5>(map_list, pl, st); break;
-            }
-            if (rc != PHM_OK) return rc;
+            if ((rc = launch_tc(true, a.out.k, map_list, pl, st)) != PHM_OK) return rc;
             if (pass == 0) {
                 tc_list_scan_kernel<<<1, 1024, 0, st>>>(w.list_count, w.list_max_rows, (unsigned long long)w.list_pool_entries, w.list_cnt,
                                                         w.list_n, w.list_off);
@@ -1908,11 +1807,9 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
         ld.perm_a = perm_a; ld.perm_c = perm_c;
         ld.list_rows = w.list_rows; ld.list_count = w.list_count; ld.list_max_rows = w.list_max_rows;
         ld.list_n = w.list_n; ld.list_off = w.list_off; ld.list_cols = w.list_cols; ld.list_km = w.list_km;
-        ld.k_neighbors = a.k_neighbors;
-        ld.knn = a.knn; ld.kmeans = a.kmeans; ld.combo = a.combo;
+        ld.out = a.out;
         ld.fallback_rows = w.fallback_rows; ld.fallback_count = w.fallback_count;
         ld.rows_listed = w.rows_listed;
-        ld.nb = a.nb;
         score_list_decide_kernel<<<sm_count() * 2, 256, 0, st>>>(ld);
         PHM_LAUNCH_CHECK();
     }
@@ -1923,10 +1820,8 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     f.refs = a.refs; f.n_refs = a.n_refs; f.n_positive = a.n_positive;
     f.cent_pos = a.cent_pos; f.n_cent_pos = a.n_cent_pos; f.cent_neg = a.cent_neg; f.n_cent_neg = a.n_cent_neg;
     f.rows = w.fallback_rows; f.count = w.fallback_count;
-    f.k_neighbors = a.k_neighbors;
-    f.knn = a.knn; f.kmeans = a.kmeans; f.combo = a.combo;
+    f.out = a.out;
     f.parts = w.fb_parts; f.tickets = w.fb_tickets;
-    f.nb = a.nb;
     PHM_CUDA_CHECK(cudaMemsetAsync(w.fb_tickets, 0, sizeof(unsigned int) * FB_GRID, st));
     score_fallback_kernel<<<FB_GRID, 256, 0, st>>>(f);                 // few rows: column slices across CTAs
     PHM_LAUNCH_CHECK();

@@ -213,8 +213,14 @@ def test_overflow_roads(golden, n_rows):
             for a, b in zip(base[:3], road[:3]):
                 assert np.array_equal(a, b, equal_nan=True), list_pass
             live = ~np.isnan(X).any(axis=1)
-            assert np.all(np.abs(road[4][live] - base[4][live]) <= 1e-13 * base[4][live]), list_pass
-            assert np.array_equal(road[3][live][clear], base[3][live][clear]), list_pass
+            if list_pass or n_rows <= 592:
+                # list pass and sliced exhaustive kernel: the default road's arithmetic and order, bit for bit
+                assert np.array_equal(road[3][live], base[3][live]), list_pass
+                assert np.array_equal(road[4][live], base[4][live]), list_pass
+            else:
+                # blocked exhaustive kernel: its own summation order (last bits of the distances)
+                assert np.all(np.abs(road[4][live] - base[4][live]) <= 1e-13 * base[4][live]), list_pass
+                assert np.array_equal(road[3][live][clear], base[3][live][clear]), list_pass
             assert np.array_equal(road[5], base[5]) and np.array_equal(road[6], base[6], equal_nan=True), list_pass
             check_refs(X, R, road[3], road[4], 3, tag=list_pass)
     finally:
