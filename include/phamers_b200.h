@@ -100,6 +100,13 @@ int phm_kmer_count_packed(const uint32_t *d_codes, const uint32_t *d_valid, cons
                           int64_t n_contigs, int k, uint32_t flags, uint32_t *d_counts, double *d_freq,
                           void *d_workspace, size_t workspace_bytes, void *stream);
 
+/* Canonical fold of rows that already exist: float64 d_rows[n_rows * 4^k] -> d_out[n_rows * phm_num_bins(k, PHM_COUNT_CANONICAL)],
+ * k = 1..6, with the definition and bin order of phm_kmer_count(..., PHM_COUNT_CANONICAL): out[c] = row[y] + row[rc(y)] for the c-th
+ * smallest y with y <= rc(y) (row[y] alone when y = rc(y)).  One add per bin pair, so integer-valued rows below 2^53 fold exactly.
+ * Needs no workspace; d_rows and d_out must not overlap.  Folding commutes with summing rows, and a row's total does not change, so
+ * fold-then-normalise equals normalising canonical counts. */
+int phm_canonical_fold(const double *d_rows, int64_t n_rows, int k, double *d_out, void *stream);
+
 /* kmer.normalize_counts on its own (scripts/kmer.py:209-221) for counts that are already on the device. */
 int phm_normalize_counts(const uint32_t *d_counts, int64_t n_rows, int64_t bins, double *d_freq, void *stream);
 /* The same for rows that are not exact 32-bit counts (the summed genome counts of kmer.count_directory, already-float features):
@@ -124,11 +131,15 @@ int phm_normalize_rows(const double *d_rows, int64_t n_rows, int64_t bins, doubl
  *     d_combo         float64[n_points]  knn + kmeans                     (may be NULL)
  *     A query row holding NaN (zero-count contig) gets NaN in all three outputs.
  *
- *     Two device paths, same results: for dim = 256 and k_neighbors in {1, 3, 5} the (query x reference) contraction runs on
+ *     Two device paths, same results: for dim = 256 or 136 and k_neighbors in {1, 3, 5} the (query x reference) contraction runs on
  *     the tcgen05 tensor cores (FP16 operands, FP32 accumulation) together with a proven per-pair error interval; the few
  *     references / centroids whose interval can reach the k nearest are kept per query and decided exactly in float64.
  *     Rows whose candidate buffer overflows (and every other shape) go through the exhaustive float64 kernel.
  *     See DESIGN.md section 5 for the error bound.
+ *     dim = 136 is the width of canonical 4-mer features (phm_canonical_fold, PHM_COUNT_CANONICAL at k = 4): their rows fill the
+ *     first 136 columns of the 256-wide FP16 operands and the rest is zero, under the same error bound.  At dim = 136 count rows
+ *     (phm_score_counts) take the tensor cores; float64 feature rows keep the exhaustive kernel unless option "score_path" = 2,
+ *     because the two roads may order exact distance ties differently and phm_score's answers at 136 stay what they were.
  * ------------------------------------------------------------------------------------------- */
 size_t phm_score_workspace_bytes(int64_t n_points, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg, int dim);
 int phm_score(const double *d_points, int64_t n_points, int dim,
@@ -140,7 +151,8 @@ int phm_score(const double *d_points, int64_t n_points, int dim,
 /* Stages 2 + 3 fused: same as phm_score, but the queries are the raw uint32 count rows of phm_kmer_count (d_counts[n_points * dim]);
  * every kernel forms feature = count / row total in float64 on the fly, exactly as kmer.normalize_counts would
  * (scripts/kmer.py:209-221, scripts/phamer.py:139), so the float64 feature matrix never exists in memory.  Needs the
- * tensor-core shape (dim = 256, k_neighbors in {1, 3, 5}, both centroid sets), PHM_E_UNSUPPORTED otherwise. */
+ * tensor-core shape (dim = 256 or 136 -- plain or canonical 4-mer counts --, k_neighbors in {1, 3, 5}, both centroid sets),
+ * PHM_E_UNSUPPORTED otherwise. */
 int phm_score_counts(const uint32_t *d_counts, int64_t n_points, int dim,
                      const double *d_refs, int64_t n_refs, int64_t n_positive,
                      const double *d_cent_pos, int64_t n_cent_pos, const double *d_cent_neg, int64_t n_cent_neg,

@@ -26,6 +26,7 @@ SIGNATURES = {
     "phm_kmer_count": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_uint32, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "phm_kmer_count_packed": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_uint32, c_void_p, c_void_p,
                                       c_void_p, c_size_t, c_void_p]),
+    "phm_canonical_fold": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "phm_normalize_counts": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "phm_normalize_rows": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "phm_distances": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),

@@ -790,6 +790,55 @@ __global__ void canonical_lut_kernel(int k, uint16_t *rc_lut, uint16_t *compact_
 }
 
 // --------------------------------------------------------------------------------------------------
+// canonical fold of rows that already exist (phm_canonical_fold): float64 [n, 4^K] -> [n, canonical bins], the counter's definition
+// and bin order.  Every CTA builds the compact bin -> representative table in shared memory (a block scan over y <= rc(y)), so the
+// call needs no workspace; then a warp per row writes out[c] = row[y] + row[rc(y)] for the representative y of c (row[y] alone
+// when y is its own reverse complement): one add per bin pair, exact for integer rows below 2^53.
+// --------------------------------------------------------------------------------------------------
+template <int K>
+__global__ void __launch_bounds__(256) canonical_fold_kernel(const double *__restrict__ in, int64_t n_rows, double *__restrict__ out) {
+    constexpr int BINS = 1 << (2 * K);
+    constexpr int PER = (BINS + 255) / 256;                            // consecutive bins per thread
+    __shared__ uint16_t rep[BINS];
+    __shared__ int warp_tot[8];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    int mine = 0;
+#pragma unroll
+    for (int j = 0; j < PER; ++j) {
+        const uint32_t y = threadIdx.x * PER + j;
+        mine += (y < (uint32_t)BINS && y <= revcomp_fast<K>(y)) ? 1 : 0;
+    }
+    int incl = mine;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int up = __shfl_up_sync(FULL, incl, o);
+        if (lane >= o) incl += up;
+    }
+    if (lane == 31) warp_tot[wid] = incl;
+    __syncthreads();
+    int base = incl - mine, n_canon = 0;
+    for (int w = 0; w < 8; ++w) {
+        base += w < wid ? warp_tot[w] : 0;
+        n_canon += warp_tot[w];
+    }
+#pragma unroll
+    for (int j = 0; j < PER; ++j) {
+        const uint32_t y = threadIdx.x * PER + j;
+        if (y < (uint32_t)BINS && y <= revcomp_fast<K>(y)) rep[base++] = (uint16_t)y;
+    }
+    __syncthreads();
+    const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t r = warp; r < n_rows; r += n_warps) {
+        const double *row = in + r * BINS;
+        for (int c = lane; c < n_canon; c += 32) {
+            const uint32_t y = rep[c], z = revcomp_fast<K>(y);
+            out[r * n_canon + c] = (z == y) ? row[y] : row[y] + row[z];
+        }
+    }
+}
+
+// --------------------------------------------------------------------------------------------------
 // simple cross-check kernel: one warp per contig, every lane re-reads the k bytes of its window, global atomics
 // --------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int ref_symbol(uint8_t c) {
@@ -1240,6 +1289,26 @@ extern "C" int phm_normalize_counts(const uint32_t *d_counts, int64_t n_rows, in
     int64_t blocks = (n_rows + 7) / 8;
     if (blocks > 148 * 16) blocks = 148 * 16;
     normalize_kernel<<<(unsigned)blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_counts, n_rows, bins, d_freq);
+    PHM_LAUNCH_CHECK();
+    return PHM_OK;
+}
+
+extern "C" int phm_canonical_fold(const double *d_rows, int64_t n_rows, int k, double *d_out, void *stream) {
+    PHM_REQUIRE(k >= 1 && k <= 6, "k must be 1..6");
+    PHM_REQUIRE(n_rows >= 0, "n_rows must be >= 0");
+    if (n_rows == 0) return PHM_OK;
+    PHM_REQUIRE(d_rows != nullptr && d_out != nullptr, "null pointer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    int64_t blocks = (n_rows + 7) / 8;
+    if (blocks > (int64_t)sm_count() * 8) blocks = (int64_t)sm_count() * 8;
+    switch (k) {
+        case 1: canonical_fold_kernel<1><<<(unsigned)blocks, 256, 0, st>>>(d_rows, n_rows, d_out); break;
+        case 2: canonical_fold_kernel<2><<<(unsigned)blocks, 256, 0, st>>>(d_rows, n_rows, d_out); break;
+        case 3: canonical_fold_kernel<3><<<(unsigned)blocks, 256, 0, st>>>(d_rows, n_rows, d_out); break;
+        case 4: canonical_fold_kernel<4><<<(unsigned)blocks, 256, 0, st>>>(d_rows, n_rows, d_out); break;
+        case 5: canonical_fold_kernel<5><<<(unsigned)blocks, 256, 0, st>>>(d_rows, n_rows, d_out); break;
+        default: canonical_fold_kernel<6><<<(unsigned)blocks, 256, 0, st>>>(d_rows, n_rows, d_out); break;
+    }
     PHM_LAUNCH_CHECK();
     return PHM_OK;
 }

@@ -83,23 +83,33 @@ struct PrepConsts {            // device-resident, written by the reference pass
     float rho;                 // max_j (dB_j + eps_acc (P_j + dB_j)) / P_j
     float pmax;                // max_j P_j
 };
-struct QueryEmit {             // where a producer of count rows writes the scorer's query operands
+struct QueryEmit {             // where a producer of 256-wide count rows writes the scorer's query operands
     __half *op;                // [n, 256] centred, 2^12-scaled FP16 rows
     float *crow;               // [n] error constant C_row (NaN for an empty contig)
     double *cnorm;             // [n] |x - 1/256|^2
     uint32_t *total;           // [n] row total of the counts (the decision kernel forms count / total without a reduction)
     const PrepConsts *consts;
 };
-constexpr int PREP_DIM = 256;
+constexpr int PREP_DIM = 256;               // width of the FP16 operands
+constexpr int CANON_DIM = 136;              // canonical 4-mer features: written into the first 136 operand columns, the rest stays zero
 constexpr double PREP_SCALE = 4096.0;
+// feature widths the tensor-core scorer takes
+__host__ __device__ constexpr bool tc_width(int dim) { return dim == PREP_DIM || dim == CANON_DIM; }
+// a W-wide float64 row spread over a warp: lane l holds features l, l + 32, ... (NCH<W> chunks); in_row is false for the chunk
+// slots beyond W, which read nothing and contribute exactly zero
+template <int W> constexpr int NCH = (W + 31) / 32;
+template <int W>
+__device__ __forceinline__ bool in_row(int lane, int i) { return W % 32 == 0 || lane + 32 * i < W; }
 
 __device__ __forceinline__ float float_up(double x) {           // a float that is >= x (x >= 0)
     float f = (float)x;
     return ((double)f >= x) ? f : __uint_as_float(__float_as_uint(f) + 1u);
 }
-// one feature: FP16 operand element and the four running sums |x|^2, |x - u|^2, |A~ - A|^2, |A|^2 (scaled units)
+// one feature of a W-wide row: FP16 operand element and the four running sums |x|^2, |x - u|^2, |A~ - A|^2, |A|^2 (scaled units),
+// u = 1/W
+template <int W = PREP_DIM>
 __device__ __forceinline__ __half prep_accumulate(double x, double &s, double &sc, double &sd, double &sh) {
-    const double xc = x - 1.0 / (double)PREP_DIM;
+    const double xc = x - 1.0 / (double)W;
     const double t = xc * PREP_SCALE;
     const __half h = __float2half_rn((float)t);
     const double hv = (double)__half2float(h);

@@ -6,6 +6,10 @@
 //
 //   d2(a, b) = |a|^2 + |b|^2 - 2 a.b          a = contig features [n, 256], b = reference rows / centroids
 //
+// Canonical 4-mer features (136 wide) take the same road: a row fills the first 136 operand columns, centred by 1/136, and the
+// other 120 columns are exactly zero on both sides, so the contraction kernel is the same and every bound below holds for the
+// 136-wide vectors.  Every kernel that reads float64 or count rows takes the width as its template parameter W.
+//
 // The a.b term is a dense contraction and runs as ONE tcgen05.mma pass (kind::f16, FP32 accumulators in tensor memory) over
 // operands that are centred by 1/256 (distances are translation invariant), scaled by 2^12 and rounded to FP16.  FP16 x FP16
 // products are exact in FP32, so the only errors are the operand roundings and the FP32 accumulation; both are BOUNDED, per
@@ -50,7 +54,7 @@ int score_list_pass = 1;          // option "score_list_pass": 0 = overflowed ro
 
 namespace tc {
 
-constexpr int KDIM = 256;                 // feature width handled by this kernel (k = 4)
+constexpr int KDIM = 256;                 // width of the FP16 operands (plain 4-mers; canonical rows are zero-padded to it)
 constexpr int BM = 128, BN = 128, BK = 64;
 constexpr int MT = 2 * BM;                // contig rows per CTA tile (two MMA row blocks share every B block)
 constexpr int NKC = KDIM / BK;            // 4 K-chunks of 128 bytes
@@ -663,25 +667,26 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, TcParams p) {
     }
 }
 
-// This lane's 8 features of a query row: from the float64 feature matrix, or from raw counts divided by the row total
-// (IEEE float64 division, exactly what kmer.normalize_counts does, scripts/kmer.py:219-220).
+// This lane's features of a W-wide query row (NCH<W> chunk slots, zero beyond W): from the float64 feature matrix, or from raw
+// counts divided by the row total (IEEE float64 division, exactly what kmer.normalize_counts does, scripts/kmer.py:219-220).
+template <int W>
 __device__ __forceinline__ void load_query_row(const double *points, const uint32_t *counts, int64_t row, int lane,
-                                               double (&x)[KDIM / 32], uint32_t *total_out = nullptr) {
+                                               double (&x)[NCH<W>], uint32_t *total_out = nullptr) {
     if (counts) {
-        uint32_t c[KDIM / 32];
+        uint32_t c[NCH<W>];
         unsigned long long total = 0;
 #pragma unroll
-        for (int i = 0; i < KDIM / 32; ++i) { c[i] = counts[row * KDIM + lane + 32 * i]; total += c[i]; }
+        for (int i = 0; i < NCH<W>; ++i) { c[i] = in_row<W>(lane, i) ? counts[row * W + lane + 32 * i] : 0u; total += c[i]; }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) total += __shfl_xor_sync(FULL, total, o);
         const double t = (double)total;
         const double r = 1.0 / t;                        // correctly rounded reciprocal, once per row
 #pragma unroll
-        for (int i = 0; i < KDIM / 32; ++i) x[i] = exact_quotient((double)c[i], t, r);
+        for (int i = 0; i < NCH<W>; ++i) x[i] = exact_quotient((double)c[i], t, r);
         if (total_out) *total_out = (uint32_t)total;
     } else {
 #pragma unroll
-        for (int i = 0; i < KDIM / 32; ++i) x[i] = points[row * KDIM + lane + 32 * i];
+        for (int i = 0; i < NCH<W>; ++i) x[i] = in_row<W>(lane, i) ? points[row * W + lane + 32 * i] : 0.0;
     }
 }
 
@@ -696,6 +701,9 @@ __device__ __forceinline__ void load_query_row(const double *points, const uint3
 // exchangeable order; a golden-ratio stride makes every prefix an even sample of the whole file.
 // is_ref = 1: reference / centroid rows: FP16 operand, nbs, P, norms, and rho / pmax by atomic max (positive floats order as ints)
 // is_ref = 0: query rows: FP16 operand, norms and C_row (reads rho / pmax, so it must run after every is_ref pass)
+// W < 256 (canonical features): the row fills the first W operand columns, centred by 1/W; the other columns are written as FP16
+// zero and enter none of the sums, so every bound below is the bound of the W-wide vectors.
+template <int W>
 __global__ void tc_prep_rows_kernel(const double *__restrict__ src, int64_t n_src, int64_t n_rows, int64_t perm_a, int64_t perm_c,
                                     const uint32_t *__restrict__ src_counts, int is_ref, int64_t n_positive, __half *__restrict__ op, double *__restrict__ norm64, double *__restrict__ cnorm64,
                                     float *__restrict__ nbs, float *__restrict__ pnorm, float *__restrict__ crow,
@@ -703,26 +711,30 @@ __global__ void tc_prep_rows_kernel(const double *__restrict__ src, int64_t n_sr
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    const double shift = 1.0 / (double)KDIM;
+    const double shift = 1.0 / (double)W;
     float rho = 0.f, pmax = 0.f;
     if (!is_ref) { rho = consts->rho; pmax = consts->pmax; }
     for (int64_t r = warp; r < n_rows; r += n_warps) {
         double s = 0.0, sc = 0.0, sd = 0.0, sh = 0.0;       // |x|^2, |x - u|^2, |B~ - B|^2, |B|^2 (scaled units)
         const int64_t sr = (r < n_src) ? (perm_a * r + perm_c) % n_src : 0;
-        double xs[KDIM / 32];
+        double xs[NCH<W>];
         uint32_t total = 0u;
-        if (r < n_src) load_query_row(src, src_counts, sr, lane, xs, &total);
+        if (r < n_src) load_query_row<W>(src, src_counts, sr, lane, xs, &total);
         if (row_total && src_counts && lane == 0 && r < n_src) row_total[sr] = total;
 #pragma unroll
         for (int i = 0; i < KDIM / 32; ++i) {
-            const double x = (r < n_src) ? xs[i] : shift;
             const int d = lane + 32 * i;
             // queries: row-major [n, 256] (fetched by 2-D TMA); references: the shared-memory image of their 128-row tile,
             // [tile][K chunk of 64][row][128 B with the 16-byte pieces XOR-swizzled by row & 7], so that a B block is ONE
             // contiguous 16 KB bulk copy instead of 128 row pieces gathered by a tensor map
             const int64_t o = is_ref ? ((((r >> 7) * NKC + (d >> 6)) * BM + (r & 127)) * BK + ((((d >> 3) & 7) ^ (int)(r & 7)) << 3) + (d & 7))
                                      : r * KDIM + d;
-            op[o] = prep_accumulate(x, s, sc, sd, sh);
+            if (W == KDIM || (i < NCH<W> && in_row<W>(lane, i))) {
+                const double x = (r < n_src) ? xs[i < NCH<W> ? i : 0] : shift;
+                op[o] = prep_accumulate<W>(x, s, sc, sd, sh);
+            } else {
+                op[o] = __float2half_rn(0.0f);
+            }
         }
         warp_sum4(s, sc, sd, sh, lane);                    // valid in lane 0
         if (lane == 0) {
@@ -797,16 +809,16 @@ struct DecideParams {
 // Squared float64 direct-difference distances of a query row (x: this lane's 8 features, lane-strided) to U rows at once.  Every
 // exact road measures its (row, reference) and (row, centroid) pairs with this: each lane's fma chain over its features in
 // ascending order, then the butterfly xor 16 ... 1, so that the roads agree bit for bit.  U > 1 keeps independent rows in flight
-// where a loop over rows is latency-bound.
-template <int U>
-__device__ __forceinline__ void warp_d2(const double (&x)[KDIM / 32], const double *const (&b)[U], int lane, double (&acc)[U]) {
+// where a loop over rows is latency-bound.  Rows are W wide; chunk slots beyond W add fma(0, 0, acc) = acc.
+template <int W, int U>
+__device__ __forceinline__ void warp_d2(const double (&x)[NCH<W>], const double *const (&b)[U], int lane, double (&acc)[U]) {
 #pragma unroll
     for (int t = 0; t < U; ++t) acc[t] = 0.0;
 #pragma unroll
-    for (int i = 0; i < KDIM / 32; ++i)
+    for (int i = 0; i < NCH<W>; ++i)
 #pragma unroll
         for (int t = 0; t < U; ++t) {
-            const double d = x[i] - b[t][lane + 32 * i];
+            const double d = in_row<W>(lane, i) ? x[i] - b[t][lane + 32 * i] : 0.0;
             acc[t] = fma(d, d, acc[t]);
         }
 #pragma unroll
@@ -814,10 +826,11 @@ __device__ __forceinline__ void warp_d2(const double (&x)[KDIM / 32], const doub
 #pragma unroll
         for (int t = 0; t < U; ++t) acc[t] += __shfl_xor_sync(FULL, acc[t], o);
 }
-__device__ __forceinline__ double warp_d2(const double (&x)[KDIM / 32], const double *b, int lane) {
+template <int W>
+__device__ __forceinline__ double warp_d2(const double (&x)[NCH<W>], const double *b, int lane) {
     const double *const rows[1] = {b};
     double acc[1];
-    warp_d2<1>(x, rows, lane, acc);
+    warp_d2<W>(x, rows, lane, acc);
     return acc[0];
 }
 
@@ -828,7 +841,7 @@ __device__ __forceinline__ double warp_min_d(double v) {
 }
 
 // The decision of a row has a SCALAR part -- which of its (at most 16) candidates can still matter, and whether the neighbour vote
-// is already settled by the proven intervals -- and a part that needs the whole 256-wide row: the exact float64 distances to the one
+// is already settled by the proven intervals -- and a part that needs the whole (W-wide) row: the exact float64 distances to the one
 // or two centroids of each class that survive, and to the band of references when the intervals leave the vote open.  Round 1 ran
 // everything warp-wide, one row at a time (795 warp instructions per row, issue-bound).  Now a warp takes 32 consecutive rows and
 //   A  every LANE settles the scalar part of its own row from the candidate slots (no shuffles, no reductions),
@@ -848,7 +861,7 @@ __device__ __forceinline__ int64_t cand_ref_index(const DecideParams &p, uint32_
 // NEIGHBORS: the call also reports the k nearest references and the nearest centroid of each class (p.nb).  A row then counts as
 // settled only when its k nearest are identified, not merely its vote: every live row re-measures its band (ROW_OPEN), and a row
 // with a dropped candidate within reach goes to the overflow road even when its vote is unanimous.  The scores do not change.
-template <bool FROM_COUNTS, bool NEIGHBORS = false>
+template <bool FROM_COUNTS, bool NEIGHBORS = false, int W = KDIM>
 __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(DecideParams p) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -964,17 +977,17 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
         unsigned todo = __ballot_sync(FULL, my_live && (has_cent || state == ROW_OPEN || p.stats != nullptr));
         // the count row (or feature row) of the NEXT row to do is fetched while the current one is worked on: the loop is a chain of
         // dependent memory accesses per row otherwise
-        uint32_t c_nxt[FROM_COUNTS ? KDIM / 32 : 1], t_nxt = 0u;
-        double x_nxt[FROM_COUNTS ? 1 : KDIM / 32];
+        uint32_t c_nxt[FROM_COUNTS ? NCH<W> : 1], t_nxt = 0u;
+        double x_nxt[FROM_COUNTS ? 1 : NCH<W>];
         auto fetch = [&](int rr) {
             const int64_t row = base + rr;
             if (FROM_COUNTS) {
 #pragma unroll
-                for (int i = 0; i < KDIM / 32; ++i) c_nxt[FROM_COUNTS ? i : 0] = p.point_counts[row * KDIM + lane + 32 * i];
+                for (int i = 0; i < NCH<W>; ++i) c_nxt[FROM_COUNTS ? i : 0] = in_row<W>(lane, i) ? p.point_counts[row * W + lane + 32 * i] : 0u;
                 t_nxt = p.row_total[row];
             } else {
 #pragma unroll
-                for (int i = 0; i < KDIM / 32; ++i) x_nxt[FROM_COUNTS ? 0 : i] = p.points[row * KDIM + lane + 32 * i];
+                for (int i = 0; i < NCH<W>; ++i) x_nxt[FROM_COUNTS ? 0 : i] = in_row<W>(lane, i) ? p.points[row * W + lane + 32 * i] : 0.0;
             }
         };
         if (todo) fetch(__ffs(todo) - 1);
@@ -984,15 +997,15 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
             const int64_t row = base + rr;
             const uint32_t info = __shfl_sync(FULL, my_info, rr);
             const uint32_t cp0 = __shfl_sync(FULL, first_p, rr), cn0 = __shfl_sync(FULL, first_n, rr);
-            double x[KDIM / 32];
+            double x[NCH<W>];
             if (FROM_COUNTS) {
                 const double t = (double)t_nxt;
                 const double r = 1.0 / t;                                 // correctly rounded reciprocal, once per row
 #pragma unroll
-                for (int i = 0; i < KDIM / 32; ++i) x[i] = exact_quotient((double)c_nxt[FROM_COUNTS ? i : 0], t, r);
+                for (int i = 0; i < NCH<W>; ++i) x[i] = exact_quotient((double)c_nxt[FROM_COUNTS ? i : 0], t, r);
             } else {
 #pragma unroll
-                for (int i = 0; i < KDIM / 32; ++i) x[i] = x_nxt[FROM_COUNTS ? 0 : i];
+                for (int i = 0; i < NCH<W>; ++i) x[i] = x_nxt[FROM_COUNTS ? 0 : i];
             }
             if (todo) fetch(__ffs(todo) - 1);
             const uint2 *ent = p.cand + row * NENT;                       // warp-uniform reads below: one broadcast each
@@ -1006,7 +1019,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                     const int s = __ffs(rest) - 1;
                     rest &= rest - 1;
                     const int64_t idx = cand_ref_index(p, ent[s].y);
-                    const double d = warp_d2(x, p.refs + idx * KDIM, lane);
+                    const double d = warp_d2<W>(x, p.refs + idx * W, lane);
                     if (lane == s) { my_d2 = d; my_idx = idx; }
                 }
                 int erank = 0;
@@ -1034,7 +1047,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                 for (int s = 0; s < CAP_R && s < cnt_r; ++s) {
                     const uint2 e = ent[s];
                     const double lo_s = (double)__uint_as_float(e.x), w_s = (double)p.cand_up[row * NENT + s] - lo_s;
-                    const double d = warp_d2(x, p.refs + cand_ref_index(p, e.y) * KDIM, lane);
+                    const double d = warp_d2<W>(x, p.refs + cand_ref_index(p, e.y) * W, lane);
                     const double exact = (d - na) * NORM_SCALE;                 // what the ranking value estimates
                     const double err = fabs(lo_s + 0.5 * w_s - exact);
                     worst_abs = fmaxf(worst_abs, (float)(err / NORM_SCALE));
@@ -1058,7 +1071,7 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                         const int64_t n_c = cls ? p.n_cent_neg : p.n_cent_pos;
                         for (int64_t c = 0; c < n_c; c += 2) {
                             const int64_t c1 = c + 1 < n_c ? c + 1 : c;
-                            const double a0 = warp_d2(x, cent + c * KDIM, lane), a1 = warp_d2(x, cent + c1 * KDIM, lane);
+                            const double a0 = warp_d2<W>(x, cent + c * W, lane), a1 = warp_d2<W>(x, cent + c1 * W, lane);
                             if (NEIGHBORS) {
                                 if (a0 < e2[cls]) { e2[cls] = a0; i2[cls] = c; }
                                 if (a1 < e2[cls]) { e2[cls] = a1; i2[cls] = c1; }
@@ -1073,9 +1086,9 @@ __global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(
                     const int sp = rest_p ? __ffs(rest_p) - 1 : 0, sn = rest_n ? __ffs(rest_n) - 1 : 0;
                     const uint32_t ip = first_round ? cp0 : ent[CAP_R + sp].y, in_ = first_round ? cn0 : ent[CAP_R + CAP_C + sn].y;
                     first_round = false;
-                    const double *const b[2] = {p.cent_pos + (int64_t)(rest_p ? ip : 0u) * KDIM, p.cent_neg + (int64_t)(rest_n ? in_ : 0u) * KDIM};
+                    const double *const b[2] = {p.cent_pos + (int64_t)(rest_p ? ip : 0u) * W, p.cent_neg + (int64_t)(rest_n ? in_ : 0u) * W};
                     double a[2];
-                    warp_d2<2>(x, b, lane, a);
+                    warp_d2<W>(x, b, lane, a);
                     const double ap = a[0], an = a[1];
                     if (NEIGHBORS) {
                         // kept slots are not in index order: the tie rule compares indices
@@ -1260,6 +1273,7 @@ __device__ __forceinline__ void finish_row(const ScoreOut &o, int64_t row, const
 
 // One warp per listed row: float64 direct-difference distance (warp_d2) to each listed reference, k smallest by (distance,
 // reference index), vote.  The centroid part of the score was settled by score_decide_kernel.
+template <int W>
 __global__ void __launch_bounds__(256) score_list_decide_kernel(ListDecideParams p) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -1274,8 +1288,8 @@ __global__ void __launch_bounds__(256) score_list_decide_kernel(ListDecideParams
             if (lane == 0) p.fallback_rows[atomicAdd(p.fallback_count, 1ull)] = row;
             continue;
         }
-        double x[KDIM / 32];
-        load_query_row(p.points, p.point_counts, row, lane, x);
+        double x[NCH<W>];
+        load_query_row<W>(p.points, p.point_counts, row, lane, x);
         TopK<TC_KMAX> top;
         top.clear();
         const uint32_t *cols = p.list_cols + off;
@@ -1286,10 +1300,10 @@ __global__ void __launch_bounds__(256) score_list_decide_kernel(ListDecideParams
             for (int t = 0; t < LD_U; ++t) {
                 const uint32_t c = c0 + t < n ? c0 + t : n - 1;
                 idx[t] = (int)((p.perm_a * (int64_t)cols[c] + p.perm_c) % p.n_refs);
-                b[t] = p.refs + (int64_t)idx[t] * KDIM;
+                b[t] = p.refs + (int64_t)idx[t] * W;
             }
             double acc[LD_U];
-            warp_d2<LD_U>(x, b, lane, acc);
+            warp_d2<W>(x, b, lane, acc);
 #pragma unroll
             for (int t = 0; t < LD_U; ++t) {
                 if (c0 + t >= n) break;
@@ -1358,6 +1372,7 @@ __device__ __forceinline__ void fallback_finish(const FallbackParams &f, int64_t
     finish_row(f.out, row, m.top.d, m.top.i, f.n_positive, fallback_km(f, m.cp, m.cn));
 }
 
+template <int W>
 __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
     __shared__ FallbackPart s_part[8];
     __shared__ FallbackPart s_all[FB_SLICES];
@@ -1373,8 +1388,8 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
         const int slice = (int)(it % slices);
         const int64_t row = f.rows[ridx];
         const int64_t c_lo = f.n_refs * slice / slices, c_hi = f.n_refs * (slice + 1) / slices;
-        double x[KDIM / 32];
-        load_query_row(f.points, f.point_counts, row, lane, x);
+        double x[NCH<W>];
+        load_query_row<W>(f.points, f.point_counts, row, lane, x);
         TopK<TC_KMAX> top;
         top.clear();
         for (int64_t c0 = c_lo + warp; c0 < c_hi; c0 += 8 * FB_U) {   // ascending index per warp (see nearer)
@@ -1382,10 +1397,10 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
 #pragma unroll
             for (int t = 0; t < FB_U; ++t) {
                 const int64_t c = c0 + 8 * t;
-                b[t] = f.refs + (c < c_hi ? c : c0) * KDIM;
+                b[t] = f.refs + (c < c_hi ? c : c0) * W;
             }
             double acc[FB_U];
-            warp_d2<FB_U>(x, b, lane, acc);                     // FB_U independent rows in flight: this loop is latency-bound
+            warp_d2<W>(x, b, lane, acc);                     // FB_U independent rows in flight: this loop is latency-bound
 #pragma unroll
             for (int t = 0; t < FB_U; ++t) {
                 const int64_t c = c0 + 8 * t;
@@ -1395,8 +1410,8 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
         }
         double cp = INFINITY, cn = INFINITY;
         if (slice == 0) {
-            for (int64_t c = warp; c < f.n_cent_pos; c += 8) cp = fmin(cp, warp_d2(x, f.cent_pos + c * KDIM, lane));
-            for (int64_t c = warp; c < f.n_cent_neg; c += 8) cn = fmin(cn, warp_d2(x, f.cent_neg + c * KDIM, lane));
+            for (int64_t c = warp; c < f.n_cent_pos; c += 8) cp = fmin(cp, warp_d2<W>(x, f.cent_pos + c * W, lane));
+            for (int64_t c = warp; c < f.n_cent_neg; c += 8) cn = fmin(cn, warp_d2<W>(x, f.cent_neg + c * W, lane));
         }
         __syncthreads();                                        // previous item's merge has finished reading shared memory
         if (lane == 0) { s_part[warp].top = top; s_part[warp].cp = cp; s_part[warp].cn = cn; }
@@ -1430,9 +1445,9 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
 // from HBM once per 32 rows instead of once per row.  Reference distances only ORDER the neighbours here; the centroid distances,
 // whose values reach the score, use the same warp_d2 as every other path.
 constexpr int FBB_ROWS = 32, FBB_TR = 32, FBB_PITCH = FBB_TR + 1;
-constexpr int FBB_SMEM = (FBB_ROWS * KDIM + KDIM * FBB_PITCH) * 8 + FBB_ROWS * TC_KMAX * 12 + 64;
+template <int W> constexpr int FBB_SMEM = (FBB_ROWS * W + W * FBB_PITCH) * 8 + FBB_ROWS * TC_KMAX * 12 + 64;
 
-template <int QW>                                                          // rows per warp
+template <int W, int QW>                                                   // row width, rows per warp
 __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned long long blk, unsigned long long count,
                                                double *s_rows, double *s_tile, double *s_d, int *s_i) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1440,14 +1455,15 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
     __syncthreads();
     // this warp's rows into shared memory; their lists start empty
     int64_t my_row[QW];
-    double x[QW][KDIM / 32];
+    double x[QW][NCH<W>];
 #pragma unroll
     for (int q = 0; q < QW; ++q) {
         const unsigned long long ridx = blk * (8 * QW) + warp * QW + q;
         my_row[q] = ridx < count ? f.rows[ridx] : -1;
-        if (my_row[q] >= 0) load_query_row(f.points, f.point_counts, my_row[q], lane, x[q]);
+        if (my_row[q] >= 0) load_query_row<W>(f.points, f.point_counts, my_row[q], lane, x[q]);
 #pragma unroll
-        for (int i = 0; i < KDIM / 32; ++i) s_rows[(warp * QW + q) * KDIM + lane + 32 * i] = my_row[q] >= 0 ? x[q][i] : 0.0;
+        for (int i = 0; i < NCH<W>; ++i)
+            if (in_row<W>(lane, i)) s_rows[(warp * QW + q) * W + lane + 32 * i] = my_row[q] >= 0 ? x[q][i] : 0.0;
         if (lane < TC_KMAX) { s_d[(warp * QW + q) * TC_KMAX + lane] = INFINITY; s_i[(warp * QW + q) * TC_KMAX + lane] = -1; }
     }
     double thr[QW];
@@ -1455,21 +1471,21 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
     for (int q = 0; q < QW; ++q) thr[q] = INFINITY;
     for (int64_t c0 = 0; c0 < f.n_refs; c0 += FBB_TR) {
         __syncthreads();                                                   // previous tile fully consumed
-        for (int idx = threadIdx.x; idx < FBB_TR * KDIM; idx += 256) {
-            const int r = idx >> 8, d = idx & 255;
-            s_tile[d * FBB_PITCH + r] = (c0 + r < f.n_refs) ? f.refs[(c0 + r) * KDIM + d] : 0.0;
+        for (int idx = threadIdx.x; idx < FBB_TR * W; idx += 256) {
+            const int r = (W == KDIM) ? idx >> 8 : idx / W, d = (W == KDIM) ? idx & 255 : idx % W;
+            s_tile[d * FBB_PITCH + r] = (c0 + r < f.n_refs) ? f.refs[(c0 + r) * W + d] : 0.0;
         }
         __syncthreads();
         double acc[QW];
 #pragma unroll
         for (int q = 0; q < QW; ++q) acc[q] = 0.0;
-        const double *xr = s_rows + warp * QW * KDIM;
+        const double *xr = s_rows + warp * QW * W;
 #pragma unroll 4
-        for (int d = 0; d < KDIM; d += 2) {
+        for (int d = 0; d < W; d += 2) {
             const double b0 = s_tile[d * FBB_PITCH + lane], b1 = s_tile[(d + 1) * FBB_PITCH + lane];
 #pragma unroll
             for (int q = 0; q < QW; ++q) {
-                const double2 xx = *reinterpret_cast<const double2 *>(xr + q * KDIM + d);
+                const double2 xx = *reinterpret_cast<const double2 *>(xr + q * W + d);
                 const double t0 = xx.x - b0, t1 = xx.y - b1;
                 acc[q] = fma(t0, t0, acc[q]);
                 acc[q] = fma(t1, t1, acc[q]);
@@ -1496,8 +1512,8 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
     for (int q = 0; q < QW; ++q) {
         if (my_row[q] < 0) continue;
         double cp = INFINITY, cn = INFINITY;
-        for (int64_t c = 0; c < f.n_cent_pos; ++c) cp = fmin(cp, warp_d2(x[q], f.cent_pos + c * KDIM, lane));
-        for (int64_t c = 0; c < f.n_cent_neg; ++c) cn = fmin(cn, warp_d2(x[q], f.cent_neg + c * KDIM, lane));
+        for (int64_t c = 0; c < f.n_cent_pos; ++c) cp = fmin(cp, warp_d2<W>(x[q], f.cent_pos + c * W, lane));
+        for (int64_t c = 0; c < f.n_cent_neg; ++c) cn = fmin(cn, warp_d2<W>(x[q], f.cent_neg + c * W, lane));
         if (lane == 0) {
             const int at = (warp * QW + q) * TC_KMAX;
             finish_row(f.out, my_row[q], s_d + at, s_i + at, f.n_positive, fallback_km(f, cp, cn));
@@ -1505,11 +1521,12 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
     }
 }
 
+template <int W>
 __global__ void __launch_bounds__(256) score_fallback_blocked_kernel(FallbackParams f) {
     extern __shared__ __align__(16) unsigned char fbb_raw[];
-    double *s_rows = reinterpret_cast<double *>(fbb_raw);                     // [32][256]
-    double *s_tile = s_rows + FBB_ROWS * KDIM;                                // [256][33]
-    double *s_d = s_tile + KDIM * FBB_PITCH;                                  // [32][TC_KMAX]
+    double *s_rows = reinterpret_cast<double *>(fbb_raw);                     // [32][W]
+    double *s_tile = s_rows + FBB_ROWS * W;                                   // [W][33]
+    double *s_d = s_tile + W * FBB_PITCH;                                     // [32][TC_KMAX]
     int *s_i = reinterpret_cast<int *>(s_d + FBB_ROWS * TC_KMAX);             // [32][TC_KMAX]
     const unsigned long long count = *f.count;
     if (count <= FB_BLOCKED_MIN) return;
@@ -1519,10 +1536,10 @@ __global__ void __launch_bounds__(256) score_fallback_blocked_kernel(FallbackPar
     const unsigned long long n_blocks = (count + 8 * qw - 1) / (8 * qw);
     for (unsigned long long blk = blockIdx.x; blk < n_blocks; blk += gridDim.x) {
         switch (qw) {
-            case 1: fallback_block<1>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
-            case 2: fallback_block<2>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
-            case 3: fallback_block<3>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
-            default: fallback_block<4>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
+            case 1: fallback_block<W, 1>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
+            case 2: fallback_block<W, 2>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
+            case 3: fallback_block<W, 3>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
+            default: fallback_block<W, 4>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
         }
     }
 }
@@ -1635,16 +1652,18 @@ size_t score_tc_workspace_bytes(int64_t n, int64_t n_refs, int64_t n_cp, int64_t
 }
 
 bool score_tc_supported(int dim, int k_neighbors, int64_t n_refs, int64_t n_cp, int64_t n_cn) {
-    return dim == KDIM && (k_neighbors == 1 || k_neighbors == 3 || k_neighbors == 5) && n_refs >= k_neighbors && n_cp > 0 && n_cn > 0;
+    return tc_width(dim) && (k_neighbors == 1 || k_neighbors == 3 || k_neighbors == 5) && n_refs >= k_neighbors && n_cp > 0 && n_cn > 0;
 }
 
-static int launch_prep(const double *src, const uint32_t *src_counts, int64_t n_src, int64_t n_rows, int64_t perm_a, int64_t perm_c, int is_ref, int64_t n_positive, __half *op,
-                       double *norm64, double *cnorm64, float *nbs, float *pnorm, float *crow, PrepConsts *consts, cudaStream_t st,
-                       uint32_t *row_total = nullptr, __half *bx = nullptr) {
+// rows of `dim` features (256 or CANON_DIM)
+static int launch_prep(int dim, const double *src, const uint32_t *src_counts, int64_t n_src, int64_t n_rows, int64_t perm_a, int64_t perm_c, int is_ref,
+                       int64_t n_positive, __half *op, double *norm64, double *cnorm64, float *nbs, float *pnorm, float *crow, PrepConsts *consts,
+                       cudaStream_t st, uint32_t *row_total = nullptr, __half *bx = nullptr) {
     if (n_rows == 0) return PHM_OK;
     int64_t blocks = (n_rows + 7) / 8;
     if (blocks > 148 * 16) blocks = 148 * 16;
-    tc_prep_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(src, n_src, n_rows, perm_a, perm_c, src_counts, is_ref, n_positive, op, norm64, cnorm64, nbs, pnorm,
+    auto kern = dim == CANON_DIM ? tc_prep_rows_kernel<CANON_DIM> : tc_prep_rows_kernel<KDIM>;
+    kern<<<(unsigned)blocks, 256, 0, st>>>(src, n_src, n_rows, perm_a, perm_c, src_counts, is_ref, n_positive, op, norm64, cnorm64, nbs, pnorm,
                                                           crow, consts, row_total, bx);
     PHM_LAUNCH_CHECK();
     return PHM_OK;
@@ -1700,11 +1719,11 @@ int score_tc_begin(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t s
     int rc;
     int64_t perm_a, perm_c;
     ref_permutation(a.n_refs, &perm_a, &perm_c);
-    if ((rc = launch_prep(a.refs, nullptr, a.n_refs, ref_pad, perm_a, perm_c, 1, a.n_positive, w.b_op, w.norm_refs, nullptr, w.nbs, w.pnorm, nullptr, w.consts, st,
+    if ((rc = launch_prep(a.dim, a.refs, nullptr, a.n_refs, ref_pad, perm_a, perm_c, 1, a.n_positive, w.b_op, w.norm_refs, nullptr, w.nbs, w.pnorm, nullptr, w.consts, st,
                           nullptr, w.bx_img)) != PHM_OK) return rc;
-    if ((rc = launch_prep(a.cent_pos, nullptr, a.n_cent_pos, cp_pad, 1, 0, 1, 0, w.b_op + ref_pad * KDIM, w.norm_cpos, nullptr, w.nbs + ref_pad,
+    if ((rc = launch_prep(a.dim, a.cent_pos, nullptr, a.n_cent_pos, cp_pad, 1, 0, 1, 0, w.b_op + ref_pad * KDIM, w.norm_cpos, nullptr, w.nbs + ref_pad,
                           w.pnorm + ref_pad, nullptr, w.consts, st, nullptr, w.bx_img + ref_pad * XK)) != PHM_OK) return rc;
-    if ((rc = launch_prep(a.cent_neg, nullptr, a.n_cent_neg, cn_pad, 1, 0, 1, 0, w.b_op + (ref_pad + cp_pad) * KDIM, w.norm_cneg, nullptr,
+    if ((rc = launch_prep(a.dim, a.cent_neg, nullptr, a.n_cent_neg, cn_pad, 1, 0, 1, 0, w.b_op + (ref_pad + cp_pad) * KDIM, w.norm_cneg, nullptr,
                           w.nbs + ref_pad + cp_pad, w.pnorm + ref_pad + cp_pad, nullptr, w.consts, st, nullptr,
                           w.bx_img + (ref_pad + cp_pad) * XK)) != PHM_OK) return rc;
     if (emit) { emit->op = w.a_op; emit->crow = w.crow; emit->cnorm = w.cnorm_points; emit->total = w.row_total; emit->consts = w.consts; }
@@ -1718,7 +1737,9 @@ int score_tc(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st) {
 }
 
 // Query side: operand preparation (unless a producer already filled the QueryEmit buffers), contraction, decision, fallback.
-int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, bool queries_prepared) {
+// W: width of the float64 / count rows
+template <int W>
+static int tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, bool queries_prepared) {
     const int64_t n = a.n_points;
     const int64_t ref_pad = round_up(a.n_refs, BN), cp_pad = round_up(a.n_cent_pos, BN), cn_pad = round_up(a.n_cent_neg, BN);
     const int64_t r_pad = ref_pad + cp_pad + cn_pad;
@@ -1728,7 +1749,7 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     int64_t perm_a, perm_c;
     ref_permutation(a.n_refs, &perm_a, &perm_c);
     if (!queries_prepared &&
-        (rc = launch_prep(a.points, a.point_counts, n, n, 1, 0, 0, 0, w.a_op, w.norm_points, w.cnorm_points, nullptr, nullptr, w.crow, w.consts, st,
+        (rc = launch_prep(W, a.points, a.point_counts, n, n, 1, 0, 0, 0, w.a_op, w.norm_points, w.cnorm_points, nullptr, nullptr, w.crow, w.consts, st,
                           w.row_total)) != PHM_OK) return rc;
 
     CUtensorMap map_a;
@@ -1772,11 +1793,11 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     const bool timed = g_decide_ring.begin(st);
     const bool nb = a.out.nb.any();
     if (a.point_counts) {
-        if (nb) score_decide_kernel<true, true><<<(unsigned)blocks, 256, 0, st>>>(r);
-        else score_decide_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(r);
+        if (nb) score_decide_kernel<true, true, W><<<(unsigned)blocks, 256, 0, st>>>(r);
+        else score_decide_kernel<true, false, W><<<(unsigned)blocks, 256, 0, st>>>(r);
     } else {
-        if (nb) score_decide_kernel<false, true><<<(unsigned)blocks, 256, 0, st>>>(r);
-        else score_decide_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(r);
+        if (nb) score_decide_kernel<false, true, W><<<(unsigned)blocks, 256, 0, st>>>(r);
+        else score_decide_kernel<false, false, W><<<(unsigned)blocks, 256, 0, st>>>(r);
     }
     PHM_LAUNCH_CHECK();
     if (timed) g_decide_ring.end(st);
@@ -1810,7 +1831,7 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
         ld.out = a.out;
         ld.fallback_rows = w.fallback_rows; ld.fallback_count = w.fallback_count;
         ld.rows_listed = w.rows_listed;
-        score_list_decide_kernel<<<sm_count() * 2, 256, 0, st>>>(ld);
+        score_list_decide_kernel<W><<<sm_count() * 2, 256, 0, st>>>(ld);
         PHM_LAUNCH_CHECK();
     }
 
@@ -1823,12 +1844,16 @@ int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t 
     f.out = a.out;
     f.parts = w.fb_parts; f.tickets = w.fb_tickets;
     PHM_CUDA_CHECK(cudaMemsetAsync(w.fb_tickets, 0, sizeof(unsigned int) * FB_GRID, st));
-    score_fallback_kernel<<<FB_GRID, 256, 0, st>>>(f);                 // few rows: column slices across CTAs
+    score_fallback_kernel<W><<<FB_GRID, 256, 0, st>>>(f);              // few rows: column slices across CTAs
     PHM_LAUNCH_CHECK();
-    PHM_CUDA_CHECK(cudaFuncSetAttribute(score_fallback_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FBB_SMEM));
-    score_fallback_blocked_kernel<<<sm_count(), 256, FBB_SMEM, st>>>(f);   // many rows: 32 per CTA share the reference stream
+    PHM_CUDA_CHECK(cudaFuncSetAttribute(score_fallback_blocked_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, FBB_SMEM<W>));
+    score_fallback_blocked_kernel<W><<<sm_count(), 256, FBB_SMEM<W>, st>>>(f);   // many rows: 32 per CTA share the reference stream
     PHM_LAUNCH_CHECK();
     return PHM_OK;
+}
+
+int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, bool queries_prepared) {
+    return a.dim == CANON_DIM ? tc_finish<CANON_DIM>(a, ws, ws_bytes, st, queries_prepared) : tc_finish<KDIM>(a, ws, ws_bytes, st, queries_prepared);
 }
 
 // statistics of the last score_tc call on this workspace

@@ -197,6 +197,29 @@ def normalize_counts(counts):
     return ops.normalize_rows_cuda(torch.from_numpy(as_f64).to("cuda")).cpu().numpy()
 
 
+def canonical_fold(counts, kmer_length):
+    """Folds every k-mer together with its reverse complement: [..., 4^k] -> [..., 136 / 512 / 2080 ...] for k = 4 / 5 / 6, the bins
+    and order of the canonical counter (canon[min(j, rc(j))] += count[j], representatives ascending).  A sequence and its reverse
+    complement have the same folded row.  int64 for integer input (exact below 2^53), float64 otherwise; the row total is kept, so
+    normalize_counts of the folded counts equals the fold of the normalised ones up to rounding."""
+    import torch
+    from . import ops, _lib
+    _lib.require_cuda()
+    arr = np.asarray(counts)
+    if arr.shape[-1:] != (4 ** int(kmer_length),):
+        raise ValueError("rows of %d bins cannot be folded at k = %d (needs %d)" % (arr.shape[-1] if arr.ndim else 0, kmer_length,
+                                                                                   4 ** int(kmer_length)))
+    integer = arr.dtype.kind in "iub"
+    rows = np.ascontiguousarray(arr.reshape(-1, arr.shape[-1]), dtype=np.float64)
+    bins = ops.num_bins(kmer_length, canonical=True)
+    if rows.shape[0] == 0:
+        folded = np.zeros((0, bins))
+    else:
+        folded = ops.canonical_fold_cuda(torch.from_numpy(rows).to("cuda"), kmer_length).cpu().numpy()
+    folded = folded.reshape(arr.shape[:-1] + (bins,))
+    return folded.astype(np.int64) if integer else folded
+
+
 def kmers(k, symbols=DNA):
     """scripts/kmer.py:224.  All k-mers in bin order."""
     out = [""]

@@ -111,6 +111,16 @@ def count_packed_cuda(codes, valid, offsets, k, canonical=False, counts=True, fr
     return out_counts, out_freq
 
 
+def canonical_fold_cuda(rows, k):
+    """Canonical fold of rows that already exist (phm_canonical_fold): float64[n, 4^k] -> float64[n, num_bins(k, canonical=True)], the
+    bins and order of count_cuda(..., canonical=True).  Integer-valued rows below 2^53 fold exactly."""
+    lib = _lib.require_cuda()
+    rows = _check(rows, "rows", torch.float64, 4 ** int(k) if 1 <= int(k) <= 6 else None)
+    out = torch.empty((rows.shape[0], num_bins(k, canonical=True)), dtype=torch.float64, device="cuda")
+    check(lib.phm_canonical_fold(ptr(rows), rows.shape[0], int(k), ptr(out), stream_ptr()))
+    return out
+
+
 def normalize_cuda(counts):
     """kmer.normalize_counts on the device: int32/uint32[n, bins] -> float64[n, bins]."""
     lib = _lib.require_cuda()
@@ -232,7 +242,8 @@ score_path_option = 0
 
 
 def set_score_path(path):
-    """'auto' (tensor cores when the shape allows), 'exact' (exhaustive float64), 'tc' (tensor cores or error)."""
+    """'auto' (tensor cores when the shape allows; at width 136 for count rows only), 'exact' (exhaustive float64), 'tc' (tensor
+    cores or error)."""
     global score_path_option
     score_path_option = {"auto": 0, "exact": 1, "tc": 2}[path]
     _lib.set_option("score_path", score_path_option)

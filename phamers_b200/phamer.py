@@ -47,6 +47,9 @@ class phamer_scorer(object):
         self.kmer_length = 4                                 # :77
         self.k_clusters = 86                                 # :78
         self.k_neighbors = 3                                 # :79
+        # strand-independent scoring: references and contigs are folded onto canonical k-mers (a k-mer and its reverse complement
+        # share a bin) before they are normalised, so a contig and its reverse complement get the same score
+        self.canonical = False
         self.scores = None
         # filled by score_neighbors(): per contig the k_neighbors nearest references (ids, 1 = phage / 0 = bacteria, distances)
         # and the nearest phage / bacteria cluster (k-means label, -1 without centroids) with its distance
@@ -61,12 +64,26 @@ class phamer_scorer(object):
         """:110-123.  Reference sets come from feature CSVs (the reference's FASTA fallback is dead code,
         SURVEY.md 8(b)); with no files given the shipped tables are used."""
         if positive_features_file and negative_features_file:
-            self.positive_ids, self.positive_data = fileIO.read_feature_file(positive_features_file, normalize=True)
-            self.negative_ids, self.negative_data = fileIO.read_feature_file(negative_features_file, normalize=True)
+            self.positive_ids, pos = fileIO.read_feature_file(positive_features_file)
+            self.negative_ids, neg = fileIO.read_feature_file(negative_features_file)
         else:
-            pid, pos, nid, neg = references.load_reference_counts()
-            self.positive_ids, self.negative_ids = pid, nid
-            self.positive_data, self.negative_data = kmer.normalize_counts(pos), kmer.normalize_counts(neg)
+            self.positive_ids, pos, self.negative_ids, neg = references.load_reference_counts()
+        self.positive_data, self.negative_data = kmer.normalize_counts(self._features(pos)), kmer.normalize_counts(self._features(neg))
+
+    def _features(self, counts):
+        """Count rows as scored: unchanged, or with self.canonical folded onto canonical k-mers.  In canonical mode rows that are
+        already canonical width are taken as they are; any other width is a ValueError."""
+        if not self.canonical:
+            return counts
+        counts = np.asarray(counts)
+        width = counts.shape[-1] if counts.ndim else 0
+        if width == 4 ** self.kmer_length:
+            return kmer.canonical_fold(counts, self.kmer_length)
+        from . import ops
+        if width == ops.num_bins(self.kmer_length, canonical=True):
+            return counts
+        raise ValueError("canonical scoring at k = %d takes rows of %d (plain) or %d (canonical) k-mer counts, not %d"
+                         % (self.kmer_length, 4 ** self.kmer_length, ops.num_bins(self.kmer_length, canonical=True), width))
 
     def load_data(self, length_requirement=None):
         """:125-142: a features CSV wins over counting the FASTA; freshly counted features are cached next to the
@@ -80,7 +97,7 @@ class phamer_scorer(object):
         else:
             logger.error("No input fasta file or features file. Exiting...")
             raise SystemExit()
-        self.data_points = kmer.normalize_counts(self.data_points)
+        self.data_points = kmer.normalize_counts(self._features(self.data_points))
         if length_requirement is None:
             length_requirement = self.length_requirement
         if length_requirement and self.fasta_file is not None and os.path.exists(self.fasta_file):
@@ -275,6 +292,8 @@ def main(argv=None):
     parser.add_argument("-l", "--length_requirement", type=int, default=5000, help="Sequence length requirement")
     parser.add_argument("-equal", "--equalize_reference", action="store_true", help="Use same number of reference data from each")
     parser.add_argument("-m", "--method", default="combo", help="Learning algorithm name")
+    parser.add_argument("-canonical", "--canonical_kmers", action="store_true",
+                        help="Fold every k-mer with its reverse complement, so that a contig scores the same on either strand")
     parser.add_argument("-neighbors", "--write_neighbors", action="store_true",
                         help="Also write phamer_neighbors.csv: the nearest references and clusters behind each score")
     parser.add_argument("-do_tsne", "--do_tsne", action="store_true", help="(out of scope)")
@@ -285,6 +304,7 @@ def main(argv=None):
     scorer = phamer_scorer()
     decide_files(scorer, args)
     scorer.scoring_method = args.method
+    scorer.canonical = args.canonical_kmers
     scorer.load_reference_data(scorer.positive_features_file, scorer.negative_features_file)
     scorer.load_data(length_requirement=args.length_requirement)
     if args.equalize_reference:
@@ -296,8 +316,9 @@ def main(argv=None):
         scorer.make_neighbors_file(args=args)
     else:
         scorer.scores = scorer.score_points()
-    # the score file's header does not depend on whether neighbours were asked for
-    score_args = argparse.Namespace(**{k: v for k, v in vars(args).items() if k != "write_neighbors"})
+    # the score file's header does not depend on whether neighbours were asked for; canonical scoring is named only when it is on
+    score_args = argparse.Namespace(**{k: v for k, v in vars(args).items()
+                                       if k != "write_neighbors" and (k != "canonical_kmers" or v)})
     scorer.make_summary_file(args=score_args)
     return scorer
 

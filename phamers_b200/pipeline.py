@@ -8,6 +8,10 @@ The whole hot path as one object: contigs in, PhaMers scores out.
 
 Stage by stage this is kmer.count_file -> kmer.normalize_counts -> phamer_scorer.score_points('combo')
 (reference scripts/phamer.py:131,139,194), with the k-mer length fixed at the width of the reference features.
+
+ContigScorer(..., canonical=True) scores canonical 4-mers (each k-mer folded with its reverse complement, 136 bins), so a contig
+and its reverse complement get the same score: references are 136 wide, contigs are counted with PHM_COUNT_CANONICAL and scored
+from the counts.
 """
 import numpy as np
 import torch
@@ -17,14 +21,17 @@ from . import _lib, ops, references
 
 class ContigScorer(object):
     def __init__(self, positive=None, negative=None, k_clusters=86, k_neighbors=3, kmer_length=4, centroids=None,
-                 equalize=True):
+                 equalize=True, canonical=False):
         _lib.require_cuda()
         if positive is None or negative is None:
-            positive, negative = references.load_reference_features(equalize=equalize)
+            positive, negative = references.load_reference_features(equalize=equalize, canonical=canonical)
         positive = np.ascontiguousarray(positive, dtype=np.float64)
         negative = np.ascontiguousarray(negative, dtype=np.float64)
-        if positive.shape[1] != 4 ** kmer_length or negative.shape[1] != 4 ** kmer_length:
-            raise ValueError("reference features are %d wide, k = %d needs %d" % (positive.shape[1], kmer_length, 4 ** kmer_length))
+        width = ops.num_bins(kmer_length, canonical)
+        if positive.shape[1] != width or negative.shape[1] != width:
+            raise ValueError("reference features are %d wide, k = %d%s needs %d"
+                             % (positive.shape[1], kmer_length, " canonical" if canonical else "", width))
+        self.canonical = canonical
         if centroids is None:
             centroids = references.reference_centroids(positive, negative, k_clusters)
         self.kmer_length = kmer_length
@@ -42,9 +49,16 @@ class ContigScorer(object):
     def score_device(self, seq, offsets, method="combo", return_counts=True):
         # one library call: the histogram kernel also emits the scorer's query operands, the scorer forms count / row total
         # wherever it needs an exact feature; the float64 feature matrix is never written
-        counts, knn, kmeans, combo = ops.count_score_cuda(seq, offsets, self.refs, self.n_positive, self.cent_pos, self.cent_neg,
-                                                          self.k_neighbors)
+        counts, knn, kmeans, combo = self._count_score(seq, offsets)
         return counts, {"knn": knn, "kmeans": kmeans, "combo": combo}[method]
+
+    def _count_score(self, seq, offsets, out_counts=None, out=None):
+        if not self.canonical:
+            return ops.count_score_cuda(seq, offsets, self.refs, self.n_positive, self.cent_pos, self.cent_neg, self.k_neighbors,
+                                        out_counts=out_counts, out=out)
+        # canonical counts, then phm_score_counts on them (the fused count + score call emits plain 256-wide operands only)
+        counts, _ = ops.count_cuda(seq, offsets, self.kmer_length, canonical=True, out_counts=out_counts)
+        return (counts,) + ops.score_cuda(counts, self.refs, self.n_positive, self.cent_pos, self.cent_neg, self.k_neighbors, out=out)
 
     # -- host buffers -----------------------------------------------------------------------------------
     HOST_CHUNKS = 8                    # upload / compute pipeline depth of score_host
@@ -77,7 +91,7 @@ class ContigScorer(object):
         scores = torch.empty((n,), dtype=torch.float64, device="cuda")
         widest = int(np.max(np.diff(cuts)))
         if self._chunk_counts is None or self._chunk_counts.shape[0] < widest:
-            self._chunk_counts = torch.empty((widest, 256), dtype=torch.int32, device="cuda")
+            self._chunk_counts = torch.empty((widest, self.refs.shape[1]), dtype=torch.int32, device="cuda")
         self._copy_stream.wait_stream(main)                                  # the staging buffer may still be read by an earlier call
         uploads, place = [], 0
         for lo, hi in zip(cuts[:-1], cuts[1:]):
@@ -93,8 +107,7 @@ class ContigScorer(object):
         for lo, hi, b0, dst, done in uploads:
             main.wait_event(done)
             part = [torch.empty((hi - lo,), dtype=torch.float64, device="cuda") if i != key else scores[lo:hi] for i in range(3)]
-            ops.count_score_cuda(dst, d_off[lo:hi + 1] - b0, self.refs, self.n_positive, self.cent_pos, self.cent_neg, self.k_neighbors,
-                                 out_counts=self._chunk_counts[:hi - lo], out=tuple(part))
+            self._count_score(dst, d_off[lo:hi + 1] - b0, out_counts=self._chunk_counts[:hi - lo], out=tuple(part))
         out = self._host_out[:n]
         out.copy_(scores, non_blocking=True)
         main.synchronize()

@@ -28,14 +28,17 @@ def load_reference_counts():
             z["negative_ids"], z["negative_counts"].astype(np.int64))
 
 
-def load_reference_features(equalize=True):
+def load_reference_features(equalize=True, canonical=False):
     """Normalised reference features as phamer.load_data builds them (scripts/phamer.py:112,119: read_feature_file(...,
-    normalize=True)); equalize truncates both to min(nP, nN) rows (scripts/phamer.py:159-175)."""
+    normalize=True)); equalize truncates both to min(nP, nN) rows (scripts/phamer.py:159-175).  canonical: the counts are folded
+    with their reverse complements (136 bins) before they are normalised."""
     from . import kmer
     _, pos, _, neg = load_reference_counts()
     if equalize:
         n = min(len(pos), len(neg))
         pos, neg = pos[:n], neg[:n]
+    if canonical:
+        pos, neg = kmer.canonical_fold(pos, 4), kmer.canonical_fold(neg, 4)
     return kmer.normalize_counts(pos), kmer.normalize_counts(neg)
 
 
