@@ -95,6 +95,31 @@ int phm_kmer_count(const uint8_t *d_seq, const int64_t *d_offsets, int64_t n_con
                    uint32_t *d_counts, double *d_freq,
                    void *d_workspace, size_t workspace_bytes, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Sliding windows: the same histogram over overlapping windows of every record, to find where in a long sequence (a prophage in a
+ * bacterial contig, a chimeric assembly) the phage-like part lies.  Coordinates are 0-based, half-open, relative to the record.
+ * For a record of length L, window w >= 1 and step s >= 1: one window [0, L) when L <= w (L = 0 included); otherwise [j s, j s + w)
+ * for j = 0, 1, ... while j s + w <= L, then [L - w, L) when the last of those ends before L -- 1 + ceil((L - w) / s) windows, each
+ * w long, numbered in ascending start order, records in order.  A window's counts are exactly phm_kmer_count's counts of the range
+ * (k-mers wholly inside it; bytes that are not symbols void the k-mers they touch); a window with none gets a NaN feature row.
+ *
+ *   phm_window_offsets      d_window_offsets int64[n_records + 1]: [0] = 0, record r owns windows [wo[r], wo[r + 1]).
+ *   phm_kmer_count_windows  counts the windows [first_window, first_window + n_windows) into rows 0 .. n_windows - 1 of d_counts /
+ *                           d_freq (phm_kmer_count's outputs and flags; PHM_COUNT_NAIVE is not accepted), and writes each window's
+ *                           (start, end) relative to its record to d_spans[2 i], [2 i + 1] (may be NULL).  The workspace
+ *                           (phm_kmer_count_windows_workspace_bytes) holds one 32-byte work item per window, or w / 65 536 of them
+ *                           for windows of 131 072 bases and more (counted in tiles); a smaller one is PHM_E_WORKSPACE.  Argument
+ *                           errors are PHM_E_ARG; the slice is checked against wo[n_records], which the call reads from the device
+ *                           (it synchronises `stream` once).  Score the rows with phm_score_counts / phm_score.
+ * ------------------------------------------------------------------------------------------- */
+int phm_window_offsets(const int64_t *d_offsets, int64_t n_records, int64_t window, int64_t step, int64_t *d_window_offsets,
+                       void *stream);
+size_t phm_kmer_count_windows_workspace_bytes(int64_t n_windows, int64_t window, int k, uint32_t flags);
+int phm_kmer_count_windows(const uint8_t *d_seq, const int64_t *d_offsets, int64_t n_records, const int64_t *d_window_offsets,
+                           int64_t window, int64_t step, int64_t first_window, int64_t n_windows, int k, uint32_t flags,
+                           uint32_t *d_counts, double *d_freq, int64_t *d_spans,
+                           void *d_workspace, size_t workspace_bytes, void *stream);
+
 /* Same histogram from the packed form produced by phm_pack_fasta (multi-k passes over one pack). */
 int phm_kmer_count_packed(const uint32_t *d_codes, const uint32_t *d_valid, const int64_t *d_offsets,
                           int64_t n_contigs, int k, uint32_t flags, uint32_t *d_counts, double *d_freq,

@@ -767,6 +767,141 @@ __global__ void __launch_bounds__(256) hist_finish_kernel(const __grid_constant_
 }
 
 // --------------------------------------------------------------------------------------------------
+// sliding windows (phm_window_offsets, phm_kmer_count_windows): every window is one work item of the list above
+// --------------------------------------------------------------------------------------------------
+// A record of length L has one window [0, L) when L <= w, else the windows [j s, j s + w) while j s + w <= L, plus [L - w, L) when
+// the last of those ends before L: 1 + ceil((L - w) / s) windows, each exactly w long.  The histogram kernel counts any range into any
+// row, so a window call only needs its own planning pass: window_plan_kernel writes one list entry per window of the slice (row =
+// index in the slice), in window order, and the unchanged kmer_hist_kernel / hist_finish_kernel take the list from there.
+__host__ __device__ __forceinline__ int64_t windows_of(int64_t len, int64_t w, int64_t s) {
+    return len <= w ? 1 : 2 + (len - w - 1) / s;                        // 1 + ceil((len - w) / s) without overflow for any s
+}
+
+// Prefix sum of the window counts in three passes that need no scratch memory beyond the output: tiles of WO_TILE records scanned
+// locally (window_offsets_kernel), the tiles' last entries scanned in place by one block (window_offsets_carry_kernel), then every
+// other entry of a tile adds the finished last entry of the tile before it (window_offsets_add_kernel).
+constexpr int WO_PER_THREAD = 8;
+constexpr int WO_TILE = 256 * WO_PER_THREAD;
+
+__global__ void __launch_bounds__(256) window_offsets_kernel(const int64_t *__restrict__ off, int64_t n, int64_t w, int64_t s,
+                                                             int64_t *__restrict__ wo) {
+    __shared__ long long s_warp[8];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t r0 = (int64_t)blockIdx.x * WO_TILE + (int64_t)threadIdx.x * WO_PER_THREAD;
+    int64_t cnt[WO_PER_THREAD], mine = 0;
+#pragma unroll
+    for (int j = 0; j < WO_PER_THREAD; ++j) {
+        const int64_t r = r0 + j;
+        cnt[j] = r < n ? windows_of(off[r + 1] - off[r], w, s) : 0;
+        mine += cnt[j];
+    }
+    long long incl = mine;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const long long up = __shfl_up_sync(FULL, incl, o);
+        if (lane >= o) incl += up;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    int64_t run = incl - mine;
+    for (int v = 0; v < warp; ++v) run += s_warp[v];
+#pragma unroll
+    for (int j = 0; j < WO_PER_THREAD; ++j) {
+        run += cnt[j];
+        if (r0 + j < n) wo[r0 + j + 1] = run;
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) wo[0] = 0;
+}
+
+__global__ void __launch_bounds__(1024) window_offsets_carry_kernel(int64_t n, int64_t *wo) {
+    __shared__ long long s_warp[32];
+    __shared__ long long s_carry;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t tiles = (n + WO_TILE - 1) / WO_TILE;
+    if (threadIdx.x == 0) s_carry = 0;
+    __syncthreads();
+    for (int64_t t0 = 0; t0 < tiles; t0 += 1024) {
+        const int64_t t = t0 + threadIdx.x;
+        const int64_t at = t < tiles ? ((t + 1) * WO_TILE < n ? (t + 1) * WO_TILE : n) : 0;   // entry of the tile's last record
+        const long long v = t < tiles ? wo[at] : 0;
+        long long incl = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const long long up = __shfl_up_sync(FULL, incl, o);
+            if (lane >= o) incl += up;
+        }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        long long before = s_carry;
+        for (int q = 0; q < warp; ++q) before += s_warp[q];
+        if (t < tiles) wo[at] = before + incl;
+        __syncthreads();
+        if (threadIdx.x == 1023) s_carry = before + incl;
+        __syncthreads();
+    }
+}
+
+__global__ void __launch_bounds__(256) window_offsets_add_kernel(int64_t n, int64_t *wo) {
+    for (int64_t r = (int64_t)WO_TILE + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t tile_end = (r / WO_TILE + 1) * WO_TILE;
+        if (r + 1 == tile_end || r + 1 == n) continue;                       // the tile's last entry is already final
+        wo[r + 1] += wo[(r / WO_TILE) * WO_TILE];
+    }
+}
+
+// One thread per window of the slice [first, first + n): its record by binary search in the window offsets, its range, and the list
+// entries of its row.  Every window gets `per` slots (the tiles of a w-long window): a window of SPLIT_MIN bases and more is cut by
+// the rule of hist_plan_fill_kernel (its row zeroed, first tile flagged for hist_finish_kernel); a shorter one (only the single window
+// of a record shorter than w can be) fills its first slot and pads the others with empty tiles, which count nothing and add nothing.
+// The header makes the histogram kernel take the list: `need` in the class the host chose (class 0 when windows are tiled, the only
+// class hist_finish_kernel walks) and n_split != 0.
+__global__ void __launch_bounds__(256) window_plan_kernel(const int64_t *__restrict__ off, const int64_t *__restrict__ wo, int64_t n_records,
+                                                          int64_t w, int64_t s, int64_t first, int64_t n, int k, uint32_t per, int cls,
+                                                          PlanHeader *plan, PlanEntry *entries, uint32_t *counts, double *freq, int out_bins,
+                                                          int64_t *spans) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        plan->need[cls] = (unsigned long long)n * per;
+        plan->n_split = 1ull;
+    }
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t g = first + i;
+        int64_t lo = 0, hi = n_records;                                     // wo[lo] <= g < wo[hi]
+        while (hi - lo > 1) {
+            const int64_t mid = lo + ((hi - lo) >> 1);
+            if (wo[mid] <= g) lo = mid; else hi = mid;
+        }
+        const int64_t rs = off[lo], len = off[lo + 1] - rs, j = g - wo[lo];
+        int64_t a = 0, b = len;
+        if (len > w) {
+            a = (j + 1 < windows_of(len, w, s)) ? j * s : len - w;
+            b = a + w;
+        }
+        if (spans) { spans[2 * i] = a; spans[2 * i + 1] = b; }
+        const int64_t c_start = rs + a, c_end = rs + b;
+        const uint32_t m = plan_tiles(b - a);
+        for (uint32_t t = 0; t < per; ++t) {
+            PlanEntry e;
+            e.contig = i;
+            e.pad = 0u;
+            if (t >= m) {
+                e.start = c_start; e.end = c_start; e.flags = ITEM_TILE;
+            } else if (m == 1u) {
+                e.start = c_start; e.end = c_end; e.flags = 0u;
+            } else {
+                e.start = (t == 0) ? c_start : ((c_start + (int64_t)t * TILE) & ~(int64_t)511);
+                e.end = (t + 1 < m) ? (((c_start + (int64_t)(t + 1) * TILE) & ~(int64_t)511) + (k - 1)) : c_end;
+                e.flags = ITEM_TILE | (t == 0 ? ITEM_FIRST_TILE : 0u);
+            }
+            entries[(unsigned long long)i * per + t] = e;
+        }
+        if (m > 1u) {
+            uint32_t *row = split_row(counts, freq, i, out_bins);
+            for (int q = 0; q < out_bins; ++q) row[q] = 0u;
+        }
+    }
+}
+
+// --------------------------------------------------------------------------------------------------
 // canonical look-up tables: rc[y] and compact[y] = rank of min(y, rc(y)) among the self-representing bins
 // --------------------------------------------------------------------------------------------------
 __global__ void canonical_lut_kernel(int k, uint16_t *rc_lut, uint16_t *compact_lut, uint16_t *canon_lut) {
@@ -1091,10 +1226,31 @@ static int launch_plan(const int64_t *off, int64_t n, int k, const CountWorkspac
     return PHM_OK;
 }
 
+// a window call (phm_kmer_count_windows): the slice [first, first + n) of the windows of the records, rows 0 .. n - 1
+struct WindowSlice {
+    const int64_t *wo; int64_t n_records, window, step, first, n;
+    int64_t *spans;
+};
+
+static int launch_window_plan(const int64_t *off, const WindowSlice &ws, int k, const CountWorkspace &w, uint32_t *counts,
+                              double *freq, int out_bins, cudaStream_t st) {
+    const uint32_t per = plan_tiles(ws.window);
+    int64_t blocks = (ws.n + 255) / 256;
+    const int64_t cap = (int64_t)sm_count() * 8;
+    if (blocks > cap) blocks = cap;
+    window_plan_kernel<<<(unsigned)blocks, 256, 0, st>>>(off, ws.wo, ws.n_records, ws.window, ws.step, ws.first, ws.n, k, per,
+                                                         per > 1u ? 0 : N_CLASS - 1, w.plan, w.entries, counts, freq, out_bins,
+                                                         ws.spans);
+    PHM_LAUNCH_CHECK();
+    return PHM_OK;
+}
+
+// win != nullptr: count the windows of a slice instead of whole records (`n` is then the slice's window count); windows always
+// take the list, whatever option hist_plan says, because no offset table describes them
 template <int K, int STRIDE, int WARPS, bool EMIT = false, bool SWZ = false, int STAGES = 0>
 static int launch_hist(const uint8_t *seq, const int64_t *off, int64_t n, uint32_t *counts, double *freq,
                        const uint16_t *rc, const uint16_t *compact, int out_bins, const CountWorkspace &w,
-                       cudaStream_t st, tc::QueryEmit emit = tc::QueryEmit()) {
+                       cudaStream_t st, tc::QueryEmit emit = tc::QueryEmit(), const WindowSlice *win = nullptr) {
     using Cfg = HistCfg<K, STRIDE>;
     const size_t smem = (size_t)WARPS * Cfg::WARP_BYTES + Cfg::ALIGN + (size_t)WARPS * STAGES * (STAGE_BYTES + 8);
     auto kern = kmer_hist_kernel<K, STRIDE, WARPS, EMIT, SWZ, STAGES>;
@@ -1106,15 +1262,19 @@ static int launch_hist(const uint8_t *seq, const int64_t *off, int64_t n, uint32
     job.seq = seq; job.off = off; job.n_contigs = n; job.counts = counts; job.freq = freq;
     job.rc_lut = rc; job.canon_lut = compact; job.out_bins = out_bins;
     job.plan = w.plan; job.entries = w.entries;
-    job.cap = hist_plan ? w.cap : 0ull;
+    job.cap = (hist_plan || win) ? w.cap : 0ull;
     const bool timed = g_hist_ring.begin(st);           // the bracket covers the whole counting stage: planning passes, histogram, finish
-    if (job.cap > 0) {
+    if (win) {
+        const int rc_plan = launch_window_plan(off, *win, K, w, counts, freq, out_bins, st);
+        if (rc_plan != PHM_OK) return rc_plan;
+    } else if (job.cap > 0) {
         const int rc_plan = launch_plan(off, n, K, w, counts, freq, out_bins, st);
         if (rc_plan != PHM_OK) return rc_plan;
     }
     constexpr int per_item = (K >= 6) ? 4 : 1;
     int64_t grid = (int64_t)per_sm * sm_count();
-    const int64_t items = (n + (int64_t)job.cap + per_item - 1) / per_item;          // upper bound: the list can hold at most cap items
+    const int64_t items = win ? (n * (int64_t)plan_tiles(win->window) + per_item - 1) / per_item          // the window list, exactly
+                              : (n + (int64_t)job.cap + per_item - 1) / per_item;  // upper bound: the list can hold at most cap items
     const int64_t need = (items + WARPS - 1) / WARPS;
     if (grid > need) grid = need < 1 ? 1 : need;
     kern<<<(unsigned)grid, WARPS * 32, smem, st>>>(job, emit);
@@ -1208,6 +1368,40 @@ static int prepare_count(int64_t n_contigs, int k, uint32_t flags, void *ws, siz
     return PHM_OK;
 }
 
+// the histogram variant of k (and of the tuning options), for a call over records or over the windows of a slice
+static int dispatch_hist(int k, const uint8_t *seq, const int64_t *off, int64_t n, uint32_t *counts, double *freq, const uint16_t *rc,
+                         const uint16_t *canon, int out_bins, const CountWorkspace &w, cudaStream_t st, const WindowSlice *win) {
+    switch (k) {
+        case 1: return launch_hist<1, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+        case 2: return launch_hist<2, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+        case 3: return launch_hist<3, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+        case 4:
+            if (hist_stride_for_k4 == 2)
+                return hist_tma ? launch_hist<4, 2, 8, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
+                                : launch_hist<4, 2, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+            return launch_hist<4, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+        case 5:
+            if ((hist_stride_for_k5 == 2 || (hist_stride_for_k5 == 0 && !rc)) && hist_warps_k5 == 18)
+                return launch_hist<5, 2, 18>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+            if (hist_stride_for_k5 == 2 || (hist_stride_for_k5 == 0 && !rc))
+                return launch_hist<5, 2, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+            if (rc && hist_canonical_swizzle)
+                return hist_tma ? launch_hist<5, 1, 8, false, true, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
+                                : launch_hist<5, 1, 8, false, true>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+            return hist_tma ? launch_hist<5, 1, 8, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
+                            : launch_hist<5, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+        case 6:
+            if (hist_warps_k6 == 4)
+                return launch_hist<6, 1, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+            if (rc && hist_canonical_swizzle)
+                return hist_tma ? launch_hist<6, 1, 11, false, true, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
+                                : launch_hist<6, 1, 13, false, true>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+            return hist_tma ? launch_hist<6, 1, 11, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
+                            : launch_hist<6, 1, 13>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+    }
+    return PHM_E_ARG;
+}
+
 extern "C" int phm_kmer_count(const uint8_t *d_seq, const int64_t *d_offsets, int64_t n_contigs, int k, uint32_t flags,
                               uint32_t *d_counts, double *d_freq, void *d_workspace, size_t workspace_bytes, void *stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1230,35 +1424,78 @@ extern "C" int phm_kmer_count(const uint8_t *d_seq, const int64_t *d_offsets, in
         if (d_freq) return phm_normalize_counts(d_counts, n_contigs, out_bins, d_freq, stream);
         return PHM_OK;
     }
-    switch (k) {
-        case 1: return launch_hist<1, 1, 8>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-        case 2: return launch_hist<2, 1, 8>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-        case 3: return launch_hist<3, 1, 8>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-        case 4:
-            if (hist_stride_for_k4 == 2)
-                return hist_tma ? launch_hist<4, 2, 8, false, false, 4>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st)
-                                : launch_hist<4, 2, 8>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-            return launch_hist<4, 1, 8>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-        case 5:
-            if ((hist_stride_for_k5 == 2 || (hist_stride_for_k5 == 0 && !rc)) && hist_warps_k5 == 18)
-                return launch_hist<5, 2, 18>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-            if (hist_stride_for_k5 == 2 || (hist_stride_for_k5 == 0 && !rc))
-                return launch_hist<5, 2, 8>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-            if (rc && hist_canonical_swizzle)
-                return hist_tma ? launch_hist<5, 1, 8, false, true, 4>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st)
-                                : launch_hist<5, 1, 8, false, true>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-            return hist_tma ? launch_hist<5, 1, 8, false, false, 4>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st)
-                            : launch_hist<5, 1, 8>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-        case 6:
-            if (hist_warps_k6 == 4)
-                return launch_hist<6, 1, 4>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-            if (rc && hist_canonical_swizzle)
-                return hist_tma ? launch_hist<6, 1, 11, false, true, 4>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st)
-                                : launch_hist<6, 1, 13, false, true>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
-            return hist_tma ? launch_hist<6, 1, 11, false, false, 4>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st)
-                            : launch_hist<6, 1, 13>(d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st);
+    return dispatch_hist(k, d_seq, d_offsets, n_contigs, d_counts, d_freq, rc, canon, out_bins, w, st, nullptr);
+}
+
+extern "C" int phm_window_offsets(const int64_t *d_offsets, int64_t n_records, int64_t window, int64_t step, int64_t *d_window_offsets,
+                                  void *stream) {
+    PHM_REQUIRE(window >= 1 && step >= 1, "window and step must be >= 1");
+    PHM_REQUIRE(n_records >= 0, "n_records must be >= 0");
+    PHM_REQUIRE(d_window_offsets != nullptr && (d_offsets != nullptr || n_records == 0), "null pointer");
+    PHM_REQUIRE(((reinterpret_cast<uintptr_t>(d_offsets) | reinterpret_cast<uintptr_t>(d_window_offsets)) & 7u) == 0,
+                "offsets must be 8-byte aligned");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (n_records == 0) {
+        PHM_CUDA_CHECK(cudaMemsetAsync(d_window_offsets, 0, sizeof(int64_t), st));
+        return PHM_OK;
     }
-    return PHM_E_ARG;
+    const int64_t tiles = (n_records + WO_TILE - 1) / WO_TILE;
+    window_offsets_kernel<<<(unsigned)tiles, 256, 0, st>>>(d_offsets, n_records, window, step, d_window_offsets);
+    PHM_LAUNCH_CHECK();
+    if (tiles > 1) {
+        window_offsets_carry_kernel<<<1, 1024, 0, st>>>(n_records, d_window_offsets);
+        PHM_LAUNCH_CHECK();
+        int64_t blocks = (n_records - WO_TILE + 255) / 256;
+        if (blocks > (int64_t)sm_count() * 16) blocks = (int64_t)sm_count() * 16;
+        window_offsets_add_kernel<<<(unsigned)blocks, 256, 0, st>>>(n_records, d_window_offsets);
+        PHM_LAUNCH_CHECK();
+    }
+    return PHM_OK;
+}
+
+extern "C" size_t phm_kmer_count_windows_workspace_bytes(int64_t n_windows, int64_t window, int, uint32_t) {
+    const size_t slots = (size_t)(n_windows > 0 ? n_windows : 0) * plan_tiles(window > 0 ? window : 1);
+    return kCountWorkspaceFixed + ((slots * sizeof(PlanEntry) + 255) & ~(size_t)255);
+}
+
+extern "C" int phm_kmer_count_windows(const uint8_t *d_seq, const int64_t *d_offsets, int64_t n_records, const int64_t *d_window_offsets,
+                                      int64_t window, int64_t step, int64_t first_window, int64_t n_windows, int k, uint32_t flags,
+                                      uint32_t *d_counts, double *d_freq, int64_t *d_spans, void *d_workspace, size_t workspace_bytes,
+                                      void *stream) {
+    // every argument is checked before the device is touched
+    PHM_REQUIRE(k >= 1 && k <= 6, "k must be 1..6");
+    PHM_REQUIRE(window >= 1 && step >= 1, "window and step must be >= 1");
+    PHM_REQUIRE((flags & ~PHM_COUNT_CANONICAL) == 0u, "flags: PHM_COUNT_CANONICAL is the only flag of a window call");
+    PHM_REQUIRE(n_records >= 0, "n_records must be >= 0");
+    PHM_REQUIRE(first_window >= 0 && n_windows >= 0, "first_window and n_windows must be >= 0");
+    PHM_REQUIRE(n_records > 0 || first_window + n_windows == 0, "the slice lies outside the windows");
+    if (n_windows == 0) return PHM_OK;
+    PHM_REQUIRE(d_seq != nullptr && d_offsets != nullptr && d_window_offsets != nullptr && d_workspace != nullptr, "null pointer");
+    PHM_REQUIRE(d_counts != nullptr || d_freq != nullptr, "both outputs are null");
+    PHM_REQUIRE((reinterpret_cast<uintptr_t>(d_seq) & 15u) == 0, "d_seq must be 16-byte aligned");
+    PHM_REQUIRE(((reinterpret_cast<uintptr_t>(d_offsets) | reinterpret_cast<uintptr_t>(d_window_offsets) |
+                  reinterpret_cast<uintptr_t>(d_freq) | reinterpret_cast<uintptr_t>(d_spans)) & 7u) == 0 &&
+                (reinterpret_cast<uintptr_t>(d_counts) & 3u) == 0, "misaligned pointer");
+    const unsigned long long slots = (unsigned long long)n_windows * plan_tiles(window);
+    if (workspace_bytes < kCountWorkspaceFixed || (workspace_bytes - kCountWorkspaceFixed) / sizeof(PlanEntry) < slots) {
+        set_error("workspace too small for %lld windows: %zu < %zu bytes", (long long)n_windows, workspace_bytes,
+                  phm_kmer_count_windows_workspace_bytes(n_windows, window, k, flags));
+        return PHM_E_WORKSPACE;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    int64_t total = 0;                                                  // the slice must lie inside [0, total windows)
+    PHM_CUDA_CHECK(cudaMemcpyAsync(&total, d_window_offsets + n_records, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    PHM_CUDA_CHECK(cudaStreamSynchronize(st));
+    if (first_window > total || n_windows > total - first_window) {
+        set_error("invalid argument: windows [%lld, %lld) lie outside the %lld windows of the records", (long long)first_window,
+                  (long long)(first_window + n_windows), (long long)total);
+        return PHM_E_ARG;
+    }
+    CountWorkspace w; const uint16_t *rc, *compact; int out_bins;
+    int rcode = prepare_count(n_windows, k, flags, d_workspace, workspace_bytes, d_offsets, &w, &rc, &compact, &out_bins, st);
+    if (rcode != PHM_OK) return rcode;
+    const WindowSlice win{d_window_offsets, n_records, window, step, first_window, n_windows, d_spans};
+    return dispatch_hist(k, d_seq, d_offsets, n_windows, d_counts, d_freq, rc, rc ? w.canon_lut : nullptr, out_bins, w, st, &win);
 }
 
 extern "C" int phm_kmer_count_packed(const uint32_t *d_codes, const uint32_t *d_valid, const int64_t *d_offsets,

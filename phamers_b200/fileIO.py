@@ -6,6 +6,8 @@ scripts/id_parser.py the path touches:
     feature CSV     read_feature_file :134, save_counts :169  ('#' header lines, then id,c0,c1,...)
     score CSV       save_phamer_scores :241, read_phamer_output :256  ('# ' header, then 'id, score')
     neighbour CSV   save_phamer_neighbors, read_phamer_neighbors  ('# ' header, then per contig its nearest references and clusters)
+    window CSV      save_phamer_windows, read_phamer_windows  ('# ' header, then 'id, start, end, score' per window)
+    region CSV      save_phamer_regions, read_phamer_regions  ('# ' header, then 'id, start, end, windows, mean_score, max_score')
 
 Host-side only (bytes and text); no arithmetic happens here.
 """
@@ -341,3 +343,60 @@ def read_phamer_neighbors(filename):
     clusters = np.array([[int(r[-4]), int(r[-2])] for r in rows], dtype=np.int64).reshape(n, 2)
     cl_dist = np.array([[float(r[-3]), float(r[-1])] for r in rows], dtype=np.float64).reshape(n, 2)
     return ids, refs, ref_labels, ref_dist, clusters, cl_dist
+
+
+# ----------------------------------------------------------------------------------------------------------
+# window and region CSVs (phamer -window): scores along each contig and the phage-like regions they show
+# ----------------------------------------------------------------------------------------------------------
+def _write_rows(file_name, header, args, columns, rows):
+    if args is not None:
+        header = generate_summary(args, header=header)
+    with open(file_name, "w") as fh:
+        for line in header.split("\n"):
+            fh.write("# " + line + "\n")
+        fh.write("# " + ", ".join(columns) + "\n")
+        for fields in rows:
+            fh.write(", ".join(fields) + "\n")
+
+
+def _read_rows(filename):
+    with open(filename, "r") as fh:
+        return [line.rstrip("\n").split(", ") for line in fh if not line.startswith("#") and line.strip()]
+
+
+def save_phamer_windows(ids, spans, scores, file_name, args=None):
+    """'# '-prefixed header lines (header 'PhaMers window file', then the column names), then one row per window:
+    'id, start, end, score' -- the contig's id, the window's 0-based half-open coordinates in the contig, its score printed by
+    numpy's float64 -> str conversion, which round-trips."""
+    spans = np.asarray(spans, dtype=np.int64).reshape(-1, 2)
+    scores = np.asarray(scores, dtype=np.float64).astype(str)
+    rows = zip(np.asarray(ids).astype(str), spans[:, 0].astype(str), spans[:, 1].astype(str), scores)
+    _write_rows(file_name, "PhaMers window file", args, ["id", "start", "end", "score"], rows)
+
+
+def read_phamer_windows(filename):
+    """The file of save_phamer_windows -> (ids [windows] str, spans int64[windows, 2], scores float64[windows])."""
+    rows = _read_rows(filename)
+    ids = np.array([r[0] for r in rows], dtype=str)
+    spans = np.array([[int(r[1]), int(r[2])] for r in rows], dtype=np.int64).reshape(len(rows), 2)
+    return ids, spans, np.array([float(r[3]) for r in rows], dtype=np.float64)
+
+
+def save_phamer_regions(ids, spans, windows, mean_scores, max_scores, file_name, args=None):
+    """'# '-prefixed header lines (header 'PhaMers region file', then the column names), then one row per region:
+    'id, start, end, windows, mean_score, max_score' -- a region is a maximal run of consecutive windows of one contig that all
+    score >= 0; start / end are those of its first / last window, scores are printed as in save_phamer_windows."""
+    spans = np.asarray(spans, dtype=np.int64).reshape(-1, 2)
+    rows = zip(np.asarray(ids).astype(str), spans[:, 0].astype(str), spans[:, 1].astype(str),
+               np.asarray(windows, dtype=np.int64).astype(str), np.asarray(mean_scores, dtype=np.float64).astype(str),
+               np.asarray(max_scores, dtype=np.float64).astype(str))
+    _write_rows(file_name, "PhaMers region file", args, ["id", "start", "end", "windows", "mean_score", "max_score"], rows)
+
+
+def read_phamer_regions(filename):
+    """The file of save_phamer_regions -> (ids str, spans int64[regions, 2], windows int64, mean_scores float64, max_scores float64)."""
+    rows = _read_rows(filename)
+    ids = np.array([r[0] for r in rows], dtype=str)
+    spans = np.array([[int(r[1]), int(r[2])] for r in rows], dtype=np.int64).reshape(len(rows), 2)
+    return (ids, spans, np.array([int(r[3]) for r in rows], dtype=np.int64), np.array([float(r[4]) for r in rows], dtype=np.float64),
+            np.array([float(r[5]) for r in rows], dtype=np.float64))

@@ -87,6 +87,50 @@ def count_cuda(seq, offsets, k, canonical=False, counts=True, freq=False, naive=
     return (out_counts if counts else None), out_freq
 
 
+def _offsets_cuda(offsets):
+    if not (isinstance(offsets, torch.Tensor) and offsets.is_cuda and offsets.dtype == torch.int64 and offsets.is_contiguous()):
+        raise TypeError("offsets must be a contiguous CUDA int64 tensor")
+    return offsets
+
+
+def window_offsets_cuda(offsets, window, step):
+    """phm_window_offsets: int64[n+1] record offsets -> int64[n+1] window offsets (entry 0 = 0; record r owns windows
+    [wo[r], wo[r+1])).  A record of length L has one window when L <= window, else 1 + ceil((L - window) / step)."""
+    lib = _lib.require_cuda()
+    offsets = _offsets_cuda(offsets)
+    n = offsets.numel() - 1
+    wo = torch.empty((n + 1,), dtype=torch.int64, device="cuda")
+    check(lib.phm_window_offsets(ptr(offsets), n, int(window), int(step), ptr(wo), stream_ptr()))
+    return wo
+
+
+def count_windows_cuda(seq, offsets, window_offsets, window, step, k, first=0, n=None, canonical=False, counts=True, freq=False,
+                       spans=False, out_counts=None):
+    """phm_kmer_count_windows: k-mer counts of the windows [first, first + n) (n = None: to the last window; reading that number
+    synchronises) into rows 0 .. n - 1.  Returns (counts int32[n, bins] or None, freq float64[n, bins] or None, spans int64[n, 2]
+    (start, end relative to the record) or None).  The call reads the total number of windows from the device once, to check the
+    slice."""
+    lib = _lib.require_cuda()
+    seq = _as_u8_cuda(seq)
+    offsets, window_offsets = _offsets_cuda(offsets), _offsets_cuda(window_offsets)
+    n_records = offsets.numel() - 1
+    if window_offsets.numel() != n_records + 1:
+        raise ValueError("window_offsets must have one entry more than there are records")
+    if n is None:
+        n = int(window_offsets[-1].item()) - int(first)
+    if int(first) < 0 or n < 0:
+        raise ValueError("the slice [%d, %d + %d) is not a range of windows" % (int(first), int(first), n))
+    flags = _lib.PHM_COUNT_CANONICAL if canonical else 0
+    bins = num_bins(k, canonical)
+    out_counts = _result(out_counts, (n, bins), torch.int32) if counts else None
+    out_freq = torch.empty((n, bins), dtype=torch.float64, device="cuda") if freq else None
+    out_spans = torch.empty((n, 2), dtype=torch.int64, device="cuda") if spans else None
+    ws = _workspace("count", lib.phm_kmer_count_windows_workspace_bytes(n, int(window), int(k), flags))
+    check(lib.phm_kmer_count_windows(ptr(seq), ptr(offsets), n_records, ptr(window_offsets), int(window), int(step), int(first), int(n),
+                                     int(k), flags, ptr(out_counts), ptr(out_freq), ptr(out_spans), ptr(ws), ws.numel(), stream_ptr()))
+    return out_counts, out_freq, out_spans
+
+
 def pack_cuda(seq):
     """K1.  uint8[n] ASCII -> (codes int32[ceil(n/16)], valid int32[ceil(n/32)])."""
     lib = _lib.require_cuda()

@@ -58,6 +58,18 @@ class phamer_scorer(object):
         self.neighbor_distances = None
         self.nearest_clusters = None
         self.nearest_cluster_distances = None
+        # filled by score_windows(): one entry per window of the contigs kept by the length screen -- the contig's id and its position
+        # in the FASTA, the window's [start, end) in the contig, its score; and by find_regions(): the phage-like regions they show
+        self.screened_length = 0
+        self.window_ids = None
+        self.window_records = None
+        self.window_spans = None
+        self.window_scores = None
+        self.region_ids = None
+        self.region_spans = None
+        self.region_windows = None
+        self.region_mean_scores = None
+        self.region_max_scores = None
 
     # ---- data -------------------------------------------------------------------------------------------
     def load_reference_data(self, positive_features_file=None, negative_features_file=None):
@@ -107,6 +119,7 @@ class phamer_scorer(object):
         """:144-157: keep contigs whose parsed sequence has at least `length_requirement` characters."""
         if length_requirement:
             self.length_requirement = length_requirement
+        self.screened_length = self.length_requirement
         ids, lengths = fileIO.get_fasta_lengths(self.fasta_file)
         long_ids = [ids[i] for i in range(len(ids)) if lengths[i] >= self.length_requirement]
         self.data_points = self.data_points[np.isin(self.data_ids, long_ids)]
@@ -186,6 +199,48 @@ class phamer_scorer(object):
         self.nearest_cluster_distances = cen_d
         return self.scores
 
+    def score_windows(self, window, step=None):
+        """Scores overlapping windows along every contig the length screen kept (all records of the FASTA when no screen ran), with
+        the scorer's references, k-mer length, k_neighbors, method and canonical mode: fills window_ids, window_records (position of
+        the contig in the FASTA), window_spans ([windows, 2], 0-based half-open, in the contig) and window_scores.  A contig of length
+        L has one window [0, L) when L <= window, else windows every `step` bases (default: window) plus one aligned to its end.
+        Needs the FASTA file: features alone say nothing about where in a contig the phage lies."""
+        from . import pipeline
+        if self.fasta_file is None or not os.path.exists(self.fasta_file):
+            raise ValueError("window scores need the FASTA file of the contigs; a features file alone has no positions")
+        if self.scoring_method not in ("knn", "kmeans", "combo"):
+            raise NotImplementedError("scoring method %r is outside the B200 hot path (knn / kmeans / combo only)" % self.scoring_method)
+        pos = np.ascontiguousarray(self.positive_data, dtype=np.float64)
+        neg = np.ascontiguousarray(self.negative_data, dtype=np.float64)
+        scorer = pipeline.ContigScorer(pos, neg, k_clusters=self.k_clusters, k_neighbors=self.k_neighbors, kmer_length=self.kmer_length,
+                                       centroids=references.reference_centroids(pos, neg, self.k_clusters), canonical=self.canonical)
+        self.window_ids, self.window_records, self.window_spans, self.window_scores = scorer.score_windows_fasta(
+            self.fasta_file, int(window), int(step or window), length_requirement=self.screened_length, method=self.scoring_method)
+        return self.window_scores
+
+    def find_regions(self):
+        """Phage-like regions from the window scores (host only): a region is a maximal run of consecutive windows of one contig whose
+        scores are all >= 0 (a NaN window ends a run; a run never crosses contigs).  Fills region_ids, region_spans ([regions, 2]: start
+        of the first window, end of the last), region_windows, region_mean_scores and region_max_scores."""
+        scores = np.asarray(self.window_scores, dtype=np.float64)
+        records = np.asarray(self.window_records, dtype=np.int64)
+        spans = np.asarray(self.window_spans, dtype=np.int64).reshape(-1, 2)
+        hit = scores >= 0
+        opens = hit.copy()
+        opens[1:] &= ~(hit[:-1] & (records[1:] == records[:-1]))
+        first = np.flatnonzero(opens)
+        run = np.cumsum(opens)[hit] - 1                                  # region of every window that scores >= 0
+        windows = np.bincount(run, minlength=len(first)).astype(np.int64)
+        last = first + windows - 1
+        starts = np.concatenate(([0], np.cumsum(windows)[:-1])).astype(np.int64)
+        in_runs = scores[hit]
+        self.region_ids = np.asarray(self.window_ids)[first]
+        self.region_spans = np.stack((spans[first, 0], spans[last, 1]), axis=1).reshape(-1, 2)
+        self.region_windows = windows
+        self.region_mean_scores = np.add.reduceat(in_runs, starts) / windows if len(first) else np.zeros(0)
+        self.region_max_scores = np.maximum.reduceat(in_runs, starts) if len(first) else np.zeros(0)
+        return self.region_spans
+
     def knn_score_points(self):
         return self._with_method("knn")
 
@@ -234,6 +289,14 @@ class phamer_scorer(object):
         self.phamer_output_filename = self.get_phamer_output_filename()
         fileIO.save_phamer_scores(self.data_ids, self.scores, self.phamer_output_filename, args=args)
 
+    def make_window_files(self, args=None):
+        """<out>/phamer_windows.csv (one row per window) and <out>/phamer_regions.csv (one row per phage-like region)."""
+        self.phamer_windows_filename = os.path.join(self.output_directory, "phamer_windows.csv")
+        self.phamer_regions_filename = os.path.join(self.output_directory, "phamer_regions.csv")
+        fileIO.save_phamer_windows(self.window_ids, self.window_spans, self.window_scores, self.phamer_windows_filename, args=args)
+        fileIO.save_phamer_regions(self.region_ids, self.region_spans, self.region_windows, self.region_mean_scores,
+                                   self.region_max_scores, self.phamer_regions_filename, args=args)
+
     def make_neighbors_file(self, args=None):
         """<out>/phamer_neighbors.csv: the rows of phamer_scores.csv with the references and clusters behind each score."""
         self.phamer_neighbors_filename = os.path.join(self.output_directory, "phamer_neighbors.csv")
@@ -277,7 +340,8 @@ def decide_files(scorer, args):
 def main(argv=None):
     """The reference's command line (scripts/phamer.py:510-599) for the hot path: count the contigs of a FASTA (or read their
     feature CSV), score them against the reference features, write <out>/phamer_scores.csv (and with -neighbors
-    <out>/phamer_neighbors.csv).  t-SNE and plots are out of scope."""
+    <out>/phamer_neighbors.csv; with -window <out>/phamer_windows.csv and <out>/phamer_regions.csv).  t-SNE and plots are out of
+    scope."""
     import argparse
     parser = argparse.ArgumentParser(description="Scores contigs based on feature similarity (B200 path)",
                                      formatter_class=argparse.ArgumentDefaultsHelpFormatter)
@@ -296,13 +360,23 @@ def main(argv=None):
                         help="Fold every k-mer with its reverse complement, so that a contig scores the same on either strand")
     parser.add_argument("-neighbors", "--write_neighbors", action="store_true",
                         help="Also write phamer_neighbors.csv: the nearest references and clusters behind each score")
+    parser.add_argument("-window", "--window_length", type=int,
+                        help="Also score windows of this many bases along each contig: phamer_windows.csv and phamer_regions.csv")
+    parser.add_argument("-step", "--window_step", type=int, help="Bases between window starts (default: the window length)")
     parser.add_argument("-do_tsne", "--do_tsne", action="store_true", help="(out of scope)")
     parser.add_argument("-plot", "--plot_tsne", action="store_true", help="(out of scope)")
     args = parser.parse_args(argv)
     if args.do_tsne or args.plot_tsne:
         raise NotImplementedError("t-SNE and plotting are outside the B200 hot path")
+    if args.window_length is not None and args.window_length < 1:
+        parser.error("-window must be >= 1")
+    if args.window_step is not None and (args.window_length is None or args.window_step < 1):
+        parser.error("-step needs -window and must be >= 1")
     scorer = phamer_scorer()
     decide_files(scorer, args)
+    if args.window_length is not None and not (scorer.fasta_file and os.path.exists(scorer.fasta_file)):
+        parser.error("-window needs the FASTA file of the contigs (-fasta, or -in with a .fasta / .fa file): "
+                     "a features file alone has no positions")
     scorer.scoring_method = args.method
     scorer.canonical = args.canonical_kmers
     scorer.load_reference_data(scorer.positive_features_file, scorer.negative_features_file)
@@ -316,9 +390,14 @@ def main(argv=None):
         scorer.make_neighbors_file(args=args)
     else:
         scorer.scores = scorer.score_points()
-    # the score file's header does not depend on whether neighbours were asked for; canonical scoring is named only when it is on
+    if args.window_length is not None:
+        scorer.score_windows(args.window_length, args.window_step)
+        scorer.find_regions()
+        scorer.make_window_files(args=args)
+    # the score file's header does not depend on whether neighbours or windows were asked for; canonical scoring is named only when
+    # it is on
     score_args = argparse.Namespace(**{k: v for k, v in vars(args).items()
-                                       if k != "write_neighbors" and (k != "canonical_kmers" or v)})
+                                       if k not in ("write_neighbors", "window_length", "window_step") and (k != "canonical_kmers" or v)})
     scorer.make_summary_file(args=score_args)
     return scorer
 

@@ -5,6 +5,8 @@ The whole hot path as one object: contigs in, PhaMers scores out.
       .score_device(seq, offsets)             device buffers -> (counts int32[n,256], scores float64[n]) on the device
       .score_host(seq, offsets)               HOST buffers (pinned recommended) -> numpy scores; copies included
       .score_fasta(path)                      FASTA file -> (ids, scores), the phamer.py flow without the files
+      .score_windows_device(seq, offsets, w, s)   scores of overlapping windows along each record, on the device
+      .score_windows_fasta(path, w, s)        FASTA file -> (ids, record index, spans, scores) of the windows
 
 Stage by stage this is kmer.count_file -> kmer.normalize_counts -> phamer_scorer.score_points('combo')
 (reference scripts/phamer.py:131,139,194), with the k-mer length fixed at the width of the reference features.
@@ -112,6 +114,48 @@ class ContigScorer(object):
         out.copy_(scores, non_blocking=True)
         main.synchronize()
         return out.numpy().copy()
+
+    # -- sliding windows ---------------------------------------------------------------------------------
+    WINDOW_SLICE = 1 << 20             # windows counted and scored per library call: bounds the count rows (1 GB at 256 bins)
+
+    def score_windows_device(self, seq, offsets, window, step, method="combo"):
+        """Scores of overlapping windows along every record (phm_window_offsets, phm_kmer_count_windows, then the scorer on the
+        count rows).  Returns, on the device, (window offsets int64[n_records + 1], spans int64[n_windows, 2] -- start, end relative
+        to the record --, scores float64[n_windows]).  Windows are counted and scored WINDOW_SLICE at a time.  Count rows go to the
+        scorer as counts where the count road takes them (k_neighbors in {1, 3, 5}); other shapes are scored from float64 feature rows
+        normalised by the same call.  A window with no countable k-mer scores NaN."""
+        key = {"knn": 0, "kmeans": 1, "combo": 2}[method]
+        wo = ops.window_offsets_cuda(offsets, window, step)
+        total = int(wo[-1].item())
+        spans = torch.empty((total, 2), dtype=torch.int64, device="cuda")
+        scores = torch.empty((total,), dtype=torch.float64, device="cuda")
+        from_counts = (self.k_neighbors in (1, 3, 5) and self.refs.shape[1] in (256, 136)
+                       and self.cent_pos.shape[0] > 0 and self.cent_neg.shape[0] > 0)
+        for first in range(0, total, self.WINDOW_SLICE):
+            n = min(self.WINDOW_SLICE, total - first)
+            counts, freq, sp = ops.count_windows_cuda(seq, offsets, wo, window, step, self.kmer_length, first=first, n=n,
+                                                      canonical=self.canonical, counts=from_counts, freq=not from_counts, spans=True)
+            spans[first:first + n] = sp
+            out = tuple(scores[first:first + n] if i == key else torch.empty((n,), dtype=torch.float64, device="cuda")
+                        for i in range(3))
+            ops.score_cuda(counts if from_counts else freq, self.refs, self.n_positive, self.cent_pos, self.cent_neg,
+                           self.k_neighbors, out=out)
+        return wo, spans, scores
+
+    def score_windows_fasta(self, path, window, step, length_requirement=0, method="combo"):
+        """score_windows_device over the records of a FASTA file.  Returns on the host (ids [n_windows] -- the id of each window's
+        record --, record_index int64[n_windows] -- its position in the file --, spans int64[n_windows, 2], scores float64[n_windows]),
+        with the windows of records shorter than length_requirement left out."""
+        from . import fileIO
+        headers, d_seq, d_off = fileIO.read_fasta_arrays_cuda(path)
+        ids = np.array([fileIO.get_id(h) for h in headers])
+        if len(ids) == 0:
+            return ids, np.zeros((0,), dtype=np.int64), np.zeros((0, 2), dtype=np.int64), np.zeros((0,), dtype=np.float64)
+        wo, spans, scores = self.score_windows_device(d_seq, d_off, window, step, method=method)
+        wo, spans, scores = wo.cpu().numpy(), spans.cpu().numpy(), scores.cpu().numpy()
+        record = np.repeat(np.arange(len(ids), dtype=np.int64), np.diff(wo))
+        keep = (np.diff(d_off.cpu().numpy()) >= length_requirement)[record]
+        return ids[record[keep]], record[keep], spans[keep], scores[keep]
 
     def score_fasta(self, path, length_requirement=0, method="combo"):
         from . import fileIO
