@@ -120,6 +120,24 @@ int phm_kmer_count_windows(const uint8_t *d_seq, const int64_t *d_offsets, int64
                            uint32_t *d_counts, double *d_freq, int64_t *d_spans,
                            void *d_workspace, size_t workspace_bytes, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Spans: the same histogram over arbitrary pieces of the records -- a phage-like region, a gene, the intervals of a BED file.
+ * d_spans is int64[n_spans * 3]: (record, start, end) per span, 0-based, half-open, relative to the record, in any order; spans may
+ * overlap, repeat, be empty or be shorter than k.  Row i of d_counts / d_freq holds span i: exactly phm_kmer_count's counts of
+ * d_seq[off[record] + start, off[record] + end) taken as a record of its own (plain or PHM_COUNT_CANONICAL, the only flag accepted);
+ * a span with no countable k-mer gets a NaN feature row.  The workspace (phm_kmer_count_spans_workspace_bytes, n_span_bases = the
+ * summed span length) holds one 32-byte work item per span plus the tiles of spans of 131 072 bases and more.
+ * Argument errors (k, flags, sizes, null or misaligned pointers) are PHM_E_ARG and a workspace without one item per span is
+ * PHM_E_WORKSPACE, both before the device is touched.  The call then validates every span on the device and synchronises `stream`
+ * once to read the result: a span whose record is not in [0, n_records), whose start is < 0, whose end is < its start or past its
+ * record's end is PHM_E_ARG naming the lowest such index and its fields, and a list that does not fit the workspace is
+ * PHM_E_WORKSPACE; in both cases no output row has been written.  Score the rows with phm_score_counts / phm_score.
+ * ------------------------------------------------------------------------------------------- */
+size_t phm_kmer_count_spans_workspace_bytes(int64_t n_spans, int64_t n_span_bases, int k, uint32_t flags);
+int phm_kmer_count_spans(const uint8_t *d_seq, const int64_t *d_offsets, int64_t n_records,
+                         const int64_t *d_spans, int64_t n_spans, int k, uint32_t flags,
+                         uint32_t *d_counts, double *d_freq, void *d_workspace, size_t workspace_bytes, void *stream);
+
 /* Same histogram from the packed form produced by phm_pack_fasta (multi-k passes over one pack). */
 int phm_kmer_count_packed(const uint32_t *d_codes, const uint32_t *d_valid, const int64_t *d_offsets,
                           int64_t n_contigs, int k, uint32_t flags, uint32_t *d_counts, double *d_freq,

@@ -28,6 +28,9 @@ SIGNATURES = {
     "phm_kmer_count_windows_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int, c_uint32]),
     "phm_kmer_count_windows": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int, c_uint32,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_kmer_count_spans_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int, c_uint32]),
+    "phm_kmer_count_spans": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int, c_uint32, c_void_p, c_void_p, c_void_p,
+                                     c_size_t, c_void_p]),
     "phm_kmer_count_packed": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_uint32, c_void_p, c_void_p,
                                       c_void_p, c_size_t, c_void_p]),
     "phm_canonical_fold": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p]),

@@ -152,6 +152,7 @@ __device__ __forceinline__ void post6(uint32_t tab, uint32_t raw1) {       // ra
 //                        the slow path.  Tiles add their folded bins to the contig's output row with global reductions (the row
 //                        is zeroed by the planning pass) and hist_finish_kernel turns the finished rows into the requested
 //                        outputs (features, scorer operands) afterwards.
+// The same two passes plan a span call (phm_kmer_count_spans), with spans instead of records as items (RecordRanges / SpanRanges below).
 // An item carries its own range, so the histogram kernel then never reads the offset table.  The plan is switched off ON THE DEVICE
 // (item i is contig i, whole, in file order, as in round 1) when no contig reaches SPLIT_MIN -- measured on BASELINE configs[1], 1 M
 // contigs of 1 - 100 kb: 4.92 ms with the list against 4.83 ms without; the tail it removes is short because a warp that is alone on
@@ -167,6 +168,7 @@ struct PlanHeader {                                                        // fi
     unsigned long long need[N_CLASS];       // list slots every class needs
     unsigned long long filled[N_CLASS];     // ... and has reserved so far
     unsigned long long n_split;             // contigs of SPLIT_MIN bases and more
+    unsigned long long first_bad;           // span calls: lowest index of an invalid span (set to ~0 before the count pass)
 };
 static_assert(sizeof(PlanEntry) == 32 && sizeof(PlanHeader) <= 256, "workspace layout");
 
@@ -177,21 +179,66 @@ __host__ __device__ __forceinline__ int plan_class(int64_t length) {
     return length >= 65536 ? 0 : (length >= 32768 ? 1 : (length >= 16384 ? 2 : 3));
 }
 
-__global__ void __launch_bounds__(256) hist_plan_count_kernel(const int64_t *__restrict__ off, int64_t n, PlanHeader *plan) {
+// Where an item's range comes from.  RecordRanges: item c is record c, [off[c], off[c + 1]).  SpanRanges (phm_kmer_count_spans):
+// item i is span i = (record, start, end) of an int64[n, 3] array, the range [off[record] + start, off[record] + end); range()
+// returns false, with an empty range, for a span that lies outside its record or names no record -- the count pass reports the
+// lowest such index and the host stops before the fill pass.  Spans take the list in any case, because no offset table describes
+// them: the count pass sets n_split itself and the fill pass never falls back to drawing items in order.
+// length() is range()'s end - start (the count pass needs no more); the record forms keep the load order the passes always had.
+struct RecordRanges {
+    static constexpr bool SPANS = false;
+    __device__ __forceinline__ bool range(const int64_t *__restrict__ off, int64_t c, int64_t &start, int64_t &end) const {
+        start = off[c]; end = off[c + 1];
+        return true;
+    }
+    __device__ __forceinline__ bool length(const int64_t *__restrict__ off, int64_t c, int64_t &len) const {
+        len = off[c + 1] - off[c];
+        return true;
+    }
+};
+struct SpanRanges {
+    static constexpr bool SPANS = true;
+    const int64_t *spans; int64_t n_records;
+    __device__ __forceinline__ bool range(const int64_t *__restrict__ off, int64_t i, int64_t &start, int64_t &end) const {
+        const int64_t r = spans[3 * i], a = spans[3 * i + 1], b = spans[3 * i + 2];
+        start = 0; end = 0;
+        if (r < 0 || r >= n_records || a < 0 || b < a) return false;
+        const int64_t rs = off[r];
+        if (b > off[r + 1] - rs) return false;
+        start = rs + a; end = rs + b;
+        return true;
+    }
+    __device__ __forceinline__ bool length(const int64_t *__restrict__ off, int64_t i, int64_t &len) const {
+        int64_t start, end;
+        const bool ok = range(off, i, start, end);
+        len = end - start;
+        return ok;
+    }
+};
+
+template <class Src>
+__global__ void __launch_bounds__(256) hist_plan_count_kernel(const int64_t *__restrict__ off, int64_t n, PlanHeader *plan, Src src) {
     __shared__ unsigned long long s_tot[N_CLASS];
     if (threadIdx.x < N_CLASS) s_tot[threadIdx.x] = 0ull;
     __syncthreads();
     unsigned long long mine[N_CLASS] = {0ull, 0ull, 0ull, 0ull};
     uint32_t n_long = 0u;
+    int64_t bad = -1;                                                   // this thread's lowest invalid span (indices ascend)
     for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t len = off[c + 1] - off[c];
+        int64_t len;
+        if (!src.length(off, c, len) && bad < 0) bad = c;
         const int q = plan_class(len);
         const unsigned long long m = plan_tiles(len);
 #pragma unroll
         for (int j = 0; j < N_CLASS; ++j) mine[j] += (q == j) ? m : 0ull;
         if (m > 1ull) n_long = 1u;
     }
-    if (__any_sync(FULL, n_long != 0u) && (threadIdx.x & 31) == 0) atomicAdd(&plan->n_split, 1ull);     // only "are there any" matters
+    if (Src::SPANS) {
+        if (bad >= 0) atomicMin(&plan->first_bad, (unsigned long long)bad);
+        if (blockIdx.x == 0 && threadIdx.x == 0) plan->n_split = 1ull;
+    } else if (__any_sync(FULL, n_long != 0u) && (threadIdx.x & 31) == 0) {
+        atomicAdd(&plan->n_split, 1ull);                                // only "are there any" matters
+    }
 #pragma unroll
     for (int j = 0; j < N_CLASS; ++j) {
 #pragma unroll
@@ -209,9 +256,11 @@ __device__ __forceinline__ uint32_t *split_row(uint32_t *counts, double *freq, i
 
 // One block takes 256 consecutive contigs per round: a block-wide exclusive scan of the slots each contig needs, per class, and ONE
 // reservation per class and round in the global counters (a reservation per contig would serialise a million atomics on four words).
+// Spans: the host has checked that the list fits, after the count pass, before it launches this pass.
+template <class Src>
 __global__ void __launch_bounds__(256) hist_plan_fill_kernel(const int64_t *__restrict__ off, int64_t n, int k, PlanHeader *plan,
                                                              PlanEntry *entries, unsigned long long cap,
-                                                             uint32_t *counts, double *freq, int out_bins) {
+                                                             uint32_t *counts, double *freq, int out_bins, Src src) {
     __shared__ uint32_t s_warp[8][N_CLASS];
     __shared__ unsigned long long s_base[N_CLASS];
     unsigned long long class_base[N_CLASS];
@@ -220,15 +269,15 @@ __global__ void __launch_bounds__(256) hist_plan_fill_kernel(const int64_t *__re
     for (int j = 0; j < N_CLASS; ++j) { class_base[j] = total; total += plan->need[j]; }
     // no plan when the list does not fit, or when no contig needs tiles (the histogram kernel tests the same): measured on 1 M
     // contigs of 1 - 100 kb, drawing them by length class gains less (a lone warp finishes its last contig quickly) than the list costs
-    if (total > cap || plan->n_split == 0ull) return;
+    if (!Src::SPANS && (total > cap || plan->n_split == 0ull)) return;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t rounds = (n + 255) / 256;
     for (int64_t r = blockIdx.x; r < rounds; r += gridDim.x) {
         const int64_t c = r * 256 + threadIdx.x;
-        int64_t c_start = 0, c_end = 0;
+        int64_t c_end = 0, c_start = 0;
         uint32_t m = 0u;
         int q = 0;
-        if (c < n) { c_start = off[c]; c_end = off[c + 1]; m = plan_tiles(c_end - c_start); q = plan_class(c_end - c_start); }
+        if (c < n) { src.range(off, c, c_start, c_end); m = plan_tiles(c_end - c_start); q = plan_class(c_end - c_start); }
         uint32_t excl = 0u;
 #pragma unroll
         for (int j = 0; j < N_CLASS; ++j) {
@@ -1219,9 +1268,53 @@ static int launch_plan(const int64_t *off, int64_t n, int k, const CountWorkspac
     int64_t blocks = (n + 255) / 256;
     const int64_t cap = (int64_t)sm_count() * 8;
     if (blocks > cap) blocks = cap;
-    hist_plan_count_kernel<<<(unsigned)blocks, 256, 0, st>>>(off, n, w.plan);
+    hist_plan_count_kernel<<<(unsigned)blocks, 256, 0, st>>>(off, n, w.plan, RecordRanges());
     PHM_LAUNCH_CHECK();
-    hist_plan_fill_kernel<<<(unsigned)blocks, 256, 0, st>>>(off, n, k, w.plan, w.entries, w.cap, counts, freq, out_bins);
+    hist_plan_fill_kernel<<<(unsigned)blocks, 256, 0, st>>>(off, n, k, w.plan, w.entries, w.cap, counts, freq, out_bins, RecordRanges());
+    PHM_LAUNCH_CHECK();
+    return PHM_OK;
+}
+
+// a span call (phm_kmer_count_spans): span i of the array is row i
+struct SpanList {
+    const int64_t *spans; int64_t n_records;
+};
+
+// The planning passes of a span call: the count pass, which also validates every span; one synchronisation to read its totals;
+// then the fill pass, only when every span is valid and the exact list fits.  *n_items: the list's length.
+static int launch_span_plan(const int64_t *off, int64_t n, const SpanList &sl, int k, const CountWorkspace &w, uint32_t *counts,
+                            double *freq, int out_bins, cudaStream_t st, unsigned long long *n_items) {
+    int64_t blocks = (n + 255) / 256;
+    const int64_t cap = (int64_t)sm_count() * 8;
+    if (blocks > cap) blocks = cap;
+    const SpanRanges src{sl.spans, sl.n_records};
+    PHM_CUDA_CHECK(cudaMemsetAsync(&w.plan->first_bad, 0xFF, sizeof(unsigned long long), st));
+    hist_plan_count_kernel<<<(unsigned)blocks, 256, 0, st>>>(off, n, w.plan, src);
+    PHM_LAUNCH_CHECK();
+    PlanHeader h;
+    PHM_CUDA_CHECK(cudaMemcpyAsync(&h, w.plan, sizeof(PlanHeader), cudaMemcpyDeviceToHost, st));
+    PHM_CUDA_CHECK(cudaStreamSynchronize(st));
+    if (h.first_bad != ~0ull) {
+        // error path only: the span's fields, and its record's offsets when it names one
+        int64_t f[3] = {0, 0, 0}, rec[2] = {0, 0};
+        PHM_CUDA_CHECK(cudaMemcpyAsync(f, sl.spans + 3 * (int64_t)h.first_bad, sizeof(f), cudaMemcpyDeviceToHost, st));
+        const bool named = f[0] >= 0 && f[0] < sl.n_records;
+        if (named) PHM_CUDA_CHECK(cudaMemcpyAsync(rec, off + f[0], sizeof(rec), cudaMemcpyDeviceToHost, st));
+        PHM_CUDA_CHECK(cudaStreamSynchronize(st));
+        const char *why = !named ? "names no record" : f[1] < 0 ? "starts before its record" : f[2] < f[1] ? "ends before it starts"
+                                                                                                      : "ends past its record";
+        set_error("invalid argument: span %llu (record %lld, start %lld, end %lld) %s (%lld records, this one %lld bases long)",
+                  h.first_bad, (long long)f[0], (long long)f[1], (long long)f[2], why, (long long)sl.n_records,
+                  (long long)(rec[1] - rec[0]));
+        return PHM_E_ARG;
+    }
+    *n_items = h.need[0] + h.need[1] + h.need[2] + h.need[3];
+    if (*n_items > w.cap) {
+        set_error("workspace too small for the %lld spans: their list needs %llu items, the workspace holds %llu", (long long)n, *n_items,
+                  w.cap);
+        return PHM_E_WORKSPACE;
+    }
+    hist_plan_fill_kernel<<<(unsigned)blocks, 256, 0, st>>>(off, n, k, w.plan, w.entries, w.cap, counts, freq, out_bins, src);
     PHM_LAUNCH_CHECK();
     return PHM_OK;
 }
@@ -1245,12 +1338,13 @@ static int launch_window_plan(const int64_t *off, const WindowSlice &ws, int k, 
     return PHM_OK;
 }
 
-// win != nullptr: count the windows of a slice instead of whole records (`n` is then the slice's window count); windows always
-// take the list, whatever option hist_plan says, because no offset table describes them
+// win != nullptr: count the windows of a slice instead of whole records (`n` is then the slice's window count); spans != nullptr:
+// count n spans.  Windows and spans always take the list, whatever option hist_plan says, because no offset table describes them
 template <int K, int STRIDE, int WARPS, bool EMIT = false, bool SWZ = false, int STAGES = 0>
 static int launch_hist(const uint8_t *seq, const int64_t *off, int64_t n, uint32_t *counts, double *freq,
                        const uint16_t *rc, const uint16_t *compact, int out_bins, const CountWorkspace &w,
-                       cudaStream_t st, tc::QueryEmit emit = tc::QueryEmit(), const WindowSlice *win = nullptr) {
+                       cudaStream_t st, tc::QueryEmit emit = tc::QueryEmit(), const WindowSlice *win = nullptr,
+                       const SpanList *spans = nullptr) {
     using Cfg = HistCfg<K, STRIDE>;
     const size_t smem = (size_t)WARPS * Cfg::WARP_BYTES + Cfg::ALIGN + (size_t)WARPS * STAGES * (STAGE_BYTES + 8);
     auto kern = kmer_hist_kernel<K, STRIDE, WARPS, EMIT, SWZ, STAGES>;
@@ -1262,10 +1356,14 @@ static int launch_hist(const uint8_t *seq, const int64_t *off, int64_t n, uint32
     job.seq = seq; job.off = off; job.n_contigs = n; job.counts = counts; job.freq = freq;
     job.rc_lut = rc; job.canon_lut = compact; job.out_bins = out_bins;
     job.plan = w.plan; job.entries = w.entries;
-    job.cap = (hist_plan || win) ? w.cap : 0ull;
+    job.cap = (hist_plan || win || spans) ? w.cap : 0ull;
     const bool timed = g_hist_ring.begin(st);           // the bracket covers the whole counting stage: planning passes, histogram, finish
+    unsigned long long span_items = 0;
     if (win) {
         const int rc_plan = launch_window_plan(off, *win, K, w, counts, freq, out_bins, st);
+        if (rc_plan != PHM_OK) return rc_plan;
+    } else if (spans) {
+        const int rc_plan = launch_span_plan(off, n, *spans, K, w, counts, freq, out_bins, st, &span_items);
         if (rc_plan != PHM_OK) return rc_plan;
     } else if (job.cap > 0) {
         const int rc_plan = launch_plan(off, n, K, w, counts, freq, out_bins, st);
@@ -1274,7 +1372,8 @@ static int launch_hist(const uint8_t *seq, const int64_t *off, int64_t n, uint32
     constexpr int per_item = (K >= 6) ? 4 : 1;
     int64_t grid = (int64_t)per_sm * sm_count();
     const int64_t items = win ? (n * (int64_t)plan_tiles(win->window) + per_item - 1) / per_item          // the window list, exactly
-                              : (n + (int64_t)job.cap + per_item - 1) / per_item;  // upper bound: the list can hold at most cap items
+                              : spans ? ((int64_t)span_items + per_item - 1) / per_item                  // the span list, exactly
+                                      : (n + (int64_t)job.cap + per_item - 1) / per_item;  // upper bound: the list can hold at most cap items
     const int64_t need = (items + WARPS - 1) / WARPS;
     if (grid > need) grid = need < 1 ? 1 : need;
     kern<<<(unsigned)grid, WARPS * 32, smem, st>>>(job, emit);
@@ -1368,36 +1467,38 @@ static int prepare_count(int64_t n_contigs, int k, uint32_t flags, void *ws, siz
     return PHM_OK;
 }
 
-// the histogram variant of k (and of the tuning options), for a call over records or over the windows of a slice
+// the histogram variant of k (and of the tuning options), for a call over records, over the windows of a slice or over spans
 static int dispatch_hist(int k, const uint8_t *seq, const int64_t *off, int64_t n, uint32_t *counts, double *freq, const uint16_t *rc,
-                         const uint16_t *canon, int out_bins, const CountWorkspace &w, cudaStream_t st, const WindowSlice *win) {
+                         const uint16_t *canon, int out_bins, const CountWorkspace &w, cudaStream_t st, const WindowSlice *win,
+                         const SpanList *sp = nullptr) {
+    const tc::QueryEmit e = tc::QueryEmit();
     switch (k) {
-        case 1: return launch_hist<1, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
-        case 2: return launch_hist<2, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
-        case 3: return launch_hist<3, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+        case 1: return launch_hist<1, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
+        case 2: return launch_hist<2, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
+        case 3: return launch_hist<3, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
         case 4:
             if (hist_stride_for_k4 == 2)
-                return hist_tma ? launch_hist<4, 2, 8, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
-                                : launch_hist<4, 2, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
-            return launch_hist<4, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+                return hist_tma ? launch_hist<4, 2, 8, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp)
+                                : launch_hist<4, 2, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
+            return launch_hist<4, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
         case 5:
             if ((hist_stride_for_k5 == 2 || (hist_stride_for_k5 == 0 && !rc)) && hist_warps_k5 == 18)
-                return launch_hist<5, 2, 18>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+                return launch_hist<5, 2, 18>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
             if (hist_stride_for_k5 == 2 || (hist_stride_for_k5 == 0 && !rc))
-                return launch_hist<5, 2, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+                return launch_hist<5, 2, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
             if (rc && hist_canonical_swizzle)
-                return hist_tma ? launch_hist<5, 1, 8, false, true, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
-                                : launch_hist<5, 1, 8, false, true>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
-            return hist_tma ? launch_hist<5, 1, 8, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
-                            : launch_hist<5, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+                return hist_tma ? launch_hist<5, 1, 8, false, true, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp)
+                                : launch_hist<5, 1, 8, false, true>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
+            return hist_tma ? launch_hist<5, 1, 8, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp)
+                            : launch_hist<5, 1, 8>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
         case 6:
             if (hist_warps_k6 == 4)
-                return launch_hist<6, 1, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+                return launch_hist<6, 1, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
             if (rc && hist_canonical_swizzle)
-                return hist_tma ? launch_hist<6, 1, 11, false, true, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
-                                : launch_hist<6, 1, 13, false, true>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
-            return hist_tma ? launch_hist<6, 1, 11, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win)
-                            : launch_hist<6, 1, 13>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, tc::QueryEmit(), win);
+                return hist_tma ? launch_hist<6, 1, 11, false, true, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp)
+                                : launch_hist<6, 1, 13, false, true>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
+            return hist_tma ? launch_hist<6, 1, 11, false, false, 4>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp)
+                            : launch_hist<6, 1, 13>(seq, off, n, counts, freq, rc, canon, out_bins, w, st, e, win, sp);
     }
     return PHM_E_ARG;
 }
@@ -1496,6 +1597,38 @@ extern "C" int phm_kmer_count_windows(const uint8_t *d_seq, const int64_t *d_off
     if (rcode != PHM_OK) return rcode;
     const WindowSlice win{d_window_offsets, n_records, window, step, first_window, n_windows, d_spans};
     return dispatch_hist(k, d_seq, d_offsets, n_windows, d_counts, d_freq, rc, rc ? w.canon_lut : nullptr, out_bins, w, st, &win);
+}
+
+// Fixed part + one list item per span, plus the extra tiles of spans of SPLIT_MIN bases and more (at most n_span_bases / TILE).
+extern "C" size_t phm_kmer_count_spans_workspace_bytes(int64_t n_spans, int64_t n_span_bases, int, uint32_t) {
+    const size_t slots = (size_t)(n_spans > 0 ? n_spans : 0) + (size_t)(n_span_bases > 0 ? n_span_bases / TILE : 0);
+    return kCountWorkspaceFixed + ((slots * sizeof(PlanEntry) + 255) & ~(size_t)255);
+}
+
+extern "C" int phm_kmer_count_spans(const uint8_t *d_seq, const int64_t *d_offsets, int64_t n_records, const int64_t *d_spans,
+                                    int64_t n_spans, int k, uint32_t flags, uint32_t *d_counts, double *d_freq, void *d_workspace,
+                                    size_t workspace_bytes, void *stream) {
+    // every argument is checked before the device is touched; the spans themselves are checked by the count pass
+    PHM_REQUIRE(k >= 1 && k <= 6, "k must be 1..6");
+    PHM_REQUIRE((flags & ~PHM_COUNT_CANONICAL) == 0u, "flags: PHM_COUNT_CANONICAL is the only flag of a span call");
+    PHM_REQUIRE(n_records >= 0 && n_spans >= 0, "n_records and n_spans must be >= 0");
+    if (n_spans == 0) return PHM_OK;
+    PHM_REQUIRE(d_seq != nullptr && d_offsets != nullptr && d_spans != nullptr && d_workspace != nullptr, "null pointer");
+    PHM_REQUIRE(d_counts != nullptr || d_freq != nullptr, "both outputs are null");
+    PHM_REQUIRE((reinterpret_cast<uintptr_t>(d_seq) & 15u) == 0, "d_seq must be 16-byte aligned");
+    PHM_REQUIRE(((reinterpret_cast<uintptr_t>(d_offsets) | reinterpret_cast<uintptr_t>(d_spans) | reinterpret_cast<uintptr_t>(d_freq)) & 7u) == 0 &&
+                (reinterpret_cast<uintptr_t>(d_counts) & 3u) == 0, "misaligned pointer");
+    if (workspace_bytes < kCountWorkspaceFixed || (workspace_bytes - kCountWorkspaceFixed) / sizeof(PlanEntry) < (unsigned long long)n_spans) {
+        set_error("workspace too small for %lld spans: %zu < %zu bytes", (long long)n_spans, workspace_bytes,
+                  phm_kmer_count_spans_workspace_bytes(n_spans, 0, k, flags));
+        return PHM_E_WORKSPACE;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CountWorkspace w; const uint16_t *rc, *compact; int out_bins;
+    int rcode = prepare_count(n_spans, k, flags, d_workspace, workspace_bytes, d_offsets, &w, &rc, &compact, &out_bins, st);
+    if (rcode != PHM_OK) return rcode;
+    const SpanList sl{d_spans, n_records};
+    return dispatch_hist(k, d_seq, d_offsets, n_spans, d_counts, d_freq, rc, rc ? w.canon_lut : nullptr, out_bins, w, st, nullptr, &sl);
 }
 
 extern "C" int phm_kmer_count_packed(const uint32_t *d_codes, const uint32_t *d_valid, const int64_t *d_offsets,

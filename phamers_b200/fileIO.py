@@ -8,6 +8,8 @@ scripts/id_parser.py the path touches:
     neighbour CSV   save_phamer_neighbors, read_phamer_neighbors  ('# ' header, then per contig its nearest references and clusters)
     window CSV      save_phamer_windows, read_phamer_windows  ('# ' header, then 'id, start, end, score' per window)
     region CSV      save_phamer_regions, read_phamer_regions  ('# ' header, then 'id, start, end, windows, mean_score, max_score')
+    BED in          read_bed  ('chrom start end [name ...]' per line)
+    span CSV        save_phamer_spans, read_phamer_spans  ('# ' header, then 'id, start, end, name, score' and the neighbour columns)
 
 Host-side only (bytes and text); no arithmetic happens here.
 """
@@ -400,3 +402,78 @@ def read_phamer_regions(filename):
     spans = np.array([[int(r[1]), int(r[2])] for r in rows], dtype=np.int64).reshape(len(rows), 2)
     return (ids, spans, np.array([int(r[3]) for r in rows], dtype=np.int64), np.array([float(r[4]) for r in rows], dtype=np.float64),
             np.array([float(r[5]) for r in rows], dtype=np.float64))
+
+
+# ----------------------------------------------------------------------------------------------------------
+# BED intervals in, span scores out (phamer -spans, -region_scores)
+# ----------------------------------------------------------------------------------------------------------
+def read_bed(path, with_lines=False):
+    """BED intervals -> (contig names [n] str, spans int64[n, 2] (start, end: 0-based, half-open), names [n] str), and with
+    with_lines=True a fourth element, where each interval came from ('<path> line <number>').  Fields are
+    separated by tabs or any whitespace: 'chrom start end [name ...]'; columns past the name are ignored and a missing name is '.'.
+    Blank lines and '#', 'track' and 'browser' lines are skipped.  A malformed line (fewer than three fields, coordinates that are
+    not integers, start < 0 or end < start) is a ValueError naming its line number."""
+    ids, spans, names, where = [], [], [], []
+    with open(path, "r") as fh:
+        for number, line in enumerate(fh, 1):
+            fields = line.split()
+            if not fields or fields[0].startswith("#") or fields[0] in ("track", "browser"):
+                continue
+            if len(fields) < 3:
+                raise ValueError("%s line %d: a BED line needs chrom, start and end: %r" % (path, number, line.rstrip("\n")))
+            try:
+                start, end = int(fields[1]), int(fields[2])
+            except ValueError:
+                raise ValueError("%s line %d: start and end must be integers: %r" % (path, number, line.rstrip("\n"))) from None
+            if start < 0 or end < start:
+                raise ValueError("%s line %d: [%d, %d) is not an interval" % (path, number, start, end))
+            ids.append(fields[0])
+            spans.append((start, end))
+            names.append(fields[3] if len(fields) > 3 else ".")
+            where.append("%s line %d" % (path, number))
+    out = np.array(ids, dtype=str), np.array(spans, dtype=np.int64).reshape(-1, 2), np.array(names, dtype=str)
+    return out + (where,) if with_lines else out
+
+
+def save_phamer_spans(ids, spans, names, scores, reference_ids, reference_labels, reference_distances, clusters, cluster_distances,
+                      file_name, args=None):
+    """'# '-prefixed header lines (header 'PhaMers span file', then the column names), then one row per span: 'id, start, end, name,
+    score' followed by the neighbour columns of save_phamer_neighbors (reference_j, class_j, distance_j for j = 1..k, then the phage
+    and bacteria cluster with their distances).  Floats are printed by numpy's float64 -> str conversion, which round-trips."""
+    spans = np.asarray(spans, dtype=np.int64).reshape(-1, 2)
+    ref_ids = np.asarray(reference_ids).astype(str)
+    k = ref_ids.shape[1] if ref_ids.ndim == 2 else 0
+    ref_ids = ref_ids.reshape(-1, k)
+    classes = np.vectorize(NEIGHBOR_CLASSES.get, otypes=[str])(np.asarray(reference_labels, dtype=np.int64).reshape(-1, k))
+    ref_dist = np.asarray(reference_distances, dtype=np.float64).reshape(-1, k).astype(str)
+    clusters = np.asarray(clusters, dtype=np.int64).reshape(-1, 2)
+    cl_dist = np.asarray(cluster_distances, dtype=np.float64).reshape(-1, 2).astype(str)
+    scores = np.asarray(scores, dtype=np.float64).astype(str)
+    columns = ["id", "start", "end", "name", "score"] + ["%s_%d" % (c, j + 1) for j in range(k) for c in ("reference", "class", "distance")]
+    columns += ["phage_cluster", "phage_cluster_distance", "bacteria_cluster", "bacteria_cluster_distance"]
+    rows = []
+    for i, (ident, name) in enumerate(zip(np.asarray(ids).astype(str), np.asarray(names).astype(str))):
+        fields = [ident, str(spans[i, 0]), str(spans[i, 1]), name, scores[i]]
+        for j in range(k):
+            fields += [ref_ids[i, j], classes[i, j], ref_dist[i, j]]
+        rows.append(fields + [str(clusters[i, 0]), cl_dist[i, 0], str(clusters[i, 1]), cl_dist[i, 1]])
+    _write_rows(file_name, "PhaMers span file", args, columns, rows)
+
+
+def read_phamer_spans(filename):
+    """The file of save_phamer_spans -> (ids str, spans int64[n, 2], names str, scores float64, reference_ids [n, k] str,
+    reference_labels [n, k] int64, reference_distances [n, k] float64, clusters [n, 2] int64, cluster_distances [n, 2] float64)."""
+    labels = {v: c for c, v in NEIGHBOR_CLASSES.items()}
+    rows = _read_rows(filename)
+    n = len(rows)
+    k = (len(rows[0]) - 9) // 3 if rows else 0
+    ids = np.array([r[0] for r in rows], dtype=str)
+    spans = np.array([[int(r[1]), int(r[2])] for r in rows], dtype=np.int64).reshape(n, 2)
+    names = np.array([r[3] for r in rows], dtype=str)
+    scores = np.array([float(r[4]) for r in rows], dtype=np.float64)
+    refs = np.array([[r[5 + 3 * j] for j in range(k)] for r in rows], dtype=str).reshape(n, k)
+    ref_labels = np.array([[labels[r[6 + 3 * j]] for j in range(k)] for r in rows], dtype=np.int64).reshape(n, k)
+    ref_dist = np.array([[float(r[7 + 3 * j]) for j in range(k)] for r in rows], dtype=np.float64).reshape(n, k)
+    clusters = np.array([[int(r[-4]), int(r[-2])] for r in rows], dtype=np.int64).reshape(n, 2)
+    cl_dist = np.array([[float(r[-3]), float(r[-1])] for r in rows], dtype=np.float64).reshape(n, 2)
+    return ids, spans, names, scores, refs, ref_labels, ref_dist, clusters, cl_dist

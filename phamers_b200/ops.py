@@ -131,6 +131,32 @@ def count_windows_cuda(seq, offsets, window_offsets, window, step, k, first=0, n
     return out_counts, out_freq, out_spans
 
 
+def count_spans_cuda(seq, offsets, spans, k, canonical=False, counts=True, freq=False, out_counts=None):
+    """phm_kmer_count_spans: k-mer counts of arbitrary spans of the records.  spans: int64 CUDA tensor [n, 3] of (record, start, end),
+    0-based half-open in the record, in any order.  Row i holds span i: the counts of count_cuda on those bases as a record of their
+    own (a span without a countable k-mer has a NaN feature row).  Returns (counts int32[n, bins] or None, freq float64[n, bins] or
+    None).  The call validates the spans on the device and synchronises once; an invalid span raises PhamersLibraryError naming
+    the lowest such index."""
+    lib = _lib.require_cuda()
+    seq = _as_u8_cuda(seq)
+    offsets = _offsets_cuda(offsets)
+    if not (isinstance(spans, torch.Tensor) and spans.is_cuda and spans.dtype == torch.int64 and spans.dim() == 2
+            and spans.shape[1] == 3):
+        raise TypeError("spans must be a CUDA int64 tensor [n, 3] of (record, start, end)")
+    spans = spans.contiguous()
+    n = spans.shape[0]
+    flags = _lib.PHM_COUNT_CANONICAL if canonical else 0
+    bins = num_bins(k, canonical)
+    out_counts = _result(out_counts, (n, bins), torch.int32) if counts else None
+    out_freq = torch.empty((n, bins), dtype=torch.float64, device="cuda") if freq else None
+    # the summed span length bounds the tiles of the list; an invalid span may make it meaningless, and the device check reports it
+    span_bases = int((spans[:, 2] - spans[:, 1]).clamp(min=0).sum().item()) if n else 0
+    ws = _workspace("count", lib.phm_kmer_count_spans_workspace_bytes(n, span_bases, int(k), flags))
+    check(lib.phm_kmer_count_spans(ptr(seq), ptr(offsets), offsets.numel() - 1, ptr(spans), n, int(k), flags, ptr(out_counts),
+                                   ptr(out_freq), ptr(ws), ws.numel(), stream_ptr()))
+    return out_counts, out_freq
+
+
 def pack_cuda(seq):
     """K1.  uint8[n] ASCII -> (codes int32[ceil(n/16)], valid int32[ceil(n/32)])."""
     lib = _lib.require_cuda()

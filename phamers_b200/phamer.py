@@ -70,6 +70,18 @@ class phamer_scorer(object):
         self.region_windows = None
         self.region_mean_scores = None
         self.region_max_scores = None
+        self.region_records = None
+        # filled by score_spans() / score_regions(): per span its contig id, [start, end), name and score, and the references and
+        # clusters behind the score (as the neighbor_* attributes)
+        self.span_ids = None
+        self.span_spans = None
+        self.span_names = None
+        self.span_scores = None
+        self.span_neighbor_ids = None
+        self.span_neighbor_labels = None
+        self.span_neighbor_distances = None
+        self.span_nearest_clusters = None
+        self.span_nearest_cluster_distances = None
 
     # ---- data -------------------------------------------------------------------------------------------
     def load_reference_data(self, positive_features_file=None, negative_features_file=None):
@@ -139,17 +151,23 @@ class phamer_scorer(object):
     # ---- scoring ----------------------------------------------------------------------------------------
     def _device_inputs(self):
         import torch
+        pts = np.ascontiguousarray(self.data_points, dtype=np.float64)
+        refs = self._device_references(pts.shape[1])                                   # raises first when there is no device
+        return (torch.from_numpy(pts).cuda(),) + refs
+
+    def _device_references(self, width):
+        """(references, positives, positive centroids, negative centroids, k_neighbors) on the device, as score_points uses them."""
+        import torch
         from . import _lib
         _lib.require_cuda()
-        pts = np.ascontiguousarray(self.data_points, dtype=np.float64)
         pos = np.ascontiguousarray(self.positive_data, dtype=np.float64)
         neg = np.ascontiguousarray(self.negative_data, dtype=np.float64)
         if self.scoring_method in ("kmeans", "combo"):
             cpos, cneg = references.reference_centroids(pos, neg, self.k_clusters)
         else:
-            cpos = cneg = np.zeros((0, pts.shape[1]))
+            cpos = cneg = np.zeros((0, width))
         refs = torch.from_numpy(np.vstack((pos, neg))).cuda()                         # :186
-        return (torch.from_numpy(pts).cuda(), refs, pos.shape[0], torch.from_numpy(np.ascontiguousarray(cpos)).cuda(),
+        return (refs, pos.shape[0], torch.from_numpy(np.ascontiguousarray(cpos)).cuda(),
                 torch.from_numpy(np.ascontiguousarray(cneg)).cuda(), self.k_neighbors)
 
     def _device_scores(self):
@@ -189,15 +207,20 @@ class phamer_scorer(object):
                                       % self.scoring_method)
         knn, km, combo, ref_i, ref_d, cen_i, cen_d = [t.cpu().numpy() for t in ops.score_neighbors_cuda(*self._device_inputs())]
         self.scores = {"knn": knn, "kmeans": km, "combo": combo}[self.scoring_method]
-        pos_ids = self.positive_ids if self.positive_ids is not None else np.arange(self.num_positive)
-        neg_ids = self.negative_ids if self.negative_ids is not None else np.arange(self.num_negative)
-        all_ids = np.concatenate((np.asarray(pos_ids).astype(str), np.asarray(neg_ids).astype(str), [""]))
-        self.neighbor_ids = all_ids[ref_i]                        # index -1 (NaN row) picks the trailing ""
-        self.neighbor_labels = np.where(ref_i < 0, -1, (ref_i < self.num_positive).astype(np.int64))
+        self.neighbor_ids, self.neighbor_labels = self._reference_names(ref_i)
         self.neighbor_distances = ref_d
         self.nearest_clusters = cen_i
         self.nearest_cluster_distances = cen_d
         return self.scores
+
+    def _reference_names(self, ref_index):
+        """Rows of the stacked references (positives first; -1 for none) -> (their ids, labels 1 = phage / 0 = bacteria / -1 none)."""
+        n_pos, n_neg = self.positive_data.shape[0], self.negative_data.shape[0]
+        pos_ids = self.positive_ids if self.positive_ids is not None else np.arange(n_pos)
+        neg_ids = self.negative_ids if self.negative_ids is not None else np.arange(n_neg)
+        all_ids = np.concatenate((np.asarray(pos_ids).astype(str), np.asarray(neg_ids).astype(str), [""]))
+        ref_index = np.asarray(ref_index, dtype=np.int64)
+        return all_ids[ref_index], np.where(ref_index < 0, -1, (ref_index < n_pos).astype(np.int64))   # -1 picks the trailing ""
 
     def score_windows(self, window, step=None):
         """Scores overlapping windows along every contig the length screen kept (all records of the FASTA when no screen ran), with
@@ -218,6 +241,60 @@ class phamer_scorer(object):
             self.fasta_file, int(window), int(step or window), length_requirement=self.screened_length, method=self.scoring_method)
         return self.window_scores
 
+    def score_spans(self, ids, spans, names=None, lines=None):
+        """Scores any spans of the contigs of the FASTA file -- ids [n] contig names (score-file ids, or the titles' first tokens as
+        BED files carry them), spans [n, 2] 0-based half-open (start, end) -- each exactly as score_neighbors scores its bases written
+        as a contig of their own, with the references behind each score.  Fills span_ids, span_spans, span_names ('.' when not
+        given), span_scores and span_neighbor_ids / _labels / _distances, span_nearest_clusters / _cluster_distances (as
+        score_neighbors).  Spans ignore the length screen: the user named them.  lines: where each span came from, named by the
+        error of a span outside its contig."""
+        from . import pipeline
+        self._check_span_inputs("span scores")
+        self.span_ids = np.asarray(ids).astype(str)
+        self.span_spans = np.asarray(spans, dtype=np.int64).reshape(-1, 2)
+        self.span_names = np.asarray(names).astype(str) if names is not None else np.full((len(self.span_ids),), ".")
+        return self._score_span_table(*pipeline.fasta_spans(self.fasta_file, self.span_ids, self.span_spans, lines))
+
+    def score_regions(self):
+        """score_spans for the regions find_regions found, in their order: each region scored as one sequence, with name '.'."""
+        import torch
+        self._check_span_inputs("region scores")
+        self.span_ids = np.asarray(self.region_ids).astype(str)
+        self.span_spans = np.asarray(self.region_spans, dtype=np.int64).reshape(-1, 2)
+        self.span_names = np.full((len(self.span_ids),), ".")
+        table = np.concatenate((np.asarray(self.region_records, dtype=np.int64).reshape(-1, 1), self.span_spans), axis=1)
+        _, d_seq, d_off = fileIO.read_fasta_arrays_cuda(self.fasta_file)
+        return self._score_span_table(d_seq, d_off, torch.from_numpy(np.ascontiguousarray(table)).cuda())
+
+    def _check_span_inputs(self, what):
+        if self.fasta_file is None or not os.path.exists(self.fasta_file):
+            raise ValueError("%s need the FASTA file of the contigs; a features file alone has no positions" % what)
+        if self.scoring_method not in ("knn", "kmeans", "combo"):
+            raise NotImplementedError("scoring method %r is outside the B200 hot path (knn / kmeans / combo only)" % self.scoring_method)
+
+    def _score_span_table(self, d_seq, d_off, table):
+        """Counts the spans of a device table [n, 3] (record, start, end) as float64 feature rows and scores them with the inputs and
+        entry point of score_neighbors, pipeline.ContigScorer.SPAN_SLICE spans per call."""
+        import torch
+        from . import ops, pipeline
+        width = ops.num_bins(self.kmer_length, self.canonical)
+        inputs = self._device_references(width)
+        key = {"knn": 0, "kmeans": 1, "combo": 2}[self.scoring_method]
+        parts = []
+        for first in range(0, table.shape[0], pipeline.ContigScorer.SPAN_SLICE):
+            _, feats = ops.count_spans_cuda(d_seq, d_off, table[first:first + pipeline.ContigScorer.SPAN_SLICE], self.kmer_length,
+                                            canonical=self.canonical, counts=False, freq=True)
+            out = ops.score_neighbors_cuda(feats, *inputs)
+            parts.append([out[key]] + list(out[3:]))
+        if not parts:
+            parts = [[torch.empty((0, n) if n else (0,), dtype=d, device="cuda") for n, d in
+                      ((0, torch.float64), (self.k_neighbors, torch.int64), (self.k_neighbors, torch.float64), (2, torch.int64),
+                       (2, torch.float64))]]
+        out = [torch.cat(col).cpu().numpy() for col in zip(*parts)]
+        self.span_scores, ref_i, self.span_neighbor_distances, self.span_nearest_clusters, self.span_nearest_cluster_distances = out
+        self.span_neighbor_ids, self.span_neighbor_labels = self._reference_names(ref_i)
+        return self.span_scores
+
     def find_regions(self):
         """Phage-like regions from the window scores (host only): a region is a maximal run of consecutive windows of one contig whose
         scores are all >= 0 (a NaN window ends a run; a run never crosses contigs).  Fills region_ids, region_spans ([regions, 2]: start
@@ -235,6 +312,7 @@ class phamer_scorer(object):
         starts = np.concatenate(([0], np.cumsum(windows)[:-1])).astype(np.int64)
         in_runs = scores[hit]
         self.region_ids = np.asarray(self.window_ids)[first]
+        self.region_records = records[first]
         self.region_spans = np.stack((spans[first, 0], spans[last, 1]), axis=1).reshape(-1, 2)
         self.region_windows = windows
         self.region_mean_scores = np.add.reduceat(in_runs, starts) / windows if len(first) else np.zeros(0)
@@ -297,6 +375,14 @@ class phamer_scorer(object):
         fileIO.save_phamer_regions(self.region_ids, self.region_spans, self.region_windows, self.region_mean_scores,
                                    self.region_max_scores, self.phamer_regions_filename, args=args)
 
+    def make_span_file(self, file_name, args=None):
+        """<out>/<file_name>: one row per span of score_spans / score_regions with its score and the references behind it."""
+        path = os.path.join(self.output_directory, file_name)
+        fileIO.save_phamer_spans(self.span_ids, self.span_spans, self.span_names, self.span_scores, self.span_neighbor_ids,
+                                 self.span_neighbor_labels, self.span_neighbor_distances, self.span_nearest_clusters,
+                                 self.span_nearest_cluster_distances, path, args=args)
+        return path
+
     def make_neighbors_file(self, args=None):
         """<out>/phamer_neighbors.csv: the rows of phamer_scores.csv with the references and clusters behind each score."""
         self.phamer_neighbors_filename = os.path.join(self.output_directory, "phamer_neighbors.csv")
@@ -340,8 +426,8 @@ def decide_files(scorer, args):
 def main(argv=None):
     """The reference's command line (scripts/phamer.py:510-599) for the hot path: count the contigs of a FASTA (or read their
     feature CSV), score them against the reference features, write <out>/phamer_scores.csv (and with -neighbors
-    <out>/phamer_neighbors.csv; with -window <out>/phamer_windows.csv and <out>/phamer_regions.csv).  t-SNE and plots are out of
-    scope."""
+    <out>/phamer_neighbors.csv; with -window <out>/phamer_windows.csv and <out>/phamer_regions.csv, and with -region_scores also
+    <out>/phamer_region_scores.csv; with -spans <out>/phamer_spans.csv).  t-SNE and plots are out of scope."""
     import argparse
     parser = argparse.ArgumentParser(description="Scores contigs based on feature similarity (B200 path)",
                                      formatter_class=argparse.ArgumentDefaultsHelpFormatter)
@@ -363,6 +449,10 @@ def main(argv=None):
     parser.add_argument("-window", "--window_length", type=int,
                         help="Also score windows of this many bases along each contig: phamer_windows.csv and phamer_regions.csv")
     parser.add_argument("-step", "--window_step", type=int, help="Bases between window starts (default: the window length)")
+    parser.add_argument("-region_scores", "--region_scores", action="store_true",
+                        help="With -window, also score each phage-like region as one sequence: phamer_region_scores.csv")
+    parser.add_argument("-spans", "--span_file",
+                        help="BED file of contig intervals to score, each as one sequence: phamer_spans.csv")
     parser.add_argument("-do_tsne", "--do_tsne", action="store_true", help="(out of scope)")
     parser.add_argument("-plot", "--plot_tsne", action="store_true", help="(out of scope)")
     args = parser.parse_args(argv)
@@ -372,10 +462,15 @@ def main(argv=None):
         parser.error("-window must be >= 1")
     if args.window_step is not None and (args.window_length is None or args.window_step < 1):
         parser.error("-step needs -window and must be >= 1")
+    if args.region_scores and args.window_length is None:
+        parser.error("-region_scores needs -window: regions are found from the window scores")
     scorer = phamer_scorer()
     decide_files(scorer, args)
     if args.window_length is not None and not (scorer.fasta_file and os.path.exists(scorer.fasta_file)):
         parser.error("-window needs the FASTA file of the contigs (-fasta, or -in with a .fasta / .fa file): "
+                     "a features file alone has no positions")
+    if args.span_file is not None and not (scorer.fasta_file and os.path.exists(scorer.fasta_file)):
+        parser.error("-spans needs the FASTA file of the contigs (-fasta, or -in with a .fasta / .fa file): "
                      "a features file alone has no positions")
     scorer.scoring_method = args.method
     scorer.canonical = args.canonical_kmers
@@ -385,18 +480,27 @@ def main(argv=None):
         scorer.equalize_reference_data()
     if not os.path.isdir(scorer.output_directory):
         os.makedirs(scorer.output_directory)
+    # the files that existed before span scoring do not name its options in their headers, so they stay what they were
+    file_args = argparse.Namespace(**{k: v for k, v in vars(args).items() if k not in ("region_scores", "span_file")})
     if args.write_neighbors:
         scorer.scores = scorer.score_neighbors()
-        scorer.make_neighbors_file(args=args)
+        scorer.make_neighbors_file(args=file_args)
     else:
         scorer.scores = scorer.score_points()
     if args.window_length is not None:
         scorer.score_windows(args.window_length, args.window_step)
         scorer.find_regions()
-        scorer.make_window_files(args=args)
-    # the score file's header does not depend on whether neighbours or windows were asked for; canonical scoring is named only when
-    # it is on
-    score_args = argparse.Namespace(**{k: v for k, v in vars(args).items()
+        scorer.make_window_files(args=file_args)
+        if args.region_scores:
+            scorer.score_regions()
+            scorer.make_span_file("phamer_region_scores.csv", args=args)
+    if args.span_file is not None:
+        ids, spans, names, lines = fileIO.read_bed(args.span_file, with_lines=True)
+        scorer.score_spans(ids, spans, names, lines=lines)
+        scorer.make_span_file("phamer_spans.csv", args=args)
+    # the score file's header does not depend on whether neighbours, windows or spans were asked for; canonical scoring is named only
+    # when it is on
+    score_args = argparse.Namespace(**{k: v for k, v in vars(file_args).items()
                                        if k not in ("write_neighbors", "window_length", "window_step") and (k != "canonical_kmers" or v)})
     scorer.make_summary_file(args=score_args)
     return scorer

@@ -7,6 +7,8 @@ The whole hot path as one object: contigs in, PhaMers scores out.
       .score_fasta(path)                      FASTA file -> (ids, scores), the phamer.py flow without the files
       .score_windows_device(seq, offsets, w, s)   scores of overlapping windows along each record, on the device
       .score_windows_fasta(path, w, s)        FASTA file -> (ids, record index, spans, scores) of the windows
+      .score_spans_device(seq, offsets, spans)    scores (and neighbours) of arbitrary (record, start, end) spans, on the device
+      .score_spans_fasta(path, ids, spans)    FASTA file + contig-named spans (a BED file) -> their scores on the host
 
 Stage by stage this is kmer.count_file -> kmer.normalize_counts -> phamer_scorer.score_points('combo')
 (reference scripts/phamer.py:131,139,194), with the k-mer length fixed at the width of the reference features.
@@ -19,6 +21,44 @@ import numpy as np
 import torch
 
 from . import _lib, ops, references
+
+
+def match_records(names, ids, tokens):
+    """Record index of every contig name: first among `ids` (the score file's ids, fileIO.get_id of each title), then, when no id
+    matches, among `tokens` (the titles' first whitespace tokens).  A name that matches no record, or more than one, is a ValueError
+    naming it."""
+    def index(keys):
+        table = {}
+        for r, key in enumerate(keys):
+            if key is not None:
+                table.setdefault(str(key), []).append(r)
+        return table
+    by_id, by_token = index(ids), index(tokens)
+    out = np.empty((len(names),), dtype=np.int64)
+    for i, name in enumerate(names):
+        hits = by_id.get(str(name)) or by_token.get(str(name))
+        if not hits:
+            raise ValueError("contig %r names no record of the FASTA file" % (name,))
+        if len(hits) > 1:
+            raise ValueError("contig %r names %d records of the FASTA file" % (name, len(hits)))
+        out[i] = hits[0]
+    return out
+
+
+def fasta_spans(path, ids, spans, lines=None):
+    """A FASTA file and contig-named spans (ids [n], spans [n, 2] start, end) -> (sequence bytes and offsets on the device, the span
+    table int64[n, 3] (record, start, end) on the device).  Names are matched by match_records; coordinates outside their record are
+    a ValueError naming lines[i] (where the span came from) when given."""
+    from . import fileIO
+    tokens, d_seq, d_off = fileIO.read_fasta_arrays_cuda(path)
+    records = match_records(ids, [fileIO.get_id(t) for t in tokens], tokens)
+    spans = np.asarray(spans, dtype=np.int64).reshape(-1, 2)
+    lengths = np.diff(d_off.cpu().numpy())
+    for i in np.flatnonzero((spans[:, 0] < 0) | (spans[:, 1] < spans[:, 0]) | (spans[:, 1] > lengths[records])):
+        where = lines[i] if lines is not None else "span %d" % i
+        raise ValueError("%s: [%d, %d) is not a range inside %s (%d bases)" % (where, spans[i, 0], spans[i, 1], ids[i], lengths[records[i]]))
+    table = np.ascontiguousarray(np.concatenate((records[:, None], spans), axis=1))
+    return d_seq, d_off, torch.from_numpy(table).cuda()
 
 
 class ContigScorer(object):
@@ -156,6 +196,45 @@ class ContigScorer(object):
         record = np.repeat(np.arange(len(ids), dtype=np.int64), np.diff(wo))
         keep = (np.diff(d_off.cpu().numpy()) >= length_requirement)[record]
         return ids[record[keep]], record[keep], spans[keep], scores[keep]
+
+    # -- spans ------------------------------------------------------------------------------------------
+    SPAN_SLICE = 1 << 20               # spans counted and scored per library call, as WINDOW_SLICE
+
+    def score_spans_device(self, seq, offsets, spans, method="combo", neighbors=False):
+        """Scores of arbitrary spans of the records (phm_kmer_count_spans, then the scorer on the count rows).  spans: int64 CUDA tensor
+        [n, 3] of (record, start, end), 0-based half-open in the record, any order.  A span scores exactly as its bases would as a
+        record of their own (score_fasta); one without a countable k-mer scores NaN.  Spans are counted and scored SPAN_SLICE at a
+        time, count rows on the count road where it takes them (k_neighbors in {1, 3, 5}), other shapes from feature rows normalised
+        by the same call.  Returns scores float64[n] on the device; with neighbors=True the tuple (scores, ref_index int64[n, k],
+        ref_distance, centroid_index int64[n, 2], centroid_distance) of ops.score_neighbors_cuda for the same rows."""
+        key = {"knn": 0, "kmeans": 1, "combo": 2}[method]
+        n_spans = spans.shape[0]
+        from_counts = (self.k_neighbors in (1, 3, 5) and self.refs.shape[1] in (256, 136)
+                       and self.cent_pos.shape[0] > 0 and self.cent_neg.shape[0] > 0)
+        parts = []
+        for first in range(0, n_spans, self.SPAN_SLICE):
+            part = spans[first:first + self.SPAN_SLICE]
+            counts, freq = ops.count_spans_cuda(seq, offsets, part, self.kmer_length, canonical=self.canonical, counts=from_counts,
+                                                freq=not from_counts)
+            args = (counts if from_counts else freq, self.refs, self.n_positive, self.cent_pos, self.cent_neg, self.k_neighbors)
+            out = ops.score_neighbors_cuda(*args) if neighbors else ops.score_cuda(*args)
+            parts.append((out[key],) + tuple(out[3:]))
+        if not parts:
+            parts = [(torch.empty((0,), dtype=torch.float64, device="cuda"), torch.empty((0, self.k_neighbors), dtype=torch.int64, device="cuda"),
+                      torch.empty((0, self.k_neighbors), dtype=torch.float64, device="cuda"),
+                      torch.empty((0, 2), dtype=torch.int64, device="cuda"), torch.empty((0, 2), dtype=torch.float64, device="cuda"))]
+        joined = tuple(torch.cat(col) for col in zip(*parts))
+        return joined if neighbors else joined[0]
+
+    def score_spans_fasta(self, path, ids, spans, method="combo", neighbors=False, lines=None):
+        """score_spans_device over the records of a FASTA file, spans named by contig: ids [n] names, spans int64[n, 2] (start, end).
+        A name is looked up among the score file's ids (fileIO.get_id of each title) first and, when none has it, among the titles'
+        first tokens (what BED files of other tools carry); a name that matches no record or several is a ValueError naming it, and
+        so are coordinates outside their record (naming lines[i], the span's source, when given).  Returns on the host what
+        score_spans_device returns, as numpy arrays."""
+        d_seq, d_off, table = fasta_spans(path, ids, spans, lines)
+        out = self.score_spans_device(d_seq, d_off, table, method=method, neighbors=neighbors)
+        return tuple(t.cpu().numpy() for t in out) if neighbors else out.cpu().numpy()
 
     def score_fasta(self, path, length_requirement=0, method="combo"):
         from . import fileIO
