@@ -259,16 +259,21 @@ int phm_count_score(const uint8_t *d_seq, const int64_t *d_offsets, int64_t n_co
 
 /* ---------------------------------------------------------------------------------------------
  * FASTA ingest on the device (the caller / data-format row either side of the path, SURVEY.md 8(f) rank 3).  Replaces the
- * tokenisation kmer.count_file gets from Bio.SeqIO (scripts/kmer.py:131-139; scripts/fileIO.py:28-42): a record starts at a
- * line beginning with '>', its sequence is every following line with '\n', '\r' and ' ' removed (k-mers span line breaks, never
- * records), text before the first '>' is ignored.  Two calls, so that the caller can size the outputs in between:
+ * tokenisation kmer.count_file gets from Bio.SeqIO over a text-mode handle (scripts/kmer.py:131-139; scripts/fileIO.py:28-42):
+ * a line ends at '\n', '\r' or "\r\n"; a record starts at a line beginning with '>', its sequence is every following line with
+ * '\n', '\r' and ' ' removed (k-mers span line breaks, never records), text before the first '>' is ignored.  Two calls, so that
+ * the caller can size the outputs in between:
  *
- *   phm_fasta_index    d_raw uint8[n_bytes] (16-byte aligned, allocation readable up to the next multiple of 16)
- *                      -> d_result int64[4]: [0] records, [1] sequence bytes, [2] 1 if the file holds a tab / VT / FF (the reference
- *                         strips those at line ends only: take the host path for such files), [3] internal
+ *   phm_fasta_index    d_raw uint8[n_bytes] (16-byte aligned, allocation readable up to the next multiple of 16; what the bytes
+ *                      past n_bytes hold does not matter)
+ *                      -> d_result int64[4]: [0] records, [1] sequence bytes, [2] 1 if the file holds a control byte other than
+ *                         '\n' '\r' (tab / VT / FF / 0x1C-0x1F among them; the reference strips those at line ends only: take
+ *                         the host path for such files), [3] internal
  *   phm_fasta_extract  -> d_seq uint8[result[1]] sequence bytes end to end (ready for phm_kmer_count), d_offsets int64[records + 1],
  *                         d_header_pos int64[records] byte position of each record's '>' in the file (the host reads the titles
- *                         there); records beyond max_records are dropped
+ *                         there); records beyond max_records are dropped: then d_offsets[max_records] is the start of the first
+ *                         dropped record (the end of the last kept one), and nothing past d_offsets[max_records] or
+ *                         d_header_pos[max_records - 1] is written
  * Both use the same d_workspace (phm_fasta_workspace_bytes), which must stay untouched between them.
  * ------------------------------------------------------------------------------------------- */
 size_t phm_fasta_workspace_bytes(int64_t n_bytes);

@@ -16,6 +16,8 @@ Third-party arithmetic the reference delegates to scikit-learn (unpinned in requ
 KNeighborsClassifier (scripts/learning.py:127-128) and KMeans (scripts/learning.py:138).
 """
 import gzip
+import re
+
 import numpy as np
 
 DNA = "ATGC"          # scripts/kmer.py:28 -- bin order A=0 T=1 G=2 C=3, first base most significant
@@ -120,10 +122,12 @@ def normalize_counts(counts):
 
 # ---- FASTA tokenisation (Biopython SimpleFastaParser semantics; scripts/kmer.py:135) ----
 def parse_fasta_text(text):
-    """Yields (title, sequence).  A record starts at a line starting with '>'; the sequence is
-    every later line rstripped and joined with blanks and CR removed."""
+    """Yields (title, sequence).  Lines end as a text-mode file (universal newlines) ends them:
+    at '\\r\\n', a lone '\\r' or '\\n'.  A record starts at a line starting with '>'; the sequence is
+    every later line rstripped and joined with blanks and CR removed.  Inputs are ASCII: under
+    UTF-8, str.rstrip() would also strip non-ASCII whitespace, which is not restated here."""
     title, chunks = None, []
-    for line in text.split("\n"):
+    for line in re.split("\r\n|\r|\n", text):
         if line.startswith(">"):
             if title is not None:
                 yield title, "".join(chunks).replace(" ", "").replace("\r", "")

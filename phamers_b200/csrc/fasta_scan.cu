@@ -2,13 +2,18 @@
 // positions, i.e. the tokenisation kmer.count_file gets from Bio.SeqIO (reference scripts/kmer.py:131-139, scripts/fileIO.py:28-42)
 // and that phamers_b200/fileIO.py::split_fasta_bytes restates on the host.
 //
-// Semantics (Bio.SeqIO FASTA parser as the reference uses it): a record starts at a line whose first byte is '>'; its sequence is
-// every following line up to the next such line, with line feeds, carriage returns and blanks removed -- k-mers span line breaks but
-// never records; text before the first '>' is ignored.  Tab / VT / FF are stripped by the reference only at line ends, which this
-// scan does not model: it reports their presence (result[2]) and the caller takes the exact host path for such (rare) files.
+// Semantics (Bio.SeqIO FASTA parser over a text-mode handle, as the reference uses it): a line ends at '\n', '\r' or "\r\n"
+// (universal newlines); a record starts at a line whose first byte is '>'; its sequence is every following line up to the next such
+// line, with line feeds, carriage returns and blanks removed -- k-mers span line breaks but never records; text before the first '>'
+// is ignored.  Tab / VT / FF / 0x1C-0x1F are stripped by the reference only at line ends (str.rstrip), which this scan does not
+// model: it reports any control byte other than '\n' '\r' (result[2]) and the caller takes the exact host path for such (rare) files.
+// The input allocation is readable up to the next multiple of 16 bytes; what those padding bytes hold does not matter, they read as
+// '\n'.
 //
 // Every byte is in one of three line states: 0 = preamble (no header seen yet), 1 = inside a header line, 2 = inside a sequence line.
-// A line start (first byte of the file, or the byte after '\n') moves the state: '>' -> 1; anything else: 1 -> 2, 0 and 2 stay.
+// A line start (first byte of the file, or the byte after '\n' or '\r') moves the state: '>' -> 1; anything else: 1 -> 2, 0 and 2
+// stay.  So the '\n' of "\r\n" starts an empty line, which keeps nothing and moves 1 -> 2 as the next real line would: LF and CRLF
+// files give the same outputs as with '\n' alone as the line end.
 // A byte is KEPT iff its state is 2 and it is none of '\n' '\r' ' '.  The state of a byte depends on everything before it, so the
 // scan works on state MAPS (3 states -> 3 states, 6 bits), whose composition is associative:
 //   pass 1  fasta_tile_kernel    per 16 KB tile: its map, the kept count for each incoming state, its number of header starts
@@ -58,10 +63,10 @@ __device__ __forceinline__ uint32_t zero_bytes(uint32_t x) {
 __device__ __forceinline__ uint32_t gather4(uint32_t z) { return (((z >> 7) * 0x00204081u) >> 21) & 0xFu; }
 
 struct Masks {
-    uint32_t nl;      // byte is '\n' (bytes at or past the end of the file count as '\n')
+    uint32_t nl;      // byte ends a line: '\n' or '\r' (bytes at or past the end of the file count as '\n')
     uint32_t keep;    // byte is none of '\n' '\r' ' '
-    uint32_t odd;     // non-zero: a control byte other than '\n' '\r' (tab / VT / FF among them) is present
-    uint32_t w[4];    // the bytes themselves
+    uint32_t odd;     // non-zero: a control byte other than '\n' '\r' (tab / VT / FF / 0x1C-0x1F among them) is present
+    uint32_t w[4];    // the bytes themselves, those past the end of the file replaced by '\n'
 };
 
 __device__ __forceinline__ Masks classify16(const uint8_t *raw, int64_t n, int64_t i0) {
@@ -76,18 +81,24 @@ __device__ __forceinline__ Masks classify16(const uint8_t *raw, int64_t n, int64
     for (int q = 0; q < 4; ++q) {
         const uint32_t z_nl = zero_bytes(m.w[q] ^ 0x0A0A0A0Au), z_cr = zero_bytes(m.w[q] ^ 0x0D0D0D0Du), z_sp = zero_bytes(m.w[q] ^ 0x20202020u);
         const uint32_t z_ctrl = zero_bytes(m.w[q] & 0xE0E0E0E0u);                    // bytes 0..31
-        nl |= gather4(z_nl) << (4 * q);
+        nl |= gather4(z_nl | z_cr) << (4 * q);
         drop |= gather4(z_nl | z_cr | z_sp) << (4 * q);
         m.odd |= z_ctrl & ~(z_nl | z_cr);
     }
     m.nl = nl;
     m.keep = ~drop & 0xFFFFu;
-    if (i0 + PER_THREAD > n) {                                       // last chunk of the file: the tail reads as '\n'
-        const int n_valid = (int)(n - i0);
+    if (i0 + PER_THREAD > n) {                   // last chunk of the file: the bytes past the end are caller padding of any content;
+        const int n_valid = (int)(n - i0);       // they are replaced by '\n', so no later reader (header_starts, byte_at, s_bytes) sees them
         const uint32_t valid = (1u << n_valid) - 1u;
         m.nl = (m.nl & valid) | (~valid & 0xFFFFu);
         m.keep &= valid;
-        m.odd = 0u;                                                  // the bytes past the end are caller padding, not file content
+        m.odd = 0u;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int v = n_valid - 4 * q;                           // valid bytes of word q
+            const uint32_t lo = v <= 0 ? 0u : (v >= 4 ? 0xFFFFFFFFu : (1u << (8 * v)) - 1u);
+            m.w[q] = (m.w[q] & lo) | (0x0A0A0A0Au & ~lo);
+        }
         for (int j = 0; j < n_valid; ++j) {
             const uint32_t c = (m.w[j >> 2] >> (8 * (j & 3))) & 255u;
             m.odd |= (c < 32u && c != 10u && c != 13u) ? 1u : 0u;
@@ -100,9 +111,10 @@ __device__ __forceinline__ uint32_t byte_at(const Masks &m, int j) {
     const uint32_t lo = (j & 4) ? m.w[1] : m.w[0], hi = (j & 4) ? m.w[3] : m.w[2];
     return (((j & 8) ? hi : lo) >> (8 * (j & 3))) & 255u;
 }
-// line starts of this thread's 16 bytes: the byte after a '\n' (the first byte of the file starts a line)
+// line starts of this thread's 16 bytes: the byte after a '\n' or '\r' (the first byte of the file starts a line)
 __device__ __forceinline__ uint32_t line_starts(const uint8_t *raw, int64_t n, int64_t i0, uint32_t nl) {
-    const uint32_t prev_nl = (i0 == 0 || i0 > n || raw[i0 - 1] == 10u) ? 1u : 0u;
+    const uint32_t prev = (i0 == 0 || i0 > n) ? 10u : raw[i0 - 1];
+    const uint32_t prev_nl = (prev == 10u || prev == 13u) ? 1u : 0u;
     return ((nl << 1) | prev_nl) & 0xFFFFu;
 }
 // which line starts are header starts ('>' as first byte of the line)
@@ -198,7 +210,7 @@ __global__ void __launch_bounds__(TILE_THREADS) fasta_tile_kernel(const uint8_t 
 // ---------------- pass 2: one CTA chains the tiles ----------------
 // Warp w owns a contiguous range of tiles and walks it 32 tiles at a time (lane = tile: coalesced loads, warp-shuffle scans), three
 // times: the range as one map; its totals once the state it starts in is known; every tile's start.
-// result[0] = records, [1] = sequence bytes kept, [2] = 1 if a tab / VT / FF was seen, [3] = tiles
+// result[0] = records, [1] = sequence bytes kept, [2] = 1 if a control byte other than '\n' '\r' was seen, [3] = tiles
 __global__ void __launch_bounds__(1024) fasta_chain_kernel(const TileSummary *__restrict__ tiles, int64_t n_tiles,
                                                            TileStart *__restrict__ starts, int64_t *__restrict__ result) {
     __shared__ uint32_t s_map[32];
@@ -351,14 +363,13 @@ __global__ void __launch_bounds__(TILE_THREADS) fasta_emit_kernel(const uint8_t 
         }
         __syncthreads();
         const uint32_t kpos = ki - nk + s_k[warp], hpos = hi - nh + s_h[warp];
-        // 3. records that start here: offset = kept bytes before the header, position of its '>'
+        // 3. records that start here: offset = kept bytes before the header, position of its '>'.  With max_records < records,
+        //    offsets[max_records] is the start of the first dropped record, which is where the last kept one ends.
         int64_t r = ts.rec_base + hpos;
         for (uint32_t hm = hs; hm; hm &= hm - 1u, ++r) {
             const int j = __ffs(hm) - 1;
-            if (r < max_records) {
-                offsets[r] = ts.seq_base + kpos + __popc(keep_mask & ((1u << j) - 1u));
-                header_pos[r] = i0 + j;
-            }
+            if (r <= max_records) offsets[r] = ts.seq_base + kpos + __popc(keep_mask & ((1u << j) - 1u));
+            if (r < max_records) header_pos[r] = i0 + j;
         }
         // 4. the kept bytes: compacted in shared memory, then written as whole 16-byte words (a byte store costs a full 32-byte sector
         //    transaction in L2, and that -- not DRAM -- bounded the first version of this kernel)

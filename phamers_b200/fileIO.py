@@ -56,7 +56,7 @@ def get_id(header):
 # ----------------------------------------------------------------------------------------------------------
 # FASTA
 # ----------------------------------------------------------------------------------------------------------
-_TRAILING = b" \t\n\r\x0b\x0c"
+_TRAILING = b" \t\n\r\x0b\x0c\x1c\x1d\x1e\x1f"      # str.isspace over ASCII: what str.rstrip() strips at a line end
 
 
 def _open_bytes(path):
@@ -69,21 +69,21 @@ def _open_bytes(path):
 
 def split_fasta_bytes(raw):
     """FASTA bytes -> (record ids [first blank-separated token of each title], uint8 array of all sequence bytes end
-    to end, int64 offsets[n+1]).  Tokenisation follows Bio.SeqIO's FASTA parser as the reference uses it
-    (scripts/kmer.py:135): a record starts at a line beginning with '>', its sequence is every following line
-    right-stripped and joined, with blanks and carriage returns removed -- so k-mers span line breaks but never
-    records.  Text before the first '>' is ignored."""
+    to end, int64 offsets[n+1]).  Tokenisation follows Bio.SeqIO's FASTA parser over a text-mode handle as the reference
+    uses it (scripts/kmer.py:135): a line ends at '\n', '\r' or '\r\n' (universal newlines); a record starts at a line
+    beginning with '>', its sequence is every following line right-stripped and joined, with blanks removed -- so k-mers
+    span line breaks but never records.  Text before the first '>' is ignored."""
     data = np.frombuffer(raw, dtype=np.uint8)
     n = data.shape[0]
     if n == 0:
         return [], np.zeros(0, dtype=np.uint8), np.zeros(1, dtype=np.int64)
-    newline = np.flatnonzero(data == 10)
+    newline = np.flatnonzero((data == 10) | (data == 13))          # line terminators: LF and CR
     line_start = np.concatenate(([0], newline + 1))
     line_start = line_start[line_start < n]
     header_start = line_start[data[line_start] == ord(">")]
     if header_start.shape[0] == 0:
         return [], np.zeros(0, dtype=np.uint8), np.zeros(1, dtype=np.int64)
-    # end of each header line (position of its '\n', or n)
+    # end of each header line (position of its '\n' or '\r', or n)
     idx = np.searchsorted(newline, header_start)
     if newline.shape[0]:
         header_end = np.where(idx < newline.shape[0], newline[np.minimum(idx, newline.shape[0] - 1)], n)
@@ -98,12 +98,12 @@ def split_fasta_bytes(raw):
         tokens = title.split(None, 1)
         ids.append(tokens[0] if tokens else "")
 
-    if any(c in raw for c in (b"\t", b"\x0b", b"\x0c")):
-        # rare: tab / VT / FF are stripped only at line ends -- exact line-by-line path
+    if any(c in raw for c in (b"\t", b"\x0b", b"\x0c", b"\x1c", b"\x1d", b"\x1e", b"\x1f")):
+        # rare: tab / VT / FF / 0x1C-0x1F are stripped only at line ends -- exact line-by-line path
         pieces, lengths = [], []
         for bs, be in zip(body_start, body_end):
-            body = b"".join(line.rstrip(_TRAILING) for line in raw[bs:be].split(b"\n"))
-            body = body.replace(b" ", b"").replace(b"\r", b"")
+            body = b"".join(line.rstrip(_TRAILING) for line in raw[bs:be].splitlines())
+            body = body.replace(b" ", b"")
             pieces.append(body)
             lengths.append(len(body))
         seq = np.frombuffer(b"".join(pieces), dtype=np.uint8)
@@ -151,8 +151,8 @@ def read_fasta_arrays_cuda(fasta_file):
     """Device-side tokenisation of a FASTA file (phm_fasta_index / phm_fasta_extract): the file is memory-mapped, its bytes go
     to the GPU once through pinned staging buffers and the sequence bytes never come back; only the title lines are read on the
     host, at the positions the device reports.  Returns (titles' first tokens, CUDA uint8 tensor of all sequence bytes end to end
-    [padded to 16], CUDA int64 offsets[n+1]).  Files holding a tab / VT / FF (stripped by the reference at line ends only) are
-    tokenised by the exact host path and uploaded.  Raises IOError when unreadable."""
+    [padded to 16], CUDA int64 offsets[n+1]).  Files holding a control byte other than '\n' '\r' (tab / VT / FF / 0x1C-0x1F are
+    stripped by the reference at line ends only) are tokenised by the exact host path and uploaded.  Raises IOError when unreadable."""
     import mmap
     import torch
     from . import ops
@@ -178,8 +178,11 @@ def read_fasta_arrays_cuda(fasta_file):
             return ids, pad.cuda(), torch.from_numpy(np.ascontiguousarray(h_off)).cuda()
         ids = []
         for hs in header_pos.cpu().tolist():
-            he = raw.find(b"\n", hs)
-            title = bytes(raw[hs + 1:(he if he >= 0 else n)]).decode("latin-1").rstrip()
+            he = n
+            for eol in (b"\n", b"\r"):                                  # the title line ends at the first '\n' or '\r'
+                e = raw.find(eol, hs, he)
+                he = e if e >= 0 else he
+            title = bytes(raw[hs + 1:he]).decode("latin-1").rstrip()
             tokens = title.split(None, 1)
             ids.append(tokens[0] if tokens else "")
         return ids, seq, offsets

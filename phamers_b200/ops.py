@@ -335,7 +335,8 @@ def fasta_scan_cuda(raw):
     """FASTA bytes on the device (contiguous CUDA uint8 tensor, 16-byte aligned) -> (seq uint8 [bases] end to end,
     offsets int64 [records + 1], header_pos int64 [records], odd_whitespace bool).  `seq` is padded to a multiple of 16
     bytes for phm_kmer_count.  One host synchronisation (the outputs are sized from the index pass).  When odd_whitespace is
-    True (tab / VT / FF in the file) the reference strips those bytes at line ends only: use the host tokeniser."""
+    True (a control byte other than '\n' '\r' in the file: tab / VT / FF / 0x1C-0x1F are stripped by the reference at line
+    ends only) use the host tokeniser.  The bytes of raw's storage past its end may hold anything."""
     lib = _lib.require_cuda()
     raw = _as_u8_cuda(raw)
     n = raw.numel()

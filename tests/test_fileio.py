@@ -1,5 +1,6 @@
 """Host-side formats either side of the path (FASTA tokenisation, feature CSV, score CSV, id parsing).  CPU only."""
 import gzip
+import io
 import os
 
 import numpy as np
@@ -83,12 +84,13 @@ def test_host_helpers():
 
 
 def test_host_tokeniser_property():
-    """Random files over the bytes that matter to the FASTA tokeniser ('>', line feeds, CR, blanks, tabs, letters): the vectorised
-    host tokeniser agrees with the oracle's line-by-line restatement of the Bio.SeqIO parser on every one of them."""
+    """Random files over the bytes that matter to the FASTA tokeniser ('>', line feeds, CR, blanks, tabs, VT, the separators 0x1C
+    and 0x1F that str.rstrip() strips, letters): the host tokeniser agrees with the oracle's line-by-line restatement of the
+    Bio.SeqIO parser on every one of them."""
     from hypothesis import given, settings, strategies as st
 
     @settings(max_examples=400, deadline=None)
-    @given(st.text(alphabet=">\n\r \tACGTNacgt|_1", min_size=0, max_size=200))
+    @given(st.text(alphabet=">\n\r \t\x0b\x1c\x1fACGTNacgt|_1", min_size=0, max_size=200))
     def check(text):
         raw = text.encode("latin-1")
         ids, seq, off = fileIO.split_fasta_bytes(raw)
@@ -98,3 +100,45 @@ def test_host_tokeniser_property():
         assert got == [s for _, s in want]
 
     check()
+
+
+def test_oracle_reads_lines_as_a_text_mode_file():
+    """parse_fasta_text splits lines as the reference's text-mode handle does (universal newlines: CRLF, a lone CR and LF each end
+    a line), so it agrees with Biopython's SimpleFastaParser run over such a handle, restated here on the handle's own lines."""
+    rng = np.random.default_rng(5)
+    alphabet = np.frombuffer(b">>\n\n\r\r \t\x0b\x0c\x1c\x1fACGTNacgt_1", dtype=np.uint8)
+    cases = [b">a_ID_1 desc\rACGTAC\r>b_ID_2\nAC\x1c\nGT\n", b"\r\r\n>x\r\r\nA\rC\r\n\r>y", b">a\r", b">a\r\n\r\nGG \t\r"]
+    cases += [rng.choice(alphabet, size=int(rng.integers(0, 120))).tobytes() for _ in range(300)]
+    for raw in cases:
+        title, chunks, want = None, [], []
+        for line in io.TextIOWrapper(io.BytesIO(raw), encoding="latin-1", newline=None):
+            if line.startswith(">"):
+                if title is not None:
+                    want.append((title, "".join(chunks).replace(" ", "").replace("\r", "")))
+                title, chunks = line[1:].rstrip(), []
+            elif title is not None:
+                chunks.append(line.rstrip())
+        if title is not None:
+            want.append((title, "".join(chunks).replace(" ", "").replace("\r", "")))
+        assert list(po.parse_fasta_text(raw.decode("latin-1"))) == want, raw
+
+
+def test_lone_carriage_returns_and_separators_at_line_ends(tmp_path):
+    """A lone CR ends a line (a classic-Mac file holds several records, not one), and 0x1C-0x1F at a line end are stripped as
+    str.rstrip() strips them: the host tokeniser, the file readers and the oracle agree."""
+    raw = b">a_ID_1 desc\rACGTAC\r>b_ID_2\nAC\x1c\nGT\n"
+    want = [("a_ID_1 desc", "ACGTAC"), ("b_ID_2", "ACGT")]
+    assert list(po.parse_fasta_text(raw.decode("latin-1"))) == want
+    ids, seq, off = fileIO.split_fasta_bytes(raw)
+    assert ids == ["a_ID_1", "b_ID_2"] and [seq.tobytes()[off[i]:off[i + 1]] for i in range(2)] == [b"ACGTAC", b"ACGT"]
+    path = tmp_path / "mac.fasta"
+    path.write_bytes(raw)
+    ids, seqs = fileIO.read_fasta(str(path))
+    ref_ids, ref_seqs = po.read_fasta(str(path))
+    assert list(ids) == list(ref_ids) == ["1", "2"] and seqs == ref_seqs == ["ACGTAC", "ACGT"]
+    for raw, want in ((b">a\rAC\t\rGT\r\n>b\r\r\nT T\x1f\r", [b"ACGT", b"TT"]),      # tab before a lone CR: exact path
+                      (b">a\r\r\nAC\rGT\x0b\n\r>b\nA\x1dC\n", [b"ACGT", b"A\x1dC"]),   # a separator inside a line is kept
+                      (b">a\rAC\rG\rT\r>b\rCC\r", [b"ACGT", b"CC"])):                    # fast path, CR only
+        ids, seq, off = fileIO.split_fasta_bytes(raw)
+        assert [seq.tobytes()[off[i]:off[i + 1]] for i in range(len(ids))] == want
+        assert [s.encode("latin-1") for _, s in po.parse_fasta_text(raw.decode("latin-1"))] == want
