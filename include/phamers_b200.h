@@ -174,7 +174,8 @@ int phm_normalize_rows(const double *d_rows, int64_t n_rows, int64_t bins, doubl
  *     d_combo         float64[n_points]  knn + kmeans                     (may be NULL)
  *     A query row holding NaN (zero-count contig) gets NaN in all three outputs.
  *
- *     Two device paths, same results: for dim = 256 or 136 and k_neighbors in {1, 3, 5} the (query x reference) contraction runs on
+ *     Two device paths, same results: for dim = 256, 136, 1024 or 512 and k_neighbors in {1, 3, 5} the (query x reference)
+ *     contraction runs on
  *     the tcgen05 tensor cores (FP16 operands, FP32 accumulation) together with a proven per-pair error interval; the few
  *     references / centroids whose interval can reach the k nearest are kept per query and decided exactly in float64.
  *     Rows whose candidate buffer overflows (and every other shape) go through the exhaustive float64 kernel.
@@ -183,6 +184,9 @@ int phm_normalize_rows(const double *d_rows, int64_t n_rows, int64_t bins, doubl
  *     first 136 columns of the 256-wide FP16 operands and the rest is zero, under the same error bound.  At dim = 136 count rows
  *     (phm_score_counts) take the tensor cores; float64 feature rows keep the exhaustive kernel unless option "score_path" = 2,
  *     because the two roads may order exact distance ties differently and phm_score's answers at 136 stay what they were.
+ *     dim = 1024 and 512 are the widths of plain and canonical 5-mer features: their FP16 operands are that wide (the workspace
+ *     grows with them, phm_score_workspace_bytes takes dim).  As at 136, count rows take the tensor cores and float64 feature rows
+ *     keep the exhaustive kernel unless option "score_path" = 2.
  * ------------------------------------------------------------------------------------------- */
 size_t phm_score_workspace_bytes(int64_t n_points, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg, int dim);
 int phm_score(const double *d_points, int64_t n_points, int dim,
@@ -194,7 +198,8 @@ int phm_score(const double *d_points, int64_t n_points, int dim,
 /* Stages 2 + 3 fused: same as phm_score, but the queries are the raw uint32 count rows of phm_kmer_count (d_counts[n_points * dim]);
  * every kernel forms feature = count / row total in float64 on the fly, exactly as kmer.normalize_counts would
  * (scripts/kmer.py:209-221, scripts/phamer.py:139), so the float64 feature matrix never exists in memory.  Needs the
- * tensor-core shape (dim = 256 or 136 -- plain or canonical 4-mer counts --, k_neighbors in {1, 3, 5}, both centroid sets),
+ * tensor-core shape (dim = 256 or 136 -- plain or canonical 4-mer counts --, 1024 or 512 -- plain or canonical 5-mer counts --,
+ * k_neighbors in {1, 3, 5}, both centroid sets),
  * PHM_E_UNSUPPORTED otherwise. */
 int phm_score_counts(const uint32_t *d_counts, int64_t n_points, int dim,
                      const double *d_refs, int64_t n_refs, int64_t n_positive,

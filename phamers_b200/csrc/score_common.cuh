@@ -92,9 +92,13 @@ struct QueryEmit {             // where a producer of 256-wide count rows writes
 };
 constexpr int PREP_DIM = 256;               // width of the FP16 operands
 constexpr int CANON_DIM = 136;              // canonical 4-mer features: written into the first 136 operand columns, the rest stays zero
+constexpr int KMER5_DIM = 1024;             // plain 5-mer features: operands 1024 wide (score_tc.cu streams the query tile)
+constexpr int CANON5_DIM = 512;             // canonical 5-mer features: operands 512 wide
 constexpr double PREP_SCALE = 4096.0;
 // feature widths the tensor-core scorer takes
-__host__ __device__ constexpr bool tc_width(int dim) { return dim == PREP_DIM || dim == CANON_DIM; }
+__host__ __device__ constexpr bool tc_width(int dim) {
+    return dim == PREP_DIM || dim == CANON_DIM || dim == KMER5_DIM || dim == CANON5_DIM;
+}
 // a W-wide float64 row spread over a warp: lane l holds features l, l + 32, ... (NCH<W> chunks); in_row is false for the chunk
 // slots beyond W, which read nothing and contribute exactly zero
 template <int W> constexpr int NCH = (W + 31) / 32;
@@ -161,7 +165,7 @@ __device__ __forceinline__ float query_crow(double sc, double sd, double sh, flo
 int score_tc_begin(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, QueryEmit *emit);
 int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, bool queries_prepared);
 bool score_tc_supported(int dim, int k_neighbors, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg);
-size_t score_tc_workspace_bytes(int64_t n_points, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg);
+size_t score_tc_workspace_bytes(int64_t n_points, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg, int dim);
 int score_tc(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st);
 int score_tc_last_ms(float *ms);
 int score_decide_last_ms(float *ms);

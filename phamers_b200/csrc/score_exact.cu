@@ -273,8 +273,8 @@ using namespace phm;
 
 extern "C" size_t phm_score_workspace_bytes(int64_t n_points, int64_t n_refs, int64_t n_cent_pos, int64_t n_cent_neg, int dim) {
     const size_t exact = (size_t)(n_points + n_refs + n_cent_pos + n_cent_neg + 8) * sizeof(double);
-    if (tc::tc_width(dim)) {                    // 256 or 136: the FP16 operands are 256 wide either way
-        const size_t tcb = tc::score_tc_workspace_bytes(n_points, n_refs, n_cent_pos, n_cent_neg);
+    if (tc::tc_width(dim)) {                    // 256 or 136: 256-wide FP16 operands; 512 or 1024: operands of that width
+        const size_t tcb = tc::score_tc_workspace_bytes(n_points, n_refs, n_cent_pos, n_cent_neg, dim);
         return tcb > exact ? tcb : exact;
     }
     return exact;
@@ -311,15 +311,19 @@ static int score_any(const double *d_points, const uint32_t *d_point_counts, int
     }
 
     const bool tc_ok = tc::score_tc_supported(dim, k_neighbors, n_refs, n_cent_pos, n_cent_neg);
-    if (score_path == 2 && !tc_ok) { set_error("tensor-core scoring needs dim = 256 or 136, k_neighbors in {1, 3, 5} and both centroid sets"); return PHM_E_UNSUPPORTED; }
-    // Float64 feature rows 136 wide keep the exhaustive kernel unless tensor cores are required: it was their road before the
-    // tensor-core road took width 136, and the two roads order exact distance ties differently (norm expansion against direct
-    // difference), so this keeps phm_score's answers at width 136 as they were.  Count rows (phm_score_counts) take the tensor cores.
+    if (score_path == 2 && !tc_ok) {
+        set_error("tensor-core scoring needs dim = 256, 136, 512 or 1024, k_neighbors in {1, 3, 5} and both centroid sets");
+        return PHM_E_UNSUPPORTED;
+    }
+    // Float64 feature rows 136, 512 or 1024 wide keep the exhaustive kernel unless tensor cores are required: it was their road
+    // before the tensor-core road took those widths, and the two roads order exact distance ties differently (norm expansion against
+    // direct difference), so this keeps phm_score's answers at those widths as they were.  Count rows (phm_score_counts) take the
+    // tensor cores.
     const bool tc_auto = tc_ok && (dim == tc::PREP_DIM || d_point_counts != nullptr);
     if ((score_path == 0 && tc_auto) || (score_path == 2 && tc_ok)) return tc::score_tc(a, d_workspace, workspace_bytes, st);
     if (d_point_counts) {
-        set_error("scoring from raw counts needs the tensor-core path (dim = 256 or 136, k_neighbors in {1, 3, 5}, both centroid sets); "
-                  "normalise first (phm_normalize_counts) and call phm_score");
+        set_error("scoring from raw counts needs the tensor-core path (dim = 256, 136, 512 or 1024, k_neighbors in {1, 3, 5}, both centroid "
+                  "sets); normalise first (phm_normalize_counts) and call phm_score");
         return PHM_E_UNSUPPORTED;
     }
 

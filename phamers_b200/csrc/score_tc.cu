@@ -9,6 +9,11 @@
 // Canonical 4-mer features (136 wide) take the same road: a row fills the first 136 operand columns, centred by 1/136, and the
 // other 120 columns are exactly zero on both sides, so the contraction kernel is the same and every bound below holds for the
 // 136-wide vectors.  Every kernel that reads float64 or count rows takes the width as its template parameter W.
+// 5-mer features (1024 plain, 512 canonical) take operands of their own width (OPW<W> = W, NK = W / 64 K-chunks); the query tile
+// is then streamed through the ring with the reference blocks instead of staying resident (score_tc_kernel<KN, LIST, NK>).  The
+// bound below is stated for any width: |b'|^2 = |b|^2 - 1/W < 1 keeps the three-way split of nbs exact, every scaled centred feature
+// lies in (-2^12/W, 2^12) inside the FP16 range, and FP16 rounds 5-mer values (about 4x smaller) with the same relative error, so
+// the scale 2^12 stays; only the accumulation allowance grows with the number of MMAs (see eps_acc).
 //
 // The a.b term is a dense contraction and runs as ONE tcgen05.mma pass (kind::f16, FP32 accumulators in tensor memory) over
 // operands that are centred by 1/256 (distances are translation invariant), scaled by 2^12 and rounded to FP16.  FP16 x FP16
@@ -19,7 +24,10 @@
 //     B = fp16(B~), B~ = 2^12 (b - 1/256)   dB = |B~ - B|_2 , P  = |B~|_2         (per reference)
 //     A~.B~ - A.B = (A~ - A).B~ + A.(B~ - B)         =>   |A~.B~ - acc| <= dA P + nA dB + eps_acc nA (P + dB)
 //
-// (Cauchy-Schwarz; eps_acc = 2^-16 covers 16 FP32-accumulated MMAs, measured usage of the whole bound <= 0.4.)  With
+// (Cauchy-Schwarz; eps_acc = 2^-16 covers 16 FP32-accumulated MMAs, measured usage of the whole bound <= 0.4.)  The allowance
+// is 2^-20 of |A| |B| per accumulating MMA of K = 16 (16x the 2^-24 of one FP32 add, for the tensor core's own accumulation order):
+// a sum of m such steps errs by at most m 2^-20 sum_i |A_i B_i| <= m 2^-20 |A| |B|, so with NK K-chunks of 64 (4 NK MMAs)
+// eps_acc = NK 2^-18: 2^-16 at 256 (NK = 4), 2^-15 at 512, 2^-14 at 1024 (EPS_ACC_OF).  With
 // rho = max_j (dB_j + eps_acc (P_j + dB_j)) / P_j over the reference set this collapses to   err_j <= C_row * P_j  with ONE
 // constant per contig row.  The ranking value x_j = 2^23 |b_j - u|^2 - acc_j therefore pins the exact value inside
 // [lo_j, up_j] = [x_j - C P_j, x_j + C P_j].  A reference can be one of the k nearest only if lo_j <= (k-th smallest up);
@@ -32,6 +40,7 @@
 // Kernel layout (one CTA per SM, persistent over 256-contig tiles, 10 warps):
 //   warp 0    TMA producer   A tile (256 contigs x 256 features FP16, 128 KB, SWIZZLE_128B) once per contig tile;
 //                            B blocks (128 references x 64 features, 16 KB) through a 4-deep mbarrier ring
+//                            (NK > 4: no resident A; every ring stage holds a B block and both 16 KB A halves of its K-chunk)
 //   warp 1    MMA issuer     one elected lane: per B block 2 x 4 tcgen05.mma (128x128x16), i.e. two 128-row halves share every
 //                            B block, into one of two 2 x 128-column accumulator sets (all 512 TMEM columns);
 //                            tcgen05.commit frees the block / publishes the accumulator set
@@ -93,6 +102,19 @@ constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)
 // block of a reference tile and the two blocks of the contig tile travel together in a fifth slot of the B ring per tile.
 constexpr int XK = 16;
 constexpr int XBLK_BYTES = BM * XK * 2;   // 4 KB
+// 5-mer rows (W = 512, 1024) take operands of their own width: NK = W / 64 K-chunks.  A 256-row A tile is then 256 or 512 KB and
+// cannot stay resident, so A is STREAMED: each ring stage carries the reference block and the two 128-row A halves of one K-chunk
+// (48 KB), and A is read from L2 once per reference tile.  NK = NKC keeps the resident-A kernel exactly as it is.
+template <int W> constexpr int OPW = W <= KDIM ? KDIM : W;           // FP16 operand width of W-wide rows
+template <int W> constexpr int NK_OF = OPW<W> / BK;                  // its K-chunks
+template <int NK> constexpr bool STREAM_A = NK > NKC;
+template <int NK> constexpr int STAGE_BYTES = STREAM_A<NK> ? 3 * BLOCK_BYTES : BLOCK_BYTES;   // [B block][A half 0][A half 1]
+template <int NK> constexpr int SMEM_BYTES_OF = (STREAM_A<NK> ? 0 : A_BYTES) + NSTAGE * STAGE_BYTES<NK> + CAND_BYTES + STG_BYTES + BAR_BYTES;
+// FP32 accumulation allowance for 4 NK MMAs of K = 16 (2^-20 of |A| |B| per MMA): 2^-16 at NK = 4, 2^-15 at 8, 2^-14 at 16
+template <int NK> constexpr double EPS_ACC_OF = (double)NK / 262144.0;
+static_assert(SMEM_BYTES_OF<NKC> == SMEM_BYTES && EPS_ACC_OF<NKC> == EPS_ACC, "the 256-wide kernel keeps its layout and bound");
+static_assert(SMEM_BYTES_OF<8> <= 232448 && SMEM_BYTES_OF<16> <= 232448, "shared memory budget of one sm_100 CTA (streamed A)");
+static_assert(NSTAGE * STAGE_BYTES<16> % 1024 == 0 && (3 * BLOCK_BYTES) % 1024 == 0, "SWIZZLE_128B blocks stay 1024-byte aligned");
 constexpr int XBLK_HALVES = XBLK_BYTES / 2;
 static_assert(3 * XBLK_BYTES <= BLOCK_BYTES, "the extra operands of a tile fit one ring slot");
 __host__ __device__ __forceinline__ int64_t xrow_offset(int64_t row) {      // in halves, K half 0 (K half 1, all zero, is 64 halves further)
@@ -428,14 +450,16 @@ __device__ __forceinline__ TcSchedule tc_schedule(const TcParams &p) {
     return s;
 }
 
-template <int KN, bool LIST>
+template <int KN, bool LIST, int NK = NKC>
 __global__ void __launch_bounds__(NTHREADS, 1)
 score_tc_kernel(const __grid_constant__ CUtensorMap map_a, TcParams p) {
+    constexpr bool STREAM = STREAM_A<NK>;
+    constexpr int SB = STAGE_BYTES<NK>;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     const uint32_t smem_base = smem_u32(smem_raw);
-    const uint32_t sm_a = smem_base;                                   // [half 0..1][chunk 0..3] blocks of 16 KB
-    const uint32_t sm_b = smem_base + A_BYTES;                         // NSTAGE blocks
-    const uint32_t sm_cand = sm_b + NSTAGE * BLOCK_BYTES;              // [16 entries][256 rows] x 8 bytes
+    const uint32_t sm_a = smem_base;                                   // [half 0..1][chunk 0..3] blocks of 16 KB (resident A only)
+    const uint32_t sm_b = smem_base + (STREAM ? 0 : A_BYTES);          // NSTAGE stages
+    const uint32_t sm_cand = sm_b + NSTAGE * SB;                       // [16 entries][256 rows] x 8 bytes
     const uint32_t sm_stg = sm_cand + CAND_BYTES;                      // [set][nbs | P][128] floats
     const uint32_t sm_x = sm_stg + STG_BYTES;                          // barriers, tmem pointer
     const uint32_t bar_a_full = sm_x + 0, bar_a_empty = sm_x + 8;
@@ -480,24 +504,29 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, TcParams p) {
                 const int mt = item / sched.n_slices, sl = item - mt * sched.n_slices;
                 const int nt_lo = LIST ? (int)((long long)p.nt_ref * sl / sched.n_slices) : 0;
                 const int nt_hi = LIST ? (int)((long long)p.nt_ref * (sl + 1) / sched.n_slices) : nt_total;
-                mbar_wait(bar_a_empty, (uint32_t)((it & 1) ^ 1));
-                mbar_expect_tx(bar_a_full, A_BYTES);
-                for (int h = 0; h < 2; ++h)
-                    for (int kc = 0; kc < NKC; ++kc)
-                        tma_load_2d(sm_a + (h * NKC + kc) * BLOCK_BYTES, &map_a, bar_a_full, kc * BK, mt * MT + h * BM);
+                if constexpr (!STREAM) {
+                    mbar_wait(bar_a_empty, (uint32_t)((it & 1) ^ 1));
+                    mbar_expect_tx(bar_a_full, A_BYTES);
+                    for (int h = 0; h < 2; ++h)
+                        for (int kc = 0; kc < NKC; ++kc)
+                            tma_load_2d(sm_a + (h * NKC + kc) * BLOCK_BYTES, &map_a, bar_a_full, kc * BK, mt * MT + h * BM);
+                }
                 for (int nt = nt_lo; nt < nt_hi; ++nt, ++tile) {
-                    for (int kc = 0; kc < NKC; ++kc) {
+                    for (int kc = 0; kc < NK; ++kc) {
                         mbar_wait(bar_b_empty + 8 * bstage, bphase ^ 1u);
-                        mbar_expect_tx(bar_b_full + 8 * bstage, BLOCK_BYTES);
-                        bulk_load(sm_b + bstage * BLOCK_BYTES, p.b_img + ((int64_t)nt * NKC + kc) * (BLOCK_BYTES / 2), BLOCK_BYTES,
+                        mbar_expect_tx(bar_b_full + 8 * bstage, STREAM ? 3 * BLOCK_BYTES : BLOCK_BYTES);
+                        bulk_load(sm_b + bstage * SB, p.b_img + ((int64_t)nt * NK + kc) * (BLOCK_BYTES / 2), BLOCK_BYTES,
                                   bar_b_full + 8 * bstage);
+                        if constexpr (STREAM)          // this K-chunk of both A halves travels with the B block (read from L2 per tile)
+                            for (int h = 0; h < 2; ++h)
+                                tma_load_2d(sm_b + bstage * SB + (1 + h) * BLOCK_BYTES, &map_a, bar_b_full + 8 * bstage, kc * BK, mt * MT + h * BM);
                         if (++bstage == NSTAGE) { bstage = 0; bphase ^= 1u; }
                     }
                     {
                         // fifth slot of the tile: the extra K columns -- the tile's references, then the two row blocks of the contig tile
                         mbar_wait(bar_b_empty + 8 * bstage, bphase ^ 1u);
                         mbar_expect_tx(bar_b_full + 8 * bstage, 3 * XBLK_BYTES);
-                        const uint32_t slot = sm_b + bstage * BLOCK_BYTES;
+                        const uint32_t slot = sm_b + bstage * SB;
                         bulk_load(slot, p.bx_img + (int64_t)nt * XBLK_HALVES, XBLK_BYTES, bar_b_full + 8 * bstage);
                         bulk_load(slot + XBLK_BYTES, p.ax_img + (int64_t)(2 * mt) * XBLK_HALVES, 2 * XBLK_BYTES, bar_b_full + 8 * bstage);
                         if (++bstage == NSTAGE) { bstage = 0; bphase ^= 1u; }
@@ -523,23 +552,24 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, TcParams p) {
             const int sl = item % sched.n_slices;
             const int nt_lo = LIST ? (int)((long long)p.nt_ref * sl / sched.n_slices) : 0;
             const int nt_hi = LIST ? (int)((long long)p.nt_ref * (sl + 1) / sched.n_slices) : nt_total;
-            mbar_wait(bar_a_full, (uint32_t)(it & 1));
+            if constexpr (!STREAM) mbar_wait(bar_a_full, (uint32_t)(it & 1));
             for (int nt = nt_lo; nt < nt_hi; ++nt, ++tile) {
                 const uint32_t set = tile & 1u;
                 mbar_wait(bar_t_empty + 8 * set, ((tile >> 1) & 1u) ^ 1u);
                 tc_fence_after();
                 const uint32_t tmem_d = tmem_base + set * (2 * BN);
 #pragma unroll
-                for (int kc = 0; kc < NKC; ++kc) {
+                for (int kc = 0; kc < NK; ++kc) {
                     mbar_wait(bar_b_full + 8 * bstage, bphase);
                     tc_fence_after();
-                    const uint32_t b_blk = b_lo + bstage * (BLOCK_BYTES >> 4);
+                    const uint32_t b_blk = b_lo + bstage * (SB >> 4);
                     if (elect_one()) {
 #pragma unroll
                         for (int h = 0; h < 2; ++h) {
 #pragma unroll
                             for (int ks = 0; ks < BK / 16; ++ks) {   // 16 halves = 32 bytes along K inside the swizzle row
-                                const uint32_t a_blk = a_lo + (h * NKC + kc) * (BLOCK_BYTES >> 4) + ks * 2;
+                                const uint32_t a_blk = STREAM ? b_blk + (1 + h) * (BLOCK_BYTES >> 4) + ks * 2
+                                                              : a_lo + (h * NKC + kc) * (BLOCK_BYTES >> 4) + ks * 2;
                                 umma_f16(tmem_d + h * BN, desc_hi | a_blk, desc_hi | (b_blk + ks * 2), (kc | ks) ? 1u : 0u);
                             }
                         }
@@ -552,7 +582,7 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, TcParams p) {
                     // the seventeenth k-step: accumulator += (2^10, 2^-1, 2^-12, C16) . (-n1, -n2, -n3, P16)
                     mbar_wait(bar_b_full + 8 * bstage, bphase);
                     tc_fence_after();
-                    const uint32_t slot = sm_b + bstage * BLOCK_BYTES;
+                    const uint32_t slot = sm_b + bstage * SB;
                     if (elect_one()) {
                         const uint64_t xb = smem_desc_plain(slot);
 #pragma unroll
@@ -564,8 +594,10 @@ score_tc_kernel(const __grid_constant__ CUtensorMap map_a, TcParams p) {
                     if (++bstage == NSTAGE) { bstage = 0; bphase ^= 1u; }
                 }
             }
-            if (elect_one()) umma_commit(bar_a_empty);            // A tile no longer read
-            __syncwarp();
+            if constexpr (!STREAM) {
+                if (elect_one()) umma_commit(bar_a_empty);        // A tile no longer read
+                __syncwarp();
+            }
         }
     } else {
         // ================= epilogue: 8 warps; thread = contig row = tensor-memory lane =================
@@ -722,14 +754,14 @@ __global__ void tc_prep_rows_kernel(const double *__restrict__ src, int64_t n_sr
         if (r < n_src) load_query_row<W>(src, src_counts, sr, lane, xs, &total);
         if (row_total && src_counts && lane == 0 && r < n_src) row_total[sr] = total;
 #pragma unroll
-        for (int i = 0; i < KDIM / 32; ++i) {
+        for (int i = 0; i < OPW<W> / 32; ++i) {
             const int d = lane + 32 * i;
-            // queries: row-major [n, 256] (fetched by 2-D TMA); references: the shared-memory image of their 128-row tile,
+            // queries: row-major [n, OPW] (fetched by 2-D TMA); references: the shared-memory image of their 128-row tile,
             // [tile][K chunk of 64][row][128 B with the 16-byte pieces XOR-swizzled by row & 7], so that a B block is ONE
             // contiguous 16 KB bulk copy instead of 128 row pieces gathered by a tensor map
-            const int64_t o = is_ref ? ((((r >> 7) * NKC + (d >> 6)) * BM + (r & 127)) * BK + ((((d >> 3) & 7) ^ (int)(r & 7)) << 3) + (d & 7))
-                                     : r * KDIM + d;
-            if (W == KDIM || (i < NCH<W> && in_row<W>(lane, i))) {
+            const int64_t o = is_ref ? ((((r >> 7) * NK_OF<W> + (d >> 6)) * BM + (r & 127)) * BK + ((((d >> 3) & 7) ^ (int)(r & 7)) << 3) + (d & 7))
+                                     : r * OPW<W> + d;
+            if (W == OPW<W> || (i < NCH<W> && in_row<W>(lane, i))) {
                 const double x = (r < n_src) ? xs[i < NCH<W> ? i : 0] : shift;
                 op[o] = prep_accumulate<W>(x, s, sc, sd, sh);
             } else {
@@ -777,7 +809,7 @@ __global__ void tc_prep_rows_kernel(const double *__restrict__ src, int64_t n_sr
                     dst[8] = make_uint4(0u, 0u, 0u, 0u);                            // K half 1: 128 bytes further
                 }
                 if (real && P > 0.0) {
-                    atomicMax(reinterpret_cast<int *>(&consts->rho), __float_as_int(float_up((dB + EPS_ACC * (P + dB)) / P)));
+                    atomicMax(reinterpret_cast<int *>(&consts->rho), __float_as_int(float_up((dB + EPS_ACC_OF<NK_OF<W>> * (P + dB)) / P)));
                     atomicMax(reinterpret_cast<int *>(&consts->pmax), __float_as_int(float_up(P)));
                 }
             } else if (real) {
@@ -861,8 +893,11 @@ __device__ __forceinline__ int64_t cand_ref_index(const DecideParams &p, uint32_
 // NEIGHBORS: the call also reports the k nearest references and the nearest centroid of each class (p.nb).  A row then counts as
 // settled only when its k nearest are identified, not merely its vote: every live row re-measures its band (ROW_OPEN), and a row
 // with a dropped candidate within reach goes to the overflow road even when its vote is unanimous.  The scores do not change.
+// 5-mer rows (W > 256): a lane holds NCH<W> = 16 or 32 doubles of the row and as many of the next one, which do not fit the
+// register budget of PHM_DECIDE_MIN_CTAS blocks per SM; those instantiations ask for one block, so that nothing spills.
+template <int W> constexpr int DECIDE_MIN_CTAS = W > KDIM ? 1 : PHM_DECIDE_MIN_CTAS;
 template <bool FROM_COUNTS, bool NEIGHBORS = false, int W = KDIM>
-__global__ void __launch_bounds__(256, PHM_DECIDE_MIN_CTAS) score_decide_kernel(DecideParams p) {
+__global__ void __launch_bounds__(256, DECIDE_MIN_CTAS<W>) score_decide_kernel(DecideParams p) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -1157,10 +1192,12 @@ __global__ void __launch_bounds__(256) tc_build_ax_kernel(const float *__restric
 }
 
 // ---------------- list pass: compaction of its rows, and the exact decision over the listed references ----------------
+template <int OW>                                                              // operand width (OPW)
 __global__ void __launch_bounds__(256) tc_list_gather_kernel(const __half *__restrict__ a_op, const float *__restrict__ crow,
                                                              const int64_t *__restrict__ list_rows, const unsigned long long *list_count,
                                                              int max_rows, __half *__restrict__ a_list, float *__restrict__ crow_list,
                                                              uint32_t *__restrict__ list_cnt, __half *__restrict__ ax_list) {
+    constexpr int V = OW * 2 / 16 / 32;                                        // 16-byte pieces of a row per lane
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -1168,14 +1205,18 @@ __global__ void __launch_bounds__(256) tc_list_gather_kernel(const __half *__res
     if (cnt > (unsigned long long)max_rows) cnt = (unsigned long long)max_rows;
     const int64_t padded = (int64_t)((cnt + MT - 1) / MT) * MT;
     for (int64_t slot = warp; slot < padded; slot += n_warps) {
-        uint4 v = make_uint4(0u, 0u, 0u, 0u);
+        uint4 v[V];
         float c = NAN;                                                 // padding rows of the last tile are not live
+#pragma unroll
+        for (int j = 0; j < V; ++j) v[j] = make_uint4(0u, 0u, 0u, 0u);
         if (slot < (int64_t)cnt) {
             const int64_t row = list_rows[slot];
-            v = reinterpret_cast<const uint4 *>(a_op)[row * (KDIM * 2 / 16) + lane];
+#pragma unroll
+            for (int j = 0; j < V; ++j) v[j] = reinterpret_cast<const uint4 *>(a_op)[row * (OW * 2 / 16) + lane + 32 * j];
             c = crow[row];
         }
-        reinterpret_cast<uint4 *>(a_list)[slot * (KDIM * 2 / 16) + lane] = v;
+#pragma unroll
+        for (int j = 0; j < V; ++j) reinterpret_cast<uint4 *>(a_list)[slot * (OW * 2 / 16) + lane + 32 * j] = v[j];
         if (lane == 0) { crow_list[slot] = c; list_cnt[slot] = 0u; write_ax_row(ax_list, slot, c); }
     }
 }
@@ -1444,8 +1485,16 @@ __global__ void __launch_bounds__(256) score_fallback_kernel(FallbackParams f) {
 // which is staged once in shared memory (transposed, padded: conflict-free for lane = reference), so the references are streamed
 // from HBM once per 32 rows instead of once per row.  Reference distances only ORDER the neighbours here; the centroid distances,
 // whose values reach the score, use the same warp_d2 as every other path.
-constexpr int FBB_ROWS = 32, FBB_TR = 32, FBB_PITCH = FBB_TR + 1;
-template <int W> constexpr int FBB_SMEM = (FBB_ROWS * W + W * FBB_PITCH) * 8 + FBB_ROWS * TC_KMAX * 12 + 64;
+// 5-mer rows (W > 256) would need 266 / 534 KB that way: a CTA takes 16 / 8 rows there, and the reference tile is staged 256
+// features at a time (the distances are summed in the same order, so they are the same bits).
+constexpr int FBB_TR = 32, FBB_PITCH = FBB_TR + 1;
+template <int W> constexpr int FBB_QW = W <= KDIM ? 4 : 4 * KDIM / W;          // most rows per warp
+template <int W> constexpr int FBB_ROWS = 8 * FBB_QW<W>;                       // rows per CTA
+template <int W> constexpr int FBB_DS = W <= KDIM ? W : KDIM;                  // features of the reference tile staged at once
+template <int W> constexpr int FBB_SMEM = (FBB_ROWS<W> * W + FBB_DS<W> * FBB_PITCH) * 8 + FBB_ROWS<W> * TC_KMAX * 12 + 64;
+template <int W> __host__ __device__ constexpr int fbb_qw(int q) { return q < FBB_QW<W> ? q : FBB_QW<W>; }
+static_assert(FBB_SMEM<256> <= 232448 && FBB_SMEM<136> <= 232448 && FBB_SMEM<512> <= 232448 && FBB_SMEM<1024> <= 232448,
+              "shared memory budget of one sm_100 CTA (blocked fallback)");
 
 template <int W, int QW>                                                   // row width, rows per warp
 __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned long long blk, unsigned long long count,
@@ -1469,26 +1518,29 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
     double thr[QW];
 #pragma unroll
     for (int q = 0; q < QW; ++q) thr[q] = INFINITY;
+    constexpr int DS = FBB_DS<W>;
     for (int64_t c0 = 0; c0 < f.n_refs; c0 += FBB_TR) {
-        __syncthreads();                                                   // previous tile fully consumed
-        for (int idx = threadIdx.x; idx < FBB_TR * W; idx += 256) {
-            const int r = (W == KDIM) ? idx >> 8 : idx / W, d = (W == KDIM) ? idx & 255 : idx % W;
-            s_tile[d * FBB_PITCH + r] = (c0 + r < f.n_refs) ? f.refs[(c0 + r) * W + d] : 0.0;
-        }
-        __syncthreads();
         double acc[QW];
 #pragma unroll
         for (int q = 0; q < QW; ++q) acc[q] = 0.0;
-        const double *xr = s_rows + warp * QW * W;
+        for (int d0 = 0; d0 < W; d0 += DS) {                               // one slice unless W > 256
+            __syncthreads();                                               // previous tile (slice) fully consumed
+            for (int idx = threadIdx.x; idx < FBB_TR * DS; idx += 256) {
+                const int r = (DS == KDIM) ? idx >> 8 : idx / DS, d = (DS == KDIM) ? idx & 255 : idx % DS;
+                s_tile[d * FBB_PITCH + r] = (c0 + r < f.n_refs) ? f.refs[(c0 + r) * W + d0 + d] : 0.0;
+            }
+            __syncthreads();
+            const double *xr = s_rows + warp * QW * W + d0;
 #pragma unroll 4
-        for (int d = 0; d < W; d += 2) {
-            const double b0 = s_tile[d * FBB_PITCH + lane], b1 = s_tile[(d + 1) * FBB_PITCH + lane];
+            for (int d = 0; d < DS; d += 2) {
+                const double b0 = s_tile[d * FBB_PITCH + lane], b1 = s_tile[(d + 1) * FBB_PITCH + lane];
 #pragma unroll
-            for (int q = 0; q < QW; ++q) {
-                const double2 xx = *reinterpret_cast<const double2 *>(xr + q * W + d);
-                const double t0 = xx.x - b0, t1 = xx.y - b1;
-                acc[q] = fma(t0, t0, acc[q]);
-                acc[q] = fma(t1, t1, acc[q]);
+                for (int q = 0; q < QW; ++q) {
+                    const double2 xx = *reinterpret_cast<const double2 *>(xr + q * W + d);
+                    const double t0 = xx.x - b0, t1 = xx.y - b1;
+                    acc[q] = fma(t0, t0, acc[q]);
+                    acc[q] = fma(t1, t1, acc[q]);
+                }
             }
         }
         const bool real = c0 + lane < f.n_refs;
@@ -1524,22 +1576,22 @@ __device__ __forceinline__ void fallback_block(const FallbackParams &f, unsigned
 template <int W>
 __global__ void __launch_bounds__(256) score_fallback_blocked_kernel(FallbackParams f) {
     extern __shared__ __align__(16) unsigned char fbb_raw[];
-    double *s_rows = reinterpret_cast<double *>(fbb_raw);                     // [32][W]
-    double *s_tile = s_rows + FBB_ROWS * W;                                   // [W][33]
-    double *s_d = s_tile + W * FBB_PITCH;                                     // [32][TC_KMAX]
-    int *s_i = reinterpret_cast<int *>(s_d + FBB_ROWS * TC_KMAX);             // [32][TC_KMAX]
+    double *s_rows = reinterpret_cast<double *>(fbb_raw);                     // [FBB_ROWS][W]
+    double *s_tile = s_rows + FBB_ROWS<W> * W;                                // [FBB_DS][33]
+    double *s_d = s_tile + FBB_DS<W> * FBB_PITCH;                             // [FBB_ROWS][TC_KMAX]
+    int *s_i = reinterpret_cast<int *>(s_d + FBB_ROWS<W> * TC_KMAX);          // [FBB_ROWS][TC_KMAX]
     const unsigned long long count = *f.count;
     if (count <= FB_BLOCKED_MIN) return;
     // rows per warp chosen so that one wave of CTAs covers all rows when it can (the work per CTA is proportional to its rows)
     int qw = (int)((count + (unsigned long long)gridDim.x * 8 - 1) / ((unsigned long long)gridDim.x * 8));
-    qw = qw > 4 ? 4 : qw;
+    qw = qw > FBB_QW<W> ? FBB_QW<W> : qw;
     const unsigned long long n_blocks = (count + 8 * qw - 1) / (8 * qw);
     for (unsigned long long blk = blockIdx.x; blk < n_blocks; blk += gridDim.x) {
         switch (qw) {
             case 1: fallback_block<W, 1>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
-            case 2: fallback_block<W, 2>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
-            case 3: fallback_block<W, 3>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
-            default: fallback_block<W, 4>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
+            case 2: fallback_block<W, fbb_qw<W>(2)>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
+            case 3: fallback_block<W, fbb_qw<W>(3)>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
+            default: fallback_block<W, fbb_qw<W>(4)>(f, blk, count, s_rows, s_tile, s_d, s_i); break;
         }
     }
 }
@@ -1559,12 +1611,13 @@ static EncodeTiledFn encode_fn() {
     return fn;
 }
 
-// [rows, 256] FP16 row-major, box = 64 features x 128 rows, 128-byte swizzle (the UMMA K-major canonical layout)
-static int make_map(CUtensorMap *map, const void *base, int64_t rows) {
+// [rows, opw] FP16 row-major (opw = OPW of the rows: 256, 512 or 1024), box = 64 features x 128 rows, 128-byte swizzle (the UMMA
+// K-major canonical layout)
+static int make_map(CUtensorMap *map, const void *base, int64_t rows, int opw) {
     EncodeTiledFn fn = encode_fn();
     if (!fn) { set_error("cuTensorMapEncodeTiled is not available from this driver"); return PHM_E_UNSUPPORTED; }
-    cuuint64_t dims[2] = {(cuuint64_t)KDIM, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)KDIM * 2};
+    cuuint64_t dims[2] = {(cuuint64_t)opw, (cuuint64_t)rows};
+    cuuint64_t strides[1] = {(cuuint64_t)opw * 2};
     cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)BM};
     cuuint32_t elem[2] = {1, 1};
     CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void *>(base), dims, strides, box, elem,
@@ -1595,7 +1648,11 @@ struct TcWorkspace {
     size_t bytes;
 };
 
-static TcWorkspace carve_tc(void *ws, int64_t n, int64_t r_pad, int64_t n_refs, int64_t n_cp, int64_t n_cn) {
+// operand width of `dim`-wide rows (host side of OPW)
+static inline int op_width(int dim) { return dim <= KDIM ? KDIM : dim; }
+
+static TcWorkspace carve_tc(void *ws, int64_t n, int64_t r_pad, int64_t n_refs, int64_t n_cp, int64_t n_cn, int dim) {
+    const int opw = op_width(dim);
     TcWorkspace w;
     size_t off = 0;
     unsigned char *base = static_cast<unsigned char *>(ws);
@@ -1607,8 +1664,8 @@ static TcWorkspace carve_tc(void *ws, int64_t n, int64_t r_pad, int64_t n_refs, 
     w.stats = reinterpret_cast<float *>(head + 64);
     w.rows_remeasured = reinterpret_cast<unsigned long long *>(head + 128);
     w.consts = reinterpret_cast<PrepConsts *>(head + 192);
-    w.a_op = reinterpret_cast<__half *>(take((size_t)n * KDIM * 2));
-    w.b_op = reinterpret_cast<__half *>(take((size_t)r_pad * KDIM * 2));
+    w.a_op = reinterpret_cast<__half *>(take((size_t)n * opw * 2));
+    w.b_op = reinterpret_cast<__half *>(take((size_t)r_pad * opw * 2));
     w.bx_img = reinterpret_cast<__half *>(take((size_t)r_pad * XK * 2));
     w.ax_img = reinterpret_cast<__half *>(take((size_t)round_up(n > 0 ? n : 1, MT) * XK * 2));
     w.nbs = reinterpret_cast<float *>(take((size_t)r_pad * 4));
@@ -1640,29 +1697,31 @@ static TcWorkspace carve_tc(void *ws, int64_t n, int64_t r_pad, int64_t n_refs, 
     w.list_pool_entries = lmax * 2048 < LIST_POOL ? lmax * 2048 : LIST_POOL;       // small problems get a small pool (at least 4 M entries)
     if (w.list_pool_entries < ((int64_t)1 << 22)) w.list_pool_entries = (int64_t)1 << 22;
     w.list_cols = reinterpret_cast<uint32_t *>(take((size_t)w.list_pool_entries * 4));
-    w.a_list = reinterpret_cast<__half *>(take((size_t)lmax * KDIM * 2));
+    w.a_list = reinterpret_cast<__half *>(take((size_t)lmax * opw * 2));
     w.ax_list = reinterpret_cast<__half *>(take((size_t)lmax * XK * 2));
     w.bytes = off;
     return w;
 }
 
-size_t score_tc_workspace_bytes(int64_t n, int64_t n_refs, int64_t n_cp, int64_t n_cn) {
+size_t score_tc_workspace_bytes(int64_t n, int64_t n_refs, int64_t n_cp, int64_t n_cn, int dim) {
     const int64_t r_pad = round_up(n_refs, BN) + round_up(n_cp, BN) + round_up(n_cn, BN);
-    return carve_tc(nullptr, n, r_pad, n_refs, n_cp, n_cn).bytes;
+    return carve_tc(nullptr, n, r_pad, n_refs, n_cp, n_cn, dim).bytes;
 }
 
 bool score_tc_supported(int dim, int k_neighbors, int64_t n_refs, int64_t n_cp, int64_t n_cn) {
     return tc_width(dim) && (k_neighbors == 1 || k_neighbors == 3 || k_neighbors == 5) && n_refs >= k_neighbors && n_cp > 0 && n_cn > 0;
 }
 
-// rows of `dim` features (256 or CANON_DIM)
+// rows of `dim` features (one of tc_width)
 static int launch_prep(int dim, const double *src, const uint32_t *src_counts, int64_t n_src, int64_t n_rows, int64_t perm_a, int64_t perm_c, int is_ref,
                        int64_t n_positive, __half *op, double *norm64, double *cnorm64, float *nbs, float *pnorm, float *crow, PrepConsts *consts,
                        cudaStream_t st, uint32_t *row_total = nullptr, __half *bx = nullptr) {
     if (n_rows == 0) return PHM_OK;
     int64_t blocks = (n_rows + 7) / 8;
     if (blocks > 148 * 16) blocks = 148 * 16;
-    auto kern = dim == CANON_DIM ? tc_prep_rows_kernel<CANON_DIM> : tc_prep_rows_kernel<KDIM>;
+    auto kern = dim == CANON_DIM ? tc_prep_rows_kernel<CANON_DIM>
+              : dim == KMER5_DIM ? tc_prep_rows_kernel<KMER5_DIM>
+              : dim == CANON5_DIM ? tc_prep_rows_kernel<CANON5_DIM> : tc_prep_rows_kernel<KDIM>;
     kern<<<(unsigned)blocks, 256, 0, st>>>(src, n_src, n_rows, perm_a, perm_c, src_counts, is_ref, n_positive, op, norm64, cnorm64, nbs, pnorm,
                                                           crow, consts, row_total, bx);
     PHM_LAUNCH_CHECK();
@@ -1674,19 +1733,20 @@ static EventRing g_decide_ring;  // ... and of the score_decide_kernel launches
 
 // score_tc_kernel for k_neighbors k: the first pass (one CTA per contig tile at most; timed for "time_kernels"), or the list pass
 // (persistent; the number of rows is read on the device)
+template <int NK>
 static int launch_tc(bool list, int k, const CUtensorMap &map, const TcParams &p, cudaStream_t st) {
     void (*kern)(CUtensorMap, TcParams);
     switch (k) {
-        case 1: kern = list ? score_tc_kernel<1, true> : score_tc_kernel<1, false>; break;
-        case 3: kern = list ? score_tc_kernel<3, true> : score_tc_kernel<3, false>; break;
-        case 5: kern = list ? score_tc_kernel<5, true> : score_tc_kernel<5, false>; break;
+        case 1: kern = list ? score_tc_kernel<1, true, NK> : score_tc_kernel<1, false, NK>; break;
+        case 3: kern = list ? score_tc_kernel<3, true, NK> : score_tc_kernel<3, false, NK>; break;
+        case 5: kern = list ? score_tc_kernel<5, true, NK> : score_tc_kernel<5, false, NK>; break;
         default: set_error("tensor-core scoring supports k_neighbors 1, 3, 5"); return PHM_E_UNSUPPORTED;
     }
-    PHM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    PHM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES_OF<NK>));
     int grid = sm_count();
     if (!list && grid > p.n_mtiles) grid = p.n_mtiles;
     const bool timed = !list && g_tc_ring.begin(st);
-    kern<<<grid, NTHREADS, SMEM_BYTES, st>>>(map, p);
+    kern<<<grid, NTHREADS, SMEM_BYTES_OF<NK>, st>>>(map, p);
     PHM_LAUNCH_CHECK();
     if (timed) g_tc_ring.end(st);
     return PHM_OK;
@@ -1711,19 +1771,20 @@ int score_tc_begin(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t s
     const int64_t n = a.n_points;
     const int64_t ref_pad = round_up(a.n_refs, BN), cp_pad = round_up(a.n_cent_pos, BN), cn_pad = round_up(a.n_cent_neg, BN);
     const int64_t r_pad = ref_pad + cp_pad + cn_pad;
-    TcWorkspace w = carve_tc(ws, n, r_pad, a.n_refs, a.n_cent_pos, a.n_cent_neg);
+    TcWorkspace w = carve_tc(ws, n, r_pad, a.n_refs, a.n_cent_pos, a.n_cent_neg, a.dim);
     if (ws_bytes < w.bytes) { set_error("workspace too small: %zu < %zu", ws_bytes, w.bytes); return PHM_E_WORKSPACE; }
     PHM_REQUIRE(n < ((int64_t)1 << 31) - MT && r_pad < ((int64_t)1 << 31), "problem too large for 32-bit TMA coordinates");
 
     PHM_CUDA_CHECK(cudaMemsetAsync(w.fallback_count, 0, 512, st));
     int rc;
     int64_t perm_a, perm_c;
+    const int64_t opw = op_width(a.dim);
     ref_permutation(a.n_refs, &perm_a, &perm_c);
     if ((rc = launch_prep(a.dim, a.refs, nullptr, a.n_refs, ref_pad, perm_a, perm_c, 1, a.n_positive, w.b_op, w.norm_refs, nullptr, w.nbs, w.pnorm, nullptr, w.consts, st,
                           nullptr, w.bx_img)) != PHM_OK) return rc;
-    if ((rc = launch_prep(a.dim, a.cent_pos, nullptr, a.n_cent_pos, cp_pad, 1, 0, 1, 0, w.b_op + ref_pad * KDIM, w.norm_cpos, nullptr, w.nbs + ref_pad,
+    if ((rc = launch_prep(a.dim, a.cent_pos, nullptr, a.n_cent_pos, cp_pad, 1, 0, 1, 0, w.b_op + ref_pad * opw, w.norm_cpos, nullptr, w.nbs + ref_pad,
                           w.pnorm + ref_pad, nullptr, w.consts, st, nullptr, w.bx_img + ref_pad * XK)) != PHM_OK) return rc;
-    if ((rc = launch_prep(a.dim, a.cent_neg, nullptr, a.n_cent_neg, cn_pad, 1, 0, 1, 0, w.b_op + (ref_pad + cp_pad) * KDIM, w.norm_cneg, nullptr,
+    if ((rc = launch_prep(a.dim, a.cent_neg, nullptr, a.n_cent_neg, cn_pad, 1, 0, 1, 0, w.b_op + (ref_pad + cp_pad) * opw, w.norm_cneg, nullptr,
                           w.nbs + ref_pad + cp_pad, w.pnorm + ref_pad + cp_pad, nullptr, w.consts, st, nullptr,
                           w.bx_img + (ref_pad + cp_pad) * XK)) != PHM_OK) return rc;
     if (emit) { emit->op = w.a_op; emit->crow = w.crow; emit->cnorm = w.cnorm_points; emit->total = w.row_total; emit->consts = w.consts; }
@@ -1743,7 +1804,7 @@ static int tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t
     const int64_t n = a.n_points;
     const int64_t ref_pad = round_up(a.n_refs, BN), cp_pad = round_up(a.n_cent_pos, BN), cn_pad = round_up(a.n_cent_neg, BN);
     const int64_t r_pad = ref_pad + cp_pad + cn_pad;
-    TcWorkspace w = carve_tc(ws, n, r_pad, a.n_refs, a.n_cent_pos, a.n_cent_neg);
+    TcWorkspace w = carve_tc(ws, n, r_pad, a.n_refs, a.n_cent_pos, a.n_cent_neg, W);
     if (ws_bytes < w.bytes) { set_error("workspace too small: %zu < %zu", ws_bytes, w.bytes); return PHM_E_WORKSPACE; }
     int rc;
     int64_t perm_a, perm_c;
@@ -1753,7 +1814,7 @@ static int tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t
                           w.row_total)) != PHM_OK) return rc;
 
     CUtensorMap map_a;
-    if ((rc = make_map(&map_a, w.a_op, n)) != PHM_OK) return rc;
+    if ((rc = make_map(&map_a, w.a_op, n, OPW<W>)) != PHM_OK) return rc;
 
     TcParams p;
     p.n_points = n;
@@ -1773,7 +1834,7 @@ static int tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t
     p.skip_scan = score_force_fallback;
     p.list_count = w.list_count; p.list_max_rows = w.list_max_rows; p.list_thr = w.list_thr; p.list_cnt = w.list_cnt;
     p.list_off = w.list_off; p.list_cols = nullptr;
-    if ((rc = launch_tc(false, a.out.k, map_a, p, st)) != PHM_OK) return rc;
+    if ((rc = launch_tc<NK_OF<W>>(false, a.out.k, map_a, p, st)) != PHM_OK) return rc;
 
     DecideParams r;
     r.points = a.points; r.point_counts = a.point_counts; r.n_points = n;
@@ -1805,17 +1866,17 @@ static int tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t
     // rows whose candidate buffer overflowed but whose threshold is final: second tensor-core pass that lists every reference
     // under the threshold, then the exact decision over the lists (row count read on the device: no host synchronisation)
     if (use_list) {
-        tc_list_gather_kernel<<<sm_count(), 256, 0, st>>>(w.a_op, w.crow, w.list_rows, w.list_count, w.list_max_rows, w.a_list, w.list_crow, w.list_cnt,
-                                                          w.ax_list);
+        tc_list_gather_kernel<OPW<W>><<<sm_count(), 256, 0, st>>>(w.a_op, w.crow, w.list_rows, w.list_count, w.list_max_rows, w.a_list, w.list_crow,
+                                                                  w.list_cnt, w.ax_list);
         PHM_LAUNCH_CHECK();
         CUtensorMap map_list;
-        if ((rc = make_map(&map_list, w.a_list, w.list_max_rows)) != PHM_OK) return rc;
+        if ((rc = make_map(&map_list, w.a_list, w.list_max_rows, OPW<W>)) != PHM_OK) return rc;
         TcParams pl = p;
         pl.crow = w.list_crow;
         pl.ax_img = w.ax_list;
         for (int pass = 0; pass < 2; ++pass) {                           // count, prefix sum, fill
             pl.list_cols = pass ? w.list_cols : nullptr;
-            if ((rc = launch_tc(true, a.out.k, map_list, pl, st)) != PHM_OK) return rc;
+            if ((rc = launch_tc<NK_OF<W>>(true, a.out.k, map_list, pl, st)) != PHM_OK) return rc;
             if (pass == 0) {
                 tc_list_scan_kernel<<<1, 1024, 0, st>>>(w.list_count, w.list_max_rows, (unsigned long long)w.list_pool_entries, w.list_cnt,
                                                         w.list_n, w.list_off);
@@ -1853,7 +1914,12 @@ static int tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t
 }
 
 int score_tc_finish(const ScoreArgs &a, void *ws, size_t ws_bytes, cudaStream_t st, bool queries_prepared) {
-    return a.dim == CANON_DIM ? tc_finish<CANON_DIM>(a, ws, ws_bytes, st, queries_prepared) : tc_finish<KDIM>(a, ws, ws_bytes, st, queries_prepared);
+    switch (a.dim) {
+        case CANON_DIM: return tc_finish<CANON_DIM>(a, ws, ws_bytes, st, queries_prepared);
+        case KMER5_DIM: return tc_finish<KMER5_DIM>(a, ws, ws_bytes, st, queries_prepared);
+        case CANON5_DIM: return tc_finish<CANON5_DIM>(a, ws, ws_bytes, st, queries_prepared);
+        default: return tc_finish<KDIM>(a, ws, ws_bytes, st, queries_prepared);
+    }
 }
 
 // statistics of the last score_tc call on this workspace

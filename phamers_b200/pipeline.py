@@ -16,6 +16,10 @@ Stage by stage this is kmer.count_file -> kmer.normalize_counts -> phamer_scorer
 ContigScorer(..., canonical=True) scores canonical 4-mers (each k-mer folded with its reverse complement, 136 bins), so a contig
 and its reverse complement get the same score: references are 136 wide, contigs are counted with PHM_COUNT_CANONICAL and scored
 from the counts.
+
+ContigScorer(..., kmer_length=5[, canonical=True]) takes 5-mer reference rows (1024 or 512 wide: the shipped tables are 4-mer, so
+the caller passes its own); score_device / score_host / score_fasta count the contigs at k = 5 and score the counts on the
+tensor-core road at that width.  Windows and spans are scored from feature rows on the exhaustive kernel, as before.
 """
 import numpy as np
 import torch
@@ -95,11 +99,11 @@ class ContigScorer(object):
         return counts, {"knn": knn, "kmeans": kmeans, "combo": combo}[method]
 
     def _count_score(self, seq, offsets, out_counts=None, out=None):
-        if not self.canonical:
+        if not self.canonical and self.kmer_length == 4:
             return ops.count_score_cuda(seq, offsets, self.refs, self.n_positive, self.cent_pos, self.cent_neg, self.k_neighbors,
                                         out_counts=out_counts, out=out)
-        # canonical counts, then phm_score_counts on them (the fused count + score call emits plain 256-wide operands only)
-        counts, _ = ops.count_cuda(seq, offsets, self.kmer_length, canonical=True, out_counts=out_counts)
+        # canonical or 5-mer counts, then phm_score_counts on them (the fused count + score call emits plain 256-wide operands only)
+        counts, _ = ops.count_cuda(seq, offsets, self.kmer_length, canonical=self.canonical, out_counts=out_counts)
         return (counts,) + ops.score_cuda(counts, self.refs, self.n_positive, self.cent_pos, self.cent_neg, self.k_neighbors, out=out)
 
     # -- host buffers -----------------------------------------------------------------------------------
