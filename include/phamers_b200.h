@@ -43,6 +43,7 @@ extern "C" {
 #define PHM_E_CUDA        -2       /* a CUDA runtime call failed; see phm_last_error() */
 #define PHM_E_WORKSPACE   -3       /* workspace too small */
 #define PHM_E_UNSUPPORTED -4       /* not an sm_100 device / option not built */
+#define PHM_E_DATA        -5       /* corrupt input data (phm_inflate: a member failed to decode); see phm_last_error() */
 
 /* flags for phm_kmer_count* */
 #define PHM_COUNT_CANONICAL  1u    /* fold reverse complements: out bins = 136 / 512 / 2080 for k = 4 / 5 / 6 */
@@ -285,6 +286,50 @@ size_t phm_fasta_workspace_bytes(int64_t n_bytes);
 int phm_fasta_index(const uint8_t *d_raw, int64_t n_bytes, int64_t *d_result, void *d_workspace, size_t workspace_bytes, void *stream);
 int phm_fasta_extract(const uint8_t *d_raw, int64_t n_bytes, const int64_t *d_result, uint8_t *d_seq, int64_t *d_offsets,
                       int64_t *d_header_pos, int64_t max_records, const void *d_workspace, size_t workspace_bytes, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * BGZF decompression on the device, in front of phm_fasta_index for compressed FASTA.  A BGZF file (what bgzip / htslib write,
+ * what samtools faidx needs) is a chain of gzip members of at most 64 KiB of output, each holding its compressed size in a 'BC'
+ * extra subfield and its CRC32 and output size (ISIZE) in its trailer; so the host finds every member and its output offset
+ * before anything is decoded, and the members are decoded in parallel, one warp each.
+ *
+ *   phm_bgzf_member    one member: its raw DEFLATE payload d_in[in_offset, in_offset + in_bytes) (between the gzip header and
+ *                      the 8-byte trailer), its output d_out[out_offset, out_offset + isize), and the trailer's CRC32.
+ *   phm_inflate        decodes every member (RFC 1951: stored, fixed and dynamic Huffman blocks, in any mix; the code sets zlib
+ *                      accepts) and checks each output's CRC32 and length.  h_members is a HOST array; outputs must be in
+ *                      ascending order and must not overlap.  Argument errors (null pointers, a payload or output range outside
+ *                      in_bytes / out_bytes, overlapping or descending outputs, in_bytes or isize above 65 536) are PHM_E_ARG,
+ *                      reported before the device is touched.  The call then synchronises `stream` once: d_status int32[n_members]
+ *                      holds each member's PHM_INFLATE_* status, and if any member failed the call returns PHM_E_DATA with a
+ *                      message naming the lowest failing member and its reason.  Every input read stays inside the member's
+ *                      payload and every write inside its output range, whatever the data; a failed member's output range
+ *                      holds unspecified bytes, every other member's output is complete.  d_in needs no alignment.
+ *                      Workspace: phm_inflate_workspace_bytes(n_members).
+ * ------------------------------------------------------------------------------------------- */
+#define PHM_BGZF_MAX_BYTES        65536   /* most output (and payload) bytes of one BGZF member */
+#define PHM_INFLATE_OK            0
+#define PHM_INFLATE_BTYPE         1       /* block type 3 */
+#define PHM_INFLATE_STORED_LEN    2       /* stored block: NLEN is not the complement of LEN */
+#define PHM_INFLATE_BAD_CODE      3       /* over-subscribed or unusable code, bad code lengths, invalid symbol */
+#define PHM_INFLATE_DISTANCE      4       /* a match reaches before the member's first output byte */
+#define PHM_INFLATE_OVERFLOW      5       /* output past ISIZE */
+#define PHM_INFLATE_TRUNCATED     6       /* payload exhausted before the final block ended */
+#define PHM_INFLATE_TRAILING      7       /* payload bytes left after the final block */
+#define PHM_INFLATE_ISIZE         8       /* final block ended with less output than ISIZE */
+#define PHM_INFLATE_CRC           9       /* CRC32 of the output differs from the trailer's */
+
+typedef struct phm_bgzf_member {
+    int64_t  in_offset;            /* first payload byte in d_in */
+    int64_t  out_offset;           /* first output byte in d_out */
+    uint32_t in_bytes;             /* payload bytes (raw DEFLATE) */
+    uint32_t isize;                /* output bytes (gzip ISIZE) */
+    uint32_t crc32;                /* CRC32 of the output (gzip trailer) */
+    uint32_t reserved;
+} phm_bgzf_member;
+
+size_t phm_inflate_workspace_bytes(int64_t n_members);
+int phm_inflate(const uint8_t *d_in, int64_t in_bytes, const phm_bgzf_member *h_members, int64_t n_members, uint8_t *d_out,
+                int64_t out_bytes, int32_t *d_status, void *d_workspace, size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Lloyd iterations of k-means on the device (SURVEY.md 8(f) rank 4).  Replaces the iterations inside the reference's

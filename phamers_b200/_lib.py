@@ -57,6 +57,8 @@ SIGNATURES = {
     "phm_fasta_workspace_bytes": (c_size_t, [c_int64]),
     "phm_fasta_index": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "phm_fasta_extract": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
+    "phm_inflate_workspace_bytes": (c_size_t, [c_int64]),
+    "phm_inflate": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "phm_last_kernel_ms": (c_int, [ctypes.c_char_p, c_void_p]),
     "phm_synth_lengths": (c_int, [c_uint64, c_int64, c_int64, c_void_p, c_void_p]),
     "phm_synth_bases": (c_int, [c_uint64, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
@@ -65,6 +67,13 @@ SIGNATURES = {
 
 class PhamersLibraryError(RuntimeError):
     pass
+
+
+class PhamersDataError(PhamersLibraryError):
+    """PHM_E_DATA: the input data is corrupt (phm_inflate: a member failed to decode)."""
+
+
+PHM_E_DATA = -5
 
 
 class Neighbors(ctypes.Structure):
@@ -106,7 +115,7 @@ def load():
 def check(rc):
     if rc != 0:
         msg = load().phm_last_error()
-        raise PhamersLibraryError("libphamers_b200 error %d: %s" % (rc, msg.decode("utf-8", "replace") if msg else ""))
+        raise (PhamersDataError if rc == PHM_E_DATA else PhamersLibraryError)("libphamers_b200 error %d: %s" % (rc, msg.decode("utf-8", "replace") if msg else ""))
 
 
 def require_cuda():

@@ -3,6 +3,7 @@ The on-disk formats either side of the hot path, mirroring the reference's scrip
 scripts/id_parser.py the path touches:
 
     FASTA in        read_fasta :28, get_fasta_ids :62 (Bio.SeqIO tokenisation) + id_parser.get_id :89
+    BGZF            bgzf_members  (the member chain of a blocked-gzip FASTA, decoded on the device by ops.inflate_cuda)
     feature CSV     read_feature_file :134, save_counts :169  ('#' header lines, then id,c0,c1,...)
     score CSV       save_phamer_scores :241, read_phamer_output :256  ('# ' header, then 'id, score')
     neighbour CSV   save_phamer_neighbors, read_phamer_neighbors  ('# ' header, then per contig its nearest references and clusters)
@@ -16,6 +17,7 @@ Host-side only (bytes and text); no arithmetic happens here.
 import gzip
 import io
 import os
+import struct
 
 import numpy as np
 
@@ -125,9 +127,9 @@ UPLOAD_CHUNK = 256 << 20             # bytes per pinned staging buffer of the fi
 
 
 def _upload(buf, n):
-    """File bytes (an mmap, or the bytes of a decompressed .gz) -> CUDA uint8 tensor padded to 16 bytes.  The copy page cache ->
-    pinned staging buffer of chunk i + 1 runs on the host while chunk i crosses PCIe (scripts/kmer.py:131-134 reads the whole
-    file through Python objects instead)."""
+    """File bytes (an mmap of a plain or BGZF file, or the bytes of a .gz inflated on the host) -> CUDA uint8 tensor padded to 16
+    bytes.  The copy page cache -> pinned staging buffer of chunk i + 1 runs on the host while chunk i crosses PCIe
+    (scripts/kmer.py:131-134 reads the whole file through Python objects instead)."""
     import torch
     d_raw = torch.empty(((n + 15) // 16 * 16 + 16,), dtype=torch.uint8, device="cuda")
     chunk = min(UPLOAD_CHUNK, max(n, 1))
@@ -147,35 +149,151 @@ def _upload(buf, n):
     return d_raw
 
 
+# phm_bgzf_member (include/phamers_b200.h): one row per member of a BGZF file
+BGZF_MEMBER = np.dtype([("in_offset", "<i8"), ("out_offset", "<i8"), ("in_bytes", "<u4"), ("isize", "<u4"), ("crc32", "<u4"),
+                        ("reserved", "<u4")])
+_BGZF_MAGIC = b"\x1f\x8b\x08\x04"          # ID1 ID2 CM, FLG = FEXTRA only
+_U16 = struct.Struct("<H").unpack_from
+
+
+def bgzf_members(buf):
+    """The member table of a BGZF file (what bgzip / htslib write): a structured array of BGZF_MEMBER, one row per member in file
+    order -- the raw DEFLATE payload's offset and size in `buf`, the member's offset in the decompressed file, its ISIZE and CRC32
+    --, or None when `buf` is not BGZF from its first byte to its last.  A member is BGZF when its header is ID1 ID2 CM = 31 139 8
+    with FLG = FEXTRA (no name, comment or header CRC) and its extra field holds a 'BC' subfield of SLEN 2 (BSIZE = member size - 1)
+    among well-formed subfields.  The chain must end exactly at the end of `buf`; the 28-byte empty EOF block is an ordinary member.
+    The walk along the chain is serial (one header per 64 KiB of output); the trailers are read with numpy."""
+    n = len(buf)
+    starts, payload, sizes = [], [], []
+    pos = 0
+    while pos < n:
+        if n - pos < 12 or buf[pos:pos + 4] != _BGZF_MAGIC:
+            return None
+        xlen = _U16(buf, pos + 10)[0]
+        if pos + 12 + xlen > n:
+            return None
+        if xlen == 6 and buf[pos + 12:pos + 16] == b"BC\x02\x00":   # bgzip's layout: BC is the only subfield
+            bsize = _U16(buf, pos + 16)[0]
+        else:
+            bsize, at, end = None, pos + 12, pos + 12 + xlen
+            while at < end:
+                if end - at < 4:
+                    return None
+                slen = _U16(buf, at + 2)[0]
+                if at + 4 + slen > end:
+                    return None
+                if buf[at:at + 2] == b"BC" and slen == 2:
+                    bsize = _U16(buf, at + 4)[0]
+                at += 4 + slen
+            if bsize is None:
+                return None
+        size = bsize + 1
+        if size < 12 + xlen + 8 or pos + size > n:
+            return None
+        starts.append(pos)
+        payload.append(pos + 12 + xlen)
+        sizes.append(size)
+        pos += size
+    if not starts:
+        return None
+    ends = np.array(starts, dtype=np.int64) + np.array(sizes, dtype=np.int64)
+    data = np.frombuffer(buf, dtype=np.uint8, count=n)
+    trailer = data[(ends - 8)[:, None] + np.arange(8)].astype(np.uint32)         # CRC32, ISIZE (little-endian)
+    crc = trailer[:, 0] | (trailer[:, 1] << 8) | (trailer[:, 2] << 16) | (trailer[:, 3] << 24)
+    isize = trailer[:, 4] | (trailer[:, 5] << 8) | (trailer[:, 6] << 16) | (trailer[:, 7] << 24)
+    if np.any(isize > 65536):
+        return None
+    table = np.zeros(len(starts), dtype=BGZF_MEMBER)
+    table["in_offset"] = payload
+    table["in_bytes"] = ends - 8 - table["in_offset"]
+    table["isize"] = isize
+    table["out_offset"][1:] = np.cumsum(isize[:-1], dtype=np.int64)
+    table["crc32"] = crc
+    return table
+
+
+def _open_fasta_device(fasta_file):
+    """(the FASTA text on the host [mmap or bytes], or None when only the device holds it; the text on the device [CUDA uint8,
+    padded to 16, or None when empty]; its size; the mmap to close or None).  A BGZF file goes to the device compressed and is
+    inflated there (ops.inflate_cuda); any other .gz is inflated on the host, as is a BGZF file whose members fail to decode on the
+    device, so that a corrupt file raises what gzip raises.  Plain files are mapped."""
+    import mmap
+    from . import _lib, ops
+    with open(fasta_file, "rb") as fh:
+        size = os.fstat(fh.fileno()).st_size
+        mapped = mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) if size else None
+    if not fasta_file.endswith(".gz"):
+        return mapped, (_upload(mapped, size) if size else None), size, mapped
+    members = bgzf_members(mapped) if size else None
+    if members is not None:
+        try:
+            d_text = ops.inflate_cuda(_upload(mapped, size)[:size], members)
+            mapped.close()
+            return None, d_text, d_text.numel(), None
+        except _lib.PhamersDataError:
+            pass
+    if mapped is not None:
+        mapped.close()
+    text = _open_bytes(fasta_file)
+    return text, (_upload(text, len(text)) if text else None), len(text), None
+
+
+def _device_titles(d_text, n, header_pos):
+    """First tokens of the title lines whose '>' is at header_pos (CUDA int64) in the device text d_text[:n]: only the title bytes
+    come back to the host -- a first window of each line, then the rest of the (rare) lines longer than it."""
+    import torch
+    window, batch = 128, 1 << 16
+    starts = header_pos + 1
+    ramp = torch.arange(window, dtype=torch.int64, device="cuda")
+    win = np.concatenate([d_text[(starts[lo:lo + batch, None] + ramp).clamp_(max=max(n - 1, 0))].cpu().numpy()
+                          for lo in range(0, starts.shape[0], batch)] or [np.zeros((0, window), dtype=np.uint8)])
+    h_starts = starts.cpu().numpy()
+    eol = (win == 10) | (win == 13) | ((h_starts[:, None] + np.arange(window)) >= n)
+    ids = []
+    for i in range(win.shape[0]):
+        row = eol[i]
+        if row.any():
+            title = win[i, :int(row.argmax())].tobytes()
+        else:
+            lo, parts = int(h_starts[i]), []
+            while True:                                                 # grow the read until the line ends
+                hi = min(n, lo + window * (1 << len(parts)))
+                piece = d_text[lo:hi].cpu().numpy()
+                cut = np.flatnonzero((piece == 10) | (piece == 13))
+                parts.append(piece[:cut[0]] if cut.shape[0] else piece)
+                if cut.shape[0] or hi == n:
+                    break
+                lo = hi
+            title = b"".join(p.tobytes() for p in parts)
+        tokens = title.decode("latin-1").rstrip().split(None, 1)
+        ids.append(tokens[0] if tokens else "")
+    return ids
+
+
 def read_fasta_arrays_cuda(fasta_file):
     """Device-side tokenisation of a FASTA file (phm_fasta_index / phm_fasta_extract): the file is memory-mapped, its bytes go
     to the GPU once through pinned staging buffers and the sequence bytes never come back; only the title lines are read on the
-    host, at the positions the device reports.  Returns (titles' first tokens, CUDA uint8 tensor of all sequence bytes end to end
-    [padded to 16], CUDA int64 offsets[n+1]).  Files holding a control byte other than '\n' '\r' (tab / VT / FF / 0x1C-0x1F are
-    stripped by the reference at line ends only) are tokenised by the exact host path and uploaded.  Raises IOError when unreadable."""
-    import mmap
+    host, at the positions the device reports.  A BGZF-compressed file (bgzf_members) crosses PCIe compressed and is inflated on
+    the device (ops.inflate_cuda); its title bytes are then copied back from the device.  Any other .gz is inflated on the host.
+    Returns (titles' first tokens, CUDA uint8 tensor of all sequence bytes end to end [padded to 16], CUDA int64 offsets[n+1]).
+    Files holding a control byte other than '\n' '\r' (tab / VT / FF / 0x1C-0x1F are stripped by the reference at line ends only)
+    are tokenised by the exact host path and uploaded.  Raises IOError when unreadable."""
     import torch
     from . import ops
-    mapped = None
-    if fasta_file.endswith(".gz"):
-        raw = _open_bytes(fasta_file)
-        n = len(raw)
-    else:
-        fh = open(fasta_file, "rb")
-        n = os.fstat(fh.fileno()).st_size
-        raw = mapped = mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) if n else b""
-        fh.close()
+    raw, d_text, n, mapped = _open_fasta_device(fasta_file)
     try:
         if n == 0:
             return [], torch.zeros((16,), dtype=torch.uint8, device="cuda"), torch.zeros((1,), dtype=torch.int64, device="cuda")
-        d_raw = _upload(raw, n)
-        seq, offsets, header_pos, odd = ops.fasta_scan_cuda(d_raw[:n])
+        seq, offsets, header_pos, odd = ops.fasta_scan_cuda(d_text[:n])
         if odd:
-            ids, h_seq, h_off = split_fasta_bytes(bytes(raw[:n]))
+            text = bytes(raw[:n]) if raw is not None else d_text[:n].cpu().numpy().tobytes()
+            ids, h_seq, h_off = split_fasta_bytes(text)
             total = int(h_off[-1])
             pad = torch.zeros((max((total + 15) // 16 * 16, 16),), dtype=torch.uint8)
             pad[:total] = torch.from_numpy(np.ascontiguousarray(h_seq[:total]).copy()) if total else pad[:0]
             return ids, pad.cuda(), torch.from_numpy(np.ascontiguousarray(h_off)).cuda()
+        if raw is None:
+            return _device_titles(d_text, n, header_pos), seq, offsets
         ids = []
         for hs in header_pos.cpu().tolist():
             he = n
@@ -189,6 +307,22 @@ def read_fasta_arrays_cuda(fasta_file):
     finally:
         if mapped is not None:
             mapped.close()
+
+
+def _is_bgzf_on_device(fasta_file):
+    """True for a BGZF file on a machine with a CUDA device: get_fasta_ids / get_fasta_lengths then read it through
+    read_fasta_arrays_cuda instead of inflating it on the host again."""
+    if not fasta_file.endswith(".gz"):
+        return False
+    import mmap
+    import torch
+    if not torch.cuda.is_available():
+        return False
+    with open(fasta_file, "rb") as fh:
+        if os.fstat(fh.fileno()).st_size == 0:
+            return False
+        with mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) as raw:
+            return bgzf_members(raw) is not None
 
 
 def read_fasta_arrays(fasta_file):
@@ -205,14 +339,22 @@ def read_fasta(fasta_file):
 
 
 def get_fasta_ids(fasta_file):
-    """scripts/fileIO.py:62-77."""
-    headers, _, _ = read_fasta_arrays(fasta_file)
+    """scripts/fileIO.py:62-77.  A BGZF file is read on the device when there is one (read_fasta_arrays_cuda)."""
+    if _is_bgzf_on_device(fasta_file):
+        headers = read_fasta_arrays_cuda(fasta_file)[0]
+    else:
+        headers = read_fasta_arrays(fasta_file)[0]
     return np.array([get_id(h) for h in headers])
 
 
 def get_fasta_lengths(fasta_file):
-    """Lengths of the parsed sequences (what phamer.screen_by_length measures, scripts/phamer.py:150-154)."""
-    headers, _, offsets = read_fasta_arrays(fasta_file)
+    """Lengths of the parsed sequences (what phamer.screen_by_length measures, scripts/phamer.py:150-154).  A BGZF file is read
+    on the device when there is one (read_fasta_arrays_cuda), so the length screen does not inflate it on the host."""
+    if _is_bgzf_on_device(fasta_file):
+        headers, _, d_off = read_fasta_arrays_cuda(fasta_file)
+        offsets = d_off.cpu().numpy()
+    else:
+        headers, _, offsets = read_fasta_arrays(fasta_file)
     return np.array([get_id(h) for h in headers]), np.diff(offsets)
 
 

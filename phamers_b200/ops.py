@@ -353,6 +353,29 @@ def fasta_scan_cuda(raw):
     return seq, offsets, header_pos[:n_records], bool(odd)
 
 
+def inflate_cuda(compressed, members, status=None):
+    """phm_inflate: the members of a BGZF file (the table of fileIO.bgzf_members) decoded on the device.  compressed: CUDA uint8
+    tensor of the file's bytes.  Returns a CUDA uint8 tensor of the decompressed file (members end to end) whose storage is padded
+    to 16 bytes past the next multiple of 16, ready for fasta_scan_cuda.  status: optional CUDA int32 tensor [members] that
+    receives each member's PHM_INFLATE_* status.  A member that fails to decode or whose CRC32 or length differs from its trailer
+    raises _lib.PhamersDataError naming the lowest such member (one host synchronisation either way)."""
+    import numpy as np
+    from .fileIO import BGZF_MEMBER
+    lib = _lib.require_cuda()
+    if not (isinstance(compressed, torch.Tensor) and compressed.is_cuda and compressed.dtype == torch.uint8
+            and compressed.is_contiguous()):
+        raise TypeError("compressed must be a contiguous CUDA uint8 tensor")
+    members = np.ascontiguousarray(members, dtype=BGZF_MEMBER)
+    n = members.shape[0]
+    total = int(members["out_offset"][-1]) + int(members["isize"][-1]) if n else 0
+    out = torch.empty(((total + 15) // 16 * 16 + 16,), dtype=torch.uint8, device="cuda")
+    status = _result(status, (n,), torch.int32) if status is not None else torch.empty((n,), dtype=torch.int32, device="cuda")
+    ws = _workspace("inflate", lib.phm_inflate_workspace_bytes(n))
+    check(lib.phm_inflate(ptr(compressed), compressed.numel(), members.ctypes.data_as(ctypes.c_void_p), n, ptr(out), total,
+                          ptr(status), ptr(ws), ws.numel(), stream_ptr()))
+    return out[:total]
+
+
 def synth_contigs(seed, first_contig, n_contigs):
     """Synthetic metagenome shard (SURVEY.md 8(d) config 2) generated on the device.
     Returns (seq uint8[total], offsets int64[n+1])."""
