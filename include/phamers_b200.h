@@ -332,6 +332,49 @@ int phm_inflate(const uint8_t *d_in, int64_t in_bytes, const phm_bgzf_member *h_
                 int64_t out_bytes, int32_t *d_status, void *d_workspace, size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Feature CSV text on the device: the k-mer count files of fileIO.save_counts / read_feature_file ('#' header lines, then one row
+ * per contig, `id,c0,c1,...`).
+ *
+ * Writing, two calls, so that the caller can size the text in between:
+ *   phm_counts_csv_layout  d_counts int64[n_rows, n_cols] (row-major), d_id_offsets int64[n_rows + 1] into the id bytes (the id of
+ *                          row r is ids[off[r], off[r+1]), clamped to [0, id_bytes))
+ *                          -> d_row_offsets int64[n_rows + 1]: where each row's text starts; d_row_offsets[n_rows] = the text size.
+ *                          Row r is its id, ',' and the decimal fields joined by ',' (just ',' when n_cols = 0), then '\n': what
+ *                          str(id) + "," + ",".join(map(str, row)) + "\n" gives for ASCII ids.  Workspace:
+ *                          phm_counts_csv_workspace_bytes(n_rows).
+ *   phm_counts_csv_format  -> d_text uint8[text_bytes] (16-byte aligned), the rows at d_row_offsets; no write lands outside d_text.
+ *
+ * Reading, two calls with the same d_workspace (phm_feature_csv_workspace_bytes(n_bytes)), untouched between them.  The grammar is
+ * the part of read_feature_file's that the device parses to the same values: bytes are printable ASCII, TAB, CR or LF; lines end
+ * at LF or CR; a line is cut at its first '#' and stripped of spaces and tabs, and skipped when nothing is left; a data line is the
+ * id (everything before its first ',') and fields [ \t]*[+-]?[0-9]{1,18}[ \t]*; every data line has the same number of fields.
+ * Anything else is a decline: the caller parses that file on the host.
+ *   phm_feature_csv_index  d_text uint8[n_bytes] (16-byte aligned, allocation readable up to the next multiple of 16; n_bytes < 2^40)
+ *                          -> d_result int64[4]: [0] data rows, [1] fields per row, [2] PHM_CSV_* (0: the device parses the file),
+ *                          [3] the 1-based line of the first decline (0 when accepted).  PHM_CSV_RAGGED is reported at the first data
+ *                          line whose field count differs from the first data line's.
+ *   phm_feature_csv_parse  (accepted files) -> d_counts int64[max_rows, n_cols] (n_cols = result[1]), d_id_ranges int64[max_rows, 2]:
+ *                          each row's id as the byte range [start, end) of d_text.  Rows past max_rows and fields past n_cols are
+ *                          not written.
+ * ------------------------------------------------------------------------------------------- */
+#define PHM_CSV_OK         0
+#define PHM_CSV_BYTE       1      /* a byte other than printable ASCII, TAB, CR and LF */
+#define PHM_CSV_NO_COMMA   2      /* a data line without ',' */
+#define PHM_CSV_FIELD      3      /* a field that is not [ \t]*[+-]?[0-9]{1,18}[ \t]* (empty, other characters, 19 or more digits) */
+#define PHM_CSV_RAGGED     4      /* data lines with different numbers of fields */
+
+size_t phm_counts_csv_workspace_bytes(int64_t n_rows);
+int phm_counts_csv_layout(const int64_t *d_counts, int64_t n_rows, int64_t n_cols, const int64_t *d_id_offsets, int64_t id_bytes,
+                          int64_t *d_row_offsets, void *d_workspace, size_t workspace_bytes, void *stream);
+int phm_counts_csv_format(const int64_t *d_counts, int64_t n_rows, int64_t n_cols, const uint8_t *d_ids, const int64_t *d_id_offsets,
+                          int64_t id_bytes, const int64_t *d_row_offsets, uint8_t *d_text, int64_t text_bytes, void *stream);
+size_t phm_feature_csv_workspace_bytes(int64_t n_bytes);
+int phm_feature_csv_index(const uint8_t *d_text, int64_t n_bytes, int64_t *d_result, void *d_workspace, size_t workspace_bytes,
+                          void *stream);
+int phm_feature_csv_parse(const uint8_t *d_text, int64_t n_bytes, int64_t *d_counts, int64_t *d_id_ranges, int64_t max_rows,
+                          int64_t n_cols, const void *d_workspace, size_t workspace_bytes, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Lloyd iterations of k-means on the device (SURVEY.md 8(f) rank 4).  Replaces the iterations inside the reference's
  * KMeans(n_clusters = k, random_state = 10).fit(data).labels_ (learning.kmeans, scripts/learning.py:131-146; run twice per
  * scoring call, scripts/phamer.py:245-248).  The caller centres the data and seeds the centres exactly as scikit-learn does

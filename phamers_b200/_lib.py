@@ -59,6 +59,12 @@ SIGNATURES = {
     "phm_fasta_extract": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "phm_inflate_workspace_bytes": (c_size_t, [c_int64]),
     "phm_inflate": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_counts_csv_workspace_bytes": (c_size_t, [c_int64]),
+    "phm_counts_csv_layout": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_counts_csv_format": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p]),
+    "phm_feature_csv_workspace_bytes": (c_size_t, [c_int64]),
+    "phm_feature_csv_index": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_feature_csv_parse": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_size_t, c_void_p]),
     "phm_last_kernel_ms": (c_int, [ctypes.c_char_p, c_void_p]),
     "phm_synth_lengths": (c_int, [c_uint64, c_int64, c_int64, c_void_p, c_void_p]),
     "phm_synth_bases": (c_int, [c_uint64, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),

@@ -23,6 +23,7 @@
 // A thread's 16 bytes are classified four at a time into 16-bit masks (SWAR zero-byte tests); the state machine then only visits
 // the line starts, of which a thread usually has none or one.
 // Traffic: the file is read twice and the sequence written once (~3 bytes per input byte); pass 2 touches 32 bytes per tile.
+#include "byte_class.cuh"
 #include "phm_common.cuh"
 
 namespace phm {
@@ -54,14 +55,7 @@ __device__ __forceinline__ uint32_t map_then(uint32_t first, uint32_t second) { 
     return map_apply(second, map_apply(first, 0)) | (map_apply(second, map_apply(first, 1)) << 2) |
            (map_apply(second, map_apply(first, 2)) << 4);
 }
-// ---- 16 bytes -> 16-bit class masks, four bytes at a time (SWAR) ----
-// 0x80 in every byte of x that is zero
-__device__ __forceinline__ uint32_t zero_bytes(uint32_t x) {
-    return ~(((x & 0x7F7F7F7Fu) + 0x7F7F7F7Fu) | x | 0x7F7F7F7Fu);
-}
-// bits 7, 15, 23, 31 -> bits 0..3 (the partial products land on distinct bits, so there are no carries)
-__device__ __forceinline__ uint32_t gather4(uint32_t z) { return (((z >> 7) * 0x00204081u) >> 21) & 0xFu; }
-
+// ---- 16 bytes -> 16-bit class masks, four bytes at a time (SWAR: zero_bytes, gather4 of byte_class.cuh) ----
 struct Masks {
     uint32_t nl;      // byte ends a line: '\n' or '\r' (bytes at or past the end of the file count as '\n')
     uint32_t keep;    // byte is none of '\n' '\r' ' '

@@ -4,7 +4,8 @@ scripts/id_parser.py the path touches:
 
     FASTA in        read_fasta :28, get_fasta_ids :62 (Bio.SeqIO tokenisation) + id_parser.get_id :89
     BGZF            bgzf_members  (the member chain of a blocked-gzip FASTA, decoded on the device by ops.inflate_cuda)
-    feature CSV     read_feature_file :134, save_counts :169  ('#' header lines, then id,c0,c1,...)
+    feature CSV     read_feature_file :134, save_counts :169  ('#' header lines, then id,c0,c1,...; formatted and parsed on the
+                    device when there is one, ops.format_counts_csv_cuda / ops.parse_feature_csv_cuda)
     score CSV       save_phamer_scores :241, read_phamer_output :256  ('# ' header, then 'id, score')
     neighbour CSV   save_phamer_neighbors, read_phamer_neighbors  ('# ' header, then per contig its nearest references and clusters)
     window CSV      save_phamer_windows, read_phamer_windows  ('# ' header, then 'id, start, end, score' per window)
@@ -12,7 +13,7 @@ scripts/id_parser.py the path touches:
     BED in          read_bed  ('chrom start end [name ...]' per line)
     span CSV        save_phamer_spans, read_phamer_spans  ('# ' header, then 'id, start, end, name, score' and the neighbour columns)
 
-Host-side only (bytes and text); no arithmetic happens here.
+Bytes and text; no arithmetic happens here.
 """
 import gzip
 import io
@@ -370,8 +371,17 @@ def generate_summary(args, line_start="", header=""):
     return line_start + header + "\n" + text
 
 
-def read_feature_file(feature_file, normalize=False, id=None):
-    """scripts/fileIO.py:134-166: (ids ndarray[str], counts int ndarray[n, bins]); normalize -> kmer.normalize_counts."""
+def _finish_features(ids, features, normalize, id):
+    if normalize:
+        from . import kmer
+        features = kmer.normalize_counts(features)
+    if id:
+        return features[ids == id]
+    return ids, features
+
+
+def _read_feature_file_host(feature_file, normalize=False, id=None):
+    """read_feature_file on the host: every file it accepts, and the only road without a device."""
     ids, rows = [], []
     opener = gzip.open if feature_file.endswith(".gz") else open
     with opener(feature_file, "rt") as fh:
@@ -383,17 +393,63 @@ def read_feature_file(feature_file, normalize=False, id=None):
             ids.append(first)
             rows.append(np.array(rest.split(","), dtype=np.int64))
     features = np.stack(rows) if rows else np.zeros((0, 0), dtype=np.int64)
-    ids = np.array(ids)
-    if normalize:
-        from . import kmer
-        features = kmer.normalize_counts(features)
-    if id:
-        return features[ids == id]
-    return ids, features
+    return _finish_features(np.array(ids), features, normalize, id)
 
 
-def save_counts(counts, ids, file_name, args=None, header="K-mer count file"):
-    """scripts/fileIO.py:169-181: '# '-prefixed header lines, then id,c0,c1,... as integers."""
+def _span_strings(raw, d_text, n, ranges):
+    """The ASCII strings at the byte ranges [start, end) of a text: sliced from the host copy when there is one, else copied back
+    from the device (a BGZF file inflated there) -- a first window of every range in one copy, then each longer range on its own."""
+    if raw is not None:
+        return [bytes(raw[a:b]).decode("ascii") for a, b in ranges.tolist()]
+    import torch
+    window, batch = 64, 1 << 16
+    ramp = torch.arange(window, dtype=torch.int64, device="cuda")
+    d_starts = torch.from_numpy(np.ascontiguousarray(ranges[:, 0])).cuda()
+    win = np.concatenate([d_text[(d_starts[lo:lo + batch, None] + ramp).clamp_(max=n - 1)].cpu().numpy()
+                          for lo in range(0, ranges.shape[0], batch)] or [np.zeros((0, window), dtype=np.uint8)])
+    out = []
+    for i, (a, b) in enumerate(ranges.tolist()):
+        piece = win[i, :b - a] if b - a <= window else d_text[a:b].cpu().numpy()
+        out.append(piece.tobytes().decode("ascii"))
+    return out
+
+
+def _read_feature_file_device(feature_file):
+    """(ids, counts) of a feature CSV parsed on the device (ops.parse_feature_csv_cuda), or None when the file is outside the device
+    grammar.  The file is opened as FASTA files are (_open_fasta_device): plain files are mapped and uploaded, BGZF files inflated on
+    the device, any other .gz on the host."""
+    from . import ops
+    raw, d_text, n, mapped = _open_fasta_device(feature_file)
+    try:
+        if n == 0:
+            return np.array([]), np.zeros((0, 0), dtype=np.int64)
+        parsed = ops.parse_feature_csv_cuda(d_text[:n])
+        if parsed is None:
+            return None
+        ranges, d_counts = parsed
+        return np.array(_span_strings(raw, d_text, n, ranges)), d_counts.cpu().numpy()
+    finally:
+        if mapped is not None:
+            mapped.close()
+
+
+def read_feature_file(feature_file, normalize=False, id=None):
+    """scripts/fileIO.py:134-166: (ids ndarray[str], counts int ndarray[n, bins]); normalize -> kmer.normalize_counts.  With a CUDA
+    device the file is parsed there (phm_feature_csv_index / phm_feature_csv_parse) when it keeps to the device grammar
+    (include/phamers_b200.h), which gives the same arrays; any other file is parsed on the host, which returns or raises what it
+    always did."""
+    import torch
+    parsed = _read_feature_file_device(feature_file) if torch.cuda.is_available() else None
+    if parsed is None:
+        return _read_feature_file_host(feature_file, normalize, id)
+    return _finish_features(parsed[0], parsed[1], normalize, id)
+
+
+FORMAT_CHUNK = 256 << 20             # text bytes one slice of save_counts may need on the device (counted at 21 bytes a field)
+
+
+def _save_counts_host(counts, ids, file_name, args=None, header="K-mer count file"):
+    """save_counts on the host: every input, and the only road without a device."""
     if args is not None:
         header = generate_summary(args, header=header)
     counts = np.asarray(counts).astype(np.int64)
@@ -404,6 +460,43 @@ def save_counts(counts, ids, file_name, args=None, header="K-mer count file"):
             fh.write("# " + line + "\n")
         for ident, row in zip(ids, counts):
             fh.write(str(ident) + "," + ",".join(map(str, row.tolist())) + "\n")
+
+
+def save_counts(counts, ids, file_name, args=None, header="K-mer count file"):
+    """scripts/fileIO.py:169-181: '# '-prefixed header lines, then id,c0,c1,... as integers.  With a CUDA device, 1-D or 2-D counts
+    and ASCII ids (str(id)), the rows are formatted on the device (ops.format_counts_csv_cuda) in slices of at most FORMAT_CHUNK bytes
+    of text, each appended to the file in order: the file is byte for byte what the host writes."""
+    import torch
+    from . import ops
+    if args is not None:
+        header = generate_summary(args, header=header)
+    table = np.asarray(counts).astype(np.int64)
+    if table.ndim not in (1, 2) or not torch.cuda.is_available():
+        return _save_counts_host(table, ids, file_name, header=header)
+    if table.ndim == 1:
+        table = table[None, :]
+    names = [str(ident) for ident, _ in zip(ids, range(table.shape[0]))]        # zip's pairing: the shorter one wins
+    if not all(name.isascii() for name in names):
+        return _save_counts_host(table, names, file_name, header=header)
+    encoded = [name.encode("ascii") for name in names]
+    row_bound = np.fromiter(map(len, encoded), dtype=np.int64, count=len(encoded)) + 21 * max(table.shape[1], 1) + 2
+    ends = np.cumsum(row_bound)
+    with open(file_name, "w") as fh:
+        for line in header.split("\n"):
+            fh.write("# " + line + "\n")
+        fh.flush()
+        lo = 0
+        while lo < len(names):
+            # rows while their text fits FORMAT_CHUNK, and at least one
+            hi = max(lo + 1, int(np.searchsorted(ends, (ends[lo - 1] if lo else 0) + FORMAT_CHUNK, side="right")))
+            id_offsets = np.zeros(hi - lo + 1, dtype=np.int64)
+            np.cumsum(row_bound[lo:hi] - (21 * max(table.shape[1], 1) + 2), out=id_offsets[1:])
+            id_bytes = np.frombuffer(b"".join(encoded[lo:hi]) or b"\0", dtype=np.uint8)
+            text = ops.format_counts_csv_cuda(torch.from_numpy(np.ascontiguousarray(table[lo:hi])).cuda(),
+                                              torch.from_numpy(id_bytes.copy()).cuda()[:int(id_offsets[-1])],
+                                              torch.from_numpy(id_offsets).cuda())
+            fh.buffer.write(text.cpu().numpy().data)
+            lo = hi
 
 
 # ----------------------------------------------------------------------------------------------------------

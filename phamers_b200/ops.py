@@ -376,6 +376,55 @@ def inflate_cuda(compressed, members, status=None):
     return out[:total]
 
 
+def format_counts_csv_cuda(counts, id_bytes, id_offsets):
+    """phm_counts_csv_layout + phm_counts_csv_format: the data rows of a feature CSV (fileIO.save_counts) written on the device.
+    counts: CUDA int64 [n, F]; id_bytes: CUDA uint8, the ids end to end; id_offsets: CUDA int64 [n + 1] into id_bytes.  Returns a CUDA
+    uint8 tensor of the text, row r being id_r + "," + ",".join(str(v) for v in counts[r]) + "\\n" ("id_r,\\n" when F = 0).  One host
+    synchronisation (the text is sized from the layout pass)."""
+    lib = _lib.require_cuda()
+    counts = _check(counts, "counts", torch.int64)
+    if counts.dim() != 2:
+        raise ValueError("counts must be [rows, fields]")
+    id_bytes = _check(id_bytes, "id_bytes", torch.uint8)
+    id_offsets = _check(id_offsets, "id_offsets", torch.int64)
+    n, f = counts.shape
+    if id_offsets.shape != (n + 1,):
+        raise ValueError("id_offsets must be [rows + 1]")
+    row_offsets = torch.empty((n + 1,), dtype=torch.int64, device="cuda")
+    ws_bytes = lib.phm_counts_csv_workspace_bytes(n)
+    ws = _workspace("csv_format", ws_bytes)
+    check(lib.phm_counts_csv_layout(ptr(counts), n, f, ptr(id_offsets), id_bytes.numel(), ptr(row_offsets), ptr(ws), ws_bytes,
+                                    stream_ptr()))
+    total = int(row_offsets[n].item())
+    text = torch.empty((max(total, 1),), dtype=torch.uint8, device="cuda")
+    check(lib.phm_counts_csv_format(ptr(counts), n, f, ptr(id_bytes), ptr(id_offsets), id_bytes.numel(), ptr(row_offsets), ptr(text),
+                                    total, stream_ptr()))
+    return text[:total]
+
+
+def parse_feature_csv_cuda(text, result=None):
+    """phm_feature_csv_index + phm_feature_csv_parse: a feature CSV on the device (contiguous CUDA uint8, 16-byte aligned, storage
+    readable up to the next multiple of 16 bytes) -> (id byte ranges int64 [rows, 2] on the host, counts CUDA int64 [rows, F]), or None
+    when the file is outside the device grammar (include/phamers_b200.h); the caller then parses it on the host.  result: optional
+    CUDA int64 tensor [4] that receives the index block (rows, fields, PHM_CSV_* reason, line of the first decline).  One host
+    synchronisation for the index, one for the id ranges."""
+    import numpy as np
+    lib = _lib.require_cuda()
+    text = _as_u8_cuda(text)
+    n = text.numel()
+    ws_bytes = lib.phm_feature_csv_workspace_bytes(n)
+    ws = _workspace("csv_parse", ws_bytes)
+    result = _result(result, (4,), torch.int64)
+    check(lib.phm_feature_csv_index(ptr(text), n, ptr(result), ptr(ws), ws_bytes, stream_ptr()))
+    rows, fields, reason, _ = result.cpu().tolist()
+    if reason != 0:
+        return None
+    counts = torch.empty((rows, fields), dtype=torch.int64, device="cuda")
+    ranges = torch.empty((max(rows, 1), 2), dtype=torch.int64, device="cuda")
+    check(lib.phm_feature_csv_parse(ptr(text), n, ptr(counts), ptr(ranges), rows, fields, ptr(ws), ws_bytes, stream_ptr()))
+    return np.ascontiguousarray(ranges[:rows].cpu().numpy()), counts
+
+
 def synth_contigs(seed, first_contig, n_contigs):
     """Synthetic metagenome shard (SURVEY.md 8(d) config 2) generated on the device.
     Returns (seq uint8[total], offsets int64[n+1])."""
