@@ -332,6 +332,39 @@ int phm_inflate(const uint8_t *d_in, int64_t in_bytes, const phm_bgzf_member *h_
                 int64_t out_bytes, int32_t *d_status, void *d_workspace, size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Single-member gzip decompression on the device (what gzip and pigz write).  The host parses the gzip header and trailer; these
+ * calls decode the raw DEFLATE payload d_payload[0, payload_bytes) (between the header and the 8-byte trailer) in parallel: the
+ * payload is cut into chunks of the option "gunzip_chunk_bytes" compressed bytes, a block finder looks for a dynamic block
+ * start in each chunk, and the pieces are decoded and chained (DESIGN.md 4.6b).  Two calls, so that the caller can size the
+ * output in between:
+ *
+ *   phm_gunzip_index    finds the blocks, decodes the stream once without writing it, verifies the chain of pieces and
+ *                       synchronises `stream`.  h_info int64[7] (HOST): [0] output bytes, [1] chunks, [2] candidate block starts
+ *                       the chain rejected, [3] repair rounds, [4] output bytes decoded by pieces that cover a whole chunk with
+ *                       no block start of its own (serially, in effect), [5] verified pieces, [6] output bytes of the longest
+ *                       piece after the first (the pieces that resolve a window).  The stream must end exactly at payload_bytes (after
+ *                       byte alignment) and its output size mod 2^32 must equal `isize`.  Workspace:
+ *                       phm_gunzip_index_workspace_bytes(payload_bytes), sized with the chunk option in force at the call.
+ *   phm_gunzip_extract  decodes again into d_out uint8[out_bytes] (out_bytes = h_info[0]; 16-byte aligned), resolves the
+ *                       back-references across pieces, and checks the CRC32 of the output against `crc32`; synchronises twice
+ *                       (after the second decode, whose errors end the call before anything reads its symbols, and at the end).
+ *                       d_index_workspace is the workspace of the index call on the same payload, untouched in between (the
+ *                       call keeps per-piece scratch there).  Workspace: phm_gunzip_extract_workspace_bytes(out_bytes): about 2
+ *                       bytes per output byte.
+ * Argument errors (null pointers, negative sizes, a workspace too small, an index workspace of another payload or size) are
+ * PHM_E_ARG / PHM_E_WORKSPACE before the device is touched (extract reads the index workspace's header first).  A stream zlib
+ * would refuse, or whose end, ISIZE or CRC32 differ from the trailer's, is PHM_E_DATA with its PHM_INFLATE_* reason; the output
+ * then holds unspecified bytes.  Every read stays inside the payload and every write inside d_out, whatever the data.
+ * ------------------------------------------------------------------------------------------- */
+size_t phm_gunzip_index_workspace_bytes(int64_t payload_bytes);
+int phm_gunzip_index(const uint8_t *d_payload, int64_t payload_bytes, uint32_t isize, int64_t *h_info, void *d_workspace,
+                     size_t workspace_bytes, void *stream);
+size_t phm_gunzip_extract_workspace_bytes(int64_t out_bytes);
+int phm_gunzip_extract(const uint8_t *d_payload, int64_t payload_bytes, uint32_t crc32, void *d_index_workspace,
+                       size_t index_workspace_bytes, uint8_t *d_out, int64_t out_bytes, void *d_workspace, size_t workspace_bytes,
+                       void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Feature CSV text on the device: the k-mer count files of fileIO.save_counts / read_feature_file ('#' header lines, then one row
  * per contig, `id,c0,c1,...`).
  *
@@ -407,7 +440,8 @@ int phm_score_stats(const void *d_workspace, uint64_t *fallback_rows, float *max
  * "score_list_pass" (0 = overflowed rows skip the listing pass and go to the exhaustive kernels),
  * "score_path" (0 = tensor cores when the shape allows, 1 = exhaustive float64 only, 2 = tensor cores or error),
  * "score_stats" (1 = collect error-interval diagnostics, slower), "time_kernels" (1 = bracket the hot kernels with CUDA
- * events for phm_last_kernel_ms). */
+ * events for phm_last_kernel_ms), "gunzip_chunk_bytes" (compressed bytes per chunk of phm_gunzip_index, 1 KiB .. 1 GiB; small
+ * values make tests cross many chunk starts). */
 int phm_set_option(const char *name, int64_t value);
 
 /* Kernels this library has launched in the calling process so far (bench.py reports the difference over its timed region). */

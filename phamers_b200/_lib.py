@@ -59,6 +59,10 @@ SIGNATURES = {
     "phm_fasta_extract": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "phm_inflate_workspace_bytes": (c_size_t, [c_int64]),
     "phm_inflate": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_gunzip_index_workspace_bytes": (c_size_t, [c_int64]),
+    "phm_gunzip_index": (c_int, [c_void_p, c_int64, c_uint32, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "phm_gunzip_extract_workspace_bytes": (c_size_t, [c_int64]),
+    "phm_gunzip_extract": (c_int, [c_void_p, c_int64, c_uint32, c_void_p, c_size_t, c_void_p, c_int64, c_void_p, c_size_t, c_void_p]),
     "phm_counts_csv_workspace_bytes": (c_size_t, [c_int64]),
     "phm_counts_csv_layout": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_size_t, c_void_p]),
     "phm_counts_csv_format": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_void_p]),
@@ -76,7 +80,8 @@ class PhamersLibraryError(RuntimeError):
 
 
 class PhamersDataError(PhamersLibraryError):
-    """PHM_E_DATA: the input data is corrupt (phm_inflate: a member failed to decode)."""
+    """PHM_E_DATA: the input data is corrupt (phm_inflate: a member failed to decode; phm_gunzip_index / phm_gunzip_extract: the
+    stream does not decode, or its CRC32, ISIZE or end differ from the trailer's)."""
 
 
 PHM_E_DATA = -5

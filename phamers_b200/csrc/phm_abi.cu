@@ -59,6 +59,7 @@ extern int score_collect_stats;
 extern int score_list_pass;
 extern int score_force_fallback;
 int kmer_hist_last_ms(float *ms);
+namespace gunzip { extern int chunk_bytes; }
 
 }  // namespace phm
 
@@ -102,6 +103,11 @@ extern "C" int phm_set_option(const char *name, int64_t value) {
     if (!strcmp(name, "score_force_fallback")) { score_force_fallback = value != 0; return PHM_OK; }
     if (!strcmp(name, "score_stats")) { score_collect_stats = value != 0; return PHM_OK; }
     if (!strcmp(name, "score_list_pass")) { score_list_pass = value != 0; return PHM_OK; }
+    if (!strcmp(name, "gunzip_chunk_bytes")) {
+        PHM_REQUIRE(value >= 1024 && value <= (1 << 30), "1 KiB .. 1 GiB");
+        gunzip::chunk_bytes = (int)value;
+        return PHM_OK;
+    }
     set_error("unknown option '%s'", name);
     return PHM_E_ARG;
 }

@@ -4,6 +4,7 @@ scripts/id_parser.py the path touches:
 
     FASTA in        read_fasta :28, get_fasta_ids :62 (Bio.SeqIO tokenisation) + id_parser.get_id :89
     BGZF            bgzf_members  (the member chain of a blocked-gzip FASTA, decoded on the device by ops.inflate_cuda)
+    gzip            gzip_member   (the header and trailer of a single-member gzip FASTA, decoded on the device by ops.gunzip_cuda)
     feature CSV     read_feature_file :134, save_counts :169  ('#' header lines, then id,c0,c1,...; formatted and parsed on the
                     device when there is one, ops.format_counts_csv_cuda / ops.parse_feature_csv_cuda)
     score CSV       save_phamer_scores :241, read_phamer_output :256  ('# ' header, then 'id, score')
@@ -213,12 +214,42 @@ def bgzf_members(buf):
     return table
 
 
+def gzip_member(buf):
+    """(payload offset, payload end, CRC32, ISIZE) of `buf` read as one gzip member whose 8-byte trailer ends the buffer, or None
+    when its header is not one Python's gzip module accepts.  The header is parsed as gzip._read_gzip_header parses it: ID1 ID2,
+    CM = 8, then FEXTRA (XLEN bytes), FNAME and FCOMMENT (up to and including a NUL) and FHCRC (2 bytes, not checked) are skipped;
+    the reserved flag bits are ignored.  Whether the DEFLATE stream in between ends exactly at the trailer, and the CRC32 and ISIZE
+    of its output, are for the decoder to check (a multi-member file gives the first header and the last trailer here)."""
+    n = len(buf)
+    if n < 10 or buf[0:3] != b"\x1f\x8b\x08":
+        return None
+    flag, pos = buf[3], 10
+    if flag & 4:                                                  # FEXTRA
+        if pos + 2 > n:
+            return None
+        pos += 2 + _U16(buf, pos)[0]
+    for bit in (8, 16):                                           # FNAME, FCOMMENT: zero-terminated
+        if flag & bit:
+            end = buf.find(b"\0", pos) if pos < n else -1
+            if end < 0:
+                return None
+            pos = end + 1
+    if flag & 2:                                                  # FHCRC
+        pos += 2
+    if pos + 8 > n:
+        return None
+    crc, isize = struct.unpack_from("<II", buf, n - 8)
+    return pos, n - 8, crc, isize
+
+
 def _open_fasta_device(fasta_file):
     """(the FASTA text on the host [mmap or bytes], or None when only the device holds it; the text on the device [CUDA uint8,
-    padded to 16, or None when empty]; its size; the mmap to close or None).  A BGZF file goes to the device compressed and is
-    inflated there (ops.inflate_cuda); any other .gz is inflated on the host, as is a BGZF file whose members fail to decode on the
-    device, so that a corrupt file raises what gzip raises.  Plain files are mapped."""
+    padded to 16, or None when empty]; its size; the mmap to close or None).  A compressed file goes to the device compressed and is
+    inflated there: BGZF by ops.inflate_cuda, a single gzip member by ops.gunzip_cuda.  Any other .gz, and any file the device
+    declines (corrupt data, trailing bytes, more than one member, not enough device memory), is inflated on the host, so that it
+    gives or raises exactly what gzip gives or raises.  Plain files are mapped."""
     import mmap
+    import torch
     from . import _lib, ops
     with open(fasta_file, "rb") as fh:
         size = os.fstat(fh.fileno()).st_size
@@ -226,12 +257,15 @@ def _open_fasta_device(fasta_file):
     if not fasta_file.endswith(".gz"):
         return mapped, (_upload(mapped, size) if size else None), size, mapped
     members = bgzf_members(mapped) if size else None
-    if members is not None:
+    member = gzip_member(mapped) if size and members is None else None
+    if members is not None or member is not None:
         try:
-            d_text = ops.inflate_cuda(_upload(mapped, size)[:size], members)
+            d_raw = _upload(mapped, size)[:size]
+            d_text = ops.inflate_cuda(d_raw, members) if members is not None else ops.gunzip_cuda(d_raw, member)
+            del d_raw
             mapped.close()
             return None, d_text, d_text.numel(), None
-        except _lib.PhamersDataError:
+        except (_lib.PhamersDataError, torch.cuda.OutOfMemoryError):
             pass
     if mapped is not None:
         mapped.close()
@@ -274,8 +308,9 @@ def _device_titles(d_text, n, header_pos):
 def read_fasta_arrays_cuda(fasta_file):
     """Device-side tokenisation of a FASTA file (phm_fasta_index / phm_fasta_extract): the file is memory-mapped, its bytes go
     to the GPU once through pinned staging buffers and the sequence bytes never come back; only the title lines are read on the
-    host, at the positions the device reports.  A BGZF-compressed file (bgzf_members) crosses PCIe compressed and is inflated on
-    the device (ops.inflate_cuda); its title bytes are then copied back from the device.  Any other .gz is inflated on the host.
+    host, at the positions the device reports.  A BGZF-compressed file (bgzf_members) or single-member gzip file (gzip_member)
+    crosses PCIe compressed and is inflated on the device (ops.inflate_cuda, ops.gunzip_cuda); its title bytes are then copied
+    back from the device.  Any other .gz, or one the device declines, is inflated on the host.
     Returns (titles' first tokens, CUDA uint8 tensor of all sequence bytes end to end [padded to 16], CUDA int64 offsets[n+1]).
     Files holding a control byte other than '\n' '\r' (tab / VT / FF / 0x1C-0x1F are stripped by the reference at line ends only)
     are tokenised by the exact host path and uploaded.  Raises IOError when unreadable."""
@@ -310,9 +345,9 @@ def read_fasta_arrays_cuda(fasta_file):
             mapped.close()
 
 
-def _is_bgzf_on_device(fasta_file):
-    """True for a BGZF file on a machine with a CUDA device: get_fasta_ids / get_fasta_lengths then read it through
-    read_fasta_arrays_cuda instead of inflating it on the host again."""
+def _is_decodable_on_device(fasta_file):
+    """True for a BGZF or single-member gzip file on a machine with a CUDA device: get_fasta_ids / get_fasta_lengths then read it
+    through read_fasta_arrays_cuda instead of inflating it on the host again."""
     if not fasta_file.endswith(".gz"):
         return False
     import mmap
@@ -323,7 +358,7 @@ def _is_bgzf_on_device(fasta_file):
         if os.fstat(fh.fileno()).st_size == 0:
             return False
         with mmap.mmap(fh.fileno(), 0, access=mmap.ACCESS_READ) as raw:
-            return bgzf_members(raw) is not None
+            return bgzf_members(raw) is not None or gzip_member(raw) is not None
 
 
 def read_fasta_arrays(fasta_file):
@@ -340,8 +375,8 @@ def read_fasta(fasta_file):
 
 
 def get_fasta_ids(fasta_file):
-    """scripts/fileIO.py:62-77.  A BGZF file is read on the device when there is one (read_fasta_arrays_cuda)."""
-    if _is_bgzf_on_device(fasta_file):
+    """scripts/fileIO.py:62-77.  A BGZF or gzip file is read on the device when there is one (read_fasta_arrays_cuda)."""
+    if _is_decodable_on_device(fasta_file):
         headers = read_fasta_arrays_cuda(fasta_file)[0]
     else:
         headers = read_fasta_arrays(fasta_file)[0]
@@ -349,9 +384,9 @@ def get_fasta_ids(fasta_file):
 
 
 def get_fasta_lengths(fasta_file):
-    """Lengths of the parsed sequences (what phamer.screen_by_length measures, scripts/phamer.py:150-154).  A BGZF file is read
-    on the device when there is one (read_fasta_arrays_cuda), so the length screen does not inflate it on the host."""
-    if _is_bgzf_on_device(fasta_file):
+    """Lengths of the parsed sequences (what phamer.screen_by_length measures, scripts/phamer.py:150-154).  A BGZF or gzip file is
+    read on the device when there is one (read_fasta_arrays_cuda), so the length screen does not inflate it on the host."""
+    if _is_decodable_on_device(fasta_file):
         headers, _, d_off = read_fasta_arrays_cuda(fasta_file)
         offsets = d_off.cpu().numpy()
     else:
@@ -416,8 +451,8 @@ def _span_strings(raw, d_text, n, ranges):
 
 def _read_feature_file_device(feature_file):
     """(ids, counts) of a feature CSV parsed on the device (ops.parse_feature_csv_cuda), or None when the file is outside the device
-    grammar.  The file is opened as FASTA files are (_open_fasta_device): plain files are mapped and uploaded, BGZF files inflated on
-    the device, any other .gz on the host."""
+    grammar.  The file is opened as FASTA files are (_open_fasta_device): plain files are mapped and uploaded, BGZF and gzip files
+    inflated on the device, any other .gz on the host."""
     from . import ops
     raw, d_text, n, mapped = _open_fasta_device(feature_file)
     try:

@@ -376,6 +376,40 @@ def inflate_cuda(compressed, members, status=None):
     return out[:total]
 
 
+def gunzip_cuda(compressed, member, stats=None):
+    """phm_gunzip_index + phm_gunzip_extract: a single-member gzip file decoded on the device.  compressed: CUDA uint8 tensor of
+    the file's bytes; member: fileIO.gzip_member of them (payload offset, payload end, CRC32, ISIZE).  Returns a CUDA uint8 tensor of
+    the decompressed bytes whose storage is padded to 16 bytes past the next multiple of 16, ready for fasta_scan_cuda.  stats:
+    optional dict that receives the index's diagnostics (chunks, rejected candidates, repair rounds, serial bytes, verified pieces,
+    output bytes of the longest piece after the first).  A stream that
+    zlib would refuse, or whose end, CRC32 or ISIZE differ from the trailer's, raises _lib.PhamersDataError; a device working set
+    that does not fit raises torch.cuda.OutOfMemoryError.  Synchronises the host a few times (the chain of pieces is verified on
+    the host between decode rounds)."""
+    lib = _lib.require_cuda()
+    if not (isinstance(compressed, torch.Tensor) and compressed.is_cuda and compressed.dtype == torch.uint8
+            and compressed.is_contiguous()):
+        raise TypeError("compressed must be a contiguous CUDA uint8 tensor")
+    begin, end, crc, isize = (int(v) for v in member)
+    if not 0 <= begin <= end <= compressed.numel():
+        raise ValueError("the payload [%d, %d) is outside the %d bytes" % (begin, end, compressed.numel()))
+    payload = compressed[begin:end]
+    n = end - begin
+    index_ws = torch.empty((lib.phm_gunzip_index_workspace_bytes(n),), dtype=torch.uint8, device="cuda")
+    info = (ctypes.c_int64 * 7)()
+    try:
+        check(lib.phm_gunzip_index(ptr(payload), n, isize, info, ptr(index_ws), index_ws.numel(), stream_ptr()))
+    finally:
+        if stats is not None:
+            stats.update(chunks=int(info[1]), rejected_candidates=int(info[2]), repair_rounds=int(info[3]),
+                         serial_bytes=int(info[4]), pieces=int(info[5]), longest_later_piece_bytes=int(info[6]))
+    total = int(info[0])
+    out = torch.empty(((total + 15) // 16 * 16 + 16,), dtype=torch.uint8, device="cuda")
+    ws = torch.empty((lib.phm_gunzip_extract_workspace_bytes(total),), dtype=torch.uint8, device="cuda")
+    check(lib.phm_gunzip_extract(ptr(payload), n, crc, ptr(index_ws), index_ws.numel(), ptr(out), total, ptr(ws), ws.numel(),
+                                 stream_ptr()))
+    return out[:total]
+
+
 def format_counts_csv_cuda(counts, id_bytes, id_offsets):
     """phm_counts_csv_layout + phm_counts_csv_format: the data rows of a feature CSV (fileIO.save_counts) written on the device.
     counts: CUDA int64 [n, F]; id_bytes: CUDA uint8, the ids end to end; id_offsets: CUDA int64 [n + 1] into id_bytes.  Returns a CUDA
